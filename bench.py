@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload auto|c2|c3|c4|c5]        our arm
   python bench.py --impl reference ...                the reference's own CPU implementation of the path
+  python bench.py ... --dump-outputs DIR              also write what the last timed step computed as DIR/<name>.npy
 
 Workloads (BASELINE.json `configs`, built by poseestimationkf_b200/workloads.py):
   c2  1 Mi independent filters x 1000 steps per GPU, inputs resident in HBM      (configs[1]; the default on 1 GPU)
@@ -44,6 +45,7 @@ NCU_FULL = os.path.join(ROOT, "profiles", "r02_replay_packed_ncu_full.json")
 FLOPS_FALLBACK = {"qr2": 364.0, "jacobi": 1292.0}
 LANE_OPS_FALLBACK = {"qr2": 237.0}
 FLOPS_COMPENSATED_EXTRA = 32      # two-sum folding of the state
+DUMP_BYTES = 64 * 10**6           # --dump-outputs: bound on all arrays together
 
 
 def parse():
@@ -67,7 +69,16 @@ def parse():
     ap.add_argument("--no-variants", action="store_true", help="skip the context measurements of the other kernels")
     ap.add_argument("--precise-state", action="store_true",
                     help="compensated two-float state (needed for R >> Q sweeps, not for the Q=1, R=0.1 headline config)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the arrays the last one returned as DIR/<name>.npy (float32, rank 0, "
+                         f"at most {DUMP_BYTES // 10**6} MB: a seeded sample of the filters beyond that); the inputs are "
+                         "seeded, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to our arm only (the reference arm returns no arrays)")
+    return args
 
 
 def kernel_source_sha() -> str:
@@ -81,6 +92,32 @@ def kernel_source_sha() -> str:
         src = re.sub(r"//[^\n]*", "", src)
         h.update(re.sub(r"\s+", "", src).encode())
     return h.hexdigest()[:16]
+
+
+def state_arrays(st) -> dict:
+    """What `replay` hands its caller in a ReplayState: x [4,N], p [10,N] (packed P/r) and, where present, the
+    compensated low part x_lo [4,N] and the tuning objective loss [N]."""
+    out = {"state_x": st.x, "state_p": st.p}
+    for name in ("x_lo", "loss"):
+        if getattr(st, name) is not None:
+            out["state_" + name] = getattr(st, name)
+    return out
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes {name: tensor [..., N]} (one N for all) as out_dir/<name>.npy in float32.  Where all N columns would
+    exceed DUMP_BYTES, every array keeps the same sample of columns, drawn with a fixed seed and kept in order."""
+    import numpy as np
+    import torch
+    n = next(iter(arrays.values())).shape[-1]
+    col_bytes = sum(4 * a.numel() // max(n, 1) for a in arrays.values())
+    keep = min(n, DUMP_BYTES // col_bytes)
+    idx = None if keep == n else torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if idx is not None:
+            a = a[..., idx.to(a.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.detach().float().cpu().numpy())
 
 
 def executed_arithmetic(wahba: str):
@@ -229,9 +266,9 @@ def run_reference(args):
     world = int(os.environ.get("WORLD_SIZE", str(args.gpus)))
     name, filters, timesteps = resolve_workload(args, world)
     base = cpu_baseline(max(5.0, args.cpu_seconds))
-    # K "steps" of the contract = K repetitions of the bounded sample (at most 3 are run); report the mean rate
+    # K steps = K repetitions of the bounded sample; report the mean rate
     vals = [base["value"]]
-    for _ in range(max(0, min(args.steps, 3) - 1)):
+    for _ in range(args.steps - 1):
         vals.append(cpu_baseline(max(5.0, args.cpu_seconds))["value"])
     v = sum(vals) / len(vals)
     base["value"] = v
@@ -539,6 +576,8 @@ def run_c2(ctx, args):
     total_ms = ctx.max_over_ranks(e_all0.elapsed_time(e_all1))
     kernel_ms = [a.elapsed_time(b) for a, b in evs]
     clocks = sampler.stop(t_wall0, t_wall1) if ctx.rank == 0 else None
+    if ctx.rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, state_arrays(fresh[-1]))
     del fresh
 
     ms_per_step = total_ms / K
@@ -633,6 +672,8 @@ def run_c5(ctx, args):
     ctx.barrier()
     t_wall1 = time.perf_counter()
     clocks = sampler.stop(t_wall0, t_wall1) if ctx.rank == 0 else None
+    if ctx.rank == 0 and args.dump_outputs:         # rank 0's shard
+        dump_outputs(args.dump_outputs, state_arrays(state))
     ms_per_step = sum(per_pass) / K
     value = N_total * T / (ms_per_step * 1e-3)
     own_rate = job.n_local * T / (ms_per_step * 1e-3)
@@ -719,6 +760,8 @@ def run_c3(ctx, args):
     ctx.barrier()
     t1w = time.perf_counter()
     clocks = sampler.stop(t0w, t1w) if ctx.rank == 0 else None
+    if ctx.rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, state_arrays(st))
     ms_per_step = ctx.max_over_ranks(e0.elapsed_time(e1)) / K
     T, Ns = w.streams.shape[0], w.streams.shape[2]
     total_filters = 64 * 64 * Ns
@@ -764,6 +807,8 @@ def run_c4(ctx, args):
         out[weights] = ms
     if ctx.rank != 0:
         return None
+    if args.dump_outputs:                           # the last timed step used the reference weights
+        dump_outputs(args.dump_outputs, {"quat": w.out})
     peaks = {}
     try:
         peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))

@@ -152,7 +152,7 @@ def test_reference_arm_contract_under_torchrun_world2():
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
-           "--master-port", "29533", os.path.join(root, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1",
+           "--master-port", str(_free_port()), os.path.join(root, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1",
            "--warmup", "1", "--cpu-seconds", "1"]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=root)
     assert out.returncode == 0, out.stderr[-2000:]
@@ -238,6 +238,34 @@ def test_bench_workload_selection_and_evidence_stamps():
     assert prof["kernel_source_sha"] == sha, "profiles/r02_replay_packed_ncu_full.json was captured from other device sources: re-profile"
     ref = bench.find_reference()
     assert ref is None or os.path.exists(os.path.join(ref, "ExtendedKalmanFilter.py"))
+
+
+def test_bench_dump_outputs_and_argument_checks(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 .npy per array; over the byte bound, the same seeded, ordered sample of filter
+    columns for every array and for every run.  --steps below 1 and a dump of the reference arm are refused."""
+    import bench
+    st = B.ReplayState.initial(1000, "cpu", r=0.1)
+    st.x = torch.randn(4, 1000, dtype=torch.float64)
+    st.loss = torch.arange(1000, dtype=torch.float32)
+    arrays = bench.state_arrays(st)
+    assert sorted(arrays) == ["state_loss", "state_p", "state_x"]
+    bench.dump_outputs(str(tmp_path / "all"), arrays)
+    for name, a in arrays.items():
+        got = np.load(tmp_path / "all" / f"{name}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, a.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 15 * 4 * 100)          # 15 floats per filter: room for 100 filters
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), arrays)
+    keep = np.load(tmp_path / "a" / "state_loss.npy").astype(np.int64)
+    assert keep.size == 100 and (np.diff(keep) > 0).all()
+    for name, a in arrays.items():
+        got = np.load(tmp_path / "a" / f"{name}.npy")
+        assert np.array_equal(got, np.load(tmp_path / "b" / f"{name}.npy"))
+        assert np.array_equal(got, a.float().numpy()[..., keep])
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
+        with pytest.raises(SystemExit):
+            bench.parse()
 
 
 def test_scale_validation_and_precision_rule_cache():
