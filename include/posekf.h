@@ -124,6 +124,29 @@ int posekf_replay_f32(int64_t n_filters, int64_t n_steps, const float* streams, 
                       uint8_t* out_flip, const float* truth, float* loss_acc, int wahba_algo, int staging,
                       int state_flags, void* stream);
 
+/* The same replay with the INNOVATION LIKELIHOOD of every filter accumulated on the device: a (Q,R) tuning objective
+ * that needs no ground truth (a recorded log has none).  It is the filter's own Gaussian model of its innovations
+ * (prediction-error decomposition), natural log, P and R unscaled:
+ *     l(Q,R) = 1/2 sum_t [ NIS_t + ln det S_t + 4 ln 2 pi ],   NIS_t = e_t^T S_t^-1 e_t,
+ *     S_t = P_t + R   (the matrix inverted at PKF/ExtendedKalmanFilter.py:63-65),
+ *     e_t = y_t - z_t (the innovation of :76, y sign-fixed by the comparator :73-75).
+ * All parameters are those of posekf_replay_f32, plus
+ *   innov_acc   [2][N] in/out, required (NULL: POSEKF_EINVAL), 4-byte aligned (8-byte for the packed kernel; AUTO
+ *               falls back to the scalar TMA kernel otherwise):  innov_acc[0][n] += sum_t NIS_t,
+ *               innov_acc[1][n] += sum_t ln det S_t over the n_steps of the launch.  Start at 0 and pass the same buffer
+ *               to every launch of a time-chunked replay (with the state flags above): the sums equal the unchunked
+ *               replay's bit for bit.  Then  NLL = (innov_acc[0] + innov_acc[1]) / 2 + 2 T ln 2 pi,
+ *               mean NIS = innov_acc[0] / T.
+ * The statistic does not perturb the filter: state, trajectory and flip mask are those of posekf_replay_f32.  Both
+ * terms are invariant under the kernels' filter-frame rotation.  Combinations of the packed staging with per-step
+ * outputs or the low-pass run in the scalar kernels (same results bit for bit). */
+int posekf_replay_innovation_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams,
+                                 const float* dt, int dt_per_step, const float* acc_ref, const float* mag_ref,
+                                 const float* q_scale, const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag,
+                                 float* state_x, float* state_x_lo, float* state_p, float* state_lpf, float* out_traj,
+                                 uint8_t* out_flip, const float* truth, float* loss_acc, float* innov_acc, int wahba_algo,
+                                 int staging, int state_flags, void* stream);
+
 /* Same replay with HOST buffers: streams_host [T][9][N] is streamed through the device in time
  * chunks (double-buffered H2D copies overlapped with the filter kernel, state carried across
  * chunks on the device), results are copied back.  This is the call an offline-replay user makes.

@@ -13,6 +13,7 @@ per-filter `[N, k]` / `[N, 4, 4]` shapes.
 """
 from __future__ import annotations
 
+import math
 import weakref
 from dataclasses import dataclass
 
@@ -83,7 +84,8 @@ class ReplayState:
     r: the float or [N] tensor the scaling refers to; lpf [6,N] or None.
     frame: "reference" (x, p in the reference's own coordinates -- what every `replay` call returns by
     default) or "filter" (left in the kernel's working frame by `replay(..., keep_filter_frame=True)`
-    between the chunks of a time-chunked replay; `to_reference_frame` converts)."""
+    between the chunks of a time-chunked replay; `to_reference_frame` converts).
+    innov [2,N]: the innovation likelihood sums (sum_t NIS_t, sum_t ln det S_t) of `replay(..., innovation=...)`."""
     x: torch.Tensor
     p: torch.Tensor
     r: object = 0.1
@@ -91,6 +93,7 @@ class ReplayState:
     loss: torch.Tensor | None = None     # [N] accumulated tuning objective (see replay(truth=...))
     x_lo: torch.Tensor | None = None     # [4,N] low-order part of the compensated (two-float) state
     frame: str = "reference"
+    innov: torch.Tensor | None = None    # [2,N] innovation likelihood sums (see replay(innovation=...))
 
     @staticmethod
     def initial(n_filters: int, device, r=0.1, with_lpf: bool = False, P0: torch.Tensor | None = None) -> "ReplayState":
@@ -113,7 +116,8 @@ class ReplayState:
 
     def clone(self) -> "ReplayState":
         c = lambda t: None if t is None else t.clone()
-        return ReplayState(self.x.clone(), self.p.clone(), self.r, c(self.lpf), c(self.loss), c(self.x_lo), self.frame)
+        return ReplayState(self.x.clone(), self.p.clone(), self.r, c(self.lpf), c(self.loss), c(self.x_lo), self.frame,
+                           c(self.innov))
 
     def to_reference_frame(self, acc_ref: torch.Tensor, mag_ref: torch.Tensor) -> "ReplayState":
         """Convert (in place) a state that `replay(..., keep_filter_frame=True)` left in the kernel's working
@@ -237,7 +241,8 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
            lpf_alpha_mag: float | None = None, out_traj: torch.Tensor | None = None, store_trajectory: bool = False,
            store_flips: bool = False, truth: torch.Tensor | None = None, loss: torch.Tensor | None = None,
            precise_state: bool | None = None, share_measurements: bool | None = None, wahba: str = "qr2",
-           staging: str = "auto", keep_filter_frame: bool = False, allow_imprecise: bool = False):
+           staging: str = "auto", keep_filter_frame: bool = False, allow_imprecise: bool = False,
+           innovation: bool | torch.Tensor | None = None):
     """Run T Prediction+Correction steps for N filters in one kernel launch.
 
     streams [T,9,Ns]; acc_ref, mag_ref [3,Ns]; dt: float seconds or [T] float32 CUDA tensor;
@@ -264,6 +269,11 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     launch.  Pass it on every chunk but the last of a time-chunked replay: the chunked replay is then
     bit-identical to the unchunked one.  `state.frame` records where the state is; a state left in the filter
     frame is accepted by the next `replay` call and converted by `state.to_reference_frame(acc_ref, mag_ref)`.
+    `innovation`: accumulate the innovation likelihood of every filter on the device -- the (Q,R) tuning objective that
+    needs no ground truth (include/posekf.h, posekf_replay_innovation_f32).  True creates a zeroed [2,N] accumulator
+    (sum_t NIS_t, sum_t ln det S_t); a tensor is used as is (pass `state.innov` back in for chunked replays).  It is
+    available as `state.innov`; `innovation_nll` turns it into per-filter NLL and mean NIS.  It does not perturb the
+    filter.  None / False: the launch is exactly that of a replay without it.
     Returns (state, traj [T,N,4] or None, flips [T,N] uint8 or None)."""
     _require_cuda(streams, acc_ref, mag_ref, out_traj)
     if streams.dim() != 3 or streams.shape[1] != 9:
@@ -299,7 +309,8 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
                 and out_traj is None and not store_trajectory and not store_flips and not use_lpf and T > 0:
             # a (Q,R) sweep: only the cells with r/q >= 100 or q/r >= 1e4 need the precise variant (+25 % time)
             mixed = _replay_sweep_mixed(streams, acc_ref, mag_ref, dt=dt, q=q, r=r, state=state, N=N, Ns=Ns, truth=truth,
-                                        loss=loss, wahba=wahba, staging=staging, keep_filter_frame=keep_filter_frame)
+                                        loss=loss, wahba=wahba, staging=staging, keep_filter_frame=keep_filter_frame,
+                                        innovation=innovation)
             if mixed is not None:
                 return mixed
         precise_state = state.x_lo is not None or needs_precise
@@ -340,18 +351,49 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
         if loss is None:
             loss = torch.zeros((N,), dtype=torch.float32, device=dev)
         state.loss = loss
-    with torch.cuda.device(dev):
-        rc = _lib.load().posekf_replay_f32(
-            N, T, _ptr(streams), Ns, _ptr(dt_t), per_step, _ptr(acc_ref), _ptr(mag_ref), _ptr(q_t), _ptr(r_t),
+    innov = _innovation_buffer(innovation, N, dev)
+    args = (N, T, _ptr(streams), Ns, _ptr(dt_t), per_step, _ptr(acc_ref), _ptr(mag_ref), _ptr(q_t), _ptr(r_t),
             -1.0 if lpf_alpha_acc is None else float(lpf_alpha_acc),
             -1.0 if lpf_alpha_mag is None else float(lpf_alpha_mag),
             _ptr(state.x), _ptr(state.x_lo if precise_state else None), _ptr(state.p), _ptr(state.lpf), _ptr(out_traj),
-            _ptr(flips), _ptr(truth),
-            _ptr(loss if truth is not None else None), _lib.WAHBA[wahba], _lib.STAGING[staging], frame_flags, _stream())
-    _lib.check(rc, "posekf_replay_f32")
+            _ptr(flips), _ptr(truth), _ptr(loss if truth is not None else None))
+    tail = (_lib.WAHBA[wahba], _lib.STAGING[staging], frame_flags, _stream())
+    with torch.cuda.device(dev):
+        if innov is None:
+            rc = _lib.load().posekf_replay_f32(*args, *tail)
+        else:
+            rc = _lib.load().posekf_replay_innovation_f32(*args, _ptr(innov), *tail)
+    _lib.check(rc, "posekf_replay_f32" if innov is None else "posekf_replay_innovation_f32")
+    if innov is not None:
+        state.innov = innov
     if wahba != "precomputed":
         state.frame = "filter" if keep_filter_frame else "reference"
     return state, out_traj, flips
+
+
+def _innovation_buffer(innovation, n: int, device):
+    """The [2,N] accumulator of replay(innovation=...): None when off, zeros for True, the caller's tensor otherwise."""
+    if innovation is None or innovation is False:
+        return None
+    if innovation is True:
+        return torch.zeros((2, n), dtype=torch.float32, device=device)
+    _require_cuda(innovation)
+    if innovation.shape != (2, n):
+        raise ValueError(f"innovation accumulator must be [2, {n}]")
+    return innovation
+
+
+def innovation_nll(innov, n_steps: int):
+    """Per-filter innovation likelihood from the [2,N] sums of `replay(..., innovation=...)` (or a ReplayState holding
+    them) over `n_steps` steps: (NLL [N], mean NIS [N]) in float64,
+        NLL = 1/2 sum_t [NIS_t + ln det S_t] + 2 T ln 2 pi,     mean NIS = sum_t NIS_t / T
+    (natural log; P and R unscaled).  A good (Q,R) minimises the NLL."""
+    a = innov.innov if isinstance(innov, ReplayState) else innov
+    if a is None:
+        raise ValueError("no innovation sums: replay with innovation=True")
+    a = a.to(torch.float64)
+    T = float(n_steps)
+    return 0.5 * (a[0] + a[1]) + 2.0 * T * math.log(2.0 * math.pi), a[0] / T
 
 
 def sweep_partition(q_t: torch.Tensor, r_t: torch.Tensor, n_streams: int):
@@ -368,7 +410,8 @@ def sweep_partition(q_t: torch.Tensor, r_t: torch.Tensor, n_streams: int):
     return expand((~need).nonzero().flatten()), expand(need.nonzero().flatten())
 
 
-def _replay_sweep_mixed(streams, acc_ref, mag_ref, *, dt, q, r, state, N, Ns, truth, loss, wahba, staging, keep_filter_frame):
+def _replay_sweep_mixed(streams, acc_ref, mag_ref, *, dt, q, r, state, N, Ns, truth, loss, wahba, staging, keep_filter_frame,
+                        innovation=None):
     """Sweep layout with automatic precision: the cells (blocks of Ns filters sharing one (q, r)) whose tuning is
     extreme run the precise variant, the others the plain one -- two launches over a cell permutation that keeps
     every filter on its own stream column (n % Ns).  Returns None when one launch serves all cells."""
@@ -380,26 +423,32 @@ def _replay_sweep_mixed(streams, acc_ref, mag_ref, *, dt, q, r, state, N, Ns, tr
     parts = []
     if truth is not None and loss is None:
         loss = torch.zeros((N,), dtype=torch.float32, device=dev)
+    innov = _innovation_buffer(innovation, N, dev)
     for idx, precise in ((idx_plain, False), (idx_precise, True)):
         sub = ReplayState(state.x[:, idx].contiguous(), state.p[:, idx].contiguous(), r_t[idx].contiguous(), None, None,
                           state.x_lo[:, idx].contiguous() if (precise and state.x_lo is not None) else None, state.frame)
         sub_loss = loss[idx].contiguous() if truth is not None else None
+        sub_innov = innov[:, idx].contiguous() if innov is not None else None
         replay(streams, acc_ref, mag_ref, dt=dt, q=q_t[idx].contiguous(), r=sub.r, state=sub, n_filters=idx.numel(), truth=truth,
                loss=sub_loss, precise_state=precise, share_measurements=False, wahba=wahba, staging=staging,
-               keep_filter_frame=keep_filter_frame)      # (the plain group holds no extreme cell by construction)
-        parts.append((idx, sub, sub_loss, precise))
+               keep_filter_frame=keep_filter_frame, innovation=sub_innov)   # (the plain group holds no extreme cell by construction)
+        parts.append((idx, sub, sub_loss, sub_innov, precise))
     if state.x_lo is None:
         state.x_lo = torch.zeros((4, N), dtype=torch.float32, device=dev)
-    for idx, sub, sub_loss, precise in parts:
+    for idx, sub, sub_loss, sub_innov, precise in parts:
         state.x[:, idx] = sub.x
         state.p[:, idx] = sub.p
         if precise:
             state.x_lo[:, idx] = sub.x_lo
         if truth is not None:
             loss[idx] = sub_loss
+        if innov is not None:
+            innov[:, idx] = sub_innov
         state.frame = sub.frame
     if truth is not None:
         state.loss = loss
+    if innov is not None:
+        state.innov = innov
     state.r = r
     return state, None, None
 

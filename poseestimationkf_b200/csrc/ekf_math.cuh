@@ -72,6 +72,18 @@ template <> inline double fma_<double>(double a, double b, double c) { return fm
 template <> inline double sqrt_<double>(double a) { return sqrt(a); }
 template <> inline double rsqrt_<double>(double a) { return 1.0 / sqrt(a); }
 #endif
+// natural logarithms of the innovation statistic (full precision: see log_pivots)
+template <typename F> PKF_HD F log_(F a) { return (F)log((double)a); }
+template <typename F> PKF_HD F log1p_(F a) { return (F)log1p((double)a); }
+#if defined(__CUDA_ARCH__)
+template <> __device__ __forceinline__ float log_<float>(float a) { return logf(a); }
+template <> __device__ __forceinline__ float log1p_<float>(float a) { return log1pf(a); }
+#else
+template <> inline float log_<float>(float a) { return logf(a); }
+template <> inline float log1p_<float>(float a) { return log1pf(a); }
+template <> inline double log_<double>(double a) { return log(a); }
+template <> inline double log1p_<double>(double a) { return log1p(a); }
+#endif
 
 template <typename F> PKF_HD F sel_(bool c, F a, F b) { return c ? a : b; }
 PKF_HD bool any_(bool m) { return m; }
@@ -197,6 +209,8 @@ template <> PKF_HD f32x2 abs_<f32x2>(f32x2 a) { return f32x2(abs_<float>(a.x), a
 template <> PKF_HD f32x2 rcp_<f32x2>(f32x2 a) { return f32x2(rcp_<float>(a.x), rcp_<float>(a.y)); }
 template <> PKF_HD f32x2 rsqrt_<f32x2>(f32x2 a) { return f32x2(rsqrt_<float>(a.x), rsqrt_<float>(a.y)); }
 template <> PKF_HD f32x2 sqrt_<f32x2>(f32x2 a) { return f32x2(sqrt_<float>(a.x), sqrt_<float>(a.y)); }
+template <> PKF_HD f32x2 log_<f32x2>(f32x2 a) { return f32x2(log_<float>(a.x), log_<float>(a.y)); }
+template <> PKF_HD f32x2 log1p_<f32x2>(f32x2 a) { return f32x2(log1p_<float>(a.x), log1p_<float>(a.y)); }
 
 // ------------------------------------------------------------------------------------------
 // types
@@ -439,6 +453,59 @@ template <typename F> struct Ldl4 {          // S = P + I = L D L^T;  N = L^-1 -
   F n10, n20, n21, n30, n31, n32, i0, i1, i2, i3, e0, e1, e2, e3;
 };
 
+// ------------------------------------------------------------------------------------------
+// Innovation likelihood (prediction-error decomposition of the filter's own Gaussian model):
+//     l(Q,R) = 1/2 sum_t [ e_t^T S_t^-1 e_t + ln det S_t + 4 ln 2 pi ],   S = P^- + R,  e = sg y/|y| - z
+// (S and e of PKF/ExtendedKalmanFilter.py:63,76).  The step carries S~ = S/r = P~ + I, so
+//     NIS = e^T S^-1 e = (1/r) e^T S~^-1 e,     ln det S = 4 ln r + ln det S~.
+// The gain stage hands over the factors it has already formed (InnovFactors); the step feeds the innovation e it
+// forms anyway.  Both terms are invariant under the filter-frame rotation (e and S are rotated by the orthogonal
+// L(p)), so no conversion back to the reference frame is needed.
+//   plain   (kalman_gain_from_s): S~ = L D L^T;  e^T S~^-1 e = sum_k i_k t_k^2, t = (I + N) e;  ln det S~ = sum_k ln d_k
+//   precise (kalman_gain_sm):     S~ = H - g x x^T;  Sherman-Morrison and the matrix-determinant lemma give
+//           e^T S~^-1 e = sum_k i_k t_k^2 (H's factors) + beta (w.e)^2,   ln det S~ = sum_k ln d_k(H) + ln(num / |x|^2)
+// (S~^-1 = I - K would cancel as K -> I: the factors are used instead.)
+// ------------------------------------------------------------------------------------------
+template <typename F> struct InnovFactors {
+  F n10, n20, n21, n30, n31, n32;   // N = L^-1 - I of S~ (plain) or of H (precise)
+  F i0, i1, i2, i3;                 // 1/d_k
+  F w0, w1, w2, w3, beta;           // precise only: w = H^-1 x, beta = g|x|^2 / x^T(I+M)w
+  F logdet;                         // ln det S~
+};
+// Running sums of one filter (true units) and the launch constants that fold 1/r and 4 ln r in per step: the sums are
+// never rescaled, so a chunked replay accumulates exactly what the unchunked one does.
+template <typename F> struct InnovAcc {
+  F nis, logdet;
+  F inv_r, log_r4;
+};
+template <typename F> PKF_HD InnovAcc<F> make_innov_acc(F nis, F logdet, F r) {
+  InnovAcc<F> a;
+  a.nis = nis; a.logdet = logdet;
+  a.inv_r = F(1) / r;
+  a.log_r4 = F(4) * log_(r);
+  return a;
+}
+// sum_k ln(1 + x_k) from the pivot excesses x_k = d_k - 1 >= 0: the excess of the product is formed first and its
+// log1p taken, so that pivots near 1 (R >> Q, where ln det S~ is small) keep their relative accuracy.
+template <typename F> PKF_HD F log_pivots(F x0, F x1, F x2, F x3) {
+  const F a = fma_(x0, x1, x0 + x1), b = fma_(x2, x3, x2 + x3);
+  return log1p_(fma_(a, b, a + b));
+}
+template <typename F, bool COMP>
+PKF_HD void innov_accumulate(InnovAcc<F>& acc, const InnovFactors<F>& f, F e0, F e1, F e2, F e3) {
+  const F t1 = fma_(f.n10, e0, e1);
+  const F t2 = fma_(f.n21, e1, fma_(f.n20, e0, e2));
+  const F t3 = fma_(f.n32, e2, fma_(f.n31, e1, fma_(f.n30, e0, e3)));
+  const F u0 = f.i0 * e0, u1 = f.i1 * t1, u2 = f.i2 * t2, u3 = f.i3 * t3;
+  F s = fma_(u3, t3, fma_(u2, t2, fma_(u1, t1, u0 * e0)));
+  if constexpr (COMP) {
+    const F we = fma_(f.w3, e3, fma_(f.w2, e2, fma_(f.w1, e1, f.w0 * e0)));
+    s = fma_(f.beta * we, we, s);
+  }
+  acc.nis = fma_(s, acc.inv_r, acc.nis);
+  acc.logdet = acc.logdet + (f.logdet + acc.log_r4);
+}
+
 template <typename F> PKF_HD Ldl4<F> ldl_unit(const Sym4<F>& P) {
   // P is the predicted covariance IN UNITS OF r (P/r), so S = P + I and rho_k = 1/d_k.
   const F p01 = P.a01, p02 = P.a02, p03 = P.a03, p12 = P.a12, p13 = P.a13, p23 = P.a23;
@@ -491,23 +558,32 @@ template <typename F> PKF_HD Sym4<F> kalman_gain_unit(const Sym4<F>& P) { return
 // kappa_k = 1 - 1/d_k.  Four additions fewer than the split-pivot form; kappa loses eps/kappa of relative accuracy,
 // i.e. 2.4e-5 at the edge of the plain variant's range (r/q = 100, kappa = 2.5e-3), which moves the state by 1e-9 --
 // beyond that range the precise variant (split pivots, kalman_gain_sm) is selected.
-template <typename F> PKF_HD Sym4<F> kalman_gain_from_s(const Sym4<F>& S) {
+template <typename F, bool INNOV = false>
+PKF_HD Sym4<F> kalman_gain_from_s(const Sym4<F>& S, InnovFactors<F>* fac = nullptr) {
   const F p01 = S.a01, p02 = S.a02, p03 = S.a03, p12 = S.a12, p13 = S.a13, p23 = S.a23;
   const F i0 = rcp_(S.a00);
   const F l10 = p01 * i0, l20 = p02 * i0, l30 = p03 * i0;
-  const F i1 = rcp_(fma_(-l10, p01, S.a11));
+  const F d1 = fma_(-l10, p01, S.a11);
+  const F i1 = rcp_(d1);
   const F t21 = fma_(-l10, p02, p12);
   const F t31 = fma_(-l10, p03, p13);
   const F l21 = t21 * i1, l31 = t31 * i1;
-  const F i2 = rcp_(fma_(-l21, t21, fma_(-l20, p02, S.a22)));
+  const F d2 = fma_(-l21, t21, fma_(-l20, p02, S.a22));
+  const F i2 = rcp_(d2);
   const F t32 = fma_(-l21, t31, fma_(-l20, p03, p23));
   const F l32 = t32 * i2;
-  const F i3 = rcp_(fma_(-l32, t32, fma_(-l31, t31, fma_(-l30, p03, S.a33))));
+  const F d3 = fma_(-l32, t32, fma_(-l31, t31, fma_(-l30, p03, S.a33)));
+  const F i3 = rcp_(d3);
   // N = L^-1 - I
   const F n10 = -l10, n21 = -l21, n32 = -l32;
   const F n20 = fma_(-l21, n10, -l20);
   const F n31 = fma_(-l32, n21, -l31);
   const F n30 = fma_(-l32, n20, fma_(-l31, n10, -l30));
+  if constexpr (INNOV) {     // the pivots d_k of S~ = P~ + I are >= 1: their excesses d_k - 1 are exact differences
+    fac->n10 = n10; fac->n20 = n20; fac->n21 = n21; fac->n30 = n30; fac->n31 = n31; fac->n32 = n32;
+    fac->i0 = i0; fac->i1 = i1; fac->i2 = i2; fac->i3 = i3;
+    fac->logdet = log_pivots(S.a00 - F(1), d1 - F(1), d2 - F(1), d3 - F(1));
+  }
   const F v30 = -(i3 * n30), v31 = -(i3 * n31), v32 = -(i3 * n32);
   const F v20 = -(i2 * n20), v21 = -(i2 * n21);
   const F v10 = -(i1 * n10);
@@ -534,7 +610,8 @@ template <typename F> PKF_HD Sym4<F> kalman_gain_from_s(const Sym4<F>& S) {
 //   den = 1 - g x^T w = x^T (I + M) w / |x|^2   (from (I + M) w + g|x|^2 w = x; no cancellation;
 //         w itself comes from the LDL^T factors of H, not from x - K_H x),
 //   K = I - S^-1 = K_H - beta w w^T,  K_H = I - H^-1 (split-pivot form above),  beta = g|x|^2 / x^T(I+M)w.
-template <typename F> PKF_HD Sym4<F> kalman_gain_sm(const Sym4<F>& M, const Quat<F>& x, F g) {
+template <typename F, bool INNOV = false>
+PKF_HD Sym4<F> kalman_gain_sm(const Sym4<F>& M, const Quat<F>& x, F g, InnovFactors<F>* fac = nullptr) {
   const F x2 = dot4(x, x);
   const F c = g * x2;
   Sym4<F> PH = M;
@@ -558,6 +635,16 @@ template <typename F> PKF_HD Sym4<F> kalman_gain_sm(const Sym4<F>& M, const Quat
   F g3 = fma_(M.a33, w3, fma_(M.a23, w2, fma_(M.a13, w1, fma_(M.a03, w0, w3))));
   F num = fma_(x.z, g3, fma_(x.y, g2, fma_(x.x, g1, x.w * g0)));
   F nb = -(c * rcp_(num));                     // -beta
+  if constexpr (INNOV) {
+    fac->n10 = f.n10; fac->n20 = f.n20; fac->n21 = f.n21; fac->n30 = f.n30; fac->n31 = f.n31; fac->n32 = f.n32;
+    fac->i0 = f.i0; fac->i1 = f.i1; fac->i2 = f.i2; fac->i3 = f.i3;
+    fac->w0 = w0; fac->w1 = w1; fac->w2 = w2; fac->w3 = w3; fac->beta = -nb;
+    // ln(num/|x|^2) = ln(1 - g x.w): through log1p while g x.w is small (R >> Q: the term is ~ -g and the quotient
+    // would round it away), through the quotient itself when it is small (Q >> R: 1 - g x.w would cancel)
+    const F u = g * fma_(x.z, w3, fma_(x.y, w2, fma_(x.x, w1, x.w * w0)));
+    const F lden = sel_(u < F(0.5), log1p_(-u), log_(num * rcp_(x2)));
+    fac->logdet = log_pivots(f.e0, f.e1, f.e2, f.e3) + lden;
+  }
   F b0 = nb * w0, b1 = nb * w1, b2 = nb * w2, b3 = nb * w3;
   Sym4<F> K;
   K.a00 = fma_(b0, w0, KH.a00); K.a01 = fma_(b0, w1, KH.a01); K.a02 = fma_(b0, w2, KH.a02); K.a03 = fma_(b0, w3, KH.a03);
@@ -1064,22 +1151,24 @@ PKF_HD void quat_fallback_unaligned(const Mat3<f32x2>& Rm, const Quat<f32x2>& z,
 // ---- the three parts of a step -------------------------------------------------------------------
 // Prediction (PKF/ExtendedKalmanFilter.py:58-68): gain K (= the post-update covariance in units of r), RK4
 // increment inc and predicted state z = x + inc.
-template <typename F, bool COMP>
+// INNOV: the gain stage also hands its factors of S~ to `fac` (innovation likelihood, see InnovFactors).
+template <typename F, bool COMP, bool INNOV = false>
 PKF_HD void ekf_predict(const Quat<F>& x, const Sym4<F>& P, const FilterConst<F>& fc, const Vec3<F>& gyro, const StepH<F>& h,
-                        Sym4<F>& K, Quat<F>& inc, Quat<F>& z) {
+                        Sym4<F>& K, Quat<F>& inc, Quat<F>& z, InnovFactors<F>* fac = nullptr) {
   Vec3<F> hw;
   hw.x = F(0.5) * gyro.x; hw.y = F(0.5) * gyro.y; hw.z = F(0.5) * gyro.z;
   if constexpr (COMP) {
     Sym4<F> M = propagate_cov<F, false>(P, hw, x, fc.g, fc.gs);               // :59-61, noise kept apart
-    K = kalman_gain_sm(M, x, fc.gs);                                          // :63-66
+    K = kalman_gain_sm<F, INNOV>(M, x, fc.gs, fac);                           // :63-66
   } else {
 #if PKF_FUSE
     Sym4<F> S = propagate_cov<F, true>(P, hw, x, fc.g, fc.gs, fc.gs1);        // :59-61 and S = P + R :63 (in units of r)
-    K = kalman_gain_from_s(S);                                                // :64-66
+    K = kalman_gain_from_s<F, INNOV>(S, fac);                                 // :64-66
     z = rk4_predict_fused(x, hw, h);                                          // :62
     inc = z;                                                                  // (unused by the plain update)
     return;
 #else
+    static_assert(!INNOV, "the innovation statistic takes its factors from the fused plain gain (PKF_FUSE)");
     Sym4<F> Pp = propagate_cov<F, true>(P, hw, x, fc.g, fc.gs);               // :59-61 (in units of r)
     K = kalman_gain_unit(Pp);                                                 // :63-66
 #endif
@@ -1161,48 +1250,52 @@ PKF_HD Quat<F> measure_quat(const FilterConst<F>& fc, const Vec3<F>& acc, const 
 }
 
 // Prediction + Correction with the measurement quaternion y (filter frame, any sign, norm 1/inv_norm) already computed.
-template <typename F, bool WANT_FLIP, bool COMP, typename FlagT>
+// INNOV: the innovation likelihood of the step is added to *innov (see InnovAcc); the filter itself is unchanged.
+template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, typename FlagT>
 PKF_HD void ekf_step_measured(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, const Vec3<F>& gyro,
                               const Quat<F>& y, F inv_norm, const StepH<F>& h, FlagT& flip, bool flip_wanted = true,
-                              typename FlipCodeOf<F>::type* code = nullptr) {
+                              typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr) {
   Sym4<F> K;
   Quat<F> inc, z;
-  ekf_predict<F, COMP>(x, P, fc, gyro, h, K, inc, z);
+  InnovFactors<F> fac;
+  ekf_predict<F, COMP, INNOV>(x, P, fc, gyro, h, K, inc, z, &fac);
   const F dyz = dot4(y, z);                       // the comparator, literally: negate when dot(y, z) < 0  :73-75
   flip = FlagT();
   if (WANT_FLIP && flip_wanted) flip = reference_flip_quat(fc, y, one_with_sign_(dyz), code);
   const F sn = copysign_(inv_norm, dyz);          // e = sg y/|y| - z, sg = sign(dot): the sign bit moves onto 1/|y| > 0  :76
   const F e0 = fma_(sn, y.w, -z.w), e1 = fma_(sn, y.x, -z.x), e2 = fma_(sn, y.y, -z.y), e3 = fma_(sn, y.z, -z.z);
+  if constexpr (INNOV) innov_accumulate<F, COMP>(*innov, fac, e0, e1, e2, e3);
   ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);
 }
 
 // The common case of ekf_step<WAHBA_QR2>: both Wahba weights are non-negative (|a_z| <= 1, i.e. a normalised
 // accelerometer), so the closed-form measurement applies and the step has no data-dependent branch.  The caller
 // guarantees the precondition (the packed kernel checks a whole tile of samples before taking this path).
-template <typename F, bool WANT_FLIP, bool COMP, typename FlagT>
+template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, typename FlagT>
 PKF_HD void ekf_step_plain_measured(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, const Vec3<F>& gyro,
                                     const Vec3<F>& acc, const Vec3<F>& mag, const StepH<F>& h, FlagT& flip, bool flip_wanted = true,
-                                    typename FlipCodeOf<F>::type* code = nullptr) {
+                                    typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr) {
   const F ka = abs_(acc.z), km = F(1) - ka;
   F inv_norm;
   const Quat<F> y = wahba_quat2_local(fc.E, acc, mag, ka, km, inv_norm);
-  ekf_step_measured<F, WANT_FLIP, COMP>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code);
+  ekf_step_measured<F, WANT_FLIP, COMP, INNOV>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code, innov);
 }
 
-template <typename F, int ALGO, bool WANT_FLIP, bool COMP, typename FlagT>
+template <typename F, int ALGO, bool WANT_FLIP, bool COMP, bool INNOV = false, typename FlagT>
 PKF_HD void ekf_step(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, const Vec3<F>& gyro,
                      const Vec3<F>& acc, const Vec3<F>& mag, const StepH<F>& h, FlagT& flip, bool flip_wanted = true,
-                     typename FlipCodeOf<F>::type* code = nullptr) {
+                     typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr) {
   // flip_wanted: launch-uniform run-time switch under WANT_FLIP -- a launch that stores the trajectory but
   // not the flip mask skips the reference's branch rule altogether
   if constexpr (ALGO == WAHBA_QR2) {
     F inv_norm;
     const Quat<F> y = measure_quat(fc, acc, mag, inv_norm);
-    ekf_step_measured<F, WANT_FLIP, COMP>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code);
+    ekf_step_measured<F, WANT_FLIP, COMP, INNOV>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code, innov);
   } else {
     Sym4<F> K;
     Quat<F> inc, z;
-    ekf_predict<F, COMP>(x, P, fc, gyro, h, K, inc, z);
+    InnovFactors<F> fac;
+    ekf_predict<F, COMP, INNOV>(x, P, fc, gyro, h, K, inc, z, &fac);
     // ---- Correction (PKF/ExtendedKalmanFilter.py:70-80) ----
     F e0, e1, e2, e3;
     if constexpr (ALGO == WAHBA_PRECOMPUTED) {
@@ -1236,6 +1329,7 @@ PKF_HD void ekf_step(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, c
         e2 = sel_(unrelated, yf.y - z.y, e2); e3 = sel_(unrelated, yf.z - z.z, e3);
       }
     }
+    if constexpr (INNOV) innov_accumulate<F, COMP>(*innov, fac, e0, e1, e2, e3);
     ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);
   }
 }

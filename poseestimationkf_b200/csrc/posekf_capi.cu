@@ -90,15 +90,16 @@ bool tma_eligible(const ReplayParams& p) {
   return true;
 }
 
-template <int ALGO, bool LPF, bool AUX, bool COMP> int launch_replay(const ReplayParams& p, bool use_tma, cudaStream_t st) {
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false>
+int launch_replay(const ReplayParams& p, bool use_tma, cudaStream_t st) {
   const unsigned grid = (unsigned)((p.N + kThreads - 1) / kThreads);
   if (!use_tma) {
-    replay_ldg_kernel<ALGO, LPF, AUX, COMP><<<grid, kThreads, 0, st>>>(p);
+    replay_ldg_kernel<ALGO, LPF, AUX, COMP, INNOV><<<grid, kThreads, 0, st>>>(p);
     return launch_status();
   }
   CUtensorMap tmap;
   if (int rc = encode_stream_map(p, kThreads, kTmaSteps, &tmap)) return rc;
-  auto kern = replay_tma_kernel<ALGO, LPF, AUX, COMP>;
+  auto kern = replay_tma_kernel<ALGO, LPF, AUX, COMP, INNOV>;
   // idempotent; set on every launch (cheap) so that it holds on every device of a multi-GPU process
   PKF_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TmaSmem)));
   kern<<<grid, kThreads, sizeof(TmaSmem), st>>>(p, tmap);
@@ -112,13 +113,15 @@ bool packed_eligible(const ReplayParams& p) {
   const void* ptrs[] = {p.acc_ref, p.mag_ref, p.q_scale, p.r_scale, p.state_x, p.state_x_lo, p.state_p, p.state_lpf};
   for (const void* q : ptrs) if ((reinterpret_cast<uintptr_t>(q) & 7) != 0) return false;
   if ((reinterpret_cast<uintptr_t>(p.loss_acc) & 7) != 0 || (reinterpret_cast<uintptr_t>(p.out_flip) & 1) != 0) return false;
+  if ((reinterpret_cast<uintptr_t>(p.innov_acc) & 7) != 0) return false;
   return true;      // out_traj / truth are already required to be 16-byte aligned
 }
 
-template <int ALGO, bool LPF, bool AUX, bool COMP> int launch_replay_packed(const ReplayParams& p, cudaStream_t st) {
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false>
+int launch_replay_packed(const ReplayParams& p, cudaStream_t st) {
   CUtensorMap tmap;
   if (int rc = encode_stream_map(p, kTile2, kTma2Steps, &tmap)) return rc;
-  auto kern = replay_tma2_kernel<ALGO, LPF, AUX, COMP>;
+  auto kern = replay_tma2_kernel<ALGO, LPF, AUX, COMP, INNOV>;
   PKF_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Tma2Smem)));
   const unsigned grid = (unsigned)((p.N + kTile2 - 1) / kTile2);
   kern<<<grid, kThreads2, sizeof(Tma2Smem), st>>>(p, tmap);
@@ -143,6 +146,21 @@ template <int ALGO, bool LPF> int launch_replay_aux(const ReplayParams& p, bool 
   return aux ? launch_replay<ALGO, LPF, true, false>(p, use_tma, st) : launch_replay<ALGO, LPF, false, false>(p, use_tma, st);
 }
 
+// Launches with the innovation likelihood.  The packed kernel carries it without per-step outputs and low-pass (the
+// (Q,R) sweep path, where the registers allow 12 warps per SM); every other combination runs in the scalar kernels on
+// the same staging (TMA or LDG), whose results are the same bit for bit.
+template <int ALGO> int launch_innovation(const ReplayParams& p, bool lpf, bool aux, bool use_tma, bool packed, cudaStream_t st) {
+  const bool comp = p.state_x_lo != nullptr;
+  if constexpr (ALGO != WAHBA_JACOBI) {
+    if (packed && !lpf && !aux)
+      return comp ? launch_replay_packed<ALGO, false, false, true, true>(p, st) : launch_replay_packed<ALGO, false, false, false, true>(p, st);
+  }
+  if constexpr (ALGO != WAHBA_PRECOMPUTED) {      // (the low-pass of a measurement stream belongs to its builder)
+    if (lpf) return comp ? launch_replay<ALGO, true, true, true, true>(p, use_tma, st) : launch_replay<ALGO, true, true, false, true>(p, use_tma, st);
+  }
+  return comp ? launch_replay<ALGO, false, true, true, true>(p, use_tma, st) : launch_replay<ALGO, false, true, false, true>(p, use_tma, st);
+}
+
 int replay_dispatch(const ReplayParams& p, int algo, int staging, cudaStream_t st) {
   const bool lpf = (p.alpha_acc >= 0.f) || (p.alpha_mag >= 0.f);
   bool use_tma, packed = false;
@@ -156,7 +174,13 @@ int replay_dispatch(const ReplayParams& p, int algo, int staging, cudaStream_t s
     packed = use_tma && kAutoPrefersPacked && algo != POSEKF_WAHBA_JACOBI && packed_eligible(p);
   } else return POSEKF_EINVAL;
   int rc;
-  if (packed)
+  if (p.innov_acc) {
+    const bool aux = p.out_traj != nullptr || p.out_flip != nullptr || p.truth != nullptr;
+    if (algo == POSEKF_WAHBA_QR2) rc = launch_innovation<WAHBA_QR2>(p, lpf, aux, use_tma, packed, st);
+    else if (algo == POSEKF_WAHBA_PRECOMPUTED) rc = launch_innovation<WAHBA_PRECOMPUTED>(p, lpf, aux, use_tma, packed, st);
+    else if (algo == POSEKF_WAHBA_JACOBI) rc = launch_innovation<WAHBA_JACOBI>(p, lpf, aux, use_tma, packed, st);
+    else return POSEKF_EINVAL;
+  } else if (packed)
     rc = algo == POSEKF_WAHBA_QR2 ? launch_packed_variant<WAHBA_QR2>(p, lpf, st) : launch_packed_variant<WAHBA_PRECOMPUTED>(p, lpf, st);
   else if (algo == POSEKF_WAHBA_PRECOMPUTED) rc = lpf ? launch_replay_aux<WAHBA_PRECOMPUTED, true>(p, use_tma, st) : launch_replay_aux<WAHBA_PRECOMPUTED, false>(p, use_tma, st);
   else if (algo == POSEKF_WAHBA_QR2) rc = lpf ? launch_replay_aux<WAHBA_QR2, true>(p, use_tma, st) : launch_replay_aux<WAHBA_QR2, false>(p, use_tma, st);
@@ -193,11 +217,15 @@ extern "C" {
 
 const char* posekf_version(void) { return "posekf_b200 0.2 sm_100a"; }
 
-int posekf_replay_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
-                      int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_scale,
-                      const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag, float* state_x, float* state_x_lo,
-                      float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth, float* loss_acc,
-                      int wahba_algo, int staging, int state_flags, void* stream) {
+}  // extern "C"
+
+namespace {
+// Validation and dispatch shared by posekf_replay_f32 and posekf_replay_innovation_f32 (innov_acc null: the former).
+int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
+                 int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_scale,
+                 const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag, float* state_x, float* state_x_lo,
+                 float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth, float* loss_acc,
+                 float* innov_acc, int wahba_algo, int staging, int state_flags, void* stream) {
   if (n_filters < 0 || n_steps < 0 || n_streams <= 0 && n_filters > 0) return POSEKF_EINVAL;
   if (state_flags & ~(POSEKF_STATE_IN_FILTER_FRAME | POSEKF_STATE_OUT_FILTER_FRAME)) return POSEKF_EINVAL;
   if (n_filters == 0) return 0;
@@ -218,14 +246,41 @@ int posekf_replay_f32(int64_t n_filters, int64_t n_steps, const float* streams, 
   if ((n_filters + kThreads - 1) / kThreads > 0x7fffffffLL || n_steps > 0x7fffffffLL) return POSEKF_EINVAL;
   if (out_traj && (reinterpret_cast<uintptr_t>(out_traj) & 15) != 0) return POSEKF_EALIGN;
   if (truth && (!loss_acc || (reinterpret_cast<uintptr_t>(truth) & 15) != 0)) return truth && !loss_acc ? POSEKF_EINVAL : POSEKF_EALIGN;
+  if ((reinterpret_cast<uintptr_t>(innov_acc) & 3) != 0) return POSEKF_EALIGN;
   ReplayParams p;
   p.N = n_filters; p.T = n_steps; p.Ns = n_streams; p.streams = streams; p.dt = dt; p.dt_per_step = dt_per_step;
   p.acc_ref = acc_ref; p.mag_ref = mag_ref; p.q_scale = q_scale; p.r_scale = r_scale;
   p.alpha_acc = lpf_alpha_acc; p.alpha_mag = lpf_alpha_mag;
   p.state_x = state_x; p.state_x_lo = state_x_lo; p.state_p = state_p; p.state_lpf = state_lpf; p.out_traj = out_traj; p.out_flip = out_flip;
   p.truth = truth; p.loss_acc = loss_acc;
+  p.innov_acc = n_steps > 0 ? innov_acc : nullptr;     // (a frame conversion has no step to add)
   p.state_flags = state_flags;
   return replay_dispatch(p, wahba_algo, staging, (cudaStream_t)stream);
+}
+}  // namespace
+
+extern "C" {
+
+int posekf_replay_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
+                      int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_scale,
+                      const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag, float* state_x, float* state_x_lo,
+                      float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth, float* loss_acc,
+                      int wahba_algo, int staging, int state_flags, void* stream) {
+  return replay_entry(n_filters, n_steps, streams, n_streams, dt, dt_per_step, acc_ref, mag_ref, q_scale, r_scale, lpf_alpha_acc,
+                      lpf_alpha_mag, state_x, state_x_lo, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, nullptr,
+                      wahba_algo, staging, state_flags, stream);
+}
+
+int posekf_replay_innovation_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
+                                 int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_scale,
+                                 const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag, float* state_x,
+                                 float* state_x_lo, float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip,
+                                 const float* truth, float* loss_acc, float* innov_acc, int wahba_algo, int staging,
+                                 int state_flags, void* stream) {
+  if (!innov_acc) return POSEKF_EINVAL;
+  return replay_entry(n_filters, n_steps, streams, n_streams, dt, dt_per_step, acc_ref, mag_ref, q_scale, r_scale, lpf_alpha_acc,
+                      lpf_alpha_mag, state_x, state_x_lo, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, innov_acc,
+                      wahba_algo, staging, state_flags, stream);
 }
 
 // ---- host-buffer replay: workspace (device staging buffers, streams, events) ----------------------

@@ -71,12 +71,12 @@ class SweepWorkload:
     streams: torch.Tensor      # [T, 9, Ns]   shared by all cells (46 MB: L2 resident)
     acc_ref: torch.Tensor
     mag_ref: torch.Tensor
-    truth: torch.Tensor        # [T, Ns, 4]   ground-truth attitude for the tuning objective
+    truth: torch.Tensor | None  # [T, Ns, 4]   ground-truth attitude for the tuning objective (None: a recording)
     qs: torch.Tensor           # [G] grid values
     rs: torch.Tensor
     q: torch.Tensor            # [G*G*Ns] per-filter; cell g = iq*G + ir owns filters g*Ns .. (g+1)*Ns
     r: torch.Tensor
-    dt: float
+    dt: float | torch.Tensor   # seconds, or [T] per-step (a recording)
 
     @property
     def n_filters(self) -> int:
@@ -107,13 +107,18 @@ def build_c3(device, grid: int = C3_GRID, n_streams: int = C3_STREAMS, n_steps: 
     return w
 
 
-def run_c3(w: SweepWorkload, *, precise_state=None, share_measurements=None) -> B.ReplayState:
-    """One sweep: every cell replays all trajectories; returns the state with `.loss` [N] (sum over steps of
-    sin^2 of the angle to the ground truth)."""
+def run_c3(w: SweepWorkload, *, precise_state=None, share_measurements=None, objective: str = "truth",
+           staging: str = "auto") -> B.ReplayState:
+    """One sweep: every cell replays all trajectories; returns the state with its tuning objective: `.loss` [N] (sum
+    over steps of sin^2 of the angle to the ground truth; objective "truth"), `.innov` [2,N] (innovation likelihood
+    sums, see `innovation_surface`; objective "innovation") or neither ("none")."""
+    if objective not in ("truth", "innovation", "none"):
+        raise ValueError("objective is 'truth', 'innovation' or 'none'")
     N = w.n_filters
     st = B.ReplayState.initial(N, w.streams.device, r=w.r)
-    B.replay(w.streams, w.acc_ref, w.mag_ref, dt=w.dt, q=w.q, r=w.r, n_filters=N, state=st, truth=w.truth,
-             precise_state=precise_state, share_measurements=share_measurements)
+    B.replay(w.streams, w.acc_ref, w.mag_ref, dt=w.dt, q=w.q, r=w.r, n_filters=N, state=st,
+             truth=w.truth if objective == "truth" else None, innovation=True if objective == "innovation" else None,
+             precise_state=precise_state, share_measurements=share_measurements, staging=staging)
     return st
 
 
@@ -121,6 +126,28 @@ def loss_surface(w: SweepWorkload, st: B.ReplayState) -> torch.Tensor:
     """[Gq, Gr] mean sin^2 per cell."""
     T, _, Ns = w.streams.shape
     return st.loss.reshape(w.qs.numel(), w.rs.numel(), Ns).mean(2) / T
+
+
+def innovation_surface(w: SweepWorkload, st: B.ReplayState):
+    """([Gq, Gr] mean innovation NLL per step, [Gq, Gr] mean NIS) per cell, float64: the tuning objective that needs no
+    ground truth (`B.innovation_nll`); the best (Q,R) is the argmin of the first."""
+    T, _, Ns = w.streams.shape
+    nll, nis = B.innovation_nll(st, T)
+    shape = (w.qs.numel(), w.rs.numel(), Ns)
+    return nll.reshape(shape).mean(2) / T, nis.reshape(shape).mean(2)
+
+
+def build_recording_sweep(log, device, grid: int = C3_GRID, lo: float = -3.0, step: float = 0.1) -> SweepWorkload:
+    """A (Q,R) grid over ONE recorded log (`logio.LogData`): the cell layout of `build_c3` (log-spaced from 1e-3 in
+    steps of 0.1 decade on both axes) with Ns = 1 stream and the log's own per-step dt.  There is no ground truth:
+    run it with `run_c3(w, objective="innovation")` and read `innovation_surface`."""
+    streams, acc_ref, mag_ref, dt = log.to_streams(device)
+    hi = lo + step * (grid - 1)
+    qs = torch.logspace(lo, hi, grid, device=device)
+    rs = torch.logspace(lo, hi, grid, device=device)
+    q = qs.repeat_interleave(grid).contiguous()
+    r = rs.repeat(grid).contiguous()
+    return SweepWorkload(streams, acc_ref, mag_ref, None, qs, rs, q, r, dt)
 
 
 # ------------------------------------------------------------------------------------------------

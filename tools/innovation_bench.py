@@ -1,0 +1,123 @@
+#!/usr/bin/env python
+"""Cost of the innovation-likelihood tuning objective on one GPU (CUDA events, warm-up, variants alternated):
+
+  * the config-3 sweep (64x64 (Q,R) grid x 256 trajectories x 5000 steps) with no objective, with the ground-truth
+    objective (loss [N]) and with the innovation objective (innov [2,N]);
+  * one recording swept over a 64x64 grid for 30 000 steps (Ns = 1, per-step dt, LDG staging), innovation objective;
+  * where the argmin of each objective lands on config 3.
+
+  python tools/innovation_bench.py [--reps 5] [--out profiles/r03_innovation_sweep.json]
+"""
+from __future__ import annotations
+
+import argparse
+import json
+import os
+import subprocess
+import sys
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+
+def card():
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                             capture_output=True, text=True, timeout=30).stdout.strip().splitlines()
+        return out[0] if out else None
+    except Exception:
+        return None
+
+
+def timed(fn, reps):
+    import torch
+    ms = []
+    for _ in range(reps):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        fn()
+        e1.record()
+        torch.cuda.synchronize()
+        ms.append(e0.elapsed_time(e1))
+    return ms
+
+
+def synthetic_recording(T, seed=30):
+    """A LogData-shaped recording with a per-step dt (jittered 100 Hz): gyro/acc/mag of one synthetic trajectory."""
+    import numpy as np
+    from poseestimationkf_b200.logio import LogData
+    from poseestimationkf_b200.synth import make_imu
+    imu = make_imu(1, T, seed=seed, sigma=0.01)
+    S = imu.streams.numpy()[:, :, 0].astype(np.float64)
+    rng = np.random.default_rng(seed)
+    t = np.concatenate([[0], np.cumsum(np.round(1e7 * (1 + 0.05 * rng.standard_normal(T))))]).astype(np.int64)
+    d = LogData()
+    d.acc_0, d.mag_0 = list(imu.acc_ref.numpy()[:, 0]), list(imu.mag_ref.numpy()[:, 0])
+    d.gyro, d.acc_1, d.mag_1 = [list(v) for v in S[:, 0:3]], [list(v) for v in S[:, 3:6]], [list(v) for v in S[:, 6:9]]
+    d.timestamp = [[int(v)] for v in t]
+    return d
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--reps", type=int, default=5)
+    ap.add_argument("--rec-steps", type=int, default=30000)
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r03_innovation_sweep.json"))
+    a = ap.parse_args()
+    import torch
+    from poseestimationkf_b200 import workloads as WL
+    assert torch.cuda.is_available(), "needs a GPU"
+    dev = torch.device("cuda:0")
+    res = {"card": card(), "torch": torch.__version__, "timing": "CUDA events around one whole sweep (state set-up, "
+           "measurement stream, two replay launches, scatter), variants alternated, after one warm-up each"}
+
+    w = WL.build_c3(dev)
+    T, _, Ns = w.streams.shape
+    fsteps = w.n_filters * T
+    objs = ("none", "truth", "innovation")
+    for o in objs:                                   # warm-up
+        WL.run_c3(w, objective=o)
+    torch.cuda.synchronize()
+    ms = {o: [] for o in objs}
+    for _ in range(a.reps):
+        for o in objs:
+            ms[o] += timed(lambda: WL.run_c3(w, objective=o), 1)
+    res["c3"] = {o: {"ms": ms[o], "ms_median": sorted(ms[o])[len(ms[o]) // 2],
+                     "gsteps_per_s": fsteps / (sorted(ms[o])[len(ms[o]) // 2] * 1e-3) / 1e9} for o in objs}
+    res["c3"]["innovation_over_truth"] = res["c3"]["innovation"]["ms_median"] / res["c3"]["truth"]["ms_median"]
+    res["c3"]["workload"] = f"64x64 (Q,R) grid x {Ns} trajectories x {T} steps = {fsteps / 1e9:.1f} G filter-steps"
+    # where the argmins land
+    st_t = WL.run_c3(w, objective="truth")
+    st_i = WL.run_c3(w, objective="innovation")
+    loss = WL.loss_surface(w, st_t)
+    nll, nis = WL.innovation_surface(w, st_i)
+    bt, bi = int(loss.argmin()), int(nll.argmin())
+    G = w.qs.numel()
+    res["c3_argmin"] = {"truth": {"q": float(w.qs[bt // G]), "r": float(w.rs[bt % G]), "mean_sin2": float(loss.min())},
+                        "innovation": {"q": float(w.qs[bi // G]), "r": float(w.rs[bi % G]), "nll_per_step": float(nll.min()),
+                                       "mean_nis": float(nis.view(-1)[bi])},
+                        "mean_nis_at_truth_argmin": float(nis.view(-1)[bt]),
+                        "mean_nis_range": [float(nis.min()), float(nis.max())]}
+    del w, st_t, st_i
+    torch.cuda.empty_cache()
+
+    rec = WL.build_recording_sweep(synthetic_recording(a.rec_steps), dev)
+    WL.run_c3(rec, objective="innovation", staging="ldg")
+    torch.cuda.synchronize()
+    rms = timed(lambda: WL.run_c3(rec, objective="innovation", staging="ldg"), a.reps)
+    med = sorted(rms)[len(rms) // 2]
+    st = WL.run_c3(rec, objective="innovation", staging="ldg")
+    nll_r, nis_r = WL.innovation_surface(rec, st)
+    br = int(nll_r.argmin())
+    res["recording"] = {"workload": f"one synthetic recording, {a.rec_steps} steps, per-step dt, 64x64 grid (4096 filters, Ns = 1)",
+                        "ms": rms, "ms_median": med, "gsteps_per_s": rec.n_filters * a.rec_steps / (med * 1e-3) / 1e9,
+                        "argmin": {"q": float(rec.qs[br // 64]), "r": float(rec.rs[br % 64]), "mean_nis": float(nis_r.view(-1)[br])}}
+    os.makedirs(os.path.dirname(a.out), exist_ok=True)
+    with open(a.out, "w") as fh:
+        json.dump(res, fh, indent=1)
+    print(json.dumps({k: v for k, v in res.items() if k != "c3"}, indent=1))
+    print(json.dumps({o: res["c3"][o]["ms_median"] for o in objs}), res["c3"]["innovation_over_truth"])
+
+
+if __name__ == "__main__":
+    main()
