@@ -147,6 +147,28 @@ int posekf_replay_innovation_f32(int64_t n_filters, int64_t n_steps, const float
                                  uint8_t* out_flip, const float* truth, float* loss_acc, float* innov_acc, int wahba_algo,
                                  int staging, int state_flags, void* stream);
 
+/* Which innovation likelihood posekf_replay_innovation_ex_f32 accumulates. */
+#define POSEKF_INNOV_FULL    0  /* the 4-D model above: the sums of posekf_replay_innovation_f32, bit for bit */
+#define POSEKF_INNOV_TANGENT 1  /* the same model in the 3-D tangent space of the prediction (below) */
+
+/* posekf_replay_innovation_f32 with a choice of model.  POSEKF_INNOV_TANGENT leaves out the direction of the
+ * prediction u_t = z_t/|z_t|: y and z are unit quaternions, so e.u ~ -|e|^2/2 carries almost no information, and P_t
+ * leaves that direction almost empty, which makes the 4-D likelihood favour ever smaller R.  With E_t any 4x3
+ * orthonormal basis of u_t-perp (the result does not depend on the choice):
+ *     l_3(Q,R) = 1/2 sum_t [ NIS3_t + ln det S3_t + 3 ln 2 pi ],   S3_t = E_t^T S_t E_t,   e3_t = E_t^T e_t,
+ *     NIS3_t = e3_t^T S3_t^-1 e3_t.
+ *   innov_acc[0][n] += sum_t NIS3_t, innov_acc[1][n] += sum_t ln det S3_t; layout, alignment, chunking and routing are
+ *               those of posekf_replay_innovation_f32.  Then  NLL = (innov_acc[0] + innov_acc[1]) / 2 + 3/2 T ln 2 pi,
+ *               mean NIS = innov_acc[0] / T (about 3 for a consistent model).
+ *   innov_model POSEKF_INNOV_FULL or POSEKF_INNOV_TANGENT; any other value: POSEKF_EINVAL.
+ * A buffer holds the sums of one model: pass it to launches of that model only. */
+int posekf_replay_innovation_ex_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams,
+                                    const float* dt, int dt_per_step, const float* acc_ref, const float* mag_ref,
+                                    const float* q_scale, const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag,
+                                    float* state_x, float* state_x_lo, float* state_p, float* state_lpf, float* out_traj,
+                                    uint8_t* out_flip, const float* truth, float* loss_acc, float* innov_acc, int innov_model,
+                                    int wahba_algo, int staging, int state_flags, void* stream);
+
 /* Same replay with HOST buffers: streams_host [T][9][N] is streamed through the device in time
  * chunks (double-buffered H2D copies overlapped with the filter kernel, state carried across
  * chunks on the device), results are copied back.  This is the call an offline-replay user makes.

@@ -14,12 +14,15 @@ _i64, _int, _f32, _vp = C.c_int64, C.c_int, C.c_float, C.c_void_p
 EINVAL, EALIGN, ENODEV = -1, -2, -3
 WAHBA = {"qr2": 0, "jacobi": 1, "precomputed": 2}
 STAGING = {"auto": 0, "ldg": 1, "tma": 2, "tma_packed": 3}
+INNOV_MODEL = {"full": 0, "tangent": 1}      # POSEKF_INNOV_*
 
 _SIGNATURES = {
     "posekf_replay_f32": [_i64, _i64, _vp, _i64, _vp, _int, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _vp, _vp,
                           _vp, _vp, _vp, _int, _int, _int, _vp],
     "posekf_replay_innovation_f32": [_i64, _i64, _vp, _i64, _vp, _int, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _vp,
                                      _vp, _vp, _vp, _vp, _vp, _int, _int, _int, _vp],
+    "posekf_replay_innovation_ex_f32": [_i64, _i64, _vp, _i64, _vp, _int, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp,
+                                        _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _int, _int, _vp],
     "posekf_replay_host_f32": [_i64, _i64, _vp, _f32, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _vp, _vp, _i64,
                                _int, _int, _int, _vp],
     "posekf_host_workspace_create": [_int, _i64, _i64, _int, C.POINTER(C.c_void_p)],

@@ -85,7 +85,8 @@ class ReplayState:
     frame: "reference" (x, p in the reference's own coordinates -- what every `replay` call returns by
     default) or "filter" (left in the kernel's working frame by `replay(..., keep_filter_frame=True)`
     between the chunks of a time-chunked replay; `to_reference_frame` converts).
-    innov [2,N]: the innovation likelihood sums (sum_t NIS_t, sum_t ln det S_t) of `replay(..., innovation=...)`."""
+    innov [2,N]: the innovation likelihood sums (sum_t NIS_t, sum_t ln det S_t) of `replay(..., innovation=...)`;
+    innov_model: the model they belong to ("full" or "tangent", see `replay(..., innovation_model=...)`)."""
     x: torch.Tensor
     p: torch.Tensor
     r: object = 0.1
@@ -94,6 +95,7 @@ class ReplayState:
     x_lo: torch.Tensor | None = None     # [4,N] low-order part of the compensated (two-float) state
     frame: str = "reference"
     innov: torch.Tensor | None = None    # [2,N] innovation likelihood sums (see replay(innovation=...))
+    innov_model: str | None = None       # "full" / "tangent": the model of `innov`
 
     @staticmethod
     def initial(n_filters: int, device, r=0.1, with_lpf: bool = False, P0: torch.Tensor | None = None) -> "ReplayState":
@@ -117,7 +119,7 @@ class ReplayState:
     def clone(self) -> "ReplayState":
         c = lambda t: None if t is None else t.clone()
         return ReplayState(self.x.clone(), self.p.clone(), self.r, c(self.lpf), c(self.loss), c(self.x_lo), self.frame,
-                           c(self.innov))
+                           c(self.innov), self.innov_model)
 
     def to_reference_frame(self, acc_ref: torch.Tensor, mag_ref: torch.Tensor) -> "ReplayState":
         """Convert (in place) a state that `replay(..., keep_filter_frame=True)` left in the kernel's working
@@ -242,7 +244,7 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
            store_flips: bool = False, truth: torch.Tensor | None = None, loss: torch.Tensor | None = None,
            precise_state: bool | None = None, share_measurements: bool | None = None, wahba: str = "qr2",
            staging: str = "auto", keep_filter_frame: bool = False, allow_imprecise: bool = False,
-           innovation: bool | torch.Tensor | None = None):
+           innovation: bool | torch.Tensor | None = None, innovation_model: str = "full"):
     """Run T Prediction+Correction steps for N filters in one kernel launch.
 
     streams [T,9,Ns]; acc_ref, mag_ref [3,Ns]; dt: float seconds or [T] float32 CUDA tensor;
@@ -274,7 +276,12 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     (sum_t NIS_t, sum_t ln det S_t); a tensor is used as is (pass `state.innov` back in for chunked replays).  It is
     available as `state.innov`; `innovation_nll` turns it into per-filter NLL and mean NIS.  It does not perturb the
     filter.  None / False: the launch is exactly that of a replay without it.
+    `innovation_model`: "full" (the 4-D model of the reference's S and e) or "tangent" (the same model in the 3-D
+    tangent space of the prediction, posekf_replay_innovation_ex_f32, whose R axis has an interior minimum).  Recorded
+    as `state.innov_model`; an accumulator that holds the sums of the other model is refused.
     Returns (state, traj [T,N,4] or None, flips [T,N] uint8 or None)."""
+    if innovation_model not in _lib.INNOV_MODEL:
+        raise ValueError("innovation_model is 'full' or 'tangent'")
     _require_cuda(streams, acc_ref, mag_ref, out_traj)
     if streams.dim() != 3 or streams.shape[1] != 9:
         raise ValueError("streams must be [T, 9, Ns]")
@@ -310,7 +317,7 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
             # a (Q,R) sweep: only the cells with r/q >= 100 or q/r >= 1e4 need the precise variant (+25 % time)
             mixed = _replay_sweep_mixed(streams, acc_ref, mag_ref, dt=dt, q=q, r=r, state=state, N=N, Ns=Ns, truth=truth,
                                         loss=loss, wahba=wahba, staging=staging, keep_filter_frame=keep_filter_frame,
-                                        innovation=innovation)
+                                        innovation=innovation, innovation_model=innovation_model)
             if mixed is not None:
                 return mixed
         precise_state = state.x_lo is not None or needs_precise
@@ -351,7 +358,7 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
         if loss is None:
             loss = torch.zeros((N,), dtype=torch.float32, device=dev)
         state.loss = loss
-    innov = _innovation_buffer(innovation, N, dev)
+    innov = _innovation_buffer(innovation, N, dev, state, innovation_model)
     args = (N, T, _ptr(streams), Ns, _ptr(dt_t), per_step, _ptr(acc_ref), _ptr(mag_ref), _ptr(q_t), _ptr(r_t),
             -1.0 if lpf_alpha_acc is None else float(lpf_alpha_acc),
             -1.0 if lpf_alpha_mag is None else float(lpf_alpha_mag),
@@ -362,38 +369,52 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
         if innov is None:
             rc = _lib.load().posekf_replay_f32(*args, *tail)
         else:
-            rc = _lib.load().posekf_replay_innovation_f32(*args, _ptr(innov), *tail)
-    _lib.check(rc, "posekf_replay_f32" if innov is None else "posekf_replay_innovation_f32")
+            rc = _lib.load().posekf_replay_innovation_ex_f32(*args, _ptr(innov), _lib.INNOV_MODEL[innovation_model], *tail)
+    _lib.check(rc, "posekf_replay_f32" if innov is None else "posekf_replay_innovation_ex_f32")
     if innov is not None:
-        state.innov = innov
+        state.innov, state.innov_model = innov, innovation_model
     if wahba != "precomputed":
         state.frame = "filter" if keep_filter_frame else "reference"
     return state, out_traj, flips
 
 
-def _innovation_buffer(innovation, n: int, device):
-    """The [2,N] accumulator of replay(innovation=...): None when off, zeros for True, the caller's tensor otherwise."""
+def _innovation_buffer(innovation, n: int, device, state=None, model: str = "full"):
+    """The [2,N] accumulator of replay(innovation=...): None when off, zeros for True, the caller's tensor otherwise.
+    The state's own accumulator is refused when it holds the sums of another model."""
     if innovation is None or innovation is False:
         return None
     if innovation is True:
         return torch.zeros((2, n), dtype=torch.float32, device=device)
+    if state is not None and innovation is state.innov and state.innov_model not in (None, model):
+        raise ValueError(f"the accumulator holds sums of the {state.innov_model!r} innovation model, not {model!r}")
     _require_cuda(innovation)
     if innovation.shape != (2, n):
         raise ValueError(f"innovation accumulator must be [2, {n}]")
     return innovation
 
 
-def innovation_nll(innov, n_steps: int):
+def innovation_nll(innov, n_steps: int, model: str | None = None):
     """Per-filter innovation likelihood from the [2,N] sums of `replay(..., innovation=...)` (or a ReplayState holding
     them) over `n_steps` steps: (NLL [N], mean NIS [N]) in float64,
-        NLL = 1/2 sum_t [NIS_t + ln det S_t] + 2 T ln 2 pi,     mean NIS = sum_t NIS_t / T
-    (natural log; P and R unscaled).  A good (Q,R) minimises the NLL."""
-    a = innov.innov if isinstance(innov, ReplayState) else innov
+        NLL = 1/2 sum_t [NIS_t + ln det S_t] + (dof/2) T ln 2 pi,     mean NIS = sum_t NIS_t / T
+    (natural log; P and R unscaled), dof = 4 for the "full" model and 3 for the "tangent" one.  A ReplayState supplies
+    its own model (`model`, when given, must agree with it); for a bare tensor `model` defaults to "full".  A good (Q,R)
+    minimises the NLL."""
+    if model is not None and model not in _lib.INNOV_MODEL:
+        raise ValueError("model is 'full' or 'tangent'")
+    if isinstance(innov, ReplayState):
+        own = innov.innov_model or "full"
+        if model is not None and model != own:
+            raise ValueError(f"the state holds sums of the {own!r} innovation model, not {model!r}")
+        model, a = own, innov.innov
+    else:
+        a = innov
     if a is None:
         raise ValueError("no innovation sums: replay with innovation=True")
+    dof = 3 if model == "tangent" else 4
     a = a.to(torch.float64)
     T = float(n_steps)
-    return 0.5 * (a[0] + a[1]) + 2.0 * T * math.log(2.0 * math.pi), a[0] / T
+    return 0.5 * (a[0] + a[1]) + 0.5 * dof * T * math.log(2.0 * math.pi), a[0] / T
 
 
 def sweep_partition(q_t: torch.Tensor, r_t: torch.Tensor, n_streams: int):
@@ -411,7 +432,7 @@ def sweep_partition(q_t: torch.Tensor, r_t: torch.Tensor, n_streams: int):
 
 
 def _replay_sweep_mixed(streams, acc_ref, mag_ref, *, dt, q, r, state, N, Ns, truth, loss, wahba, staging, keep_filter_frame,
-                        innovation=None):
+                        innovation=None, innovation_model="full"):
     """Sweep layout with automatic precision: the cells (blocks of Ns filters sharing one (q, r)) whose tuning is
     extreme run the precise variant, the others the plain one -- two launches over a cell permutation that keeps
     every filter on its own stream column (n % Ns).  Returns None when one launch serves all cells."""
@@ -423,7 +444,7 @@ def _replay_sweep_mixed(streams, acc_ref, mag_ref, *, dt, q, r, state, N, Ns, tr
     parts = []
     if truth is not None and loss is None:
         loss = torch.zeros((N,), dtype=torch.float32, device=dev)
-    innov = _innovation_buffer(innovation, N, dev)
+    innov = _innovation_buffer(innovation, N, dev, state, innovation_model)
     for idx, precise in ((idx_plain, False), (idx_precise, True)):
         sub = ReplayState(state.x[:, idx].contiguous(), state.p[:, idx].contiguous(), r_t[idx].contiguous(), None, None,
                           state.x_lo[:, idx].contiguous() if (precise and state.x_lo is not None) else None, state.frame)
@@ -431,7 +452,8 @@ def _replay_sweep_mixed(streams, acc_ref, mag_ref, *, dt, q, r, state, N, Ns, tr
         sub_innov = innov[:, idx].contiguous() if innov is not None else None
         replay(streams, acc_ref, mag_ref, dt=dt, q=q_t[idx].contiguous(), r=sub.r, state=sub, n_filters=idx.numel(), truth=truth,
                loss=sub_loss, precise_state=precise, share_measurements=False, wahba=wahba, staging=staging,
-               keep_filter_frame=keep_filter_frame, innovation=sub_innov)   # (the plain group holds no extreme cell by construction)
+               keep_filter_frame=keep_filter_frame, innovation=sub_innov,
+               innovation_model=innovation_model)   # (the plain group holds no extreme cell by construction)
         parts.append((idx, sub, sub_loss, sub_innov, precise))
     if state.x_lo is None:
         state.x_lo = torch.zeros((4, N), dtype=torch.float32, device=dev)
@@ -448,7 +470,7 @@ def _replay_sweep_mixed(streams, acc_ref, mag_ref, *, dt, q, r, state, N, Ns, tr
     if truth is not None:
         state.loss = loss
     if innov is not None:
-        state.innov = innov
+        state.innov, state.innov_model = innov, innovation_model
     state.r = r
     return state, None, None
 

@@ -465,6 +465,15 @@ template <typename F> struct Ldl4 {          // S = P + I = L D L^T;  N = L^-1 -
 //   precise (kalman_gain_sm):     S~ = H - g x x^T;  Sherman-Morrison and the matrix-determinant lemma give
 //           e^T S~^-1 e = sum_k i_k t_k^2 (H's factors) + beta (w.e)^2,   ln det S~ = sum_k ln d_k(H) + ln(num / |x|^2)
 // (S~^-1 = I - K would cancel as K -> I: the factors are used instead.)
+//
+// TAN (tangent-space likelihood): the same model restricted to the 3-D tangent space of the prediction u = z/|z| --
+// e_3 = E^T e, S_3 = E^T S E for any orthonormal basis E of u-perp, and
+//     l_3(Q,R) = 1/2 sum_t [ e_3^T S_3^-1 e_3 + ln det S_3 + 3 ln 2 pi ].
+// The 4-D model also scores the direction of u, where a unit-quaternion innovation has almost no component
+// (e.u ~ -|e|^2/2) and P^- almost no variance, which drives its R axis towards zero.  No basis is formed: with
+// c = z^T S~^-1 z, b = z^T S~^-1 e, s = e^T S~^-1 e the Schur complement of u gives
+//     NIS_3 = (s - b^2/c) / r,     ln det S_3 = 3 ln r + ln det S~ + ln(c/|z|^2),   c/|z|^2 = 1 - z^T K z / |z|^2,
+// with c and b from the same factors as s (v = (I + N) z; precise: + beta (w.z)^2, + beta (w.z)(w.e)).
 // ------------------------------------------------------------------------------------------
 template <typename F> struct InnovFactors {
   F n10, n20, n21, n30, n31, n32;   // N = L^-1 - I of S~ (plain) or of H (precise)
@@ -472,17 +481,23 @@ template <typename F> struct InnovFactors {
   F w0, w1, w2, w3, beta;           // precise only: w = H^-1 x, beta = g|x|^2 / x^T(I+M)w
   F logdet;                         // ln det S~
 };
-// Running sums of one filter (true units) and the launch constants that fold 1/r and 4 ln r in per step: the sums are
-// never rescaled, so a chunked replay accumulates exactly what the unchunked one does.
+// Running sums of one filter (true units) and the launch constants that fold 1/r and dof ln r (4, TAN: 3) in per step:
+// the sums are never rescaled, so a chunked replay accumulates exactly what the unchunked one does.
 template <typename F> struct InnovAcc {
   F nis, logdet;
-  F inv_r, log_r4;
+  F inv_r, log_rd;
 };
-template <typename F> PKF_HD InnovAcc<F> make_innov_acc(F nis, F logdet, F r) {
+// 3 ln r, rounded once per lane: the packed lanes form it with scalar multiplications, which the compiler does not fuse
+// into the per-step addition (a packed product by 3 would be, and that fused sum differs from the scalar kernels' in the
+// last bit; 4 ln r is exact either way)
+template <typename F> PKF_HD F log_r3_(F r) { return F(3) * log_(r); }
+template <> PKF_HD f32x2 log_r3_<f32x2>(f32x2 r) { return f32x2(log_r3_<float>(r.x), log_r3_<float>(r.y)); }
+template <typename F, bool TAN = false> PKF_HD InnovAcc<F> make_innov_acc(F nis, F logdet, F r) {
   InnovAcc<F> a;
   a.nis = nis; a.logdet = logdet;
   a.inv_r = F(1) / r;
-  a.log_r4 = F(4) * log_(r);
+  if constexpr (TAN) a.log_rd = log_r3_(r);
+  else a.log_rd = F(4) * log_(r);
   return a;
 }
 // sum_k ln(1 + x_k) from the pivot excesses x_k = d_k - 1 >= 0: the excess of the product is formed first and its
@@ -491,8 +506,10 @@ template <typename F> PKF_HD F log_pivots(F x0, F x1, F x2, F x3) {
   const F a = fma_(x0, x1, x0 + x1), b = fma_(x2, x3, x2 + x3);
   return log1p_(fma_(a, b, a + b));
 }
-template <typename F, bool COMP>
-PKF_HD void innov_accumulate(InnovAcc<F>& acc, const InnovFactors<F>& f, F e0, F e1, F e2, F e3) {
+// K = I - S~^-1 (the step's gain) and z are read by TAN only.
+template <typename F, bool COMP, bool TAN = false>
+PKF_HD void innov_accumulate(InnovAcc<F>& acc, const InnovFactors<F>& f, const Sym4<F>& K, const Quat<F>& z,
+                             F e0, F e1, F e2, F e3) {
   const F t1 = fma_(f.n10, e0, e1);
   const F t2 = fma_(f.n21, e1, fma_(f.n20, e0, e2));
   const F t3 = fma_(f.n32, e2, fma_(f.n31, e1, fma_(f.n30, e0, e3)));
@@ -502,8 +519,35 @@ PKF_HD void innov_accumulate(InnovAcc<F>& acc, const InnovFactors<F>& f, F e0, F
     const F we = fma_(f.w3, e3, fma_(f.w2, e2, fma_(f.w1, e1, f.w0 * e0)));
     s = fma_(f.beta * we, we, s);
   }
-  acc.nis = fma_(s, acc.inv_r, acc.nis);
-  acc.logdet = acc.logdet + (f.logdet + acc.log_r4);
+  if constexpr (!TAN) {
+    acc.nis = fma_(s, acc.inv_r, acc.nis);
+    acc.logdet = acc.logdet + (f.logdet + acc.log_rd);
+  } else {
+    const F v1 = fma_(f.n10, z.w, z.x);
+    const F v2 = fma_(f.n21, z.x, fma_(f.n20, z.w, z.y));
+    const F v3 = fma_(f.n32, z.y, fma_(f.n31, z.x, fma_(f.n30, z.w, z.z)));
+    const F g0 = f.i0 * z.w, g1 = f.i1 * v1, g2 = f.i2 * v2, g3 = f.i3 * v3;
+    F c = fma_(g3, v3, fma_(g2, v2, fma_(g1, v1, g0 * z.w)));
+    F b = fma_(g3, t3, fma_(g2, t2, fma_(g1, t1, g0 * e0)));
+    if constexpr (COMP) {
+      const F we = fma_(f.w3, e3, fma_(f.w2, e2, fma_(f.w1, e1, f.w0 * e0)));   // (the same value as above)
+      const F wz = fma_(f.w3, z.z, fma_(f.w2, z.y, fma_(f.w1, z.x, f.w0 * z.w)));
+      const F bwz = f.beta * wz;
+      c = fma_(bwz, wz, c);
+      b = fma_(bwz, we, b);
+    }
+    // ln(c/|z|^2) = ln(1 - z^T K z/|z|^2): through log1p while z^T K z/|z|^2 is small (R >> Q, and Q >> R with a slow
+    // state: there the empty direction of P^- is the previous x, close to z), through the quotient beyond
+    const F k0 = fma_(F(2), fma_(K.a03, z.z, fma_(K.a02, z.y, K.a01 * z.x)), K.a00 * z.w);
+    const F k1 = fma_(F(2), fma_(K.a13, z.z, K.a12 * z.y), K.a11 * z.x);
+    const F k2 = fma_(F(2), K.a23 * z.z, K.a22 * z.y);
+    const F zkz = fma_(K.a33 * z.z, z.z, fma_(k2, z.y, fma_(k1, z.x, k0 * z.w)));
+    const F iz2 = rcp_(dot4(z, z));
+    const F kz = zkz * iz2;
+    const F lc = sel_(kz < F(0.5), log1p_(-kz), log_(c * iz2));
+    acc.nis = fma_(fma_(-b, b * rcp_(c), s), acc.inv_r, acc.nis);
+    acc.logdet = acc.logdet + ((f.logdet + lc) + acc.log_rd);
+  }
 }
 
 template <typename F> PKF_HD Ldl4<F> ldl_unit(const Sym4<F>& P) {
@@ -1251,7 +1295,8 @@ PKF_HD Quat<F> measure_quat(const FilterConst<F>& fc, const Vec3<F>& acc, const 
 
 // Prediction + Correction with the measurement quaternion y (filter frame, any sign, norm 1/inv_norm) already computed.
 // INNOV: the innovation likelihood of the step is added to *innov (see InnovAcc); the filter itself is unchanged.
-template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, typename FlagT>
+// TAN: its tangent-space form (see innov_accumulate).
+template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, typename FlagT>
 PKF_HD void ekf_step_measured(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, const Vec3<F>& gyro,
                               const Quat<F>& y, F inv_norm, const StepH<F>& h, FlagT& flip, bool flip_wanted = true,
                               typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr) {
@@ -1264,24 +1309,24 @@ PKF_HD void ekf_step_measured(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<
   if (WANT_FLIP && flip_wanted) flip = reference_flip_quat(fc, y, one_with_sign_(dyz), code);
   const F sn = copysign_(inv_norm, dyz);          // e = sg y/|y| - z, sg = sign(dot): the sign bit moves onto 1/|y| > 0  :76
   const F e0 = fma_(sn, y.w, -z.w), e1 = fma_(sn, y.x, -z.x), e2 = fma_(sn, y.y, -z.y), e3 = fma_(sn, y.z, -z.z);
-  if constexpr (INNOV) innov_accumulate<F, COMP>(*innov, fac, e0, e1, e2, e3);
+  if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3);
   ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);
 }
 
 // The common case of ekf_step<WAHBA_QR2>: both Wahba weights are non-negative (|a_z| <= 1, i.e. a normalised
 // accelerometer), so the closed-form measurement applies and the step has no data-dependent branch.  The caller
 // guarantees the precondition (the packed kernel checks a whole tile of samples before taking this path).
-template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, typename FlagT>
+template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, typename FlagT>
 PKF_HD void ekf_step_plain_measured(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, const Vec3<F>& gyro,
                                     const Vec3<F>& acc, const Vec3<F>& mag, const StepH<F>& h, FlagT& flip, bool flip_wanted = true,
                                     typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr) {
   const F ka = abs_(acc.z), km = F(1) - ka;
   F inv_norm;
   const Quat<F> y = wahba_quat2_local(fc.E, acc, mag, ka, km, inv_norm);
-  ekf_step_measured<F, WANT_FLIP, COMP, INNOV>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code, innov);
+  ekf_step_measured<F, WANT_FLIP, COMP, INNOV, TAN>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code, innov);
 }
 
-template <typename F, int ALGO, bool WANT_FLIP, bool COMP, bool INNOV = false, typename FlagT>
+template <typename F, int ALGO, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, typename FlagT>
 PKF_HD void ekf_step(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, const Vec3<F>& gyro,
                      const Vec3<F>& acc, const Vec3<F>& mag, const StepH<F>& h, FlagT& flip, bool flip_wanted = true,
                      typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr) {
@@ -1290,7 +1335,7 @@ PKF_HD void ekf_step(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, c
   if constexpr (ALGO == WAHBA_QR2) {
     F inv_norm;
     const Quat<F> y = measure_quat(fc, acc, mag, inv_norm);
-    ekf_step_measured<F, WANT_FLIP, COMP, INNOV>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code, innov);
+    ekf_step_measured<F, WANT_FLIP, COMP, INNOV, TAN>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code, innov);
   } else {
     Sym4<F> K;
     Quat<F> inc, z;
@@ -1329,7 +1374,7 @@ PKF_HD void ekf_step(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, c
         e2 = sel_(unrelated, yf.y - z.y, e2); e3 = sel_(unrelated, yf.z - z.z, e3);
       }
     }
-    if constexpr (INNOV) innov_accumulate<F, COMP>(*innov, fac, e0, e1, e2, e3);
+    if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3);
     ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);
   }
 }

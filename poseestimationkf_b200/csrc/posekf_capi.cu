@@ -90,16 +90,16 @@ bool tma_eligible(const ReplayParams& p) {
   return true;
 }
 
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false>
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false>
 int launch_replay(const ReplayParams& p, bool use_tma, cudaStream_t st) {
   const unsigned grid = (unsigned)((p.N + kThreads - 1) / kThreads);
   if (!use_tma) {
-    replay_ldg_kernel<ALGO, LPF, AUX, COMP, INNOV><<<grid, kThreads, 0, st>>>(p);
+    replay_ldg_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN><<<grid, kThreads, 0, st>>>(p);
     return launch_status();
   }
   CUtensorMap tmap;
   if (int rc = encode_stream_map(p, kThreads, kTmaSteps, &tmap)) return rc;
-  auto kern = replay_tma_kernel<ALGO, LPF, AUX, COMP, INNOV>;
+  auto kern = replay_tma_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN>;
   // idempotent; set on every launch (cheap) so that it holds on every device of a multi-GPU process
   PKF_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TmaSmem)));
   kern<<<grid, kThreads, sizeof(TmaSmem), st>>>(p, tmap);
@@ -117,11 +117,11 @@ bool packed_eligible(const ReplayParams& p) {
   return true;      // out_traj / truth are already required to be 16-byte aligned
 }
 
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false>
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false>
 int launch_replay_packed(const ReplayParams& p, cudaStream_t st) {
   CUtensorMap tmap;
   if (int rc = encode_stream_map(p, kTile2, kTma2Steps, &tmap)) return rc;
-  auto kern = replay_tma2_kernel<ALGO, LPF, AUX, COMP, INNOV>;
+  auto kern = replay_tma2_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN>;
   PKF_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Tma2Smem)));
   const unsigned grid = (unsigned)((p.N + kTile2 - 1) / kTile2);
   kern<<<grid, kThreads2, sizeof(Tma2Smem), st>>>(p, tmap);
@@ -146,22 +146,32 @@ template <int ALGO, bool LPF> int launch_replay_aux(const ReplayParams& p, bool 
   return aux ? launch_replay<ALGO, LPF, true, false>(p, use_tma, st) : launch_replay<ALGO, LPF, false, false>(p, use_tma, st);
 }
 
-// Launches with the innovation likelihood.  The packed kernel carries it without per-step outputs and low-pass (the
-// (Q,R) sweep path, where the registers allow 12 warps per SM); every other combination runs in the scalar kernels on
-// the same staging (TMA or LDG), whose results are the same bit for bit.
-template <int ALGO> int launch_innovation(const ReplayParams& p, bool lpf, bool aux, bool use_tma, bool packed, cudaStream_t st) {
+// Launches with the innovation likelihood (TAN: its tangent-space form).  The packed kernel carries it without per-step
+// outputs and low-pass (the (Q,R) sweep path, where the registers allow 12 warps per SM); every other combination runs
+// in the scalar kernels on the same staging (TMA or LDG), whose results are the same bit for bit.
+template <int ALGO, bool TAN = false>
+int launch_innovation(const ReplayParams& p, bool lpf, bool aux, bool use_tma, bool packed, cudaStream_t st) {
   const bool comp = p.state_x_lo != nullptr;
   if constexpr (ALGO != WAHBA_JACOBI) {
     if (packed && !lpf && !aux)
-      return comp ? launch_replay_packed<ALGO, false, false, true, true>(p, st) : launch_replay_packed<ALGO, false, false, false, true>(p, st);
+      return comp ? launch_replay_packed<ALGO, false, false, true, true, TAN>(p, st) : launch_replay_packed<ALGO, false, false, false, true, TAN>(p, st);
   }
   if constexpr (ALGO != WAHBA_PRECOMPUTED) {      // (the low-pass of a measurement stream belongs to its builder)
-    if (lpf) return comp ? launch_replay<ALGO, true, true, true, true>(p, use_tma, st) : launch_replay<ALGO, true, true, false, true>(p, use_tma, st);
+    if (lpf) return comp ? launch_replay<ALGO, true, true, true, true, TAN>(p, use_tma, st) : launch_replay<ALGO, true, true, false, true, TAN>(p, use_tma, st);
   }
-  return comp ? launch_replay<ALGO, false, true, true, true>(p, use_tma, st) : launch_replay<ALGO, false, true, false, true>(p, use_tma, st);
+  return comp ? launch_replay<ALGO, false, true, true, true, TAN>(p, use_tma, st) : launch_replay<ALGO, false, true, false, true, TAN>(p, use_tma, st);
 }
 
-int replay_dispatch(const ReplayParams& p, int algo, int staging, cudaStream_t st) {
+template <bool TAN> int launch_innovation_algo(const ReplayParams& p, int algo, bool lpf, bool aux, bool use_tma, bool packed,
+                                               cudaStream_t st) {
+  if (algo == POSEKF_WAHBA_QR2) return launch_innovation<WAHBA_QR2, TAN>(p, lpf, aux, use_tma, packed, st);
+  if (algo == POSEKF_WAHBA_PRECOMPUTED) return launch_innovation<WAHBA_PRECOMPUTED, TAN>(p, lpf, aux, use_tma, packed, st);
+  if (algo == POSEKF_WAHBA_JACOBI) return launch_innovation<WAHBA_JACOBI, TAN>(p, lpf, aux, use_tma, packed, st);
+  return POSEKF_EINVAL;
+}
+
+// innov_model: POSEKF_INNOV_* of the sums in p.innov_acc (read only when it is set).
+int replay_dispatch(const ReplayParams& p, int algo, int staging, int innov_model, cudaStream_t st) {
   const bool lpf = (p.alpha_acc >= 0.f) || (p.alpha_mag >= 0.f);
   bool use_tma, packed = false;
   if (staging == POSEKF_STAGE_LDG) use_tma = false;
@@ -176,10 +186,8 @@ int replay_dispatch(const ReplayParams& p, int algo, int staging, cudaStream_t s
   int rc;
   if (p.innov_acc) {
     const bool aux = p.out_traj != nullptr || p.out_flip != nullptr || p.truth != nullptr;
-    if (algo == POSEKF_WAHBA_QR2) rc = launch_innovation<WAHBA_QR2>(p, lpf, aux, use_tma, packed, st);
-    else if (algo == POSEKF_WAHBA_PRECOMPUTED) rc = launch_innovation<WAHBA_PRECOMPUTED>(p, lpf, aux, use_tma, packed, st);
-    else if (algo == POSEKF_WAHBA_JACOBI) rc = launch_innovation<WAHBA_JACOBI>(p, lpf, aux, use_tma, packed, st);
-    else return POSEKF_EINVAL;
+    rc = innov_model == POSEKF_INNOV_TANGENT ? launch_innovation_algo<true>(p, algo, lpf, aux, use_tma, packed, st)
+                                             : launch_innovation_algo<false>(p, algo, lpf, aux, use_tma, packed, st);
   } else if (packed)
     rc = algo == POSEKF_WAHBA_QR2 ? launch_packed_variant<WAHBA_QR2>(p, lpf, st) : launch_packed_variant<WAHBA_PRECOMPUTED>(p, lpf, st);
   else if (algo == POSEKF_WAHBA_PRECOMPUTED) rc = lpf ? launch_replay_aux<WAHBA_PRECOMPUTED, true>(p, use_tma, st) : launch_replay_aux<WAHBA_PRECOMPUTED, false>(p, use_tma, st);
@@ -220,12 +228,13 @@ const char* posekf_version(void) { return "posekf_b200 0.2 sm_100a"; }
 }  // extern "C"
 
 namespace {
-// Validation and dispatch shared by posekf_replay_f32 and posekf_replay_innovation_f32 (innov_acc null: the former).
+// Validation and dispatch shared by posekf_replay_f32 and posekf_replay_innovation(_ex)_f32 (innov_acc null: the first).
+// innov_model: POSEKF_INNOV_FULL or POSEKF_INNOV_TANGENT (checked by the caller).
 int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
                  int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_scale,
                  const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag, float* state_x, float* state_x_lo,
                  float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth, float* loss_acc,
-                 float* innov_acc, int wahba_algo, int staging, int state_flags, void* stream) {
+                 float* innov_acc, int innov_model, int wahba_algo, int staging, int state_flags, void* stream) {
   if (n_filters < 0 || n_steps < 0 || n_streams <= 0 && n_filters > 0) return POSEKF_EINVAL;
   if (state_flags & ~(POSEKF_STATE_IN_FILTER_FRAME | POSEKF_STATE_OUT_FILTER_FRAME)) return POSEKF_EINVAL;
   if (n_filters == 0) return 0;
@@ -255,7 +264,7 @@ int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64
   p.truth = truth; p.loss_acc = loss_acc;
   p.innov_acc = n_steps > 0 ? innov_acc : nullptr;     // (a frame conversion has no step to add)
   p.state_flags = state_flags;
-  return replay_dispatch(p, wahba_algo, staging, (cudaStream_t)stream);
+  return replay_dispatch(p, wahba_algo, staging, innov_model, (cudaStream_t)stream);
 }
 }  // namespace
 
@@ -268,7 +277,7 @@ int posekf_replay_f32(int64_t n_filters, int64_t n_steps, const float* streams, 
                       int wahba_algo, int staging, int state_flags, void* stream) {
   return replay_entry(n_filters, n_steps, streams, n_streams, dt, dt_per_step, acc_ref, mag_ref, q_scale, r_scale, lpf_alpha_acc,
                       lpf_alpha_mag, state_x, state_x_lo, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, nullptr,
-                      wahba_algo, staging, state_flags, stream);
+                      POSEKF_INNOV_FULL, wahba_algo, staging, state_flags, stream);
 }
 
 int posekf_replay_innovation_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
@@ -280,7 +289,19 @@ int posekf_replay_innovation_f32(int64_t n_filters, int64_t n_steps, const float
   if (!innov_acc) return POSEKF_EINVAL;
   return replay_entry(n_filters, n_steps, streams, n_streams, dt, dt_per_step, acc_ref, mag_ref, q_scale, r_scale, lpf_alpha_acc,
                       lpf_alpha_mag, state_x, state_x_lo, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, innov_acc,
-                      wahba_algo, staging, state_flags, stream);
+                      POSEKF_INNOV_FULL, wahba_algo, staging, state_flags, stream);
+}
+
+int posekf_replay_innovation_ex_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams,
+                                    const float* dt, int dt_per_step, const float* acc_ref, const float* mag_ref,
+                                    const float* q_scale, const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag,
+                                    float* state_x, float* state_x_lo, float* state_p, float* state_lpf, float* out_traj,
+                                    uint8_t* out_flip, const float* truth, float* loss_acc, float* innov_acc, int innov_model,
+                                    int wahba_algo, int staging, int state_flags, void* stream) {
+  if (!innov_acc || (innov_model != POSEKF_INNOV_FULL && innov_model != POSEKF_INNOV_TANGENT)) return POSEKF_EINVAL;
+  return replay_entry(n_filters, n_steps, streams, n_streams, dt, dt_per_step, acc_ref, mag_ref, q_scale, r_scale, lpf_alpha_acc,
+                      lpf_alpha_mag, state_x, state_x_lo, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, innov_acc,
+                      innov_model, wahba_algo, staging, state_flags, stream);
 }
 
 // ---- host-buffer replay: workspace (device staging buffers, streams, events) ----------------------

@@ -28,7 +28,8 @@ struct ReplayParams {
   const float* truth;   // [T][Ns][4] reference track for the tuning objective, or null
   float* loss_acc;      // [N] in/out: sum over steps of 1 - (x . truth)^2
   int state_flags;      // POSEKF_STATE_IN_FILTER_FRAME | POSEKF_STATE_OUT_FILTER_FRAME (include/posekf.h)
-  float* innov_acc;     // [2][N] in/out innovation likelihood sums (NIS, ln det S), or null; read by INNOV kernels only
+  float* innov_acc;     // [2][N] in/out innovation likelihood sums (NIS, ln det S; TAN kernels: of the tangent-space
+                        // model), or null; read by INNOV kernels only
                         // (last: the parameter offsets of the other kernels are unchanged)
 };
 constexpr int kStateInFilterFrame = 1, kStateOutFilterFrame = 2;
@@ -42,13 +43,13 @@ struct FilterRegs {
   InnovAcc<float> in;   // innovation likelihood sums (INNOV kernels only)
 };
 
-template <int ALGO, bool LPF, bool COMP, bool INNOV = false>
+template <int ALGO, bool LPF, bool COMP, bool INNOV = false, bool TAN = false>
 __device__ __forceinline__ void load_filter(const ReplayParams& p, int64_t n, int64_t col, FilterRegs& f) {
   const int64_t N = p.N, Ns = p.Ns;
   Vec3<float> ra = {p.acc_ref[col], p.acc_ref[Ns + col], p.acc_ref[2 * Ns + col]};
   Vec3<float> rm = {p.mag_ref[col], p.mag_ref[Ns + col], p.mag_ref[2 * Ns + col]};
   f.fc = make_filter_const<float>(ra, rm, p.q_scale[n], p.r_scale[n]);
-  if (INNOV) f.in = make_innov_acc<float>(p.innov_acc[n], p.innov_acc[N + n], p.r_scale[n]);
+  if (INNOV) f.in = make_innov_acc<float, TAN>(p.innov_acc[n], p.innov_acc[N + n], p.r_scale[n]);
   f.x = {p.state_x[n], p.state_x[N + n], p.state_x[2 * N + n], p.state_x[3 * N + n]};
   f.xlo = {0.f, 0.f, 0.f, 0.f};
   if (COMP) f.xlo = {p.state_x_lo[n], p.state_x_lo[N + n], p.state_x_lo[2 * N + n], p.state_x_lo[3 * N + n]};
@@ -64,7 +65,7 @@ __device__ __forceinline__ void load_filter(const ReplayParams& p, int64_t n, in
   if (uses_filter_frame<ALGO>() && !(p.state_flags & kStateInFilterFrame)) enter_filter_frame(f.fc, f.x, f.xlo, f.P, COMP);
 }
 
-template <int ALGO, bool LPF, bool COMP, bool INNOV = false>
+template <int ALGO, bool LPF, bool COMP, bool INNOV = false, bool TAN = false>
 __device__ __forceinline__ void store_filter(const ReplayParams& p, int64_t n, FilterRegs& f) {
   const int64_t N = p.N;
   if (uses_filter_frame<ALGO>() && !(p.state_flags & kStateOutFilterFrame)) leave_filter_frame(f.fc, f.x, f.xlo, f.P, COMP);
@@ -100,7 +101,7 @@ template <bool AUX> __device__ __forceinline__ AuxPtrs make_aux(const ReplayPara
   return a;
 }
 
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false>
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false>
 __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f, const float (&s)[kChannels], float h,
                                             AuxPtrs& aux) {
   Vec3<float> w = {s[0], s[1], s[2]}, a = {s[3], s[4], s[5]}, m = {s[6], s[7], s[8]};
@@ -112,8 +113,8 @@ __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f
   // flip-mask byte: the float32 decision, plus the tie marker and per-branch alternatives that flip_fixup_kernel settles
   // in float64 after the launch (raw samples only: a low-passed sample is not in the stream any more)
   unsigned code = 0;
-  ekf_step<float, ALGO, AUX, COMP, INNOV>(f.x, f.xlo, f.P, f.fc, w, a, m, StepH<float>(h), flip, aux.flips != nullptr,
-                                          (AUX && !LPF && ALGO == WAHBA_QR2) ? &code : nullptr, INNOV ? &f.in : nullptr);
+  ekf_step<float, ALGO, AUX, COMP, INNOV, TAN>(f.x, f.xlo, f.P, f.fc, w, a, m, StepH<float>(h), flip, aux.flips != nullptr,
+                                               (AUX && !LPF && ALGO == WAHBA_QR2) ? &code : nullptr, INNOV ? &f.in : nullptr);
   if (!(AUX && !LPF && ALGO == WAHBA_QR2)) code = flip ? 1u : 0u;
   if (AUX) {
     // per-step outputs are in the reference frame (the reference's X_k)
@@ -144,8 +145,9 @@ __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f
 // Replay, LDG staging: coalesced loads straight to registers, next step prefetched while the
 // current one is computed.
 // ---------------------------------------------------------------------------------------------
-// (INNOV: the innovation likelihood; its instantiations always have AUX and are built for 3 CTAs per SM, <= 168 registers)
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false>
+// (INNOV: the innovation likelihood, TAN: its tangent-space form; their instantiations always have AUX and are built for
+//  3 CTAs per SM, <= 168 registers)
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false>
 __global__ void __launch_bounds__(kThreads, INNOV ? 3 : ((ALGO == WAHBA_JACOBI || (COMP && LPF && AUX)) ? 4 : ((COMP || LPF) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
     replay_ldg_kernel(const ReplayParams p) {
   const int64_t n = (int64_t)blockIdx.x * kThreads + threadIdx.x;
@@ -153,7 +155,7 @@ __global__ void __launch_bounds__(kThreads, INNOV ? 3 : ((ALGO == WAHBA_JACOBI |
   const int64_t Ns = p.Ns;
   const int64_t col = (Ns == p.N) ? n : (n % Ns);
   FilterRegs f;
-  load_filter<ALGO, LPF, COMP, INNOV>(p, n, col, f);
+  load_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, col, f);
   AuxPtrs aux = make_aux<AUX>(p, n, col, true);
   const float* s = p.streams + col;
   const int64_t step_stride = kChannels * Ns;
@@ -167,11 +169,11 @@ __global__ void __launch_bounds__(kThreads, INNOV ? 3 : ((ALGO == WAHBA_JACOBI |
 #pragma unroll
     for (int c = 0; c < kChannels; ++c) nxt[c] = ldg_stream(s + c * Ns);
     const float h = p.dt_per_step ? __ldg(p.dt + t) : dt0;
-    filter_step<ALGO, LPF, AUX, COMP, INNOV>(p, f, cur, h, aux);
+    filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN>(p, f, cur, h, aux);
 #pragma unroll
     for (int c = 0; c < kChannels; ++c) cur[c] = nxt[c];
   }
-  store_filter<ALGO, LPF, COMP, INNOV>(p, n, f);
+  store_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, f);
   if (AUX && aux.truth) p.loss_acc[n] = aux.loss;
 }
 
@@ -188,7 +190,7 @@ struct __align__(128) TmaSmem {
 };
 constexpr uint32_t kTileBytes = kTmaSteps * kChannels * kThreads * sizeof(float);
 
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false>
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false>
 __global__ void __launch_bounds__(kThreads, INNOV ? 3 : (ALGO == WAHBA_JACOBI ? 4 : ((COMP && (LPF || AUX)) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
     replay_tma_kernel(const ReplayParams p, const __grid_constant__ CUtensorMap tmap) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -219,7 +221,7 @@ __global__ void __launch_bounds__(kThreads, INNOV ? 3 : (ALGO == WAHBA_JACOBI ? 
   }
 
   FilterRegs f;
-  if (valid) load_filter<ALGO, LPF, COMP, INNOV>(p, n, (int64_t)col0 + tid, f);
+  if (valid) load_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, (int64_t)col0 + tid, f);
   AuxPtrs aux = make_aux<AUX>(p, n, (int64_t)col0 + tid, valid);
   const float dt0 = p.dt[0];
 
@@ -244,7 +246,7 @@ __global__ void __launch_bounds__(kThreads, INNOV ? 3 : (ALGO == WAHBA_JACOBI ? 
 #pragma unroll
           for (int c = 0; c < kChannels; ++c) s[c] = sm.tile[stage][tt][c][tid];
           const float h = p.dt_per_step ? __ldg(p.dt + k * kTmaSteps + tt) : dt0;
-          filter_step<ALGO, LPF, AUX, COMP, INNOV>(p, f, s, h, aux);
+          filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN>(p, f, s, h, aux);
         }
       }
     }
@@ -252,7 +254,7 @@ __global__ void __launch_bounds__(kThreads, INNOV ? 3 : (ALGO == WAHBA_JACOBI ? 
     if ((tid & 31) == 0) mbar_arrive(&sm.empty[stage]);
     if (++stage == kTmaStages) { stage = 0; parity ^= 1; }
   }
-  if (valid) store_filter<ALGO, LPF, COMP, INNOV>(p, n, f);
+  if (valid) store_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, f);
   if (AUX && valid && aux.truth) p.loss_acc[n] = aux.loss;
 }
 
@@ -280,8 +282,9 @@ struct FilterRegs2 {
 };
 
 // (the precise variant with per-step outputs needs ~190 registers: 8 warps per SM instead of 12.  INNOV: the innovation
-//  likelihood, instantiated without per-step outputs and low-pass -- the sweep path; replay_dispatch routes the rest)
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false>
+//  likelihood (TAN: tangent-space form), instantiated without per-step outputs and low-pass -- the sweep path;
+//  replay_dispatch routes the rest)
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false>
 __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) < PKF_MIN_CTAS2 ? (256 / kThreads2) : PKF_MIN_CTAS2) : PKF_MIN_CTAS2)
     replay_tma2_kernel(const ReplayParams p, const __grid_constant__ CUtensorMap tmap) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -318,7 +321,7 @@ __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) 
     Vec3<f32x2> ra = {ld2(p.acc_ref + col), ld2(p.acc_ref + Ns + col), ld2(p.acc_ref + 2 * Ns + col)};
     Vec3<f32x2> rm = {ld2(p.mag_ref + col), ld2(p.mag_ref + Ns + col), ld2(p.mag_ref + 2 * Ns + col)};
     f.fc = make_filter_const<f32x2>(ra, rm, ld2(p.q_scale + n), ld2(p.r_scale + n));
-    if (INNOV) f.in = make_innov_acc<f32x2>(ld2(p.innov_acc + n), ld2(p.innov_acc + N + n), ld2(p.r_scale + n));
+    if (INNOV) f.in = make_innov_acc<f32x2, TAN>(ld2(p.innov_acc + n), ld2(p.innov_acc + N + n), ld2(p.r_scale + n));
     f.x = {ld2(p.state_x + n), ld2(p.state_x + N + n), ld2(p.state_x + 2 * N + n), ld2(p.state_x + 3 * N + n)};
     f.xlo = {f32x2(0.f), f32x2(0.f), f32x2(0.f), f32x2(0.f)};
     if (COMP) f.xlo = {ld2(p.state_x_lo + n), ld2(p.state_x_lo + N + n), ld2(p.state_x_lo + 2 * N + n), ld2(p.state_x_lo + 3 * N + n)};
@@ -381,10 +384,10 @@ __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) 
         mask2 flip;
         constexpr bool kTieCode = AUX && !LPF && ALGO == WAHBA_QR2;     // see filter_step
         FlipCode2 code = {0u, 0u};
-        if constexpr (FAST && ALGO == WAHBA_QR2) ekf_step_plain_measured<f32x2, AUX, COMP, INNOV>(f.x, f.xlo, f.P, f.fc, w, a, m, sh, flip, flips != nullptr,
-                                                                                                   kTieCode ? &code : nullptr, INNOV ? &f.in : nullptr);
-        else ekf_step<f32x2, ALGO, AUX, COMP, INNOV>(f.x, f.xlo, f.P, f.fc, w, a, m, sh, flip, flips != nullptr, kTieCode ? &code : nullptr,
-                                                     INNOV ? &f.in : nullptr);
+        if constexpr (FAST && ALGO == WAHBA_QR2) ekf_step_plain_measured<f32x2, AUX, COMP, INNOV, TAN>(f.x, f.xlo, f.P, f.fc, w, a, m, sh, flip, flips != nullptr,
+                                                                                                        kTieCode ? &code : nullptr, INNOV ? &f.in : nullptr);
+        else ekf_step<f32x2, ALGO, AUX, COMP, INNOV, TAN>(f.x, f.xlo, f.P, f.fc, w, a, m, sh, flip, flips != nullptr, kTieCode ? &code : nullptr,
+                                                          INNOV ? &f.in : nullptr);
         if (!kTieCode) code = FlipCode2{flip.x ? 1u : 0u, flip.y ? 1u : 0u};
         if (AUX) {
           Quat<f32x2> xr = f.x;     // per-step outputs are in the reference frame

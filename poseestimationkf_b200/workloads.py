@@ -111,14 +111,17 @@ def run_c3(w: SweepWorkload, *, precise_state=None, share_measurements=None, obj
            staging: str = "auto") -> B.ReplayState:
     """One sweep: every cell replays all trajectories; returns the state with its tuning objective: `.loss` [N] (sum
     over steps of sin^2 of the angle to the ground truth; objective "truth"), `.innov` [2,N] (innovation likelihood
-    sums, see `innovation_surface`; objective "innovation") or neither ("none")."""
-    if objective not in ("truth", "innovation", "none"):
-        raise ValueError("objective is 'truth', 'innovation' or 'none'")
+    sums, see `innovation_surface`; objective "innovation" for the 4-D model, "innovation_tangent" for the tangent-space
+    one) or neither ("none")."""
+    innov_model = {"innovation": "full", "innovation_tangent": "tangent"}.get(objective)
+    if innov_model is None and objective not in ("truth", "none"):
+        raise ValueError("objective is 'truth', 'innovation', 'innovation_tangent' or 'none'")
     N = w.n_filters
     st = B.ReplayState.initial(N, w.streams.device, r=w.r)
     B.replay(w.streams, w.acc_ref, w.mag_ref, dt=w.dt, q=w.q, r=w.r, n_filters=N, state=st,
-             truth=w.truth if objective == "truth" else None, innovation=True if objective == "innovation" else None,
-             precise_state=precise_state, share_measurements=share_measurements, staging=staging)
+             truth=w.truth if objective == "truth" else None, innovation=True if innov_model else None,
+             innovation_model=innov_model or "full", precise_state=precise_state, share_measurements=share_measurements,
+             staging=staging)
     return st
 
 
@@ -130,7 +133,7 @@ def loss_surface(w: SweepWorkload, st: B.ReplayState) -> torch.Tensor:
 
 def innovation_surface(w: SweepWorkload, st: B.ReplayState):
     """([Gq, Gr] mean innovation NLL per step, [Gq, Gr] mean NIS) per cell, float64: the tuning objective that needs no
-    ground truth (`B.innovation_nll`); the best (Q,R) is the argmin of the first."""
+    ground truth (`B.innovation_nll`, in the model of the state's sums); the best (Q,R) is the argmin of the first."""
     T, _, Ns = w.streams.shape
     nll, nis = B.innovation_nll(st, T)
     shape = (w.qs.numel(), w.rs.numel(), Ns)
@@ -140,7 +143,8 @@ def innovation_surface(w: SweepWorkload, st: B.ReplayState):
 def build_recording_sweep(log, device, grid: int = C3_GRID, lo: float = -3.0, step: float = 0.1) -> SweepWorkload:
     """A (Q,R) grid over ONE recorded log (`logio.LogData`): the cell layout of `build_c3` (log-spaced from 1e-3 in
     steps of 0.1 decade on both axes) with Ns = 1 stream and the log's own per-step dt.  There is no ground truth:
-    run it with `run_c3(w, objective="innovation")` and read `innovation_surface`."""
+    run it with `run_c3(w, objective="innovation_tangent")` (or "innovation") and read `innovation_surface`; pass
+    `lo` = -7 or so to reach the R that the tangent objective picks on low-noise sensors."""
     streams, acc_ref, mag_ref, dt = log.to_streams(device)
     hi = lo + step * (grid - 1)
     qs = torch.logspace(lo, hi, grid, device=device)
