@@ -169,6 +169,29 @@ int posekf_replay_innovation_ex_f32(int64_t n_filters, int64_t n_steps, const fl
                                     uint8_t* out_flip, const float* truth, float* loss_acc, float* innov_acc, int innov_model,
                                     int wahba_algo, int staging, int state_flags, void* stream);
 
+/* A batch of recordings in one launch, each with its own time steps and length (Python Kalman Filter/main_file.py:25,
+ * 38-47: every recording differences its own timestamps against its own previousT).  The parameters of
+ * posekf_replay_innovation_ex_f32, plus:
+ *   dt_cols     [T][Ns] seconds, or NULL: filter n steps with dt_cols[t][n % Ns] (overrides dt / dt_per_step; dt may
+ *               then be NULL).  Not 16-byte aligned: POSEKF_STAGE_AUTO runs the LDG kernel, an explicit TMA staging
+ *               returns POSEKF_EALIGN (as for streams).
+ *   n_valid     [Ns] int32, or NULL: stream c has n_valid[c] steps in this launch; the caller guarantees
+ *               0 <= n_valid[c] <= T (it is not read on the host).  A step t >= n_valid[n % Ns] leaves filter n as it
+ *               is: state, P, low-pass state, loss_acc and innov_acc are unchanged, the trajectory slot gets the held
+ *               state (reference frame) and the flip byte is 0.  The samples and dt of such a step are never used:
+ *               they may hold anything, NaN included.  For a time-chunked replay pass the lengths counted from the
+ *               chunk's first step, clamped to [0, chunk length].
+ *   innov_acc   may be NULL (no innovation sums); innov_model must be POSEKF_INNOV_FULL or POSEKF_INNOV_TANGENT.
+ * With dt_cols and n_valid both NULL the call is posekf_replay_innovation_ex_f32 (innov_acc non-NULL) or
+ * posekf_replay_f32 (innov_acc NULL).  Filters with all of their steps live give the same bits as one launch per
+ * recording with that recording's dt[T]; every staging and variant is supported. */
+int posekf_replay_batch_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
+                            int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_scale,
+                            const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag, float* state_x, float* state_x_lo,
+                            float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth,
+                            float* loss_acc, float* innov_acc, int innov_model, int wahba_algo, int staging, int state_flags,
+                            void* stream, const float* dt_cols, const int32_t* n_valid);
+
 /* Same replay with HOST buffers: streams_host [T][9][N] is streamed through the device in time
  * chunks (double-buffered H2D copies overlapped with the filter kernel, state carried across
  * chunks on the device), results are copied back.  This is the call an offline-replay user makes.

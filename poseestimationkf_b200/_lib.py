@@ -23,6 +23,8 @@ _SIGNATURES = {
                                      _vp, _vp, _vp, _vp, _vp, _int, _int, _int, _vp],
     "posekf_replay_innovation_ex_f32": [_i64, _i64, _vp, _i64, _vp, _int, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp,
                                         _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _int, _int, _vp],
+    "posekf_replay_batch_f32": [_i64, _i64, _vp, _i64, _vp, _int, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _vp, _vp,
+                                _vp, _vp, _vp, _vp, _int, _int, _int, _int, _vp, _vp, _vp],
     "posekf_replay_host_f32": [_i64, _i64, _vp, _f32, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _vp, _vp, _i64,
                                _int, _int, _int, _vp],
     "posekf_host_workspace_create": [_int, _i64, _i64, _int, C.POINTER(C.c_void_p)],

@@ -244,10 +244,12 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
            store_flips: bool = False, truth: torch.Tensor | None = None, loss: torch.Tensor | None = None,
            precise_state: bool | None = None, share_measurements: bool | None = None, wahba: str = "qr2",
            staging: str = "auto", keep_filter_frame: bool = False, allow_imprecise: bool = False,
-           innovation: bool | torch.Tensor | None = None, innovation_model: str = "full"):
+           innovation: bool | torch.Tensor | None = None, innovation_model: str = "full",
+           lengths: torch.Tensor | None = None):
     """Run T Prediction+Correction steps for N filters in one kernel launch.
 
-    streams [T,9,Ns]; acc_ref, mag_ref [3,Ns]; dt: float seconds or [T] float32 CUDA tensor;
+    streams [T,9,Ns]; acc_ref, mag_ref [3,Ns]; dt: float seconds, [T] float32 CUDA tensor (one clock for every
+    filter) or [T,Ns] (per stream: filter n steps with column n % Ns -- a batch of recordings, `logio.stack_logs`);
     q, r: floats or [N] tensors (Q=q*I3, R=r*I4).  `n_filters` > Ns replays every trajectory
     N/Ns times (filter n reads column n % Ns) -- the Q/R sweep layout.  `state` is updated in place
     (created with the reference's initial values when None).  `truth` [T,Ns,4] enables the on-device
@@ -279,6 +281,11 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     `innovation_model`: "full" (the 4-D model of the reference's S and e) or "tangent" (the same model in the 3-D
     tangent space of the prediction, posekf_replay_innovation_ex_f32, whose R axis has an interior minimum).  Recorded
     as `state.innov_model`; an accumulator that holds the sums of the other model is refused.
+    `lengths`: [Ns] int32 CUDA tensor, the number of steps of THIS call that stream c has (0..T; checked with one
+    read-back).  A filter whose stream has ended is held: its state, loss and innovation sums stay as they are, its
+    trajectory rows repeat its final state and its flip bytes are 0; the samples and dt of those steps are never used
+    (they may be NaN).  For a time-chunked replay pass each chunk its own lengths (`logio.LogBatch.window`).
+    A [T,Ns] dt or `lengths` runs the batched kernels (include/posekf.h, posekf_replay_batch_f32).
     Returns (state, traj [T,N,4] or None, flips [T,N] uint8 or None)."""
     if innovation_model not in _lib.INNOV_MODEL:
         raise ValueError("innovation_model is 'full' or 'tangent'")
@@ -291,6 +298,14 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
         raise ValueError("acc_ref / mag_ref must be [3, Ns]")
     dev = streams.device
     use_lpf = lpf_alpha_acc is not None or lpf_alpha_mag is not None
+    dt_cols = None
+    if isinstance(dt, torch.Tensor) and dt.dim() == 2:
+        _require_cuda(dt)
+        if dt.shape != (T, Ns):
+            raise ValueError(f"a per-stream dt tensor must be [T, Ns] = [{T}, {Ns}]")
+        dt_cols = dt
+    if lengths is not None:
+        _check_lengths(lengths, Ns, T)
     if share_measurements is None:
         share_measurements = N > Ns and N >= 4 * Ns and wahba == "qr2" and not use_lpf and T > 0
     if share_measurements:
@@ -317,7 +332,7 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
             # a (Q,R) sweep: only the cells with r/q >= 100 or q/r >= 1e4 need the precise variant (+25 % time)
             mixed = _replay_sweep_mixed(streams, acc_ref, mag_ref, dt=dt, q=q, r=r, state=state, N=N, Ns=Ns, truth=truth,
                                         loss=loss, wahba=wahba, staging=staging, keep_filter_frame=keep_filter_frame,
-                                        innovation=innovation, innovation_model=innovation_model)
+                                        innovation=innovation, innovation_model=innovation_model, lengths=lengths)
             if mixed is not None:
                 return mixed
         precise_state = state.x_lo is not None or needs_precise
@@ -332,10 +347,12 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     _require_cuda(state.x, state.p, state.lpf)
     if state.x.shape != (4, N) or state.p.shape != (10, N):
         raise ValueError("state has the wrong shape for this batch")
-    if isinstance(dt, torch.Tensor):
+    if dt_cols is not None:
+        dt_t, per_step = None, 0
+    elif isinstance(dt, torch.Tensor):
         _require_cuda(dt)
         if dt.shape != (T,):
-            raise ValueError("dt tensor must be [T]")
+            raise ValueError("dt tensor must be [T] or [T, Ns]")
         dt_t, per_step = dt, 1
     else:
         dt_t, per_step = _scalar_tensor(dt, dev), 0
@@ -365,17 +382,35 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
             _ptr(state.x), _ptr(state.x_lo if precise_state else None), _ptr(state.p), _ptr(state.lpf), _ptr(out_traj),
             _ptr(flips), _ptr(truth), _ptr(loss if truth is not None else None))
     tail = (_lib.WAHBA[wahba], _lib.STAGING[staging], frame_flags, _stream())
+    batch = dt_cols is not None or lengths is not None
     with torch.cuda.device(dev):
-        if innov is None:
+        if batch:
+            rc = _lib.load().posekf_replay_batch_f32(*args, _ptr(innov), _lib.INNOV_MODEL[innovation_model], *tail, _ptr(dt_cols),
+                                                     _ptr(lengths))
+        elif innov is None:
             rc = _lib.load().posekf_replay_f32(*args, *tail)
         else:
             rc = _lib.load().posekf_replay_innovation_ex_f32(*args, _ptr(innov), _lib.INNOV_MODEL[innovation_model], *tail)
-    _lib.check(rc, "posekf_replay_f32" if innov is None else "posekf_replay_innovation_ex_f32")
+    _lib.check(rc, "posekf_replay_batch_f32" if batch else
+               ("posekf_replay_f32" if innov is None else "posekf_replay_innovation_ex_f32"))
     if innov is not None:
         state.innov, state.innov_model = innov, innovation_model
     if wahba != "precomputed":
         state.frame = "filter" if keep_filter_frame else "reference"
     return state, out_traj, flips
+
+
+def _check_lengths(lengths, n_streams: int, n_steps: int) -> None:
+    """replay(lengths=...): an [Ns] int32 CUDA tensor with every value in [0, T] (one reduction and one read-back)."""
+    if not isinstance(lengths, torch.Tensor) or lengths.dtype != torch.int32 or not lengths.is_contiguous() \
+            or lengths.shape != (n_streams,):
+        raise ValueError(f"lengths must be a contiguous int32 tensor of shape ({n_streams},)")
+    if n_streams:
+        lo, hi = torch.stack((lengths.min(), lengths.max())).tolist()
+        if lo < 0 or hi > n_steps:
+            raise ValueError(f"lengths must lie in [0, {n_steps}] (the steps of this call), got [{lo}, {hi}]")
+    if not lengths.is_cuda:
+        raise _lib.PosekfError("poseestimationkf_b200 runs on CUDA tensors only (no CPU fallback)")
 
 
 def _innovation_buffer(innovation, n: int, device, state=None, model: str = "full"):
@@ -393,9 +428,10 @@ def _innovation_buffer(innovation, n: int, device, state=None, model: str = "ful
     return innovation
 
 
-def innovation_nll(innov, n_steps: int, model: str | None = None):
+def innovation_nll(innov, n_steps, model: str | None = None):
     """Per-filter innovation likelihood from the [2,N] sums of `replay(..., innovation=...)` (or a ReplayState holding
-    them) over `n_steps` steps: (NLL [N], mean NIS [N]) in float64,
+    them) over `n_steps` steps (an int, or an [N] tensor of per-filter step counts -- a batch of recordings of different
+    lengths; a filter with 0 steps has NLL 0 and mean NIS nan): (NLL [N], mean NIS [N]) in float64,
         NLL = 1/2 sum_t [NIS_t + ln det S_t] + (dof/2) T ln 2 pi,     mean NIS = sum_t NIS_t / T
     (natural log; P and R unscaled), dof = 4 for the "full" model and 3 for the "tangent" one.  A ReplayState supplies
     its own model (`model`, when given, must agree with it); for a bare tensor `model` defaults to "full".  A good (Q,R)
@@ -413,7 +449,7 @@ def innovation_nll(innov, n_steps: int, model: str | None = None):
         raise ValueError("no innovation sums: replay with innovation=True")
     dof = 3 if model == "tangent" else 4
     a = a.to(torch.float64)
-    T = float(n_steps)
+    T = n_steps.to(device=a.device, dtype=torch.float64) if isinstance(n_steps, torch.Tensor) else float(n_steps)
     return 0.5 * (a[0] + a[1]) + 0.5 * dof * T * math.log(2.0 * math.pi), a[0] / T
 
 
@@ -432,7 +468,7 @@ def sweep_partition(q_t: torch.Tensor, r_t: torch.Tensor, n_streams: int):
 
 
 def _replay_sweep_mixed(streams, acc_ref, mag_ref, *, dt, q, r, state, N, Ns, truth, loss, wahba, staging, keep_filter_frame,
-                        innovation=None, innovation_model="full"):
+                        innovation=None, innovation_model="full", lengths=None):
     """Sweep layout with automatic precision: the cells (blocks of Ns filters sharing one (q, r)) whose tuning is
     extreme run the precise variant, the others the plain one -- two launches over a cell permutation that keeps
     every filter on its own stream column (n % Ns).  Returns None when one launch serves all cells."""
@@ -452,8 +488,8 @@ def _replay_sweep_mixed(streams, acc_ref, mag_ref, *, dt, q, r, state, N, Ns, tr
         sub_innov = innov[:, idx].contiguous() if innov is not None else None
         replay(streams, acc_ref, mag_ref, dt=dt, q=q_t[idx].contiguous(), r=sub.r, state=sub, n_filters=idx.numel(), truth=truth,
                loss=sub_loss, precise_state=precise, share_measurements=False, wahba=wahba, staging=staging,
-               keep_filter_frame=keep_filter_frame, innovation=sub_innov,
-               innovation_model=innovation_model)   # (the plain group holds no extreme cell by construction)
+               keep_filter_frame=keep_filter_frame, innovation=sub_innov, innovation_model=innovation_model,
+               lengths=lengths)   # (the plain group holds no extreme cell by construction)
         parts.append((idx, sub, sub_loss, sub_innov, precise))
     if state.x_lo is None:
         state.x_lo = torch.zeros((4, N), dtype=torch.float32, device=dev)

@@ -64,6 +64,11 @@ __device__ __forceinline__ float ldg_stream(const float* p) {
   asm volatile("ld.global.nc.L1::no_allocate.f32 %0, [%1];" : "=f"(v) : "l"(p));
   return v;
 }
+__device__ __forceinline__ f32x2 ldg2_stream(const float* p) {
+  float a, b;
+  asm volatile("ld.global.nc.L1::no_allocate.v2.f32 {%0, %1}, [%2];" : "=f"(a), "=f"(b) : "l"(p));
+  return f32x2(a, b);
+}
 __device__ __forceinline__ void stg_stream(float* p, float v) {
   asm volatile("st.global.cs.f32 [%0], %1;" ::"l"(p), "f"(v) : "memory");
 }

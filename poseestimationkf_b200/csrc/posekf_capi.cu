@@ -84,22 +84,23 @@ int encode_stream_map(const ReplayParams& p, int columns, int steps, CUtensorMap
 
 bool tma_eligible(const ReplayParams& p) {
   if ((reinterpret_cast<uintptr_t>(p.streams) & 15) != 0) return false;
+  if ((reinterpret_cast<uintptr_t>(p.dt_cols) & 15) != 0) return false;   // (the TMA kernels read it with 8-byte loads)
   if (p.Ns % 4 != 0) return false;                        // global strides must be multiples of 16 bytes
   if (p.Ns != p.N && (p.Ns % kThreads) != 0) return false;   // a CTA's 128 columns must not wrap
   if (p.T > INT32_MAX || p.Ns > INT32_MAX) return false;
   return true;
 }
 
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false>
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false>
 int launch_replay(const ReplayParams& p, bool use_tma, cudaStream_t st) {
   const unsigned grid = (unsigned)((p.N + kThreads - 1) / kThreads);
   if (!use_tma) {
-    replay_ldg_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN><<<grid, kThreads, 0, st>>>(p);
+    replay_ldg_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH><<<grid, kThreads, 0, st>>>(p);
     return launch_status();
   }
   CUtensorMap tmap;
   if (int rc = encode_stream_map(p, kThreads, kTmaSteps, &tmap)) return rc;
-  auto kern = replay_tma_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN>;
+  auto kern = replay_tma_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH>;
   // idempotent; set on every launch (cheap) so that it holds on every device of a multi-GPU process
   PKF_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TmaSmem)));
   kern<<<grid, kThreads, sizeof(TmaSmem), st>>>(p, tmap);
@@ -117,56 +118,83 @@ bool packed_eligible(const ReplayParams& p) {
   return true;      // out_traj / truth are already required to be 16-byte aligned
 }
 
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false>
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false>
 int launch_replay_packed(const ReplayParams& p, cudaStream_t st) {
   CUtensorMap tmap;
   if (int rc = encode_stream_map(p, kTile2, kTma2Steps, &tmap)) return rc;
-  auto kern = replay_tma2_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN>;
-  PKF_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Tma2Smem)));
+  auto kern = replay_tma2_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH>;
+  const int smem = (int)sizeof(Tma2Smem) + (BATCH ? (int)kBatchSmem2 : 0);
+  PKF_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   const unsigned grid = (unsigned)((p.N + kTile2 - 1) / kTile2);
-  kern<<<grid, kThreads2, sizeof(Tma2Smem), st>>>(p, tmap);
+  kern<<<grid, kThreads2, smem, st>>>(p, tmap);
   return launch_status();
 }
 
-template <int ALGO> int launch_packed_variant(const ReplayParams& p, bool lpf, cudaStream_t st) {
-  const bool comp = p.state_x_lo != nullptr;
+template <int ALGO, bool LPF, bool BATCH = false> int launch_replay_aux(const ReplayParams& p, bool use_tma, cudaStream_t st) {
   const bool aux = p.out_traj != nullptr || p.out_flip != nullptr || p.truth != nullptr;
-  if (lpf) {
-    if (aux) return comp ? launch_replay_packed<ALGO, true, true, true>(p, st) : launch_replay_packed<ALGO, true, true, false>(p, st);
-    return comp ? launch_replay_packed<ALGO, true, false, true>(p, st) : launch_replay_packed<ALGO, true, false, false>(p, st);
-  }
-  if (aux) return comp ? launch_replay_packed<ALGO, false, true, true>(p, st) : launch_replay_packed<ALGO, false, true, false>(p, st);
-  return comp ? launch_replay_packed<ALGO, false, false, true>(p, st) : launch_replay_packed<ALGO, false, false, false>(p, st);
+  const bool comp = p.state_x_lo != nullptr;
+  if (comp) return aux ? launch_replay<ALGO, LPF, true, true, false, false, BATCH>(p, use_tma, st) : launch_replay<ALGO, LPF, false, true, false, false, BATCH>(p, use_tma, st);
+  return aux ? launch_replay<ALGO, LPF, true, false, false, false, BATCH>(p, use_tma, st) : launch_replay<ALGO, LPF, false, false, false, false, BATCH>(p, use_tma, st);
 }
 
-template <int ALGO, bool LPF> int launch_replay_aux(const ReplayParams& p, bool use_tma, cudaStream_t st) {
-  const bool aux = p.out_traj != nullptr || p.out_flip != nullptr || p.truth != nullptr;
+template <int ALGO, bool BATCH = false> int launch_packed_variant(const ReplayParams& p, bool lpf, cudaStream_t st) {
   const bool comp = p.state_x_lo != nullptr;
-  if (comp) return aux ? launch_replay<ALGO, LPF, true, true>(p, use_tma, st) : launch_replay<ALGO, LPF, false, true>(p, use_tma, st);
-  return aux ? launch_replay<ALGO, LPF, true, false>(p, use_tma, st) : launch_replay<ALGO, LPF, false, false>(p, use_tma, st);
+  const bool aux = p.out_traj != nullptr || p.out_flip != nullptr || p.truth != nullptr;
+  if constexpr (BATCH) {
+    // the precise packed step with per-step outputs or the low-pass, plus the copies a held lane needs, does not fit the
+    // registers of 3 CTAs per SM: the scalar TMA kernel runs those (same results bit for bit)
+    if (comp && (aux || lpf)) return lpf ? launch_replay_aux<ALGO, true, true>(p, true, st) : launch_replay_aux<ALGO, false, true>(p, true, st);
+    if (lpf) return aux ? launch_replay_packed<ALGO, true, true, false, false, false, true>(p, st) : launch_replay_packed<ALGO, true, false, false, false, false, true>(p, st);
+    if (aux) return launch_replay_packed<ALGO, false, true, false, false, false, true>(p, st);
+    return comp ? launch_replay_packed<ALGO, false, false, true, false, false, true>(p, st) : launch_replay_packed<ALGO, false, false, false, false, false, true>(p, st);
+  } else {
+    if (lpf) {
+      if (aux) return comp ? launch_replay_packed<ALGO, true, true, true>(p, st) : launch_replay_packed<ALGO, true, true, false>(p, st);
+      return comp ? launch_replay_packed<ALGO, true, false, true>(p, st) : launch_replay_packed<ALGO, true, false, false>(p, st);
+    }
+    if (aux) return comp ? launch_replay_packed<ALGO, false, true, true>(p, st) : launch_replay_packed<ALGO, false, true, false>(p, st);
+    return comp ? launch_replay_packed<ALGO, false, false, true>(p, st) : launch_replay_packed<ALGO, false, false, false>(p, st);
+  }
 }
 
 // Launches with the innovation likelihood (TAN: its tangent-space form).  The packed kernel carries it without per-step
 // outputs and low-pass (the (Q,R) sweep path, where the registers allow 12 warps per SM); every other combination runs
 // in the scalar kernels on the same staging (TMA or LDG), whose results are the same bit for bit.
-template <int ALGO, bool TAN = false>
+template <int ALGO, bool TAN = false, bool BATCH = false>
 int launch_innovation(const ReplayParams& p, bool lpf, bool aux, bool use_tma, bool packed, cudaStream_t st) {
   const bool comp = p.state_x_lo != nullptr;
   if constexpr (ALGO != WAHBA_JACOBI) {
     if (packed && !lpf && !aux)
-      return comp ? launch_replay_packed<ALGO, false, false, true, true, TAN>(p, st) : launch_replay_packed<ALGO, false, false, false, true, TAN>(p, st);
+      return comp ? launch_replay_packed<ALGO, false, false, true, true, TAN, BATCH>(p, st) : launch_replay_packed<ALGO, false, false, false, true, TAN, BATCH>(p, st);
   }
   if constexpr (ALGO != WAHBA_PRECOMPUTED) {      // (the low-pass of a measurement stream belongs to its builder)
-    if (lpf) return comp ? launch_replay<ALGO, true, true, true, true, TAN>(p, use_tma, st) : launch_replay<ALGO, true, true, false, true, TAN>(p, use_tma, st);
+    if (lpf) return comp ? launch_replay<ALGO, true, true, true, true, TAN, BATCH>(p, use_tma, st) : launch_replay<ALGO, true, true, false, true, TAN, BATCH>(p, use_tma, st);
   }
-  return comp ? launch_replay<ALGO, false, true, true, true, TAN>(p, use_tma, st) : launch_replay<ALGO, false, true, false, true, TAN>(p, use_tma, st);
+  return comp ? launch_replay<ALGO, false, true, true, true, TAN, BATCH>(p, use_tma, st) : launch_replay<ALGO, false, true, false, true, TAN, BATCH>(p, use_tma, st);
 }
 
-template <bool TAN> int launch_innovation_algo(const ReplayParams& p, int algo, bool lpf, bool aux, bool use_tma, bool packed,
-                                               cudaStream_t st) {
-  if (algo == POSEKF_WAHBA_QR2) return launch_innovation<WAHBA_QR2, TAN>(p, lpf, aux, use_tma, packed, st);
-  if (algo == POSEKF_WAHBA_PRECOMPUTED) return launch_innovation<WAHBA_PRECOMPUTED, TAN>(p, lpf, aux, use_tma, packed, st);
-  if (algo == POSEKF_WAHBA_JACOBI) return launch_innovation<WAHBA_JACOBI, TAN>(p, lpf, aux, use_tma, packed, st);
+template <bool TAN, bool BATCH = false>
+int launch_innovation_algo(const ReplayParams& p, int algo, bool lpf, bool aux, bool use_tma, bool packed, cudaStream_t st) {
+  if (algo == POSEKF_WAHBA_QR2) return launch_innovation<WAHBA_QR2, TAN, BATCH>(p, lpf, aux, use_tma, packed, st);
+  if (algo == POSEKF_WAHBA_PRECOMPUTED) return launch_innovation<WAHBA_PRECOMPUTED, TAN, BATCH>(p, lpf, aux, use_tma, packed, st);
+  if (algo == POSEKF_WAHBA_JACOBI) return launch_innovation<WAHBA_JACOBI, TAN, BATCH>(p, lpf, aux, use_tma, packed, st);
+  return POSEKF_EINVAL;
+}
+
+// The kernels of a launch, chosen from its buffers.  BATCH: per-stream dt columns or lengths (ReplayParams::dt_cols /
+// n_valid); every combination the other kernels accept has a BATCH twin on the same staging.
+template <bool BATCH>
+int launch_kernels(const ReplayParams& p, int algo, bool lpf, bool use_tma, bool packed, int innov_model, cudaStream_t st) {
+  if (p.innov_acc) {
+    const bool aux = p.out_traj != nullptr || p.out_flip != nullptr || p.truth != nullptr;
+    return innov_model == POSEKF_INNOV_TANGENT ? launch_innovation_algo<true, BATCH>(p, algo, lpf, aux, use_tma, packed, st)
+                                               : launch_innovation_algo<false, BATCH>(p, algo, lpf, aux, use_tma, packed, st);
+  }
+  if (packed)
+    return algo == POSEKF_WAHBA_QR2 ? launch_packed_variant<WAHBA_QR2, BATCH>(p, lpf, st) : launch_packed_variant<WAHBA_PRECOMPUTED, BATCH>(p, lpf, st);
+  if (algo == POSEKF_WAHBA_PRECOMPUTED) return lpf ? launch_replay_aux<WAHBA_PRECOMPUTED, true, BATCH>(p, use_tma, st) : launch_replay_aux<WAHBA_PRECOMPUTED, false, BATCH>(p, use_tma, st);
+  if (algo == POSEKF_WAHBA_QR2) return lpf ? launch_replay_aux<WAHBA_QR2, true, BATCH>(p, use_tma, st) : launch_replay_aux<WAHBA_QR2, false, BATCH>(p, use_tma, st);
+  if (algo == POSEKF_WAHBA_JACOBI) return lpf ? launch_replay_aux<WAHBA_JACOBI, true, BATCH>(p, use_tma, st) : launch_replay_aux<WAHBA_JACOBI, false, BATCH>(p, use_tma, st);
   return POSEKF_EINVAL;
 }
 
@@ -183,17 +211,10 @@ int replay_dispatch(const ReplayParams& p, int algo, int staging, int innov_mode
     use_tma = tma_eligible(p);
     packed = use_tma && kAutoPrefersPacked && algo != POSEKF_WAHBA_JACOBI && packed_eligible(p);
   } else return POSEKF_EINVAL;
-  int rc;
-  if (p.innov_acc) {
-    const bool aux = p.out_traj != nullptr || p.out_flip != nullptr || p.truth != nullptr;
-    rc = innov_model == POSEKF_INNOV_TANGENT ? launch_innovation_algo<true>(p, algo, lpf, aux, use_tma, packed, st)
-                                             : launch_innovation_algo<false>(p, algo, lpf, aux, use_tma, packed, st);
-  } else if (packed)
-    rc = algo == POSEKF_WAHBA_QR2 ? launch_packed_variant<WAHBA_QR2>(p, lpf, st) : launch_packed_variant<WAHBA_PRECOMPUTED>(p, lpf, st);
-  else if (algo == POSEKF_WAHBA_PRECOMPUTED) rc = lpf ? launch_replay_aux<WAHBA_PRECOMPUTED, true>(p, use_tma, st) : launch_replay_aux<WAHBA_PRECOMPUTED, false>(p, use_tma, st);
-  else if (algo == POSEKF_WAHBA_QR2) rc = lpf ? launch_replay_aux<WAHBA_QR2, true>(p, use_tma, st) : launch_replay_aux<WAHBA_QR2, false>(p, use_tma, st);
-  else if (algo == POSEKF_WAHBA_JACOBI) rc = lpf ? launch_replay_aux<WAHBA_JACOBI, true>(p, use_tma, st) : launch_replay_aux<WAHBA_JACOBI, false>(p, use_tma, st);
-  else return POSEKF_EINVAL;
+  const bool batch = p.dt_cols != nullptr || p.n_valid != nullptr;
+  int rc = batch ? launch_kernels<true>(p, algo, lpf, use_tma, packed, innov_model, st)
+                 : launch_kernels<false>(p, algo, lpf, use_tma, packed, innov_model, st);
+  // (held steps of a batched launch carry flip byte 0, which the fix-up leaves alone)
   if (rc == 0 && p.out_flip && p.T > 0 && algo == POSEKF_WAHBA_QR2 && !lpf) {
     // the flip-mask bytes the kernel marked as float32 ties of the reference's sign rule are settled in float64
     const FlipFixupParams fp{p.N, p.T, p.Ns, p.streams, p.acc_ref, p.mag_ref, p.out_flip};
@@ -228,13 +249,16 @@ const char* posekf_version(void) { return "posekf_b200 0.2 sm_100a"; }
 }  // extern "C"
 
 namespace {
-// Validation and dispatch shared by posekf_replay_f32 and posekf_replay_innovation(_ex)_f32 (innov_acc null: the first).
+// Validation and dispatch shared by posekf_replay_f32, posekf_replay_innovation(_ex)_f32 and posekf_replay_batch_f32
+// (innov_acc null: the first; dt_cols and n_valid null: all but the last).
 // innov_model: POSEKF_INNOV_FULL or POSEKF_INNOV_TANGENT (checked by the caller).
 int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
                  int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_scale,
                  const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag, float* state_x, float* state_x_lo,
                  float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth, float* loss_acc,
-                 float* innov_acc, int innov_model, int wahba_algo, int staging, int state_flags, void* stream) {
+                 float* innov_acc, int innov_model, int wahba_algo, int staging, int state_flags, void* stream,
+                 const float* dt_cols = nullptr, const int32_t* n_valid = nullptr) {
+  if (dt_cols && !dt) { dt = dt_cols; dt_per_step = 0; }    // (the kernels read dt[0] unconditionally; it is unused then)
   if (n_filters < 0 || n_steps < 0 || n_streams <= 0 && n_filters > 0) return POSEKF_EINVAL;
   if (state_flags & ~(POSEKF_STATE_IN_FILTER_FRAME | POSEKF_STATE_OUT_FILTER_FRAME)) return POSEKF_EINVAL;
   if (n_filters == 0) return 0;
@@ -256,6 +280,7 @@ int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64
   if (out_traj && (reinterpret_cast<uintptr_t>(out_traj) & 15) != 0) return POSEKF_EALIGN;
   if (truth && (!loss_acc || (reinterpret_cast<uintptr_t>(truth) & 15) != 0)) return truth && !loss_acc ? POSEKF_EINVAL : POSEKF_EALIGN;
   if ((reinterpret_cast<uintptr_t>(innov_acc) & 3) != 0) return POSEKF_EALIGN;
+  if ((reinterpret_cast<uintptr_t>(dt_cols) & 3) != 0 || (reinterpret_cast<uintptr_t>(n_valid) & 3) != 0) return POSEKF_EALIGN;
   ReplayParams p;
   p.N = n_filters; p.T = n_steps; p.Ns = n_streams; p.streams = streams; p.dt = dt; p.dt_per_step = dt_per_step;
   p.acc_ref = acc_ref; p.mag_ref = mag_ref; p.q_scale = q_scale; p.r_scale = r_scale;
@@ -264,6 +289,8 @@ int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64
   p.truth = truth; p.loss_acc = loss_acc;
   p.innov_acc = n_steps > 0 ? innov_acc : nullptr;     // (a frame conversion has no step to add)
   p.state_flags = state_flags;
+  p.dt_cols = n_steps > 0 ? dt_cols : nullptr;
+  p.n_valid = n_steps > 0 ? n_valid : nullptr;
   return replay_dispatch(p, wahba_algo, staging, innov_model, (cudaStream_t)stream);
 }
 }  // namespace
@@ -302,6 +329,18 @@ int posekf_replay_innovation_ex_f32(int64_t n_filters, int64_t n_steps, const fl
   return replay_entry(n_filters, n_steps, streams, n_streams, dt, dt_per_step, acc_ref, mag_ref, q_scale, r_scale, lpf_alpha_acc,
                       lpf_alpha_mag, state_x, state_x_lo, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, innov_acc,
                       innov_model, wahba_algo, staging, state_flags, stream);
+}
+
+int posekf_replay_batch_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
+                            int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_scale,
+                            const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag, float* state_x, float* state_x_lo,
+                            float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth,
+                            float* loss_acc, float* innov_acc, int innov_model, int wahba_algo, int staging, int state_flags,
+                            void* stream, const float* dt_cols, const int32_t* n_valid) {
+  if (innov_model != POSEKF_INNOV_FULL && innov_model != POSEKF_INNOV_TANGENT) return POSEKF_EINVAL;
+  return replay_entry(n_filters, n_steps, streams, n_streams, dt, dt_per_step, acc_ref, mag_ref, q_scale, r_scale, lpf_alpha_acc,
+                      lpf_alpha_mag, state_x, state_x_lo, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, innov_acc,
+                      innov_model, wahba_algo, staging, state_flags, stream, dt_cols, n_valid);
 }
 
 // ---- host-buffer replay: workspace (device staging buffers, streams, events) ----------------------

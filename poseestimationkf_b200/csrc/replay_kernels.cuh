@@ -30,7 +30,10 @@ struct ReplayParams {
   int state_flags;      // POSEKF_STATE_IN_FILTER_FRAME | POSEKF_STATE_OUT_FILTER_FRAME (include/posekf.h)
   float* innov_acc;     // [2][N] in/out innovation likelihood sums (NIS, ln det S; TAN kernels: of the tangent-space
                         // model), or null; read by INNOV kernels only
-                        // (last: the parameter offsets of the other kernels are unchanged)
+  // batched recordings (read by BATCH kernels only; filter n uses column n % Ns of both):
+  const float* dt_cols;     // [T][Ns] per-stream time steps (overrides dt / dt_per_step), or null
+  const int32_t* n_valid;   // [Ns] steps of this launch that stream n % Ns has (0..T); later steps hold the filter, or null
+                            // (last: the parameter offsets of the other kernels are unchanged)
 };
 constexpr int kStateInFilterFrame = 1, kStateOutFilterFrame = 2;
 
@@ -141,13 +144,30 @@ __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f
   }
 }
 
+// A step at or past the length of the filter's stream (BATCH kernels): the filter is left as it is, the trajectory slot
+// gets the held state, the flip byte is 0 (unmarked: flip_fixup_kernel leaves it alone) and the objectives add nothing.
+// The step's sample and dt are not read.
+template <int ALGO, bool AUX>
+__device__ __forceinline__ void hold_step(const ReplayParams& p, const FilterRegs& f, AuxPtrs& aux) {
+  if (AUX) {
+    if (aux.traj) {
+      Quat<float> xr = f.x;
+      if (uses_filter_frame<ALGO>()) xr = state_in_reference_frame(f.fc, f.x);
+      stg_stream4(aux.traj, xr.w, xr.x, xr.y, xr.z);
+      aux.traj += p.N;
+    }
+    if (aux.flips) { *aux.flips = 0; aux.flips += p.N; }
+    if (aux.truth) aux.truth += p.Ns;
+  }
+}
+
 // ---------------------------------------------------------------------------------------------
 // Replay, LDG staging: coalesced loads straight to registers, next step prefetched while the
 // current one is computed.
 // ---------------------------------------------------------------------------------------------
 // (INNOV: the innovation likelihood, TAN: its tangent-space form; their instantiations always have AUX and are built for
-//  3 CTAs per SM, <= 168 registers)
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false>
+//  3 CTAs per SM, <= 168 registers.  BATCH: per-stream dt columns and lengths, ReplayParams::dt_cols / n_valid)
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false>
 __global__ void __launch_bounds__(kThreads, INNOV ? 3 : ((ALGO == WAHBA_JACOBI || (COMP && LPF && AUX)) ? 4 : ((COMP || LPF) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
     replay_ldg_kernel(const ReplayParams p) {
   const int64_t n = (int64_t)blockIdx.x * kThreads + threadIdx.x;
@@ -161,20 +181,55 @@ __global__ void __launch_bounds__(kThreads, INNOV ? 3 : ((ALGO == WAHBA_JACOBI |
   const int64_t step_stride = kChannels * Ns;
   float cur[kChannels], nxt[kChannels];
   const int T = (int)p.T;     // T == 0: a frame conversion of the state only (no stream is read)
+  // BATCH: this stream's length and time-step column (prefetched with the samples)
+  const int nv = (BATCH && p.n_valid) ? p.n_valid[col] : T;
+  const float* dc = (BATCH && p.dt_cols) ? p.dt_cols + col : nullptr;
+  float hcur = 0.f, hnxt = 0.f;
 #pragma unroll
   for (int c = 0; c < kChannels; ++c) cur[c] = T > 0 ? ldg_stream(s + c * Ns) : 0.f;
+  if (BATCH && dc && T > 0) hcur = ldg_stream(dc);
   const float dt0 = T > 0 ? p.dt[0] : 0.f;
   for (int t = 0; t < T; ++t) {
     if (t + 1 < T) s += step_stride;
 #pragma unroll
     for (int c = 0; c < kChannels; ++c) nxt[c] = ldg_stream(s + c * Ns);
-    const float h = p.dt_per_step ? __ldg(p.dt + t) : dt0;
-    filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN>(p, f, cur, h, aux);
+    if (BATCH && dc) hnxt = ldg_stream(dc + (int64_t)(t + 1 < T ? t + 1 : t) * Ns);
+    const float h = (BATCH && dc) ? hcur : (p.dt_per_step ? __ldg(p.dt + t) : dt0);
+    if (!BATCH || t < nv) filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN>(p, f, cur, h, aux);
+    else hold_step<ALGO, AUX>(p, f, aux);
 #pragma unroll
     for (int c = 0; c < kChannels; ++c) cur[c] = nxt[c];
+    if (BATCH) hcur = hnxt;
   }
   store_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, f);
   if (AUX && aux.truth) p.loss_acc[n] = aux.loss;
+}
+
+// BATCH kernels: the stream length(s) of the thread's filter(s) and the per-step dt of the current and the next tile
+// (registers; the next tile's are loaded one tile ahead, like the samples)
+template <bool BATCH, typename V, int S> struct BatchRegs {};
+template <typename V, int S> struct BatchRegs<true, V, S> {
+  int nv, nv1, min_nv;
+  const float* dc;
+  V cur[S], next[S];
+};
+
+// dt of the S steps of tile k (0 past T): a column of dt_cols, or the launch's dt / dt[T]
+template <int S>
+__device__ __forceinline__ void load_dt_tile(float (&h)[S], const ReplayParams& p, const float* dc, int k, int T, float dt0) {
+#pragma unroll
+  for (int tt = 0; tt < S; ++tt) {
+    const int t = k * S + tt;
+    h[tt] = t >= T ? 0.f : (dc ? ldg_stream(dc + (int64_t)t * p.Ns) : (p.dt_per_step ? __ldg(p.dt + t) : dt0));
+  }
+}
+template <int S>
+__device__ __forceinline__ void load_dt_tile(f32x2 (&h)[S], const ReplayParams& p, const float* dc, int k, int T, float dt0) {
+#pragma unroll
+  for (int tt = 0; tt < S; ++tt) {
+    const int t = k * S + tt;
+    h[tt] = t >= T ? f32x2(0.f) : (dc ? ldg2_stream(dc + (int64_t)t * p.Ns) : f32x2(p.dt_per_step ? __ldg(p.dt + t) : dt0));
+  }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -190,7 +245,7 @@ struct __align__(128) TmaSmem {
 };
 constexpr uint32_t kTileBytes = kTmaSteps * kChannels * kThreads * sizeof(float);
 
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false>
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false>
 __global__ void __launch_bounds__(kThreads, INNOV ? 3 : (ALGO == WAHBA_JACOBI ? 4 : ((COMP && (LPF || AUX)) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
     replay_tma_kernel(const ReplayParams p, const __grid_constant__ CUtensorMap tmap) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -224,6 +279,14 @@ __global__ void __launch_bounds__(kThreads, INNOV ? 3 : (ALGO == WAHBA_JACOBI ? 
   if (valid) load_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, (int64_t)col0 + tid, f);
   AuxPtrs aux = make_aux<AUX>(p, n, (int64_t)col0 + tid, valid);
   const float dt0 = p.dt[0];
+  // BATCH: this stream's length, and the time steps of the next tile held in registers (loaded one tile ahead: the
+  // shared-memory ring has no room left at this kernel's occupancy)
+  [[maybe_unused]] BatchRegs<BATCH, float, kTmaSteps> bt;
+  if constexpr (BATCH) {
+    bt.nv = (valid && p.n_valid) ? p.n_valid[col0 + tid] : T;
+    bt.dc = p.dt_cols ? p.dt_cols + col0 + tid : nullptr;
+    if (valid) load_dt_tile(bt.next, p, bt.dc, 0, T, dt0);
+  }
 
   int stage = 0;
   uint32_t parity = 0;
@@ -236,17 +299,29 @@ __global__ void __launch_bounds__(kThreads, INNOV ? 3 : (ALGO == WAHBA_JACOBI ? 
       mbar_expect_tx(&sm.full[ps], kTileBytes);
       tma_load_3d(&sm.tile[ps][0][0][0], &tmap, &sm.full[ps], col0, 0, (k - 1 + kTmaStages) * kTmaSteps);
     }
+    if constexpr (BATCH) {
+#pragma unroll
+      for (int tt = 0; tt < kTmaSteps; ++tt) bt.cur[tt] = bt.next[tt];
+      if (valid && k + 1 < n_chunks) load_dt_tile(bt.next, p, bt.dc, k + 1, T, dt0);
+    }
     mbar_wait(&sm.full[stage], parity);
     if (valid) {
       const int steps = min(kTmaSteps, T - k * kTmaSteps);     // < kTmaSteps only in the last chunk
 #pragma unroll
       for (int tt = 0; tt < kTmaSteps; ++tt) {
         if (tt < steps) {
+          if constexpr (BATCH) {
+            if (k * kTmaSteps + tt >= bt.nv) { hold_step<ALGO, AUX>(p, f, aux); continue; }
+          }
           float s[kChannels];
 #pragma unroll
           for (int c = 0; c < kChannels; ++c) s[c] = sm.tile[stage][tt][c][tid];
-          const float h = p.dt_per_step ? __ldg(p.dt + k * kTmaSteps + tt) : dt0;
-          filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN>(p, f, s, h, aux);
+          if constexpr (BATCH) {
+            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN>(p, f, s, bt.cur[tt], aux);
+          } else {
+            const float h = p.dt_per_step ? __ldg(p.dt + k * kTmaSteps + tt) : dt0;
+            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN>(p, f, s, h, aux);
+          }
         }
       }
     }
@@ -272,6 +347,7 @@ struct __align__(128) Tma2Smem {
   uint64_t empty[kTma2Stages];
 };
 constexpr uint32_t kTile2Bytes = kTma2Steps * kChannels * kTile2 * sizeof(float);
+constexpr uint32_t kBatchSmem2 = (kThreads2 / 32) * sizeof(int);     // BATCH: per-warp minima of the stream lengths
 
 struct FilterRegs2 {
   Quat<f32x2> x, xlo;
@@ -281,10 +357,30 @@ struct FilterRegs2 {
   InnovAcc<f32x2> in;
 };
 
+template <bool HOLD> struct HeldLanes {};
+template <> struct HeldLanes<true> { mask2 live; FilterRegs2 f0; f32x2 loss0; };
+
+// BATCH: the lanes that were past their stream's length (live false) get back the values they had before the step
+template <bool LPF, bool COMP, bool INNOV>
+__device__ __forceinline__ void hold_lanes(mask2 live, FilterRegs2& f, const FilterRegs2& f0) {
+  f.x = {sel_(live, f.x.w, f0.x.w), sel_(live, f.x.x, f0.x.x), sel_(live, f.x.y, f0.x.y), sel_(live, f.x.z, f0.x.z)};
+  if (COMP) f.xlo = {sel_(live, f.xlo.w, f0.xlo.w), sel_(live, f.xlo.x, f0.xlo.x), sel_(live, f.xlo.y, f0.xlo.y), sel_(live, f.xlo.z, f0.xlo.z)};
+  f.P = {sel_(live, f.P.a00, f0.P.a00), sel_(live, f.P.a01, f0.P.a01), sel_(live, f.P.a02, f0.P.a02), sel_(live, f.P.a03, f0.P.a03),
+         sel_(live, f.P.a11, f0.P.a11), sel_(live, f.P.a12, f0.P.a12), sel_(live, f.P.a13, f0.P.a13), sel_(live, f.P.a22, f0.P.a22),
+         sel_(live, f.P.a23, f0.P.a23), sel_(live, f.P.a33, f0.P.a33)};
+  if (LPF) {
+    f.la = {sel_(live, f.la.x, f0.la.x), sel_(live, f.la.y, f0.la.y), sel_(live, f.la.z, f0.la.z)};
+    f.lm = {sel_(live, f.lm.x, f0.lm.x), sel_(live, f.lm.y, f0.lm.y), sel_(live, f.lm.z, f0.lm.z)};
+  }
+  if (INNOV) { f.in.nis = sel_(live, f.in.nis, f0.in.nis); f.in.logdet = sel_(live, f.in.logdet, f0.in.logdet); }
+}
+
 // (the precise variant with per-step outputs needs ~190 registers: 8 warps per SM instead of 12.  INNOV: the innovation
 //  likelihood (TAN: tangent-space form), instantiated without per-step outputs and low-pass -- the sweep path;
-//  replay_dispatch routes the rest)
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false>
+//  replay_dispatch routes the rest.  BATCH: per-stream dt columns and lengths; a tile runs as the one-block fast tile
+//  when every filter of the CTA is live for all of its steps, and otherwise steps both lanes and keeps the old values of
+//  a lane past its length)
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false>
 __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) < PKF_MIN_CTAS2 ? (256 / kThreads2) : PKF_MIN_CTAS2) : PKF_MIN_CTAS2)
     replay_tma2_kernel(const ReplayParams p, const __grid_constant__ CUtensorMap tmap) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -297,6 +393,15 @@ __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) 
   const int T = (int)p.T;
   const int n_chunks = (T + kTma2Steps - 1) / kTma2Steps;
   const int64_t N = p.N, Ns = p.Ns;
+  // BATCH: the lengths of this thread's two streams and their minimum over the CTA (reduced once, here)
+  [[maybe_unused]] BatchRegs<BATCH, f32x2, kTma2Steps> bt;
+  if constexpr (BATCH) {
+    int* warp_min = reinterpret_cast<int*>(smem_raw + sizeof(Tma2Smem));     // kBatchSmem2 bytes past the ring
+    bt.nv = bt.nv1 = bt.min_nv = T;
+    if (valid && p.n_valid) { bt.nv = p.n_valid[col0 + 2 * tid]; bt.nv1 = p.n_valid[col0 + 2 * tid + 1]; }
+    const int m = __reduce_min_sync(0xffffffffu, valid ? min(bt.nv, bt.nv1) : T);
+    if ((tid & 31) == 0) warp_min[tid >> 5] = m;
+  }
 
   if (tid == 0) {
 #pragma unroll
@@ -304,6 +409,11 @@ __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) 
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncthreads();
+  if constexpr (BATCH) {
+    const int* warp_min = reinterpret_cast<const int*>(smem_raw + sizeof(Tma2Smem));
+#pragma unroll
+    for (int w = 0; w < kThreads2 / 32; ++w) bt.min_nv = min(bt.min_nv, warp_min[w]);
+  }
   if (tid == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(&tmap) : "memory");
 #pragma unroll
@@ -348,6 +458,12 @@ __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) 
     if (p.out_flip) flips = p.out_flip + n;
     if (p.truth) { truth = reinterpret_cast<const float4*>(p.truth) + ((int64_t)col0 + 2 * tid); loss = ld2(p.loss_acc + n); }
   }
+  // BATCH: the per-lane time steps of the next tile, held in registers (loaded one tile ahead: the shared-memory ring has
+  // no room left for them at 3 CTAs per SM)
+  if constexpr (BATCH) {
+    bt.dc = p.dt_cols ? p.dt_cols + col0 + 2 * tid : nullptr;
+    if (valid) load_dt_tile(bt.next, p, bt.dc, 0, T, dt0);
+  }
 
   int stage = 0;
   uint32_t parity = 0;
@@ -363,6 +479,11 @@ __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) 
     if (tid == 0 && (k + kTma2Stages - 1 + PKF_L2_PREFETCH) < n_chunks)
       tma_prefetch_l2_3d(&tmap, col0, 0, (k + kTma2Stages - 1 + PKF_L2_PREFETCH) * kTma2Steps);
 #endif
+    if constexpr (BATCH) {
+#pragma unroll
+      for (int tt = 0; tt < kTma2Steps; ++tt) bt.cur[tt] = bt.next[tt];
+      if (valid && k + 1 < n_chunks) load_dt_tile(bt.next, p, bt.dc, k + 1, T, dt0);
+    }
     mbar_wait(&sm.full[stage], parity);
     if (valid) {
       const int steps = min(kTma2Steps, T - k * kTma2Steps);
@@ -375,7 +496,18 @@ __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) 
 #pragma unroll
         for (int c = 0; c < kChannels; ++c) s[c] = ld2(&sm.tile[stage][tt][c][2 * tid]);
         StepH<f32x2> sh = sh0;                         // launch constant (the fast path runs only then) ...
-        if (!FAST && p.dt_per_step) sh = StepH<f32x2>(f32x2(__ldg(p.dt + k * kTma2Steps + tt)));     // ... unless dt comes per step
+        if constexpr (BATCH) sh = StepH<f32x2>(bt.cur[tt]);     // (per lane: rounds as the scalar StepH<float> of each lane)
+        else if (!FAST && p.dt_per_step) sh = StepH<f32x2>(f32x2(__ldg(p.dt + k * kTma2Steps + tt)));     // ... unless dt comes per step
+        // BATCH, general path: the lanes past their stream's length get their values from before the step back
+        [[maybe_unused]] HeldLanes<BATCH && !FAST> held;
+        if constexpr (BATCH) {
+          if constexpr (!FAST) {
+            const int t = k * kTma2Steps + tt;
+            held.live = mask2{t < bt.nv, t < bt.nv1};
+            held.f0 = f;
+            held.loss0 = loss;
+          }
+        }
         Vec3<f32x2> w = {s[0], s[1], s[2]}, a = {s[3], s[4], s[5]}, m = {s[6], s[7], s[8]};
         if (LPF) {
           if (p.alpha_acc >= 0.f) { lowpass<f32x2>(f.la, a, f32x2(p.alpha_acc), f32x2(1.f - p.alpha_acc)); a = f.la; }
@@ -389,6 +521,12 @@ __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) 
         else ekf_step<f32x2, ALGO, AUX, COMP, INNOV, TAN>(f.x, f.xlo, f.P, f.fc, w, a, m, sh, flip, flips != nullptr, kTieCode ? &code : nullptr,
                                                           INNOV ? &f.in : nullptr);
         if (!kTieCode) code = FlipCode2{flip.x ? 1u : 0u, flip.y ? 1u : 0u};
+        if constexpr (BATCH && !FAST) {
+          if (!(held.live.x && held.live.y)) {
+            hold_lanes<LPF, COMP, INNOV>(held.live, f, held.f0);
+            code = FlipCode2{held.live.x ? code.x : 0u, held.live.y ? code.y : 0u};
+          }
+        }
         if (AUX) {
           Quat<f32x2> xr = f.x;     // per-step outputs are in the reference frame
           if (uses_filter_frame<ALGO>() && (traj || truth)) xr = state_in_reference_frame(f.fc, f.x);
@@ -408,13 +546,18 @@ __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) 
             const f32x2 m01 = fma_(xw, qx, -(xx * qw)), m02 = fma_(xw, qy, -(xy * qw)), m03 = fma_(xw, qz, -(xz * qw));
             const f32x2 m12 = fma_(xx, qy, -(xy * qx)), m13 = fma_(xx, qz, -(xz * qx)), m23 = fma_(xy, qz, -(xz * qy));
             loss = loss + fma_(m23, m23, fma_(m13, m13, fma_(m12, m12, fma_(m03, m03, fma_(m02, m02, m01 * m01)))));
+            if constexpr (BATCH && !FAST) loss = sel_(held.live, loss, held.loss0);
           }
         }
       };
       bool fast = false;
-      if constexpr (ALGO == WAHBA_PRECOMPUTED && PKF_FAST_TILE) fast = steps == kTma2Steps && !p.dt_per_step;   // no branch in that step at all
+      // (BATCH: the time steps come per lane from registers; every filter of the CTA is live for the whole tile)
+      bool whole;
+      if constexpr (BATCH) whole = k * kTma2Steps + kTma2Steps <= bt.min_nv;
+      else whole = !p.dt_per_step;
+      if constexpr (ALGO == WAHBA_PRECOMPUTED && PKF_FAST_TILE) fast = steps == kTma2Steps && whole;   // no branch in that step at all
       if constexpr (ALGO == WAHBA_QR2 && !LPF && PKF_FAST_TILE) {
-        if (steps == kTma2Steps && !p.dt_per_step) {
+        if (steps == kTma2Steps && whole) {
           // |a_z| <= 1 for every sample of the tile (both lanes): the accelerometer weight 1 - |a_z| is non-negative
           float az = 0.f;
 #pragma unroll

@@ -48,6 +48,66 @@ class LogData:
                 f32(np.asarray(self.mag_0, dtype=np.float64)[:, None]), f32(dt))
 
 
+@dataclass
+class LogBatch:
+    """Several recordings stacked for one `batched.replay` launch (`stack_logs`): column c is recording c.
+    streams [T,9,Ns] float32, acc_ref / mag_ref [3,Ns], dt [T,Ns] float32 seconds, lengths [Ns] int32 (steps of each
+    recording), n_logs: the number of real recordings (columns n_logs..Ns-1 are padding of length 0)."""
+    streams: object
+    acc_ref: object
+    mag_ref: object
+    dt: object
+    lengths: object
+    n_logs: int
+
+    def window(self, t0: int, t1: int) -> "LogBatch":
+        """Steps [t0, t1) for a time-chunked replay: the slices, and lengths counted from t0, clamped to [0, t1 - t0]
+        (pass `keep_filter_frame=True` on every chunk but the last)."""
+        import torch
+        lengths = torch.clamp(self.lengths - t0, 0, t1 - t0).to(torch.int32)
+        return LogBatch(self.streams[t0:t1], self.acc_ref, self.mag_ref, self.dt[t0:t1], lengths, self.n_logs)
+
+
+def stack_logs(logs, device="cuda", pad_cols_to: int = 4) -> LogBatch:
+    """Stack recordings (`LogData`) of different lengths and timestamps into one batch.  Each recording's dt is its own
+    timestamps differenced in float64 ns on the host, bit for bit the dt of its `to_streams` (main_file.py:25: every
+    recording keeps its own previousT).  The steps past a recording's end repeat its last sample with dt = 0 (a
+    recording without samples repeats its reference vectors with zero rate); the number of columns is rounded up to a
+    multiple of `pad_cols_to` (4 keeps the TMA staging) with empty recordings of length 0."""
+    import torch
+    K = len(logs)
+    Tmax = max([lg.n_steps() for lg in logs], default=0)
+    Ns = -(-K // pad_cols_to) * pad_cols_to if pad_cols_to > 1 else K
+    streams = np.zeros((Tmax, 9, Ns), dtype=np.float32)
+    acc_ref = np.zeros((3, Ns), dtype=np.float32)
+    mag_ref = np.zeros((3, Ns), dtype=np.float32)
+    acc_ref[2] = 1.0
+    mag_ref[0] = 1.0
+    dt = np.zeros((Tmax, Ns), dtype=np.float32)
+    lengths = np.zeros((Ns,), dtype=np.int32)
+    for c, lg in enumerate(logs):
+        T = lg.n_steps()
+        acc_ref[:, c] = np.asarray(lg.acc_0, dtype=np.float64)
+        mag_ref[:, c] = np.asarray(lg.mag_0, dtype=np.float64)
+        lengths[c] = T
+        if T == 0:
+            continue
+        # the arithmetic of to_streams, one recording at a time
+        s = np.concatenate([np.asarray(lg.gyro[:T], dtype=np.float64), np.asarray(lg.acc_1, dtype=np.float64),
+                            np.asarray(lg.mag_1[:T], dtype=np.float64)], axis=1)
+        t_ns = np.asarray(lg.timestamp, dtype=np.float64)[:, 0]
+        streams[:T, :, c] = s.astype(np.float32)
+        streams[T:, :, c] = streams[T - 1, :, c]
+        dt[:T, c] = np.ascontiguousarray(np.diff(t_ns)[:T] * 1e-9, dtype=np.float32)
+    for c in range(Ns):
+        if lengths[c] == 0:
+            streams[:, 3:6, c] = acc_ref[:, c]
+            streams[:, 6:9, c] = mag_ref[:, c]
+    dev = torch.device(device)
+    t = lambda a: torch.from_numpy(a).to(dev)
+    return LogBatch(t(streams), t(acc_ref), t(mag_ref), t(dt), t(lengths), K)
+
+
 def _values(line: str):
     """ReadFile.py:14-21 (`getArray`): text after the first ':' split on ','."""
     return [float(v) for v in line.split(":")[1].split(",")]

@@ -76,7 +76,8 @@ class SweepWorkload:
     rs: torch.Tensor
     q: torch.Tensor            # [G*G*Ns] per-filter; cell g = iq*G + ir owns filters g*Ns .. (g+1)*Ns
     r: torch.Tensor
-    dt: float | torch.Tensor   # seconds, or [T] per-step (a recording)
+    dt: float | torch.Tensor   # seconds, [T] per-step (a recording) or [T, Ns] per stream (a batch of recordings)
+    lengths: torch.Tensor | None = None     # [Ns] int32 steps of each stream (a batch of recordings), None: all T
 
     @property
     def n_filters(self) -> int:
@@ -121,7 +122,7 @@ def run_c3(w: SweepWorkload, *, precise_state=None, share_measurements=None, obj
     B.replay(w.streams, w.acc_ref, w.mag_ref, dt=w.dt, q=w.q, r=w.r, n_filters=N, state=st,
              truth=w.truth if objective == "truth" else None, innovation=True if innov_model else None,
              innovation_model=innov_model or "full", precise_state=precise_state, share_measurements=share_measurements,
-             staging=staging)
+             staging=staging, lengths=w.lengths)
     return st
 
 
@@ -152,6 +153,36 @@ def build_recording_sweep(log, device, grid: int = C3_GRID, lo: float = -3.0, st
     q = qs.repeat_interleave(grid).contiguous()
     r = rs.repeat(grid).contiguous()
     return SweepWorkload(streams, acc_ref, mag_ref, None, qs, rs, q, r, dt)
+
+
+def build_multi_recording_sweep(logs, device, grid: int = C3_GRID, lo: float = -7.0, step: float = 0.1) -> SweepWorkload:
+    """A (Q,R) grid over a SET of recorded logs, all in one launch: the cell layout of `build_c3` with Ns = len(logs)
+    streams (rounded up to a multiple of 4 with empty ones), each with its own dt and length (`logio.stack_logs`).  Run
+    it with `run_c3(w, objective="innovation_tangent")` and read `pooled_innovation_surface`, whose argmin is the one
+    (Q,R) that best explains every recording together."""
+    from .logio import stack_logs
+    b = stack_logs(logs, device)
+    Ns = b.streams.shape[2]
+    hi = lo + step * (grid - 1)
+    qs = torch.logspace(lo, hi, grid, device=device)
+    rs = torch.logspace(lo, hi, grid, device=device)
+    q = qs.repeat_interleave(grid).repeat_interleave(Ns).contiguous()
+    r = rs.repeat(grid).repeat_interleave(Ns).contiguous()
+    return SweepWorkload(b.streams, b.acc_ref, b.mag_ref, None, qs, rs, q, r, b.dt, b.lengths)
+
+
+def pooled_innovation_surface(w: SweepWorkload, st: B.ReplayState):
+    """([Gq, Gr] pooled innovation NLL per step, [Gq, Gr] pooled mean NIS) per cell, float64: the joint likelihood of
+    all recordings of the sweep under the cell's one (Q,R), sum_k NLL_k / sum_k L_k, and sum_k sum_t NIS / sum_k L_k
+    (L_k: the length of recording k; streams of length 0 add nothing).  Its argmin is the pooled tuning."""
+    T, _, Ns = w.streams.shape
+    L = (w.lengths if w.lengths is not None else torch.full((Ns,), T, dtype=torch.int32, device=w.streams.device))
+    L = L.to(torch.float64)
+    n_steps = L.repeat(st.x.shape[1] // Ns)
+    nll, _ = B.innovation_nll(st, n_steps)
+    shape = (w.qs.numel(), w.rs.numel(), Ns)
+    total = L.sum()
+    return nll.reshape(shape).sum(2) / total, st.innov[0].to(torch.float64).reshape(shape).sum(2) / total
 
 
 # ------------------------------------------------------------------------------------------------
