@@ -192,6 +192,35 @@ int posekf_replay_batch_f32(int64_t n_filters, int64_t n_steps, const float* str
                             float* loss_acc, float* innov_acc, int innov_model, int wahba_algo, int staging, int state_flags,
                             void* stream, const float* dt_cols, const int32_t* n_valid);
 
+/* Innovation gating: the replay of posekf_replay_batch_f32 (same parameters, same rules) with outlier measurements
+ * rejected by their tangent-space normalised innovation squared.  A live step is GATED iff
+ *     NIS3_t = e3^T S3^-1 e3 > gate_nis3          (S = P^- + r I, e = y - z after the comparator, u = z/|z|; see
+ *                                                  posekf_replay_innovation_ex_f32 for e3 and S3)
+ * computed the same way whichever innov_model the launch accumulates.  The comparison is strict: a NaN statistic is
+ * not gated (NaN propagates as in the reference).  Under a consistent model NIS3 ~ chi^2_3: 16.27 is its 0.999
+ * quantile.  On a gated step:
+ *   state       X_t = z_t / |z_t|, the normalised prediction (the update with e = 0); x_lo carries it the same way;
+ *   covariance  P_t = P^-_t, the propagated covariance: state_p holds P^-/r;
+ *   flip byte, loss_acc, low-pass state: as without the gate (the comparator still runs, the fix-up still applies);
+ *   innov_acc   still adds the step's terms: the prediction-error decomposition stays the exact likelihood of the
+ *               observations under the predictor that produced z and S, so the NLL stays a (Q,R) objective.
+ * Held steps (t >= n_valid) are never gated and never counted.  gate_nis3 = +inf gives the bits of the same launch
+ * without the gate; a chunked replay equals the unchunked one (the gate carries no state beyond X and P).  With q = 0
+ * a run of rejected steps can never reopen the gate: P^- does not grow.
+ *   gate_nis3   the threshold; NaN: POSEKF_EINVAL.
+ *   gate_count  [N] int32 in/out, or NULL: += the number of gated steps of filter n (4-byte aligned, else
+ *               POSEKF_EALIGN).
+ *   out_gated   [T][N] uint8, or NULL: 1 where the step was gated, else 0 (held steps 0).
+ * The packed kernel reads gate_count 8 bytes and writes out_gated 2 bytes at a time: buffers not aligned for that run
+ * the scalar TMA kernel (same results).  Which kernel runs which combination: DESIGN.md section 5, f8. */
+int posekf_replay_gated_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
+                            int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_scale,
+                            const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag, float* state_x, float* state_x_lo,
+                            float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth,
+                            float* loss_acc, float* innov_acc, int innov_model, int wahba_algo, int staging, int state_flags,
+                            void* stream, const float* dt_cols, const int32_t* n_valid, float gate_nis3, int32_t* gate_count,
+                            uint8_t* out_gated);
+
 /* Same replay with HOST buffers: streams_host [T][9][N] is streamed through the device in time
  * chunks (double-buffered H2D copies overlapped with the filter kernel, state carried across
  * chunks on the device), results are copied back.  This is the call an offline-replay user makes.

@@ -86,7 +86,8 @@ class ReplayState:
     default) or "filter" (left in the kernel's working frame by `replay(..., keep_filter_frame=True)`
     between the chunks of a time-chunked replay; `to_reference_frame` converts).
     innov [2,N]: the innovation likelihood sums (sum_t NIS_t, sum_t ln det S_t) of `replay(..., innovation=...)`;
-    innov_model: the model they belong to ("full" or "tangent", see `replay(..., innovation_model=...)`)."""
+    innov_model: the model they belong to ("full" or "tangent", see `replay(..., innovation_model=...)`).
+    gate_count [N] int32: the number of steps the innovation gate rejected (see `replay(..., gate=...)`)."""
     x: torch.Tensor
     p: torch.Tensor
     r: object = 0.1
@@ -96,6 +97,7 @@ class ReplayState:
     frame: str = "reference"
     innov: torch.Tensor | None = None    # [2,N] innovation likelihood sums (see replay(innovation=...))
     innov_model: str | None = None       # "full" / "tangent": the model of `innov`
+    gate_count: torch.Tensor | None = None   # [N] int32 gated steps (see replay(gate=...))
 
     @staticmethod
     def initial(n_filters: int, device, r=0.1, with_lpf: bool = False, P0: torch.Tensor | None = None) -> "ReplayState":
@@ -119,7 +121,7 @@ class ReplayState:
     def clone(self) -> "ReplayState":
         c = lambda t: None if t is None else t.clone()
         return ReplayState(self.x.clone(), self.p.clone(), self.r, c(self.lpf), c(self.loss), c(self.x_lo), self.frame,
-                           c(self.innov), self.innov_model)
+                           c(self.innov), self.innov_model, c(self.gate_count))
 
     def to_reference_frame(self, acc_ref: torch.Tensor, mag_ref: torch.Tensor) -> "ReplayState":
         """Convert (in place) a state that `replay(..., keep_filter_frame=True)` left in the kernel's working
@@ -245,7 +247,8 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
            precise_state: bool | None = None, share_measurements: bool | None = None, wahba: str = "qr2",
            staging: str = "auto", keep_filter_frame: bool = False, allow_imprecise: bool = False,
            innovation: bool | torch.Tensor | None = None, innovation_model: str = "full",
-           lengths: torch.Tensor | None = None):
+           lengths: torch.Tensor | None = None, gate: float | None = None, gate_count: torch.Tensor | None = None,
+           out_gated: torch.Tensor | None = None):
     """Run T Prediction+Correction steps for N filters in one kernel launch.
 
     streams [T,9,Ns]; acc_ref, mag_ref [3,Ns]; dt: float seconds, [T] float32 CUDA tensor (one clock for every
@@ -286,9 +289,21 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     trajectory rows repeat its final state and its flip bytes are 0; the samples and dt of those steps are never used
     (they may be NaN).  For a time-chunked replay pass each chunk its own lengths (`logio.LogBatch.window`).
     A [T,Ns] dt or `lengths` runs the batched kernels (include/posekf.h, posekf_replay_batch_f32).
+    `gate`: innovation gating (include/posekf.h, posekf_replay_gated_f32) -- a step whose tangent-space normalised
+    innovation squared NIS3 exceeds `gate` is not corrected: the filter keeps its prediction and its propagated
+    covariance (an outlier measurement, e.g. a magnetic disturbance, is rejected).  NIS3 ~ chi^2_3 under a consistent
+    model: `GATE_CHI2_3_999` = 16.27 rejects one step in a thousand of a consistent filter.  float('inf') gives the
+    bits of the ungated replay.  The flip mask, the loss, the low-pass and the innovation sums still see every step.
+    `gate_count`: [N] int32 CUDA tensor incremented by each filter's number of gated steps (created zeroed when None;
+    pass `state.gate_count` back in for chunked replays); available as `state.gate_count`.  `out_gated`: a [T,N]
+    uint8 CUDA tensor that receives 1 where a step was gated (0 elsewhere and on held steps).  Both need `gate`.
     Returns (state, traj [T,N,4] or None, flips [T,N] uint8 or None)."""
     if innovation_model not in _lib.INNOV_MODEL:
         raise ValueError("innovation_model is 'full' or 'tangent'")
+    if gate is None and (gate_count is not None or out_gated is not None):
+        raise ValueError("gate_count / out_gated need gate=<threshold>")
+    if gate is not None and math.isnan(float(gate)):
+        raise ValueError("gate must be a number (NaN decides nothing)")
     _require_cuda(streams, acc_ref, mag_ref, out_traj)
     if streams.dim() != 3 or streams.shape[1] != 9:
         raise ValueError("streams must be [T, 9, Ns]")
@@ -328,11 +343,13 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     state.r = r
     if precise_state is None:
         if (isinstance(q, torch.Tensor) or isinstance(r, torch.Tensor)) and N > Ns and N % Ns == 0 \
-                and out_traj is None and not store_trajectory and not store_flips and not use_lpf and T > 0:
+                and out_traj is None and not store_trajectory and not store_flips and not use_lpf and T > 0 \
+                and out_gated is None:
             # a (Q,R) sweep: only the cells with r/q >= 100 or q/r >= 1e4 need the precise variant (+25 % time)
             mixed = _replay_sweep_mixed(streams, acc_ref, mag_ref, dt=dt, q=q, r=r, state=state, N=N, Ns=Ns, truth=truth,
                                         loss=loss, wahba=wahba, staging=staging, keep_filter_frame=keep_filter_frame,
-                                        innovation=innovation, innovation_model=innovation_model, lengths=lengths)
+                                        innovation=innovation, innovation_model=innovation_model, lengths=lengths,
+                                        gate=gate, gate_count=gate_count)
             if mixed is not None:
                 return mixed
         precise_state = state.x_lo is not None or needs_precise
@@ -376,6 +393,8 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
             loss = torch.zeros((N,), dtype=torch.float32, device=dev)
         state.loss = loss
     innov = _innovation_buffer(innovation, N, dev, state, innovation_model)
+    if gate is not None:
+        gate_count = _gate_buffers(gate_count, out_gated, N, T, dev)
     args = (N, T, _ptr(streams), Ns, _ptr(dt_t), per_step, _ptr(acc_ref), _ptr(mag_ref), _ptr(q_t), _ptr(r_t),
             -1.0 if lpf_alpha_acc is None else float(lpf_alpha_acc),
             -1.0 if lpf_alpha_mag is None else float(lpf_alpha_mag),
@@ -384,17 +403,22 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     tail = (_lib.WAHBA[wahba], _lib.STAGING[staging], frame_flags, _stream())
     batch = dt_cols is not None or lengths is not None
     with torch.cuda.device(dev):
-        if batch:
+        if gate is not None:
+            rc = _lib.load().posekf_replay_gated_f32(*args, _ptr(innov), _lib.INNOV_MODEL[innovation_model], *tail, _ptr(dt_cols),
+                                                     _ptr(lengths), float(gate), _ptr(gate_count), _ptr(out_gated))
+        elif batch:
             rc = _lib.load().posekf_replay_batch_f32(*args, _ptr(innov), _lib.INNOV_MODEL[innovation_model], *tail, _ptr(dt_cols),
                                                      _ptr(lengths))
         elif innov is None:
             rc = _lib.load().posekf_replay_f32(*args, *tail)
         else:
             rc = _lib.load().posekf_replay_innovation_ex_f32(*args, _ptr(innov), _lib.INNOV_MODEL[innovation_model], *tail)
-    _lib.check(rc, "posekf_replay_batch_f32" if batch else
+    _lib.check(rc, "posekf_replay_gated_f32" if gate is not None else "posekf_replay_batch_f32" if batch else
                ("posekf_replay_f32" if innov is None else "posekf_replay_innovation_ex_f32"))
     if innov is not None:
         state.innov, state.innov_model = innov, innovation_model
+    if gate is not None:
+        state.gate_count = gate_count
     if wahba != "precomputed":
         state.frame = "filter" if keep_filter_frame else "reference"
     return state, out_traj, flips
@@ -411,6 +435,25 @@ def _check_lengths(lengths, n_streams: int, n_steps: int) -> None:
             raise ValueError(f"lengths must lie in [0, {n_steps}] (the steps of this call), got [{lo}, {hi}]")
     if not lengths.is_cuda:
         raise _lib.PosekfError("poseestimationkf_b200 runs on CUDA tensors only (no CPU fallback)")
+
+
+# the 0.999 quantile of chi^2 with 3 degrees of freedom: a gate threshold that rejects one step in a thousand of a
+# consistent filter (replay(gate=...))
+GATE_CHI2_3_999 = 16.266236196238129
+
+
+def _gate_buffers(gate_count, out_gated, n: int, n_steps: int, device):
+    """replay(gate=...): checks out_gated [T,N] uint8 and returns the [N] int32 gate_count (zeros when None)."""
+    for t, shape, dtype, name in ((gate_count, (n,), torch.int32, "gate_count"), (out_gated, (n_steps, n), torch.uint8, "out_gated")):
+        if t is None:
+            continue
+        if not isinstance(t, torch.Tensor) or t.dtype != dtype or tuple(t.shape) != shape or not t.is_contiguous():
+            raise ValueError(f"{name} must be a contiguous {dtype} tensor of shape {shape}")
+        if not t.is_cuda:
+            raise _lib.PosekfError("poseestimationkf_b200 runs on CUDA tensors only (no CPU fallback)")
+    if gate_count is None:
+        gate_count = torch.zeros((n,), dtype=torch.int32, device=device)
+    return gate_count
 
 
 def _innovation_buffer(innovation, n: int, device, state=None, model: str = "full"):
@@ -468,7 +511,7 @@ def sweep_partition(q_t: torch.Tensor, r_t: torch.Tensor, n_streams: int):
 
 
 def _replay_sweep_mixed(streams, acc_ref, mag_ref, *, dt, q, r, state, N, Ns, truth, loss, wahba, staging, keep_filter_frame,
-                        innovation=None, innovation_model="full", lengths=None):
+                        innovation=None, innovation_model="full", lengths=None, gate=None, gate_count=None):
     """Sweep layout with automatic precision: the cells (blocks of Ns filters sharing one (q, r)) whose tuning is
     extreme run the precise variant, the others the plain one -- two launches over a cell permutation that keeps
     every filter on its own stream column (n % Ns).  Returns None when one launch serves all cells."""
@@ -481,19 +524,22 @@ def _replay_sweep_mixed(streams, acc_ref, mag_ref, *, dt, q, r, state, N, Ns, tr
     if truth is not None and loss is None:
         loss = torch.zeros((N,), dtype=torch.float32, device=dev)
     innov = _innovation_buffer(innovation, N, dev, state, innovation_model)
+    if gate is not None:
+        gate_count = _gate_buffers(gate_count, None, N, streams.shape[0], dev)
     for idx, precise in ((idx_plain, False), (idx_precise, True)):
         sub = ReplayState(state.x[:, idx].contiguous(), state.p[:, idx].contiguous(), r_t[idx].contiguous(), None, None,
                           state.x_lo[:, idx].contiguous() if (precise and state.x_lo is not None) else None, state.frame)
         sub_loss = loss[idx].contiguous() if truth is not None else None
         sub_innov = innov[:, idx].contiguous() if innov is not None else None
+        sub_gc = gate_count[idx].contiguous() if gate is not None else None
         replay(streams, acc_ref, mag_ref, dt=dt, q=q_t[idx].contiguous(), r=sub.r, state=sub, n_filters=idx.numel(), truth=truth,
                loss=sub_loss, precise_state=precise, share_measurements=False, wahba=wahba, staging=staging,
                keep_filter_frame=keep_filter_frame, innovation=sub_innov, innovation_model=innovation_model,
-               lengths=lengths)   # (the plain group holds no extreme cell by construction)
-        parts.append((idx, sub, sub_loss, sub_innov, precise))
+               lengths=lengths, gate=gate, gate_count=sub_gc)   # (the plain group holds no extreme cell by construction)
+        parts.append((idx, sub, sub_loss, sub_innov, precise, sub_gc))
     if state.x_lo is None:
         state.x_lo = torch.zeros((4, N), dtype=torch.float32, device=dev)
-    for idx, sub, sub_loss, sub_innov, precise in parts:
+    for idx, sub, sub_loss, sub_innov, precise, sub_gc in parts:
         state.x[:, idx] = sub.x
         state.p[:, idx] = sub.p
         if precise:
@@ -502,11 +548,15 @@ def _replay_sweep_mixed(streams, acc_ref, mag_ref, *, dt, q, r, state, N, Ns, tr
             loss[idx] = sub_loss
         if innov is not None:
             innov[:, idx] = sub_innov
+        if gate is not None:
+            gate_count[idx] = sub_gc
         state.frame = sub.frame
     if truth is not None:
         state.loss = loss
     if innov is not None:
         state.innov, state.innov_model = innov, innovation_model
+    if gate is not None:
+        state.gate_count = gate_count
     state.r = r
     return state, None, None
 

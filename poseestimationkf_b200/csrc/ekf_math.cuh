@@ -550,6 +550,49 @@ PKF_HD void innov_accumulate(InnovAcc<F>& acc, const InnovFactors<F>& f, const S
   }
 }
 
+// ------------------------------------------------------------------------------------------
+// Innovation gate (GATE): a step whose tangent-space NIS is implausible under the filter's own model is not corrected.
+//     gated  <=>  NIS_3 = (s - b^2/c) / r  >  gamma,   evaluated as  s - b^2/c > gamma r   (r > 0; strict: a NaN
+//                                                                                       statistic is never gated)
+// with s, b, c of innov_accumulate (TAN), formed here with the same operations, so the decision is the same whichever
+// model a launch accumulates and needs no logarithm (gamma r is one launch constant per filter: two registers fewer than
+// 1/r and gamma in the packed kernel).  On a gated step the innovation is zeroed per lane
+// (X = z + K 0 = z, then normalised: the prediction) and the covariance becomes the propagated P^- instead of K; the
+// innovation sums, the flip byte and the loss still see the step.  Under a consistent model NIS_3 ~ chi^2_3.
+// ------------------------------------------------------------------------------------------
+template <typename F> struct GateParams {
+  F thr;       // gamma r: the threshold on r NIS_3 (+inf: never gated)
+};
+template <typename F> PKF_HD GateParams<F> make_gate_params(F r, float gamma) {
+  GateParams<F> g;
+  g.thr = F(gamma) * r;
+  return g;
+}
+// r NIS_3 = s - b^2/c (the covariance in units of r)
+template <typename F, bool COMP>
+PKF_HD F tangent_nis_r(const InnovFactors<F>& f, const Quat<F>& z, F e0, F e1, F e2, F e3) {
+  const F t1 = fma_(f.n10, e0, e1);
+  const F t2 = fma_(f.n21, e1, fma_(f.n20, e0, e2));
+  const F t3 = fma_(f.n32, e2, fma_(f.n31, e1, fma_(f.n30, e0, e3)));
+  const F u0 = f.i0 * e0, u1 = f.i1 * t1, u2 = f.i2 * t2, u3 = f.i3 * t3;
+  F s = fma_(u3, t3, fma_(u2, t2, fma_(u1, t1, u0 * e0)));
+  const F v1 = fma_(f.n10, z.w, z.x);
+  const F v2 = fma_(f.n21, z.x, fma_(f.n20, z.w, z.y));
+  const F v3 = fma_(f.n32, z.y, fma_(f.n31, z.x, fma_(f.n30, z.w, z.z)));
+  const F g0 = f.i0 * z.w, g1 = f.i1 * v1, g2 = f.i2 * v2, g3 = f.i3 * v3;
+  F c = fma_(g3, v3, fma_(g2, v2, fma_(g1, v1, g0 * z.w)));
+  F b = fma_(g3, t3, fma_(g2, t2, fma_(g1, t1, g0 * e0)));
+  if constexpr (COMP) {
+    const F we = fma_(f.w3, e3, fma_(f.w2, e2, fma_(f.w1, e1, f.w0 * e0)));
+    s = fma_(f.beta * we, we, s);
+    const F wz = fma_(f.w3, z.z, fma_(f.w2, z.y, fma_(f.w1, z.x, f.w0 * z.w)));
+    const F bwz = f.beta * wz;
+    c = fma_(bwz, wz, c);
+    b = fma_(bwz, we, b);
+  }
+  return fma_(-b, b * rcp_(c), s);
+}
+
 template <typename F> PKF_HD Ldl4<F> ldl_unit(const Sym4<F>& P) {
   // P is the predicted covariance IN UNITS OF r (P/r), so S = P + I and rho_k = 1/d_k.
   const F p01 = P.a01, p02 = P.a02, p03 = P.a03, p12 = P.a12, p13 = P.a13, p23 = P.a23;
@@ -602,7 +645,8 @@ template <typename F> PKF_HD Sym4<F> kalman_gain_unit(const Sym4<F>& P) { return
 // kappa_k = 1 - 1/d_k.  Four additions fewer than the split-pivot form; kappa loses eps/kappa of relative accuracy,
 // i.e. 2.4e-5 at the edge of the plain variant's range (r/q = 100, kappa = 2.5e-3), which moves the state by 1e-9 --
 // beyond that range the precise variant (split pivots, kalman_gain_sm) is selected.
-template <typename F, bool INNOV = false>
+// FAC hands the factors to `fac`; LOGDET adds ln det S~ (the innovation gate reads the factors only).
+template <typename F, bool FAC = false, bool LOGDET = FAC>
 PKF_HD Sym4<F> kalman_gain_from_s(const Sym4<F>& S, InnovFactors<F>* fac = nullptr) {
   const F p01 = S.a01, p02 = S.a02, p03 = S.a03, p12 = S.a12, p13 = S.a13, p23 = S.a23;
   const F i0 = rcp_(S.a00);
@@ -623,10 +667,10 @@ PKF_HD Sym4<F> kalman_gain_from_s(const Sym4<F>& S, InnovFactors<F>* fac = nullp
   const F n20 = fma_(-l21, n10, -l20);
   const F n31 = fma_(-l32, n21, -l31);
   const F n30 = fma_(-l32, n20, fma_(-l31, n10, -l30));
-  if constexpr (INNOV) {     // the pivots d_k of S~ = P~ + I are >= 1: their excesses d_k - 1 are exact differences
+  if constexpr (FAC) {       // the pivots d_k of S~ = P~ + I are >= 1: their excesses d_k - 1 are exact differences
     fac->n10 = n10; fac->n20 = n20; fac->n21 = n21; fac->n30 = n30; fac->n31 = n31; fac->n32 = n32;
     fac->i0 = i0; fac->i1 = i1; fac->i2 = i2; fac->i3 = i3;
-    fac->logdet = log_pivots(S.a00 - F(1), d1 - F(1), d2 - F(1), d3 - F(1));
+    if constexpr (LOGDET) fac->logdet = log_pivots(S.a00 - F(1), d1 - F(1), d2 - F(1), d3 - F(1));
   }
   const F v30 = -(i3 * n30), v31 = -(i3 * n31), v32 = -(i3 * n32);
   const F v20 = -(i2 * n20), v21 = -(i2 * n21);
@@ -654,7 +698,7 @@ PKF_HD Sym4<F> kalman_gain_from_s(const Sym4<F>& S, InnovFactors<F>* fac = nullp
 //   den = 1 - g x^T w = x^T (I + M) w / |x|^2   (from (I + M) w + g|x|^2 w = x; no cancellation;
 //         w itself comes from the LDL^T factors of H, not from x - K_H x),
 //   K = I - S^-1 = K_H - beta w w^T,  K_H = I - H^-1 (split-pivot form above),  beta = g|x|^2 / x^T(I+M)w.
-template <typename F, bool INNOV = false>
+template <typename F, bool FAC = false, bool LOGDET = FAC>
 PKF_HD Sym4<F> kalman_gain_sm(const Sym4<F>& M, const Quat<F>& x, F g, InnovFactors<F>* fac = nullptr) {
   const F x2 = dot4(x, x);
   const F c = g * x2;
@@ -679,15 +723,17 @@ PKF_HD Sym4<F> kalman_gain_sm(const Sym4<F>& M, const Quat<F>& x, F g, InnovFact
   F g3 = fma_(M.a33, w3, fma_(M.a23, w2, fma_(M.a13, w1, fma_(M.a03, w0, w3))));
   F num = fma_(x.z, g3, fma_(x.y, g2, fma_(x.x, g1, x.w * g0)));
   F nb = -(c * rcp_(num));                     // -beta
-  if constexpr (INNOV) {
+  if constexpr (FAC) {
     fac->n10 = f.n10; fac->n20 = f.n20; fac->n21 = f.n21; fac->n30 = f.n30; fac->n31 = f.n31; fac->n32 = f.n32;
     fac->i0 = f.i0; fac->i1 = f.i1; fac->i2 = f.i2; fac->i3 = f.i3;
     fac->w0 = w0; fac->w1 = w1; fac->w2 = w2; fac->w3 = w3; fac->beta = -nb;
-    // ln(num/|x|^2) = ln(1 - g x.w): through log1p while g x.w is small (R >> Q: the term is ~ -g and the quotient
-    // would round it away), through the quotient itself when it is small (Q >> R: 1 - g x.w would cancel)
-    const F u = g * fma_(x.z, w3, fma_(x.y, w2, fma_(x.x, w1, x.w * w0)));
-    const F lden = sel_(u < F(0.5), log1p_(-u), log_(num * rcp_(x2)));
-    fac->logdet = log_pivots(f.e0, f.e1, f.e2, f.e3) + lden;
+    if constexpr (LOGDET) {
+      // ln(num/|x|^2) = ln(1 - g x.w): through log1p while g x.w is small (R >> Q: the term is ~ -g and the quotient
+      // would round it away), through the quotient itself when it is small (Q >> R: 1 - g x.w would cancel)
+      const F u = g * fma_(x.z, w3, fma_(x.y, w2, fma_(x.x, w1, x.w * w0)));
+      const F lden = sel_(u < F(0.5), log1p_(-u), log_(num * rcp_(x2)));
+      fac->logdet = log_pivots(f.e0, f.e1, f.e2, f.e3) + lden;
+    }
   }
   F b0 = nb * w0, b1 = nb * w1, b2 = nb * w2, b3 = nb * w3;
   Sym4<F> K;
@@ -1196,23 +1242,35 @@ PKF_HD void quat_fallback_unaligned(const Mat3<f32x2>& Rm, const Quat<f32x2>& z,
 // Prediction (PKF/ExtendedKalmanFilter.py:58-68): gain K (= the post-update covariance in units of r), RK4
 // increment inc and predicted state z = x + inc.
 // INNOV: the gain stage also hands its factors of S~ to `fac` (innovation likelihood, see InnovFactors).
-template <typename F, bool COMP, bool INNOV = false>
+// GATE: the factors go to `fac` for the gate statistic as well, and the propagated covariance P^- (units of r) to *Pm.
+template <typename F, bool COMP, bool INNOV = false, bool GATE = false>
 PKF_HD void ekf_predict(const Quat<F>& x, const Sym4<F>& P, const FilterConst<F>& fc, const Vec3<F>& gyro, const StepH<F>& h,
-                        Sym4<F>& K, Quat<F>& inc, Quat<F>& z, InnovFactors<F>* fac = nullptr) {
+                        Sym4<F>& K, Quat<F>& inc, Quat<F>& z, InnovFactors<F>* fac = nullptr, Sym4<F>* Pm = nullptr) {
   Vec3<F> hw;
   hw.x = F(0.5) * gyro.x; hw.y = F(0.5) * gyro.y; hw.z = F(0.5) * gyro.z;
   if constexpr (COMP) {
     Sym4<F> M = propagate_cov<F, false>(P, hw, x, fc.g, fc.gs);               // :59-61, noise kept apart
-    K = kalman_gain_sm<F, INNOV>(M, x, fc.gs, fac);                           // :63-66
+    K = kalman_gain_sm<F, INNOV || GATE, INNOV>(M, x, fc.gs, fac);            // :63-66
+    if constexpr (GATE) {     // P^- = M + gs (|x|^2 I - x x^T), the diagonal formed as kalman_gain_sm forms H's
+      const F x2 = dot4(x, x);
+      const F yw = fc.gs * x.w, yx = fc.gs * x.x, yy = fc.gs * x.y, yz = fc.gs * x.z;
+      Pm->a00 = fma_(-yw, x.w, fma_(fc.gs, x2, M.a00)); Pm->a11 = fma_(-yx, x.x, fma_(fc.gs, x2, M.a11));
+      Pm->a22 = fma_(-yy, x.y, fma_(fc.gs, x2, M.a22)); Pm->a33 = fma_(-yz, x.z, fma_(fc.gs, x2, M.a33));
+      Pm->a01 = fma_(-yw, x.x, M.a01); Pm->a02 = fma_(-yw, x.y, M.a02); Pm->a03 = fma_(-yw, x.z, M.a03);
+      Pm->a12 = fma_(-yx, x.y, M.a12); Pm->a13 = fma_(-yx, x.z, M.a13); Pm->a23 = fma_(-yy, x.z, M.a23);
+    }
   } else {
 #if PKF_FUSE
     Sym4<F> S = propagate_cov<F, true>(P, hw, x, fc.g, fc.gs, fc.gs1);        // :59-61 and S = P + R :63 (in units of r)
-    K = kalman_gain_from_s<F, INNOV>(S, fac);                                 // :64-66
+    K = kalman_gain_from_s<F, INNOV || GATE, INNOV>(S, fac);                  // :64-66
+    // GATE: P^- itself, its diagonal constant gs instead of gs + 1 (S - I would round P^-'s diagonal at ulp(1): 9 bits
+    // of a 2.5e-3 entry); the off-diagonal entries are S's, shared with it
+    if constexpr (GATE) *Pm = propagate_cov<F, true>(P, hw, x, fc.g, fc.gs, fc.gs);
     z = rk4_predict_fused(x, hw, h);                                          // :62
     inc = z;                                                                  // (unused by the plain update)
     return;
 #else
-    static_assert(!INNOV, "the innovation statistic takes its factors from the fused plain gain (PKF_FUSE)");
+    static_assert(!INNOV && !GATE, "the innovation statistic takes its factors from the fused plain gain (PKF_FUSE)");
     Sym4<F> Pp = propagate_cov<F, true>(P, hw, x, fc.g, fc.gs);               // :59-61 (in units of r)
     K = kalman_gain_unit(Pp);                                                 // :63-66
 #endif
@@ -1293,54 +1351,73 @@ PKF_HD Quat<F> measure_quat(const FilterConst<F>& fc, const Vec3<F>& acc, const 
   return y;
 }
 
+// GATE (see GateParams): the step's gate decision goes to *gated; a gated lane keeps its prediction and P^-.
+template <typename F, bool COMP, typename FlagT>
+PKF_HD void gate_apply(const GateParams<F>& gp, const InnovFactors<F>& fac, const Quat<F>& z, const Sym4<F>& Pm, Sym4<F>& K,
+                       F& e0, F& e1, F& e2, F& e3, FlagT& gated) {
+  const auto g = tangent_nis_r<F, COMP>(fac, z, e0, e1, e2, e3) > gp.thr;
+  gated = g;
+  e0 = sel_(g, F(0), e0); e1 = sel_(g, F(0), e1); e2 = sel_(g, F(0), e2); e3 = sel_(g, F(0), e3);
+  K.a00 = sel_(g, Pm.a00, K.a00); K.a01 = sel_(g, Pm.a01, K.a01); K.a02 = sel_(g, Pm.a02, K.a02); K.a03 = sel_(g, Pm.a03, K.a03);
+  K.a11 = sel_(g, Pm.a11, K.a11); K.a12 = sel_(g, Pm.a12, K.a12); K.a13 = sel_(g, Pm.a13, K.a13);
+  K.a22 = sel_(g, Pm.a22, K.a22); K.a23 = sel_(g, Pm.a23, K.a23); K.a33 = sel_(g, Pm.a33, K.a33);
+}
+
 // Prediction + Correction with the measurement quaternion y (filter frame, any sign, norm 1/inv_norm) already computed.
 // INNOV: the innovation likelihood of the step is added to *innov (see InnovAcc); the filter itself is unchanged.
-// TAN: its tangent-space form (see innov_accumulate).
-template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, typename FlagT>
+// TAN: its tangent-space form (see innov_accumulate).  GATE: the innovation gate (see GateParams), decision in *gated.
+template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, bool GATE = false, typename FlagT>
 PKF_HD void ekf_step_measured(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, const Vec3<F>& gyro,
                               const Quat<F>& y, F inv_norm, const StepH<F>& h, FlagT& flip, bool flip_wanted = true,
-                              typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr) {
-  Sym4<F> K;
+                              typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr,
+                              const GateParams<F>* gate = nullptr, FlagT* gated = nullptr) {
+  Sym4<F> K, Pm;
   Quat<F> inc, z;
   InnovFactors<F> fac;
-  ekf_predict<F, COMP, INNOV>(x, P, fc, gyro, h, K, inc, z, &fac);
+  ekf_predict<F, COMP, INNOV, GATE>(x, P, fc, gyro, h, K, inc, z, &fac, &Pm);
   const F dyz = dot4(y, z);                       // the comparator, literally: negate when dot(y, z) < 0  :73-75
   flip = FlagT();
   if (WANT_FLIP && flip_wanted) flip = reference_flip_quat(fc, y, one_with_sign_(dyz), code);
   const F sn = copysign_(inv_norm, dyz);          // e = sg y/|y| - z, sg = sign(dot): the sign bit moves onto 1/|y| > 0  :76
-  const F e0 = fma_(sn, y.w, -z.w), e1 = fma_(sn, y.x, -z.x), e2 = fma_(sn, y.y, -z.y), e3 = fma_(sn, y.z, -z.z);
+  F e0 = fma_(sn, y.w, -z.w), e1 = fma_(sn, y.x, -z.x), e2 = fma_(sn, y.y, -z.y), e3 = fma_(sn, y.z, -z.z);
   if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3);
+  if constexpr (GATE) gate_apply<F, COMP>(*gate, fac, z, Pm, K, e0, e1, e2, e3, *gated);
   ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);
 }
 
 // The common case of ekf_step<WAHBA_QR2>: both Wahba weights are non-negative (|a_z| <= 1, i.e. a normalised
 // accelerometer), so the closed-form measurement applies and the step has no data-dependent branch.  The caller
 // guarantees the precondition (the packed kernel checks a whole tile of samples before taking this path).
-template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, typename FlagT>
+template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, bool GATE = false, typename FlagT>
 PKF_HD void ekf_step_plain_measured(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, const Vec3<F>& gyro,
                                     const Vec3<F>& acc, const Vec3<F>& mag, const StepH<F>& h, FlagT& flip, bool flip_wanted = true,
-                                    typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr) {
+                                    typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr,
+                                    const GateParams<F>* gate = nullptr, FlagT* gated = nullptr) {
   const F ka = abs_(acc.z), km = F(1) - ka;
   F inv_norm;
   const Quat<F> y = wahba_quat2_local(fc.E, acc, mag, ka, km, inv_norm);
-  ekf_step_measured<F, WANT_FLIP, COMP, INNOV, TAN>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code, innov);
+  ekf_step_measured<F, WANT_FLIP, COMP, INNOV, TAN, GATE>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code, innov,
+                                                          gate, gated);
 }
 
-template <typename F, int ALGO, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, typename FlagT>
+template <typename F, int ALGO, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, bool GATE = false,
+          typename FlagT>
 PKF_HD void ekf_step(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, const Vec3<F>& gyro,
                      const Vec3<F>& acc, const Vec3<F>& mag, const StepH<F>& h, FlagT& flip, bool flip_wanted = true,
-                     typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr) {
+                     typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr,
+                     const GateParams<F>* gate = nullptr, FlagT* gated = nullptr) {
   // flip_wanted: launch-uniform run-time switch under WANT_FLIP -- a launch that stores the trajectory but
   // not the flip mask skips the reference's branch rule altogether
   if constexpr (ALGO == WAHBA_QR2) {
     F inv_norm;
     const Quat<F> y = measure_quat(fc, acc, mag, inv_norm);
-    ekf_step_measured<F, WANT_FLIP, COMP, INNOV, TAN>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code, innov);
+    ekf_step_measured<F, WANT_FLIP, COMP, INNOV, TAN, GATE>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code, innov,
+                                                            gate, gated);
   } else {
-    Sym4<F> K;
+    Sym4<F> K, Pm;
     Quat<F> inc, z;
     InnovFactors<F> fac;
-    ekf_predict<F, COMP, INNOV>(x, P, fc, gyro, h, K, inc, z, &fac);
+    ekf_predict<F, COMP, INNOV, GATE>(x, P, fc, gyro, h, K, inc, z, &fac, &Pm);
     // ---- Correction (PKF/ExtendedKalmanFilter.py:70-80) ----
     F e0, e1, e2, e3;
     if constexpr (ALGO == WAHBA_PRECOMPUTED) {
@@ -1375,6 +1452,7 @@ PKF_HD void ekf_step(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, c
       }
     }
     if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3);
+    if constexpr (GATE) gate_apply<F, COMP>(*gate, fac, z, Pm, K, e0, e1, e2, e3, *gated);
     ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);
   }
 }

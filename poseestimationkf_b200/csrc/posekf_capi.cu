@@ -91,19 +91,21 @@ bool tma_eligible(const ReplayParams& p) {
   return true;
 }
 
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false>
-int launch_replay(const ReplayParams& p, bool use_tma, cudaStream_t st) {
+// ga: the gate's arguments (one GateArgs; GATE launches only, the others pass none)
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false, bool GATE = false,
+          typename... GA>
+int launch_replay(const ReplayParams& p, bool use_tma, cudaStream_t st, const GA&... ga) {
   const unsigned grid = (unsigned)((p.N + kThreads - 1) / kThreads);
   if (!use_tma) {
-    replay_ldg_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH><<<grid, kThreads, 0, st>>>(p);
+    replay_ldg_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH, GATE, GA...><<<grid, kThreads, 0, st>>>(p, ga...);
     return launch_status();
   }
   CUtensorMap tmap;
   if (int rc = encode_stream_map(p, kThreads, kTmaSteps, &tmap)) return rc;
-  auto kern = replay_tma_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH>;
+  auto kern = replay_tma_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH, GATE, GA...>;
   // idempotent; set on every launch (cheap) so that it holds on every device of a multi-GPU process
   PKF_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TmaSmem)));
-  kern<<<grid, kThreads, sizeof(TmaSmem), st>>>(p, tmap);
+  kern<<<grid, kThreads, sizeof(TmaSmem), st>>>(p, tmap, ga...);
   return launch_status();
 }
 
@@ -118,15 +120,16 @@ bool packed_eligible(const ReplayParams& p) {
   return true;      // out_traj / truth are already required to be 16-byte aligned
 }
 
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false>
-int launch_replay_packed(const ReplayParams& p, cudaStream_t st) {
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false, bool GATE = false,
+          typename... GA>
+int launch_replay_packed(const ReplayParams& p, cudaStream_t st, const GA&... ga) {
   CUtensorMap tmap;
   if (int rc = encode_stream_map(p, kTile2, kTma2Steps, &tmap)) return rc;
-  auto kern = replay_tma2_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH>;
+  auto kern = replay_tma2_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH, GATE, GA...>;
   const int smem = (int)sizeof(Tma2Smem) + (BATCH ? (int)kBatchSmem2 : 0);
   PKF_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   const unsigned grid = (unsigned)((p.N + kTile2 - 1) / kTile2);
-  kern<<<grid, kThreads2, smem, st>>>(p, tmap);
+  kern<<<grid, kThreads2, smem, st>>>(p, tmap, ga...);
   return launch_status();
 }
 
@@ -198,8 +201,59 @@ int launch_kernels(const ReplayParams& p, int algo, bool lpf, bool use_tma, bool
   return POSEKF_EINVAL;
 }
 
-// innov_model: POSEKF_INNOV_* of the sums in p.innov_acc (read only when it is set).
-int replay_dispatch(const ReplayParams& p, int algo, int staging, int innov_model, cudaStream_t st) {
+// Launches with the innovation gate.  The scalar gated kernels are the BATCH kernels, which step exactly as the others
+// when dt_cols and n_valid are null (bit for bit, see launch_kernels), so the gate adds one set of them, not two; they
+// always have AUX (their per-step outputs are checked per pointer).  The packed kernel carries the plain variant with
+// and without per-step outputs and the precise variant without them, all without low-pass and innovation sums (a
+// trajectory replay and the (Q,R) sweep); with per-stream dt or lengths only the plain variant without per-step
+// outputs, because the copies a held lane needs push the others past the 168 registers of 3 CTAs per SM.  Every other
+// combination runs in the scalar kernels on the same staging (the TMA kernel for a packed staging), whose results are
+// the same bit for bit.
+template <int ALGO, bool TAN>
+int launch_gated_innovation(const ReplayParams& p, const GateArgs& ga, bool lpf, bool use_tma, cudaStream_t st) {
+  const bool comp = p.state_x_lo != nullptr;
+  if constexpr (ALGO != WAHBA_PRECOMPUTED) {
+    if (lpf) return comp ? launch_replay<ALGO, true, true, true, true, TAN, true, true>(p, use_tma, st, ga) : launch_replay<ALGO, true, true, false, true, TAN, true, true>(p, use_tma, st, ga);
+  }
+  return comp ? launch_replay<ALGO, false, true, true, true, TAN, true, true>(p, use_tma, st, ga) : launch_replay<ALGO, false, true, false, true, TAN, true, true>(p, use_tma, st, ga);
+}
+
+template <int ALGO>
+int launch_gated(const ReplayParams& p, const GateArgs& ga, bool lpf, bool use_tma, bool packed, int innov_model, cudaStream_t st) {
+  const bool comp = p.state_x_lo != nullptr;
+  const bool aux = p.out_traj != nullptr || p.out_flip != nullptr || p.truth != nullptr || ga.out_gated != nullptr;
+  if (p.innov_acc) return innov_model == POSEKF_INNOV_TANGENT ? launch_gated_innovation<ALGO, true>(p, ga, lpf, use_tma, st)
+                                                              : launch_gated_innovation<ALGO, false>(p, ga, lpf, use_tma, st);
+  // (the packed kernel reads gate_count as int2 and stores out_gated as uchar2)
+  packed = packed && (reinterpret_cast<uintptr_t>(ga.gate_count) & 7) == 0 && (reinterpret_cast<uintptr_t>(ga.out_gated) & 1) == 0;
+  if constexpr (ALGO != WAHBA_JACOBI) {
+    const bool batch = p.dt_cols != nullptr || p.n_valid != nullptr;
+    if (packed && !lpf && !comp && !aux) {
+      return batch ? launch_replay_packed<ALGO, false, false, false, false, false, true, true>(p, st, ga)
+                   : launch_replay_packed<ALGO, false, false, false, false, false, false, true>(p, st, ga);
+    }
+    if (packed && !lpf && !batch && !(comp && aux)) {
+      return comp ? launch_replay_packed<ALGO, false, false, true, false, false, false, true>(p, st, ga)
+                  : launch_replay_packed<ALGO, false, true, false, false, false, false, true>(p, st, ga);
+    }
+  }
+  if constexpr (ALGO != WAHBA_PRECOMPUTED) {
+    if (lpf) return comp ? launch_replay<ALGO, true, true, true, false, false, true, true>(p, use_tma, st, ga) : launch_replay<ALGO, true, true, false, false, false, true, true>(p, use_tma, st, ga);
+  }
+  return comp ? launch_replay<ALGO, false, true, true, false, false, true, true>(p, use_tma, st, ga) : launch_replay<ALGO, false, true, false, false, false, true, true>(p, use_tma, st, ga);
+}
+
+int launch_gated_algo(const ReplayParams& p, const GateArgs& ga, int algo, bool lpf, bool use_tma, bool packed, int innov_model,
+                      cudaStream_t st) {
+  if (algo == POSEKF_WAHBA_QR2) return launch_gated<WAHBA_QR2>(p, ga, lpf, use_tma, packed, innov_model, st);
+  if (algo == POSEKF_WAHBA_PRECOMPUTED) return launch_gated<WAHBA_PRECOMPUTED>(p, ga, lpf, use_tma, packed, innov_model, st);
+  if (algo == POSEKF_WAHBA_JACOBI) return launch_gated<WAHBA_JACOBI>(p, ga, lpf, use_tma, packed, innov_model, st);
+  return POSEKF_EINVAL;
+}
+
+// innov_model: POSEKF_INNOV_* of the sums in p.innov_acc (read only when it is set).  gate: run the gated kernels with
+// these arguments (null: the ungated ones).
+int replay_dispatch(const ReplayParams& p, int algo, int staging, int innov_model, cudaStream_t st, const GateArgs* gate = nullptr) {
   const bool lpf = (p.alpha_acc >= 0.f) || (p.alpha_mag >= 0.f);
   bool use_tma, packed = false;
   if (staging == POSEKF_STAGE_LDG) use_tma = false;
@@ -212,8 +266,9 @@ int replay_dispatch(const ReplayParams& p, int algo, int staging, int innov_mode
     packed = use_tma && kAutoPrefersPacked && algo != POSEKF_WAHBA_JACOBI && packed_eligible(p);
   } else return POSEKF_EINVAL;
   const bool batch = p.dt_cols != nullptr || p.n_valid != nullptr;
-  int rc = batch ? launch_kernels<true>(p, algo, lpf, use_tma, packed, innov_model, st)
-                 : launch_kernels<false>(p, algo, lpf, use_tma, packed, innov_model, st);
+  int rc = gate ? launch_gated_algo(p, *gate, algo, lpf, use_tma, packed, innov_model, st)
+                : batch ? launch_kernels<true>(p, algo, lpf, use_tma, packed, innov_model, st)
+                        : launch_kernels<false>(p, algo, lpf, use_tma, packed, innov_model, st);
   // (held steps of a batched launch carry flip byte 0, which the fix-up leaves alone)
   if (rc == 0 && p.out_flip && p.T > 0 && algo == POSEKF_WAHBA_QR2 && !lpf) {
     // the flip-mask bytes the kernel marked as float32 ties of the reference's sign rule are settled in float64
@@ -249,15 +304,16 @@ const char* posekf_version(void) { return "posekf_b200 0.2 sm_100a"; }
 }  // extern "C"
 
 namespace {
-// Validation and dispatch shared by posekf_replay_f32, posekf_replay_innovation(_ex)_f32 and posekf_replay_batch_f32
-// (innov_acc null: the first; dt_cols and n_valid null: all but the last).
+// Validation and dispatch shared by posekf_replay_f32, posekf_replay_innovation(_ex)_f32, posekf_replay_batch_f32 and
+// posekf_replay_gated_f32 (innov_acc null: the first; dt_cols and n_valid null: the first three; gate: the last).
 // innov_model: POSEKF_INNOV_FULL or POSEKF_INNOV_TANGENT (checked by the caller).
 int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
                  int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_scale,
                  const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag, float* state_x, float* state_x_lo,
                  float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth, float* loss_acc,
                  float* innov_acc, int innov_model, int wahba_algo, int staging, int state_flags, void* stream,
-                 const float* dt_cols = nullptr, const int32_t* n_valid = nullptr) {
+                 const float* dt_cols = nullptr, const int32_t* n_valid = nullptr, bool gate = false, float gate_nis3 = 0.f,
+                 int32_t* gate_count = nullptr, uint8_t* out_gated = nullptr) {
   if (dt_cols && !dt) { dt = dt_cols; dt_per_step = 0; }    // (the kernels read dt[0] unconditionally; it is unused then)
   if (n_filters < 0 || n_steps < 0 || n_streams <= 0 && n_filters > 0) return POSEKF_EINVAL;
   if (state_flags & ~(POSEKF_STATE_IN_FILTER_FRAME | POSEKF_STATE_OUT_FILTER_FRAME)) return POSEKF_EINVAL;
@@ -281,6 +337,7 @@ int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64
   if (truth && (!loss_acc || (reinterpret_cast<uintptr_t>(truth) & 15) != 0)) return truth && !loss_acc ? POSEKF_EINVAL : POSEKF_EALIGN;
   if ((reinterpret_cast<uintptr_t>(innov_acc) & 3) != 0) return POSEKF_EALIGN;
   if ((reinterpret_cast<uintptr_t>(dt_cols) & 3) != 0 || (reinterpret_cast<uintptr_t>(n_valid) & 3) != 0) return POSEKF_EALIGN;
+  if ((reinterpret_cast<uintptr_t>(gate_count) & 3) != 0) return POSEKF_EALIGN;
   ReplayParams p;
   p.N = n_filters; p.T = n_steps; p.Ns = n_streams; p.streams = streams; p.dt = dt; p.dt_per_step = dt_per_step;
   p.acc_ref = acc_ref; p.mag_ref = mag_ref; p.q_scale = q_scale; p.r_scale = r_scale;
@@ -291,7 +348,8 @@ int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64
   p.state_flags = state_flags;
   p.dt_cols = n_steps > 0 ? dt_cols : nullptr;
   p.n_valid = n_steps > 0 ? n_valid : nullptr;
-  return replay_dispatch(p, wahba_algo, staging, innov_model, (cudaStream_t)stream);
+  const GateArgs ga{gate_nis3, gate_count, out_gated};
+  return replay_dispatch(p, wahba_algo, staging, innov_model, (cudaStream_t)stream, gate && n_steps > 0 ? &ga : nullptr);
 }
 }  // namespace
 
@@ -341,6 +399,21 @@ int posekf_replay_batch_f32(int64_t n_filters, int64_t n_steps, const float* str
   return replay_entry(n_filters, n_steps, streams, n_streams, dt, dt_per_step, acc_ref, mag_ref, q_scale, r_scale, lpf_alpha_acc,
                       lpf_alpha_mag, state_x, state_x_lo, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, innov_acc,
                       innov_model, wahba_algo, staging, state_flags, stream, dt_cols, n_valid);
+}
+
+int posekf_replay_gated_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
+                            int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_scale,
+                            const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag, float* state_x, float* state_x_lo,
+                            float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth,
+                            float* loss_acc, float* innov_acc, int innov_model, int wahba_algo, int staging, int state_flags,
+                            void* stream, const float* dt_cols, const int32_t* n_valid, float gate_nis3, int32_t* gate_count,
+                            uint8_t* out_gated) {
+  if (innov_model != POSEKF_INNOV_FULL && innov_model != POSEKF_INNOV_TANGENT) return POSEKF_EINVAL;
+  if (gate_nis3 != gate_nis3) return POSEKF_EINVAL;      // NaN: no decision could ever be made with it
+  return replay_entry(n_filters, n_steps, streams, n_streams, dt, dt_per_step, acc_ref, mag_ref, q_scale, r_scale, lpf_alpha_acc,
+                      lpf_alpha_mag, state_x, state_x_lo, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, innov_acc,
+                      innov_model, wahba_algo, staging, state_flags, stream, dt_cols, n_valid, true, gate_nis3, gate_count,
+                      out_gated);
 }
 
 // ---- host-buffer replay: workspace (device staging buffers, streams, events) ----------------------

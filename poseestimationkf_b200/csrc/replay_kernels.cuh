@@ -46,6 +46,28 @@ struct FilterRegs {
   InnovAcc<float> in;   // innovation likelihood sums (INNOV kernels only)
 };
 
+// The innovation gate's arguments.  They are the last kernel parameter of the GATE kernels only (a parameter pack that
+// is empty in the others), and the gate's per-filter registers live in a struct of their own (GateRegs; empty
+// NoGateRegs elsewhere): the ungated kernels keep the parameters, registers and code of a build without the gate.
+struct GateArgs {
+  float gate_nis3;          // threshold on the tangent-space NIS of a step (ekf_math.cuh, GateParams)
+  int32_t* gate_count;      // [N] in/out: steps gated so far, or null
+  uint8_t* out_gated;       // [T][N] 1 where the step was gated, 0 elsewhere (held steps: 0), or null
+};
+__device__ __forceinline__ GateArgs gate_args_(const GateArgs& g) { return g; }     // (GATE kernels: their one argument)
+struct GateRegs {
+  GateParams<float> gp;
+  int count;                // steps gated
+  uint8_t* out;             // this filter's slot in out_gated (AUX kernels), advanced by N per step, or null
+};
+struct NoGateRegs {};
+template <bool GATE> using GateRegsOf = typename std::conditional<GATE, GateRegs, NoGateRegs>::type;
+template <bool AUX> __device__ __forceinline__ void load_gate(const ReplayParams& p, const GateArgs& ga, int64_t n, GateRegs& g) {
+  g.gp = make_gate_params<float>(p.r_scale[n], ga.gate_nis3);
+  g.count = ga.gate_count ? ga.gate_count[n] : 0;
+  g.out = (AUX && ga.out_gated) ? ga.out_gated + n : nullptr;
+}
+
 template <int ALGO, bool LPF, bool COMP, bool INNOV = false, bool TAN = false>
 __device__ __forceinline__ void load_filter(const ReplayParams& p, int64_t n, int64_t col, FilterRegs& f) {
   const int64_t N = p.N, Ns = p.Ns;
@@ -104,9 +126,9 @@ template <bool AUX> __device__ __forceinline__ AuxPtrs make_aux(const ReplayPara
   return a;
 }
 
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false>
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool GATE = false>
 __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f, const float (&s)[kChannels], float h,
-                                            AuxPtrs& aux) {
+                                            AuxPtrs& aux, GateRegsOf<GATE>& g) {
   Vec3<float> w = {s[0], s[1], s[2]}, a = {s[3], s[4], s[5]}, m = {s[6], s[7], s[8]};
   if (LPF) {   // SRV/KalmanFilter.cpp:285,298 -- filtered values feed Wahba, not renormalised
     if (p.alpha_acc >= 0.f) { lowpass<float>(f.la, a, p.alpha_acc, 1.f - p.alpha_acc); a = f.la; }
@@ -116,8 +138,17 @@ __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f
   // flip-mask byte: the float32 decision, plus the tie marker and per-branch alternatives that flip_fixup_kernel settles
   // in float64 after the launch (raw samples only: a low-passed sample is not in the stream any more)
   unsigned code = 0;
-  ekf_step<float, ALGO, AUX, COMP, INNOV, TAN>(f.x, f.xlo, f.P, f.fc, w, a, m, StepH<float>(h), flip, aux.flips != nullptr,
-                                               (AUX && !LPF && ALGO == WAHBA_QR2) ? &code : nullptr, INNOV ? &f.in : nullptr);
+  if constexpr (GATE) {
+    bool gated = false;
+    ekf_step<float, ALGO, AUX, COMP, INNOV, TAN, true>(f.x, f.xlo, f.P, f.fc, w, a, m, StepH<float>(h), flip, aux.flips != nullptr,
+                                                       (AUX && !LPF && ALGO == WAHBA_QR2) ? &code : nullptr, INNOV ? &f.in : nullptr,
+                                                       &g.gp, &gated);
+    g.count += gated ? 1 : 0;
+    if (g.out) { *g.out = gated ? 1 : 0; g.out += p.N; }
+  } else {
+    ekf_step<float, ALGO, AUX, COMP, INNOV, TAN>(f.x, f.xlo, f.P, f.fc, w, a, m, StepH<float>(h), flip, aux.flips != nullptr,
+                                                 (AUX && !LPF && ALGO == WAHBA_QR2) ? &code : nullptr, INNOV ? &f.in : nullptr);
+  }
   if (!(AUX && !LPF && ALGO == WAHBA_QR2)) code = flip ? 1u : 0u;
   if (AUX) {
     // per-step outputs are in the reference frame (the reference's X_k)
@@ -147,8 +178,9 @@ __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f
 // A step at or past the length of the filter's stream (BATCH kernels): the filter is left as it is, the trajectory slot
 // gets the held state, the flip byte is 0 (unmarked: flip_fixup_kernel leaves it alone) and the objectives add nothing.
 // The step's sample and dt are not read.
-template <int ALGO, bool AUX>
-__device__ __forceinline__ void hold_step(const ReplayParams& p, const FilterRegs& f, AuxPtrs& aux) {
+template <int ALGO, bool AUX, bool GATE = false>
+__device__ __forceinline__ void hold_step(const ReplayParams& p, const FilterRegs& f, AuxPtrs& aux, GateRegsOf<GATE>& g) {
+  if constexpr (GATE) { if (g.out) { *g.out = 0; g.out += p.N; } }
   if (AUX) {
     if (aux.traj) {
       Quat<float> xr = f.x;
@@ -167,9 +199,11 @@ __device__ __forceinline__ void hold_step(const ReplayParams& p, const FilterReg
 // ---------------------------------------------------------------------------------------------
 // (INNOV: the innovation likelihood, TAN: its tangent-space form; their instantiations always have AUX and are built for
 //  3 CTAs per SM, <= 168 registers.  BATCH: per-stream dt columns and lengths, ReplayParams::dt_cols / n_valid)
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false>
-__global__ void __launch_bounds__(kThreads, INNOV ? 3 : ((ALGO == WAHBA_JACOBI || (COMP && LPF && AUX)) ? 4 : ((COMP || LPF) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
-    replay_ldg_kernel(const ReplayParams p) {
+//  GATE: the innovation gate, its arguments in the pack ga (one GateArgs; empty in the other kernels))
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false, bool GATE = false,
+          typename... GA>
+__global__ void __launch_bounds__(kThreads, (INNOV || GATE) ? 3 : ((ALGO == WAHBA_JACOBI || (COMP && LPF && AUX)) ? 4 : ((COMP || LPF) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
+    replay_ldg_kernel(const ReplayParams p, GA... ga) {
   const int64_t n = (int64_t)blockIdx.x * kThreads + threadIdx.x;
   if (n >= p.N) return;
   const int64_t Ns = p.Ns;
@@ -177,6 +211,8 @@ __global__ void __launch_bounds__(kThreads, INNOV ? 3 : ((ALGO == WAHBA_JACOBI |
   FilterRegs f;
   load_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, col, f);
   AuxPtrs aux = make_aux<AUX>(p, n, col, true);
+  [[maybe_unused]] GateRegsOf<GATE> g;
+  if constexpr (GATE) load_gate<AUX>(p, gate_args_(ga...), n, g);
   const float* s = p.streams + col;
   const int64_t step_stride = kChannels * Ns;
   float cur[kChannels], nxt[kChannels];
@@ -195,14 +231,15 @@ __global__ void __launch_bounds__(kThreads, INNOV ? 3 : ((ALGO == WAHBA_JACOBI |
     for (int c = 0; c < kChannels; ++c) nxt[c] = ldg_stream(s + c * Ns);
     if (BATCH && dc) hnxt = ldg_stream(dc + (int64_t)(t + 1 < T ? t + 1 : t) * Ns);
     const float h = (BATCH && dc) ? hcur : (p.dt_per_step ? __ldg(p.dt + t) : dt0);
-    if (!BATCH || t < nv) filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN>(p, f, cur, h, aux);
-    else hold_step<ALGO, AUX>(p, f, aux);
+    if (!BATCH || t < nv) filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE>(p, f, cur, h, aux, g);
+    else hold_step<ALGO, AUX, GATE>(p, f, aux, g);
 #pragma unroll
     for (int c = 0; c < kChannels; ++c) cur[c] = nxt[c];
     if (BATCH) hcur = hnxt;
   }
   store_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, f);
   if (AUX && aux.truth) p.loss_acc[n] = aux.loss;
+  if constexpr (GATE) { const GateArgs a = gate_args_(ga...); if (a.gate_count) a.gate_count[n] = g.count; }
 }
 
 // BATCH kernels: the stream length(s) of the thread's filter(s) and the per-step dt of the current and the next tile
@@ -245,9 +282,10 @@ struct __align__(128) TmaSmem {
 };
 constexpr uint32_t kTileBytes = kTmaSteps * kChannels * kThreads * sizeof(float);
 
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false>
-__global__ void __launch_bounds__(kThreads, INNOV ? 3 : (ALGO == WAHBA_JACOBI ? 4 : ((COMP && (LPF || AUX)) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
-    replay_tma_kernel(const ReplayParams p, const __grid_constant__ CUtensorMap tmap) {
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false, bool GATE = false,
+          typename... GA>
+__global__ void __launch_bounds__(kThreads, (INNOV || GATE) ? 3 : (ALGO == WAHBA_JACOBI ? 4 : ((COMP && (LPF || AUX)) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
+    replay_tma_kernel(const ReplayParams p, const __grid_constant__ CUtensorMap tmap, GA... ga) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   TmaSmem& sm = *reinterpret_cast<TmaSmem*>(smem_raw);
   const int tid = threadIdx.x;
@@ -278,6 +316,8 @@ __global__ void __launch_bounds__(kThreads, INNOV ? 3 : (ALGO == WAHBA_JACOBI ? 
   FilterRegs f;
   if (valid) load_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, (int64_t)col0 + tid, f);
   AuxPtrs aux = make_aux<AUX>(p, n, (int64_t)col0 + tid, valid);
+  [[maybe_unused]] GateRegsOf<GATE> g;
+  if constexpr (GATE) { if (valid) load_gate<AUX>(p, gate_args_(ga...), n, g); }
   const float dt0 = p.dt[0];
   // BATCH: this stream's length, and the time steps of the next tile held in registers (loaded one tile ahead: the
   // shared-memory ring has no room left at this kernel's occupancy)
@@ -311,16 +351,16 @@ __global__ void __launch_bounds__(kThreads, INNOV ? 3 : (ALGO == WAHBA_JACOBI ? 
       for (int tt = 0; tt < kTmaSteps; ++tt) {
         if (tt < steps) {
           if constexpr (BATCH) {
-            if (k * kTmaSteps + tt >= bt.nv) { hold_step<ALGO, AUX>(p, f, aux); continue; }
+            if (k * kTmaSteps + tt >= bt.nv) { hold_step<ALGO, AUX, GATE>(p, f, aux, g); continue; }
           }
           float s[kChannels];
 #pragma unroll
           for (int c = 0; c < kChannels; ++c) s[c] = sm.tile[stage][tt][c][tid];
           if constexpr (BATCH) {
-            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN>(p, f, s, bt.cur[tt], aux);
+            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE>(p, f, s, bt.cur[tt], aux, g);
           } else {
             const float h = p.dt_per_step ? __ldg(p.dt + k * kTmaSteps + tt) : dt0;
-            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN>(p, f, s, h, aux);
+            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE>(p, f, s, h, aux, g);
           }
         }
       }
@@ -330,6 +370,7 @@ __global__ void __launch_bounds__(kThreads, INNOV ? 3 : (ALGO == WAHBA_JACOBI ? 
     if (++stage == kTmaStages) { stage = 0; parity ^= 1; }
   }
   if (valid) store_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, f);
+  if constexpr (GATE) { const GateArgs a = gate_args_(ga...); if (valid && a.gate_count) a.gate_count[n] = g.count; }
   if (AUX && valid && aux.truth) p.loss_acc[n] = aux.loss;
 }
 
@@ -379,10 +420,13 @@ __device__ __forceinline__ void hold_lanes(mask2 live, FilterRegs2& f, const Fil
 //  likelihood (TAN: tangent-space form), instantiated without per-step outputs and low-pass -- the sweep path;
 //  replay_dispatch routes the rest.  BATCH: per-stream dt columns and lengths; a tile runs as the one-block fast tile
 //  when every filter of the CTA is live for all of its steps, and otherwise steps both lanes and keeps the old values of
-//  a lane past its length)
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false>
+//  a lane past its length.  GATE: the innovation gate, instantiated for the plain variant with and without per-step
+//  outputs and for the precise one without them (BATCH: the plain one without them), no low-pass, no innovation sums;
+//  replay_dispatch routes the rest)
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false, bool GATE = false,
+          typename... GA>
 __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) < PKF_MIN_CTAS2 ? (256 / kThreads2) : PKF_MIN_CTAS2) : PKF_MIN_CTAS2)
-    replay_tma2_kernel(const ReplayParams p, const __grid_constant__ CUtensorMap tmap) {
+    replay_tma2_kernel(const ReplayParams p, const __grid_constant__ CUtensorMap tmap, GA... ga) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   Tma2Smem& sm = *reinterpret_cast<Tma2Smem*>(smem_raw);
   const int tid = threadIdx.x;
@@ -446,16 +490,28 @@ __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) 
     adopt_state(f.fc, f.x, f.xlo);
     if (uses_filter_frame<ALGO>() && !(p.state_flags & kStateInFilterFrame)) enter_filter_frame(f.fc, f.x, f.xlo, f.P, COMP);
   }
+  // GATE: the gate's launch constants and the two lanes' counts of gated steps
+  [[maybe_unused]] GateParams<f32x2> gp;
+  [[maybe_unused]] int gc0 = 0, gc1 = 0;
+  if constexpr (GATE) {
+    if (valid) {
+      const GateArgs a = gate_args_(ga...);
+      gp = make_gate_params<f32x2>(ld2(p.r_scale + n), a.gate_nis3);
+      if (a.gate_count) { const int2 c = *reinterpret_cast<const int2*>(a.gate_count + n); gc0 = c.x; gc1 = c.y; }
+    }
+  }
   const float dt0 = p.dt[0];
   const StepH<f32x2> sh0{f32x2(dt0), f32x2(dt0 * dt0), f32x2(dt0 * (-1.f / 6.f))};
   // auxiliary outputs: this thread's pair of adjacent slots
   float4* traj = nullptr;
   uint8_t* flips = nullptr;
   const float4* truth = nullptr;
+  [[maybe_unused]] uint8_t* gflags = nullptr;
   f32x2 loss(0.f);
   if (AUX && valid) {
     if (p.out_traj) traj = reinterpret_cast<float4*>(p.out_traj) + n;
     if (p.out_flip) flips = p.out_flip + n;
+    if constexpr (GATE) { const GateArgs a = gate_args_(ga...); if (a.out_gated) gflags = a.out_gated + n; }
     if (p.truth) { truth = reinterpret_cast<const float4*>(p.truth) + ((int64_t)col0 + 2 * tid); loss = ld2(p.loss_acc + n); }
   }
   // BATCH: the per-lane time steps of the next tile, held in registers (loaded one tile ahead: the shared-memory ring has
@@ -516,15 +572,32 @@ __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) 
         mask2 flip;
         constexpr bool kTieCode = AUX && !LPF && ALGO == WAHBA_QR2;     // see filter_step
         FlipCode2 code = {0u, 0u};
-        if constexpr (FAST && ALGO == WAHBA_QR2) ekf_step_plain_measured<f32x2, AUX, COMP, INNOV, TAN>(f.x, f.xlo, f.P, f.fc, w, a, m, sh, flip, flips != nullptr,
-                                                                                                        kTieCode ? &code : nullptr, INNOV ? &f.in : nullptr);
-        else ekf_step<f32x2, ALGO, AUX, COMP, INNOV, TAN>(f.x, f.xlo, f.P, f.fc, w, a, m, sh, flip, flips != nullptr, kTieCode ? &code : nullptr,
-                                                          INNOV ? &f.in : nullptr);
+        [[maybe_unused]] mask2 gated = {false, false};
+        if constexpr (GATE) {
+          if constexpr (FAST && ALGO == WAHBA_QR2) ekf_step_plain_measured<f32x2, AUX, COMP, INNOV, TAN, true>(f.x, f.xlo, f.P, f.fc, w, a, m, sh, flip, flips != nullptr,
+                                                                                                            kTieCode ? &code : nullptr, INNOV ? &f.in : nullptr, &gp, &gated);
+          else ekf_step<f32x2, ALGO, AUX, COMP, INNOV, TAN, true>(f.x, f.xlo, f.P, f.fc, w, a, m, sh, flip, flips != nullptr, kTieCode ? &code : nullptr,
+                                                                  INNOV ? &f.in : nullptr, &gp, &gated);
+        } else {
+          if constexpr (FAST && ALGO == WAHBA_QR2) ekf_step_plain_measured<f32x2, AUX, COMP, INNOV, TAN>(f.x, f.xlo, f.P, f.fc, w, a, m, sh, flip, flips != nullptr,
+                                                                                                          kTieCode ? &code : nullptr, INNOV ? &f.in : nullptr);
+          else ekf_step<f32x2, ALGO, AUX, COMP, INNOV, TAN>(f.x, f.xlo, f.P, f.fc, w, a, m, sh, flip, flips != nullptr, kTieCode ? &code : nullptr,
+                                                            INNOV ? &f.in : nullptr);
+        }
         if (!kTieCode) code = FlipCode2{flip.x ? 1u : 0u, flip.y ? 1u : 0u};
         if constexpr (BATCH && !FAST) {
           if (!(held.live.x && held.live.y)) {
             hold_lanes<LPF, COMP, INNOV>(held.live, f, held.f0);
             code = FlipCode2{held.live.x ? code.x : 0u, held.live.y ? code.y : 0u};
+          }
+          if constexpr (GATE) gated = gated && held.live;     // a held step is never gated
+        }
+        if constexpr (GATE) {
+          gc0 += gated.x ? 1 : 0;
+          gc1 += gated.y ? 1 : 0;
+          if (AUX && gflags) {
+            *reinterpret_cast<uchar2*>(gflags) = make_uchar2(gated.x ? 1 : 0, gated.y ? 1 : 0);
+            gflags += N;
           }
         }
         if (AUX) {
@@ -598,6 +671,10 @@ __global__ void __launch_bounds__(kThreads2, (AUX && COMP) ? ((256 / kThreads2) 
     }
     if (AUX && p.truth) st2(p.loss_acc + n, loss);
     if (INNOV) { st2(p.innov_acc + n, f.in.nis); st2(p.innov_acc + N + n, f.in.logdet); }
+    if constexpr (GATE) {
+      const GateArgs a = gate_args_(ga...);
+      if (a.gate_count) *reinterpret_cast<int2*>(a.gate_count + n) = make_int2(gc0, gc1);
+    }
   }
 }
 

@@ -138,3 +138,39 @@ def make_imu(n_filters: int, n_steps: int, *, seed: int = 0, sigma: float = 0.0,
         if keep_truth:
             q_true[i] = q
     return SyntheticIMU(out, acc0_meas.to(torch.float32), mag0_meas.to(torch.float32), q_true, dt)
+
+
+def add_disturbances(streams: torch.Tensor, *, seed: int = 1, n_mag: int = 3, n_acc: int = 0,
+                     mag_strength=(0.15, 0.5), acc_strength=(0.15, 0.5), length=(100, 300),
+                     margin=(200, 300)) -> torch.Tensor:
+    """Inject sensor disturbances into a `[T, 9, N]` stream IN PLACE and return the disturbed-step mask `[T, N]` (bool).
+
+    Every recording (column) gets `n_mag` magnetometer disturbances (a magnetic field distortion near metal) and
+    `n_acc` accelerometer ones (a burst of linear acceleration).  Each starts at a uniform step in
+    [margin[0], T - margin[1]), lasts a uniform number of steps in [length[0], length[1]] and adds u * d to the unit
+    sample, with u ~ U(strength) and d a random unit vector fixed for the disturbance; the sample is then renormalised.
+    Overlapping disturbances add up.  The draws come from a CPU generator seeded with `seed`, so the result does not
+    depend on the device.  Sample 0 (the reference vectors of `make_imu`) is outside every disturbance."""
+    T, C, N = streams.shape
+    if C != N_CHANNELS:
+        raise ValueError("streams must be [T, 9, N]")
+    if T - margin[1] <= margin[0]:
+        raise ValueError(f"T = {T} leaves no room for a disturbance between the margins {margin}")
+    dev = streams.device
+    g = torch.Generator(device="cpu")
+    g.manual_seed(seed)
+    f64 = dict(dtype=torch.float64)
+    t = torch.arange(T, device=dev)[:, None]
+    mask = torch.zeros((T, N), dtype=torch.bool, device=dev)
+    for rows, count, (lo, hi) in ((MAG, n_mag, mag_strength), (ACC, n_acc, acc_strength)):
+        for _ in range(count):
+            start = torch.randint(margin[0], T - margin[1], (N,), generator=g).to(dev)
+            dur = torch.randint(length[0], length[1] + 1, (N,), generator=g).to(dev)
+            u = (lo + (hi - lo) * torch.rand(N, generator=g, **f64)).to(dev)
+            d = _unit(torch.randn(3, N, generator=g, **f64)).to(dev)
+            on = (t >= start[None]) & (t < (start + dur)[None])                       # [T,N]
+            v = streams[:, rows].to(torch.float64) + (u * d)[None] * on[:, None].to(torch.float64)
+            v = v / torch.linalg.vector_norm(v, dim=1, keepdim=True)
+            streams[:, rows] = torch.where(on[:, None], v.to(torch.float32), streams[:, rows])
+            mask |= on
+    return mask

@@ -109,11 +109,12 @@ def build_c3(device, grid: int = C3_GRID, n_streams: int = C3_STREAMS, n_steps: 
 
 
 def run_c3(w: SweepWorkload, *, precise_state=None, share_measurements=None, objective: str = "truth",
-           staging: str = "auto") -> B.ReplayState:
+           staging: str = "auto", gate: float | None = None) -> B.ReplayState:
     """One sweep: every cell replays all trajectories; returns the state with its tuning objective: `.loss` [N] (sum
     over steps of sin^2 of the angle to the ground truth; objective "truth"), `.innov` [2,N] (innovation likelihood
     sums, see `innovation_surface`; objective "innovation" for the 4-D model, "innovation_tangent" for the tangent-space
-    one) or neither ("none")."""
+    one) or neither ("none").  `gate`: replay with the innovation gate at that NIS3 threshold (`B.replay(gate=...)`;
+    the per-filter counts of gated steps are in `.gate_count`)."""
     innov_model = {"innovation": "full", "innovation_tangent": "tangent"}.get(objective)
     if innov_model is None and objective not in ("truth", "none"):
         raise ValueError("objective is 'truth', 'innovation', 'innovation_tangent' or 'none'")
@@ -122,7 +123,7 @@ def run_c3(w: SweepWorkload, *, precise_state=None, share_measurements=None, obj
     B.replay(w.streams, w.acc_ref, w.mag_ref, dt=w.dt, q=w.q, r=w.r, n_filters=N, state=st,
              truth=w.truth if objective == "truth" else None, innovation=True if innov_model else None,
              innovation_model=innov_model or "full", precise_state=precise_state, share_measurements=share_measurements,
-             staging=staging, lengths=w.lengths)
+             staging=staging, lengths=w.lengths, gate=gate)
     return st
 
 
