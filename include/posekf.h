@@ -221,6 +221,34 @@ int posekf_replay_gated_f32(int64_t n_filters, int64_t n_steps, const float* str
                             void* stream, const float* dt_cols, const int32_t* n_valid, float gate_nis3, int32_t* gate_count,
                             uint8_t* out_gated);
 
+/* General Q and R matrices: the replay of posekf_replay_batch_f32 (same parameters and rules, minus q_scale / r_scale)
+ * for filters whose process noise Q is any symmetric positive semidefinite 3x3 and whose measurement noise R is any
+ * symmetric positive definite 4x4 -- the reference's KalmanFilter with its Q and R attributes assigned
+ * (PKF/ExtendedKalmanFilter.py:58-80).  Each step is
+ *     P^- = A P A^T + B(x) Q B(x)^T      (A = 0.5 Omega(w), the reference's own; B at the state before the step)
+ *     z   = RK4 prediction               (restructured as in posekf_replay_f32, DESIGN.md section 3)
+ *     S = P^- + R,  K = P^- S^-1,  y = the Wahba quaternion sign-fixed against z by the comparator
+ *     X = (z + K (y - z)) / |.|,  P = P^- - K P^-.
+ *   q_tri   [6][nq]: the upper triangle of Q, row-major (Q00 Q01 Q02 Q11 Q12 Q22); nq = 1 (one Q for the launch) or
+ *           n_filters (filter n uses column n).  4-byte aligned, else POSEKF_EALIGN.
+ *   r_tri   [10][nr]: the upper triangle of R in the order of state_p (R00 R01 R02 R03 R11 R12 R13 R22 R23 R33); nr = 1
+ *           or n_filters.
+ *   state_p holds P itself, NOT P/r as in the scalar entry points: convert when a state moves between the two.
+ * Precondition (not checked here, like r > 0 and q >= 0 of the scalar entry points): R positive definite, Q positive
+ * semidefinite, both symmetric.  POSEKF_EINVAL: innov_acc or state_x_lo non-NULL (no innovation sums and no precise
+ * variant with general matrices), nq or nr neither 1 nor n_filters, q_tri or r_tri NULL, and everything
+ * posekf_replay_batch_f32 refuses.  There is no gated twin.  The float64 flip fix-up, the tuning loss (truth/loss_acc),
+ * the low-pass, all three Wahba modes, per-stream dt / lengths and the filter-frame state flags work as in
+ * posekf_replay_batch_f32.  A chunked replay equals the unchunked one bit for bit; every staging gives the same bits
+ * (a packed staging runs the scalar TMA kernel).  The float32 step meets the 1e-5 rad tolerance of the float64
+ * reference for eigenvalue ratios lambda(R)/lambda(Q) <= 100 and lambda(Q)/lambda(R) <= 1e4 (DESIGN.md, f9). */
+int posekf_replay_general_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
+                              int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_tri, int64_t nq,
+                              const float* r_tri, int64_t nr, float lpf_alpha_acc, float lpf_alpha_mag, float* state_x,
+                              float* state_x_lo, float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip,
+                              const float* truth, float* loss_acc, float* innov_acc, int innov_model, int wahba_algo,
+                              int staging, int state_flags, void* stream, const float* dt_cols, const int32_t* n_valid);
+
 /* Same replay with HOST buffers: streams_host [T][9][N] is streamed through the device in time
  * chunks (double-buffered H2D copies overlapped with the filter kernel, state carried across
  * chunks on the device), results are copied back.  This is the call an offline-replay user makes.

@@ -81,7 +81,8 @@ class ReplayState:
     """Filter state carried between `replay` calls (time-chunked replay, checkpoint/resume).
     x [4,N]; p [10,N] packed upper triangle of P/r (the covariance in units of each filter's r --
     the form the kernel works in, so that chunked and unchunked replays are bit-identical);
-    r: the float or [N] tensor the scaling refers to; lpf [6,N] or None.
+    r: the float or [N] tensor the scaling refers to -- 1.0 after a replay with general Q / R matrices, whose kernels
+    carry P itself (`replay` converts p whenever the next call needs the other form); lpf [6,N] or None.
     frame: "reference" (x, p in the reference's own coordinates -- what every `replay` call returns by
     default) or "filter" (left in the kernel's working frame by `replay(..., keep_filter_frame=True)`
     between the chunks of a time-chunked replay; `to_reference_frame` converts).
@@ -210,6 +211,73 @@ def _scales_need_precise(q, r) -> bool:
     return bool(flags[1])
 
 
+_TRI3 = [(0, 0), (0, 1), (0, 2), (1, 1), (1, 2), (2, 2)]
+
+
+def _is_matrix(v) -> bool:
+    """A q / r argument that selects the general-matrix replay: a [k,k] or [N,k,k] tensor or array."""
+    return hasattr(v, "shape") and len(v.shape) >= 2
+
+
+def _as_matrices(v, k: int, n: int, device, name: str) -> torch.Tensor:
+    """[1,k,k] or [n,k,k] float64 on `device` from a [k,k] / [n,k,k] matrix, or from a float / [n] tensor (v I_k)."""
+    if isinstance(v, torch.Tensor) and not v.is_cuda and torch.device(device).type == "cuda":
+        raise _lib.PosekfError("poseestimationkf_b200 runs on CUDA tensors only (no CPU fallback); matrices may be numpy "
+                               "arrays or CUDA tensors of any float dtype")
+    t = torch.as_tensor(v, dtype=torch.float64, device=device)
+    eye = torch.eye(k, dtype=torch.float64, device=device)
+    if t.dim() == 0:
+        return (t * eye)[None]
+    if t.dim() == 1 and t.shape == (n,):
+        return t[:, None, None] * eye[None]
+    if t.dim() == 2 and t.shape == (k, k):
+        return t[None]
+    if t.dim() == 3 and t.shape == (n, k, k):
+        return t
+    raise ValueError(f"{name} must be a float, an [N] tensor, a [{k},{k}] or an [N,{k},{k}] matrix (N = {n}), "
+                     f"got shape {tuple(t.shape)}")
+
+
+_general_cache: dict = {}
+
+
+def general_qr_tri(q, r, n: int, device):
+    """The matrices of a general-matrix replay (include/posekf.h, posekf_replay_general_f32) as the kernels read them:
+    (q_tri [6,Nq], r_tri [10,Nr]) float32 upper triangles, Nq / Nr = 1 for one matrix shared by the launch, else n.
+    q: [3,3] / [N,3,3] (Q), or a float / [N] tensor (q I3); r: [4,4] / [N,4,4] (R), or a float / [N] tensor (r I4).
+    Checks, on the float32 values the kernels use: symmetry (to 1e-6 of the largest entry), R positive definite and Q
+    positive semidefinite (torch.linalg.eigvalsh; an eigenvalue down to -1e-6 of the largest counts as 0).  One
+    read-back, cached per tensor pair and version (pass the SAME tensor objects to every chunk of a chunked replay)."""
+    key = tuple(id(t) if isinstance(t, torch.Tensor) else None for t in (q, r))
+    hit = _general_cache.get(key) if all(k is not None for k in key) else None
+    if hit is not None:
+        refs, versions, dev, n0, out = hit
+        if all(ref() is t and t._version == ver for t, ref, ver in zip((q, r), refs, versions)) and dev == str(device) and n0 == n:
+            return out
+    Q = _as_matrices(q, 3, n, device, "q").to(torch.float32).to(torch.float64)
+    R = _as_matrices(r, 4, n, device, "r").to(torch.float32).to(torch.float64)
+    bad = []
+    for M, name in ((Q, "Q"), (R, "R")):
+        asym = (M - M.transpose(1, 2)).abs().amax() > 1e-6 * M.abs().amax()
+        lam = torch.linalg.eigvalsh(torch.triu(M) + torch.triu(M, 1).transpose(1, 2))
+        low = lam.amin() <= 0 if name == "R" else lam.amin() < -1e-6 * lam.amax().clamp(min=0)
+        bad += [asym, low | ~torch.isfinite(lam).all()]
+    asym_q, neg_q, asym_r, neg_r = torch.stack(bad).tolist()
+    if asym_q or asym_r:
+        raise ValueError("Q and R must be symmetric")
+    if neg_r:
+        raise ValueError("R must be positive definite")
+    if neg_q:
+        raise ValueError("Q must be positive semidefinite")
+    out = (torch.stack([Q[:, i, j] for i, j in _TRI3]).to(torch.float32).contiguous(),
+           torch.stack([R[:, i, j] for i, j in _TRI]).to(torch.float32).contiguous())
+    if all(k is not None for k in key):
+        if len(_general_cache) > 64:
+            _general_cache.clear()
+        _general_cache[key] = (tuple(weakref.ref(t) for t in (q, r)), tuple(t._version for t in (q, r)), str(device), n, out)
+    return out
+
+
 def _per_filter(v, n, device):
     if isinstance(v, torch.Tensor):
         _require_cuda(v)
@@ -253,7 +321,12 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
 
     streams [T,9,Ns]; acc_ref, mag_ref [3,Ns]; dt: float seconds, [T] float32 CUDA tensor (one clock for every
     filter) or [T,Ns] (per stream: filter n steps with column n % Ns -- a batch of recordings, `logio.stack_logs`);
-    q, r: floats or [N] tensors (Q=q*I3, R=r*I4).  `n_filters` > Ns replays every trajectory
+    q, r: floats or [N] tensors (Q=q*I3, R=r*I4), or general matrices: q [3,3] / [N,3,3] and r [4,4] / [N,4,4] (numpy
+    arrays or CUDA tensors; either may stay a float or [N] tensor).  A matrix runs the general-matrix replay
+    (include/posekf.h, posekf_replay_general_f32): the reference's KalmanFilter with its Q and R attributes assigned,
+    symmetric Q positive semidefinite and R positive definite (checked, `general_qr_tri`).  It has no precise variant,
+    no innovation sums and no gate; trajectories, flips, the loss, the low-pass, every Wahba mode, per-stream dt and
+    lengths work as with scalars, and `state.p` then holds P itself (`state.r` = 1.0).  `n_filters` > Ns replays every trajectory
     N/Ns times (filter n reads column n % Ns) -- the Q/R sweep layout.  `state` is updated in place
     (created with the reference's initial values when None).  `truth` [T,Ns,4] enables the on-device
     tuning objective: `loss` [N] (created zeroed when None; pass it back in for chunked replays) is
@@ -328,21 +401,31 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
             raise ValueError("share_measurements needs raw streams, N > Ns and no low-pass stage")
         streams, _ = measurement_stream(streams, acc_ref, mag_ref, algo=wahba)
         wahba = "precomputed"
-    if isinstance(q, torch.Tensor):
-        _require_cuda(q)
-    if isinstance(r, torch.Tensor):
-        _require_cuda(r)
-    needs_precise = _scales_need_precise(q, r)      # also validates r > 0, q >= 0
+    general = _is_matrix(q) or _is_matrix(r)
+    if general:
+        if (innovation is not None and innovation is not False) or gate is not None:
+            raise ValueError("general Q / R matrices: the replay has no innovation sums and no gate")
+        if precise_state or (state is not None and state.x_lo is not None):
+            raise ValueError("general Q / R matrices: the replay has no precise variant (precise_state, a two-float state)")
+        q_tri, r_tri = general_qr_tri(q, r, N, dev)
+        needs_precise, units = False, 1.0        # the general kernels carry P itself
+    else:
+        if isinstance(q, torch.Tensor):
+            _require_cuda(q)
+        if isinstance(r, torch.Tensor):
+            _require_cuda(r)
+        needs_precise = _scales_need_precise(q, r)      # also validates r > 0, q >= 0
+        units = r
     if state is None:
-        state = ReplayState.initial(N, dev, r=r, with_lpf=use_lpf)
-    elif not _same_scale(state.r, r):
+        state = ReplayState.initial(N, dev, r=units, with_lpf=use_lpf)
+    elif not _same_scale(state.r, units):
         # the covariance is stored in units of the r it was created with: re-express it in units of the new r
         old = state.r if isinstance(state.r, torch.Tensor) else float(state.r)
-        new = r if isinstance(r, torch.Tensor) else float(r)
+        new = units if isinstance(units, torch.Tensor) else float(units)
         state.p.mul_(old / new)
-    state.r = r
+    state.r = units
     if precise_state is None:
-        if (isinstance(q, torch.Tensor) or isinstance(r, torch.Tensor)) and N > Ns and N % Ns == 0 \
+        if not general and (isinstance(q, torch.Tensor) or isinstance(r, torch.Tensor)) and N > Ns and N % Ns == 0 \
                 and out_traj is None and not store_trajectory and not store_flips and not use_lpf and T > 0 \
                 and out_gated is None:
             # a (Q,R) sweep: only the cells with r/q >= 100 or q/r >= 1e4 need the precise variant (+25 % time)
@@ -373,7 +456,7 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
         dt_t, per_step = dt, 1
     else:
         dt_t, per_step = _scalar_tensor(dt, dev), 0
-    q_t, r_t = _per_filter(q, N, dev), _per_filter(r, N, dev)
+    q_t, r_t = (None, None) if general else (_per_filter(q, N, dev), _per_filter(r, N, dev))
     if wahba == "precomputed":
         # no Wahba stage in the kernel: its working frame is the reference frame
         state.to_reference_frame(acc_ref, mag_ref)
@@ -403,7 +486,11 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     tail = (_lib.WAHBA[wahba], _lib.STAGING[staging], frame_flags, _stream())
     batch = dt_cols is not None or lengths is not None
     with torch.cuda.device(dev):
-        if gate is not None:
+        if general:
+            rc = _lib.load().posekf_replay_general_f32(
+                N, T, _ptr(streams), Ns, _ptr(dt_t), per_step, _ptr(acc_ref), _ptr(mag_ref), _ptr(q_tri), q_tri.shape[1],
+                _ptr(r_tri), r_tri.shape[1], *args[10:], None, _lib.INNOV_MODEL["full"], *tail, _ptr(dt_cols), _ptr(lengths))
+        elif gate is not None:
             rc = _lib.load().posekf_replay_gated_f32(*args, _ptr(innov), _lib.INNOV_MODEL[innovation_model], *tail, _ptr(dt_cols),
                                                      _ptr(lengths), float(gate), _ptr(gate_count), _ptr(out_gated))
         elif batch:
@@ -413,7 +500,8 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
             rc = _lib.load().posekf_replay_f32(*args, *tail)
         else:
             rc = _lib.load().posekf_replay_innovation_ex_f32(*args, _ptr(innov), _lib.INNOV_MODEL[innovation_model], *tail)
-    _lib.check(rc, "posekf_replay_gated_f32" if gate is not None else "posekf_replay_batch_f32" if batch else
+    _lib.check(rc, "posekf_replay_general_f32" if general else "posekf_replay_gated_f32" if gate is not None else
+               "posekf_replay_batch_f32" if batch else
                ("posekf_replay_f32" if innov is None else "posekf_replay_innovation_ex_f32"))
     if innov is not None:
         state.innov, state.innov_model = innov, innovation_model

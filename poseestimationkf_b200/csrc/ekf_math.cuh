@@ -1363,18 +1363,164 @@ PKF_HD void gate_apply(const GateParams<F>& gp, const InnovFactors<F>& fac, cons
   K.a22 = sel_(g, Pm.a22, K.a22); K.a23 = sel_(g, Pm.a23, K.a23); K.a33 = sel_(g, Pm.a33, K.a33);
 }
 
+// ------------------------------------------------------------------------------------------
+// GENERAL Q AND R (GEN): Q any symmetric positive semidefinite 3x3, R any symmetric positive definite 4x4 -- the
+// reference's KalmanFilter with its Q and R attributes assigned (PKF/ExtendedKalmanFilter.py:58-79).  Neither the
+// closed form of B Q B^T nor the units-of-r scaling applies, so P is carried unscaled (plain variant only).
+//   B(x) Q B(x)^T: B(x) v = (0, v) (x) x / 2 is linear in x.  With Q4 = Q/4 and 2B (entries +-x_i),
+//     M = (2B) Q4 (4x3),   P^-_ij = (A P A^T)_ij + sum_c M_ic (2B)_jc          (propagate_cov_general)
+//   and the first step of a launch handed a non-unit state gets |x|^2 B(x^) Q B(x^)^T through fc.gs (fc.g = 1, see
+//   adopt_state), so the second factor is formed from gs x.
+//   Gain: S = P^- + R = L D L^T (kalman_gain_general).  K = P^- S^-1 = I - R S^-1, and with G = L^-1 R, H = D^-1 G:
+//     K e = e - H^T (L^-1 e),     P^+ = P^- - K P^- = K R = R - R S^-1 R = R - G^T H
+//   (upper triangle only, symmetric by construction; no backward substitution).  For R = r I this is the isotropic
+//   step's own algebra (K = I - r S^-1, P^+ = r K), so it loses accuracy where that one does (see kalman_gain_from_s).
+//   Filter frame: with x' = p (x) x, L(p) B(x) v = B(x') Rot(p) v, so the recursion stays equivariant when Q and R are
+//   carried as Rot(p) Q Rot(p)^T and L(p) R L(p)^T (make_gen_qr).
+// ------------------------------------------------------------------------------------------
+template <typename F> struct Sym3 { F a00, a01, a02, a11, a12, a22; };      // upper triangle, row-major
+template <typename F> struct GenQR {
+  Sym3<F> q4;     // Q/4 in the step's frame
+  Sym4<F> R;      // R in the step's frame
+};
+template <typename F> struct GainGen {
+  Sym4<F> Pp;                          // P^+
+  F l10, l20, l30, l21, l31, l32;      // L of S = L D L^T
+  F h[4][4];                           // H = D^-1 L^-1 R
+};
+struct NoGainGen {};
+template <typename F, bool GEN> struct GainGenOf { typedef GainGen<F> type; };   // (empty in the other instantiations)
+template <typename F> struct GainGenOf<F, false> { typedef NoGainGen type; };
+
+// q [6], r [10]: the upper triangles of Q and R in the reference frame (row-major, the order of Sym4).  filter_frame:
+// express them in the filter frame of fc (p = conj(qE), Rot(p) = E^T).
+template <typename F>
+PKF_HD GenQR<F> make_gen_qr(const FilterConst<F>& fc, const F (&q)[6], const F (&r)[10], bool filter_frame) {
+  F Q[3][3] = {{q[0], q[1], q[2]}, {q[1], q[3], q[4]}, {q[2], q[4], q[5]}};
+  Sym4<F> R = {r[0], r[1], r[2], r[3], r[4], r[5], r[6], r[7], r[8], r[9]};
+  if (filter_frame) {
+    const F e[3][3] = {{fc.E.e1.x, fc.E.e1.y, fc.E.e1.z}, {fc.E.e2.x, fc.E.e2.y, fc.E.e2.z}, {fc.E.e3.x, fc.E.e3.y, fc.E.e3.z}};
+    F QE[3][3], Qf[3][3];     // Q e_j, then e_i^T Q e_j
+    for (int i = 0; i < 3; ++i)
+      for (int j = 0; j < 3; ++j) QE[i][j] = fma_(Q[i][2], e[j][2], fma_(Q[i][1], e[j][1], Q[i][0] * e[j][0]));
+    for (int i = 0; i < 3; ++i)
+      for (int j = 0; j < 3; ++j) Qf[i][j] = fma_(e[i][2], QE[2][j], fma_(e[i][1], QE[1][j], e[i][0] * QE[0][j]));
+    for (int i = 0; i < 3; ++i)
+      for (int j = 0; j < 3; ++j) Q[i][j] = Qf[i][j];
+    R = rotate_cov(qconj(fc.qE), R);
+  }
+  GenQR<F> g;
+  g.q4 = {F(0.25) * Q[0][0], F(0.25) * Q[0][1], F(0.25) * Q[0][2], F(0.25) * Q[1][1], F(0.25) * Q[1][2], F(0.25) * Q[2][2]};
+  g.R = R;
+  return g;
+}
+
+// P^- = A P A^T + B(x) Q B(x)^T, Q = 4 q4; s = |x|^2 of the state handed to the launch on its first step, else 1.
+template <typename F>
+PKF_HD Sym4<F> propagate_cov_general(const Sym4<F>& P, const Vec3<F>& hw, const Quat<F>& x, F s, const Sym3<F>& q4) {
+  Sym4<F> N = propagate_cov<F, false>(P, hw, x, F(0), F(0));
+  const F Q[3][3] = {{q4.a00, q4.a01, q4.a02}, {q4.a01, q4.a11, q4.a12}, {q4.a02, q4.a12, q4.a22}};
+  // rows of 2B(x): column c is (0, e_c) (x) x
+  const F b[4][3] = {{-x.x, -x.y, -x.z}, {x.w, x.z, -x.y}, {-x.z, x.w, x.x}, {x.y, -x.x, x.w}};
+  const Quat<F> y = {s * x.w, s * x.x, s * x.y, s * x.z};
+  const F bs[4][3] = {{-y.x, -y.y, -y.z}, {y.w, y.z, -y.y}, {-y.z, y.w, y.x}, {y.y, -y.x, y.w}};
+  F M[4][3];
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+  for (int i = 0; i < 4; ++i) {
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for (int c = 0; c < 3; ++c) M[i][c] = fma_(b[i][2], Q[2][c], fma_(b[i][1], Q[1][c], b[i][0] * Q[0][c]));
+  }
+  auto add = [&](F n, int i, int j) { return fma_(M[i][2], bs[j][2], fma_(M[i][1], bs[j][1], fma_(M[i][0], bs[j][0], n))); };
+  N.a00 = add(N.a00, 0, 0); N.a01 = add(N.a01, 0, 1); N.a02 = add(N.a02, 0, 2); N.a03 = add(N.a03, 0, 3);
+  N.a11 = add(N.a11, 1, 1); N.a12 = add(N.a12, 1, 2); N.a13 = add(N.a13, 1, 3);
+  N.a22 = add(N.a22, 2, 2); N.a23 = add(N.a23, 2, 3);
+  N.a33 = add(N.a33, 3, 3);
+  return N;
+}
+
+// S = P^- + R = L D L^T, H = D^-1 L^-1 R and P^+ = R - (L^-1 R)^T H (see GENERAL Q AND R above).
+template <typename F> PKF_HD GainGen<F> kalman_gain_general(const Sym4<F>& Pm, const Sym4<F>& R) {
+  const F s00 = Pm.a00 + R.a00, s01 = Pm.a01 + R.a01, s02 = Pm.a02 + R.a02, s03 = Pm.a03 + R.a03;
+  const F s11 = Pm.a11 + R.a11, s12 = Pm.a12 + R.a12, s13 = Pm.a13 + R.a13;
+  const F s22 = Pm.a22 + R.a22, s23 = Pm.a23 + R.a23, s33 = Pm.a33 + R.a33;
+  GainGen<F> g;
+  const F i0 = rcp_(s00);
+  g.l10 = s01 * i0; g.l20 = s02 * i0; g.l30 = s03 * i0;
+  const F i1 = rcp_(fma_(-g.l10, s01, s11));
+  const F t21 = fma_(-g.l10, s02, s12), t31 = fma_(-g.l10, s03, s13);
+  g.l21 = t21 * i1; g.l31 = t31 * i1;
+  const F i2 = rcp_(fma_(-g.l21, t21, fma_(-g.l20, s02, s22)));
+  const F t32 = fma_(-g.l21, t31, fma_(-g.l20, s03, s23));
+  g.l32 = t32 * i2;
+  const F i3 = rcp_(fma_(-g.l32, t32, fma_(-g.l31, t31, fma_(-g.l30, s03, s33))));
+  const F Rm[4][4] = {{R.a00, R.a01, R.a02, R.a03}, {R.a01, R.a11, R.a12, R.a13}, {R.a02, R.a12, R.a22, R.a23},
+                      {R.a03, R.a13, R.a23, R.a33}};
+  F G[4][4];      // L^-1 R, column by column
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+  for (int j = 0; j < 4; ++j) {
+    G[0][j] = Rm[0][j];
+    G[1][j] = fma_(-g.l10, G[0][j], Rm[1][j]);
+    G[2][j] = fma_(-g.l21, G[1][j], fma_(-g.l20, G[0][j], Rm[2][j]));
+    G[3][j] = fma_(-g.l32, G[2][j], fma_(-g.l31, G[1][j], fma_(-g.l30, G[0][j], Rm[3][j])));
+    g.h[0][j] = i0 * G[0][j]; g.h[1][j] = i1 * G[1][j]; g.h[2][j] = i2 * G[2][j]; g.h[3][j] = i3 * G[3][j];
+  }
+  auto pp = [&](int i, int j) {
+    return fma_(-G[3][i], g.h[3][j], fma_(-G[2][i], g.h[2][j], fma_(-G[1][i], g.h[1][j], fma_(-G[0][i], g.h[0][j], Rm[i][j]))));
+  };
+  g.Pp = {pp(0, 0), pp(0, 1), pp(0, 2), pp(0, 3), pp(1, 1), pp(1, 2), pp(1, 3), pp(2, 2), pp(2, 3), pp(3, 3)};
+  return g;
+}
+
+// Prediction with general Q and R: the gain stage and the RK4 prediction z (plain-variant form)
+template <typename F>
+PKF_HD void ekf_predict_general(const Quat<F>& x, const Sym4<F>& P, const FilterConst<F>& fc, const GenQR<F>& gq,
+                                const Vec3<F>& gyro, const StepH<F>& h, GainGen<F>& gg, Quat<F>& z) {
+  Vec3<F> hw;
+  hw.x = F(0.5) * gyro.x; hw.y = F(0.5) * gyro.y; hw.z = F(0.5) * gyro.z;
+  gg = kalman_gain_general(propagate_cov_general(P, hw, x, fc.gs, gq.q4), gq.R);     // :59-66
+  z = rk4_predict_fused(x, hw, h);                                                       // :62
+}
+
+// X = z + K e, normalised; P = P^+                                                         :77-79
+template <typename F>
+PKF_HD void ekf_update_general(Quat<F>& x, Sym4<F>& P, FilterConst<F>& fc, const GainGen<F>& gg, const Quat<F>& z,
+                               F e0, F e1, F e2, F e3) {
+  const F t0 = e0;                                 // t = L^-1 e
+  const F t1 = fma_(-gg.l10, t0, e1);
+  const F t2 = fma_(-gg.l21, t1, fma_(-gg.l20, t0, e2));
+  const F t3 = fma_(-gg.l32, t2, fma_(-gg.l31, t1, fma_(-gg.l30, t0, e3)));
+  auto ke = [&](int i, F ei) { return fma_(-gg.h[3][i], t3, fma_(-gg.h[2][i], t2, fma_(-gg.h[1][i], t1, fma_(-gg.h[0][i], t0, ei)))); };
+  Quat<F> xn;
+  xn.w = z.w + ke(0, e0); xn.x = z.x + ke(1, e1); xn.y = z.y + ke(2, e2); xn.z = z.z + ke(3, e3);
+  const F d = rsqrt_(dot4(xn, xn)) - F(1);
+  x.w = fma_(xn.w, d, xn.w); x.x = fma_(xn.x, d, xn.x); x.y = fma_(xn.y, d, xn.y); x.z = fma_(xn.z, d, xn.z);
+  P = gg.Pp;
+  fc.gs = fc.g;        // the state leaves every step normalised
+}
+
 // Prediction + Correction with the measurement quaternion y (filter frame, any sign, norm 1/inv_norm) already computed.
 // INNOV: the innovation likelihood of the step is added to *innov (see InnovAcc); the filter itself is unchanged.
 // TAN: its tangent-space form (see innov_accumulate).  GATE: the innovation gate (see GateParams), decision in *gated.
-template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, bool GATE = false, typename FlagT>
+// GEN: general Q and R from *gen (see GENERAL Q AND R); P is unscaled, plain variant only.
+template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, bool GATE = false, bool GEN = false,
+          typename FlagT>
 PKF_HD void ekf_step_measured(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, const Vec3<F>& gyro,
                               const Quat<F>& y, F inv_norm, const StepH<F>& h, FlagT& flip, bool flip_wanted = true,
                               typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr,
-                              const GateParams<F>* gate = nullptr, FlagT* gated = nullptr) {
+                              const GateParams<F>* gate = nullptr, FlagT* gated = nullptr, const GenQR<F>* gen = nullptr) {
+  static_assert(!GEN || !(COMP || INNOV || GATE), "general Q and R: plain variant, no innovation sums, no gate");
   Sym4<F> K, Pm;
   Quat<F> inc, z;
   InnovFactors<F> fac;
-  ekf_predict<F, COMP, INNOV, GATE>(x, P, fc, gyro, h, K, inc, z, &fac, &Pm);
+  [[maybe_unused]] typename GainGenOf<F, GEN>::type gg;
+  if constexpr (GEN) ekf_predict_general(x, P, fc, *gen, gyro, h, gg, z);
+  else ekf_predict<F, COMP, INNOV, GATE>(x, P, fc, gyro, h, K, inc, z, &fac, &Pm);
   const F dyz = dot4(y, z);                       // the comparator, literally: negate when dot(y, z) < 0  :73-75
   flip = FlagT();
   if (WANT_FLIP && flip_wanted) flip = reference_flip_quat(fc, y, one_with_sign_(dyz), code);
@@ -1382,7 +1528,8 @@ PKF_HD void ekf_step_measured(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<
   F e0 = fma_(sn, y.w, -z.w), e1 = fma_(sn, y.x, -z.x), e2 = fma_(sn, y.y, -z.y), e3 = fma_(sn, y.z, -z.z);
   if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3);
   if constexpr (GATE) gate_apply<F, COMP>(*gate, fac, z, Pm, K, e0, e1, e2, e3, *gated);
-  ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);
+  if constexpr (GEN) ekf_update_general(x, P, fc, gg, z, e0, e1, e2, e3);
+  else ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);
 }
 
 // The common case of ekf_step<WAHBA_QR2>: both Wahba weights are non-negative (|a_z| <= 1, i.e. a normalised
@@ -1401,23 +1548,26 @@ PKF_HD void ekf_step_plain_measured(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, Filter
 }
 
 template <typename F, int ALGO, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, bool GATE = false,
-          typename FlagT>
+          bool GEN = false, typename FlagT>
 PKF_HD void ekf_step(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, const Vec3<F>& gyro,
                      const Vec3<F>& acc, const Vec3<F>& mag, const StepH<F>& h, FlagT& flip, bool flip_wanted = true,
                      typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr,
-                     const GateParams<F>* gate = nullptr, FlagT* gated = nullptr) {
+                     const GateParams<F>* gate = nullptr, FlagT* gated = nullptr, const GenQR<F>* gen = nullptr) {
   // flip_wanted: launch-uniform run-time switch under WANT_FLIP -- a launch that stores the trajectory but
   // not the flip mask skips the reference's branch rule altogether
   if constexpr (ALGO == WAHBA_QR2) {
     F inv_norm;
     const Quat<F> y = measure_quat(fc, acc, mag, inv_norm);
-    ekf_step_measured<F, WANT_FLIP, COMP, INNOV, TAN, GATE>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code, innov,
-                                                            gate, gated);
+    ekf_step_measured<F, WANT_FLIP, COMP, INNOV, TAN, GATE, GEN>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code,
+                                                                 innov, gate, gated, gen);
   } else {
+    static_assert(!GEN || !(COMP || INNOV || GATE), "general Q and R: plain variant, no innovation sums, no gate");
     Sym4<F> K, Pm;
     Quat<F> inc, z;
     InnovFactors<F> fac;
-    ekf_predict<F, COMP, INNOV, GATE>(x, P, fc, gyro, h, K, inc, z, &fac, &Pm);
+    [[maybe_unused]] typename GainGenOf<F, GEN>::type gg;
+    if constexpr (GEN) ekf_predict_general(x, P, fc, *gen, gyro, h, gg, z);
+    else ekf_predict<F, COMP, INNOV, GATE>(x, P, fc, gyro, h, K, inc, z, &fac, &Pm);
     // ---- Correction (PKF/ExtendedKalmanFilter.py:70-80) ----
     F e0, e1, e2, e3;
     if constexpr (ALGO == WAHBA_PRECOMPUTED) {
@@ -1453,7 +1603,8 @@ PKF_HD void ekf_step(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, c
     }
     if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3);
     if constexpr (GATE) gate_apply<F, COMP>(*gate, fac, z, Pm, K, e0, e1, e2, e3, *gated);
-    ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);
+    if constexpr (GEN) ekf_update_general(x, P, fc, gg, z, e0, e1, e2, e3);
+    else ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);
   }
 }
 

@@ -91,18 +91,19 @@ bool tma_eligible(const ReplayParams& p) {
   return true;
 }
 
-// ga: the gate's arguments (one GateArgs; GATE launches only, the others pass none)
+// ga: the gate's arguments (one GateArgs; GATE launches only) or the general Q and R (one GenQRArgs; GEN launches only);
+// the others pass none
 template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false, bool GATE = false,
-          typename... GA>
+          bool GEN = false, typename... GA>
 int launch_replay(const ReplayParams& p, bool use_tma, cudaStream_t st, const GA&... ga) {
   const unsigned grid = (unsigned)((p.N + kThreads - 1) / kThreads);
   if (!use_tma) {
-    replay_ldg_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH, GATE, GA...><<<grid, kThreads, 0, st>>>(p, ga...);
+    replay_ldg_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH, GATE, GEN, GA...><<<grid, kThreads, 0, st>>>(p, ga...);
     return launch_status();
   }
   CUtensorMap tmap;
   if (int rc = encode_stream_map(p, kThreads, kTmaSteps, &tmap)) return rc;
-  auto kern = replay_tma_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH, GATE, GA...>;
+  auto kern = replay_tma_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH, GATE, GEN, GA...>;
   // idempotent; set on every launch (cheap) so that it holds on every device of a multi-GPU process
   PKF_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TmaSmem)));
   kern<<<grid, kThreads, sizeof(TmaSmem), st>>>(p, tmap, ga...);
@@ -251,9 +252,29 @@ int launch_gated_algo(const ReplayParams& p, const GateArgs& ga, int algo, bool 
   return POSEKF_EINVAL;
 }
 
+// Launches with general Q and R matrices (posekf_replay_general_f32): the scalar BATCH kernels with GEN, which step
+// exactly as without BATCH when dt_cols and n_valid are null, with AUX (per-step outputs checked per pointer), on the
+// launch's staging (the TMA kernel for a packed staging: the packed kernel has no GEN twin, its 124-168 registers leave
+// no room for the 16 of Q and R at 3 CTAs per SM).  Plain variant only, no innovation sums, no gate.
+template <int ALGO>
+int launch_general(const ReplayParams& p, const GenQRArgs& gq, bool lpf, bool use_tma, cudaStream_t st) {
+  if constexpr (ALGO != WAHBA_PRECOMPUTED) {
+    if (lpf) return launch_replay<ALGO, true, true, false, false, false, true, false, true>(p, use_tma, st, gq);
+  }
+  return launch_replay<ALGO, false, true, false, false, false, true, false, true>(p, use_tma, st, gq);
+}
+
+int launch_general_algo(const ReplayParams& p, const GenQRArgs& gq, int algo, bool lpf, bool use_tma, cudaStream_t st) {
+  if (algo == POSEKF_WAHBA_QR2) return launch_general<WAHBA_QR2>(p, gq, lpf, use_tma, st);
+  if (algo == POSEKF_WAHBA_PRECOMPUTED) return launch_general<WAHBA_PRECOMPUTED>(p, gq, lpf, use_tma, st);
+  if (algo == POSEKF_WAHBA_JACOBI) return launch_general<WAHBA_JACOBI>(p, gq, lpf, use_tma, st);
+  return POSEKF_EINVAL;
+}
+
 // innov_model: POSEKF_INNOV_* of the sums in p.innov_acc (read only when it is set).  gate: run the gated kernels with
-// these arguments (null: the ungated ones).
-int replay_dispatch(const ReplayParams& p, int algo, int staging, int innov_model, cudaStream_t st, const GateArgs* gate = nullptr) {
+// these arguments (null: the ungated ones).  gen: run the general-matrix kernels with these matrices.
+int replay_dispatch(const ReplayParams& p, int algo, int staging, int innov_model, cudaStream_t st, const GateArgs* gate = nullptr,
+                    const GenQRArgs* gen = nullptr) {
   const bool lpf = (p.alpha_acc >= 0.f) || (p.alpha_mag >= 0.f);
   bool use_tma, packed = false;
   if (staging == POSEKF_STAGE_LDG) use_tma = false;
@@ -266,7 +287,8 @@ int replay_dispatch(const ReplayParams& p, int algo, int staging, int innov_mode
     packed = use_tma && kAutoPrefersPacked && algo != POSEKF_WAHBA_JACOBI && packed_eligible(p);
   } else return POSEKF_EINVAL;
   const bool batch = p.dt_cols != nullptr || p.n_valid != nullptr;
-  int rc = gate ? launch_gated_algo(p, *gate, algo, lpf, use_tma, packed, innov_model, st)
+  int rc = gen ? launch_general_algo(p, *gen, algo, lpf, use_tma, st)
+           : gate ? launch_gated_algo(p, *gate, algo, lpf, use_tma, packed, innov_model, st)
                 : batch ? launch_kernels<true>(p, algo, lpf, use_tma, packed, innov_model, st)
                         : launch_kernels<false>(p, algo, lpf, use_tma, packed, innov_model, st);
   // (held steps of a batched launch carry flip byte 0, which the fix-up leaves alone)
@@ -304,8 +326,9 @@ const char* posekf_version(void) { return "posekf_b200 0.2 sm_100a"; }
 }  // extern "C"
 
 namespace {
-// Validation and dispatch shared by posekf_replay_f32, posekf_replay_innovation(_ex)_f32, posekf_replay_batch_f32 and
-// posekf_replay_gated_f32 (innov_acc null: the first; dt_cols and n_valid null: the first three; gate: the last).
+// Validation and dispatch shared by posekf_replay_f32, posekf_replay_innovation(_ex)_f32, posekf_replay_batch_f32,
+// posekf_replay_gated_f32 and posekf_replay_general_f32 (innov_acc null: the first; dt_cols and n_valid null: the first
+// three; gate: the gated one; gen: the general one, whose q_scale and r_scale are null).
 // innov_model: POSEKF_INNOV_FULL or POSEKF_INNOV_TANGENT (checked by the caller).
 int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
                  int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_scale,
@@ -313,7 +336,7 @@ int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64
                  float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth, float* loss_acc,
                  float* innov_acc, int innov_model, int wahba_algo, int staging, int state_flags, void* stream,
                  const float* dt_cols = nullptr, const int32_t* n_valid = nullptr, bool gate = false, float gate_nis3 = 0.f,
-                 int32_t* gate_count = nullptr, uint8_t* out_gated = nullptr) {
+                 int32_t* gate_count = nullptr, uint8_t* out_gated = nullptr, const GenQRArgs* gen = nullptr) {
   if (dt_cols && !dt) { dt = dt_cols; dt_per_step = 0; }    // (the kernels read dt[0] unconditionally; it is unused then)
   if (n_filters < 0 || n_steps < 0 || n_streams <= 0 && n_filters > 0) return POSEKF_EINVAL;
   if (state_flags & ~(POSEKF_STATE_IN_FILTER_FRAME | POSEKF_STATE_OUT_FILTER_FRAME)) return POSEKF_EINVAL;
@@ -322,11 +345,11 @@ int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64
     // nothing to replay; a launch is still needed when the state has to change frames
     const bool in_f = state_flags & POSEKF_STATE_IN_FILTER_FRAME, out_f = state_flags & POSEKF_STATE_OUT_FILTER_FRAME;
     if (in_f == out_f || wahba_algo == POSEKF_WAHBA_PRECOMPUTED) return 0;
-    if (!acc_ref || !mag_ref || !q_scale || !r_scale || !state_x || !state_p) return POSEKF_EINVAL;
+    if (!acc_ref || !mag_ref || (!gen && (!q_scale || !r_scale)) || !state_x || !state_p) return POSEKF_EINVAL;
     if (n_streams > n_filters || (n_filters % n_streams) != 0) return POSEKF_EINVAL;
     staging = POSEKF_STAGE_LDG;
   } else if (!streams || !dt) return POSEKF_EINVAL;
-  if (!acc_ref || !mag_ref || !q_scale || !r_scale || !state_x || !state_p) return POSEKF_EINVAL;
+  if (!acc_ref || !mag_ref || (!gen && (!q_scale || !r_scale)) || !state_x || !state_p) return POSEKF_EINVAL;
   if (n_streams > n_filters || (n_filters % n_streams) != 0) return POSEKF_EINVAL;
   const bool lpf = lpf_alpha_acc >= 0.f || lpf_alpha_mag >= 0.f;
   if (lpf && !state_lpf) return POSEKF_EINVAL;
@@ -349,7 +372,7 @@ int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64
   p.dt_cols = n_steps > 0 ? dt_cols : nullptr;
   p.n_valid = n_steps > 0 ? n_valid : nullptr;
   const GateArgs ga{gate_nis3, gate_count, out_gated};
-  return replay_dispatch(p, wahba_algo, staging, innov_model, (cudaStream_t)stream, gate && n_steps > 0 ? &ga : nullptr);
+  return replay_dispatch(p, wahba_algo, staging, innov_model, (cudaStream_t)stream, gate && n_steps > 0 ? &ga : nullptr, gen);
 }
 }  // namespace
 
@@ -414,6 +437,23 @@ int posekf_replay_gated_f32(int64_t n_filters, int64_t n_steps, const float* str
                       lpf_alpha_mag, state_x, state_x_lo, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, innov_acc,
                       innov_model, wahba_algo, staging, state_flags, stream, dt_cols, n_valid, true, gate_nis3, gate_count,
                       out_gated);
+}
+
+int posekf_replay_general_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,
+                              int dt_per_step, const float* acc_ref, const float* mag_ref, const float* q_tri, int64_t nq,
+                              const float* r_tri, int64_t nr, float lpf_alpha_acc, float lpf_alpha_mag, float* state_x,
+                              float* state_x_lo, float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip,
+                              const float* truth, float* loss_acc, float* innov_acc, int innov_model, int wahba_algo,
+                              int staging, int state_flags, void* stream, const float* dt_cols, const int32_t* n_valid) {
+  if (innov_model != POSEKF_INNOV_FULL && innov_model != POSEKF_INNOV_TANGENT) return POSEKF_EINVAL;
+  if (innov_acc || state_x_lo) return POSEKF_EINVAL;     // no innovation sums, no precise variant with general matrices
+  if (n_filters > 0 && (!q_tri || !r_tri || (nq != 1 && nq != n_filters) || (nr != 1 && nr != n_filters))) return POSEKF_EINVAL;
+  if ((reinterpret_cast<uintptr_t>(q_tri) & 3) != 0 || (reinterpret_cast<uintptr_t>(r_tri) & 3) != 0) return POSEKF_EALIGN;
+  const GenQRArgs gq{q_tri, nq, r_tri, nr};
+  return replay_entry(n_filters, n_steps, streams, n_streams, dt, dt_per_step, acc_ref, mag_ref, nullptr, nullptr, lpf_alpha_acc,
+                      lpf_alpha_mag, state_x, nullptr, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, nullptr,
+                      innov_model, wahba_algo, staging, state_flags, stream, dt_cols, n_valid, false, 0.f, nullptr, nullptr,
+                      &gq);
 }
 
 // ---- host-buffer replay: workspace (device staging buffers, streams, events) ----------------------

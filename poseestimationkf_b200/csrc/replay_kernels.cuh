@@ -68,17 +68,41 @@ template <bool AUX> __device__ __forceinline__ void load_gate(const ReplayParams
   g.out = (AUX && ga.out_gated) ? ga.out_gated + n : nullptr;
 }
 
-template <int ALGO, bool LPF, bool COMP, bool INNOV = false, bool TAN = false>
+// General Q and R (GEN kernels): the upper triangles of the matrices, the last kernel parameter of those kernels only
+// (like GateArgs).  Filter n uses column (nq == 1 ? 0 : n) of q_tri and (nr == 1 ? 0 : n) of r_tri; the kernel carries
+// them in the filter frame, Q/4 and R in a register struct of their own (GenRegs; empty NoGenRegs elsewhere).
+struct GenQRArgs {
+  const float* q_tri;       // [6][nq]
+  int64_t nq;
+  const float* r_tri;       // [10][nr]
+  int64_t nr;
+};
+__device__ __forceinline__ GenQRArgs gen_args_(const GenQRArgs& g) { return g; }     // (GEN kernels: their one argument)
+struct GenRegs { GenQR<float> m; };
+struct NoGenRegs {};
+template <bool GEN> using GenRegsOf = typename std::conditional<GEN, GenRegs, NoGenRegs>::type;
+template <int ALGO> __device__ __forceinline__ void load_gen(const GenQRArgs& a, int64_t n, const FilterConst<float>& fc, GenRegs& g) {
+  const int64_t iq = a.nq == 1 ? 0 : n, ir = a.nr == 1 ? 0 : n;
+  float q[6], r[10];
+#pragma unroll
+  for (int k = 0; k < 6; ++k) q[k] = a.q_tri[k * a.nq + iq];
+#pragma unroll
+  for (int k = 0; k < 10; ++k) r[k] = a.r_tri[k * a.nr + ir];
+  g.m = make_gen_qr<float>(fc, q, r, uses_filter_frame<ALGO>());
+}
+
+// (GEN: q_scale / r_scale are not read; the covariance is unscaled, the process noise scale fc.g is 1)
+template <int ALGO, bool LPF, bool COMP, bool INNOV = false, bool TAN = false, bool GEN = false>
 __device__ __forceinline__ void load_filter(const ReplayParams& p, int64_t n, int64_t col, FilterRegs& f) {
   const int64_t N = p.N, Ns = p.Ns;
   Vec3<float> ra = {p.acc_ref[col], p.acc_ref[Ns + col], p.acc_ref[2 * Ns + col]};
   Vec3<float> rm = {p.mag_ref[col], p.mag_ref[Ns + col], p.mag_ref[2 * Ns + col]};
-  f.fc = make_filter_const<float>(ra, rm, p.q_scale[n], p.r_scale[n]);
+  f.fc = make_filter_const<float>(ra, rm, GEN ? 4.f : p.q_scale[n], GEN ? 1.f : p.r_scale[n]);
   if (INNOV) f.in = make_innov_acc<float, TAN>(p.innov_acc[n], p.innov_acc[N + n], p.r_scale[n]);
   f.x = {p.state_x[n], p.state_x[N + n], p.state_x[2 * N + n], p.state_x[3 * N + n]};
   f.xlo = {0.f, 0.f, 0.f, 0.f};
   if (COMP) f.xlo = {p.state_x_lo[n], p.state_x_lo[N + n], p.state_x_lo[2 * N + n], p.state_x_lo[3 * N + n]};
-  const float* sp = p.state_p + n;   // P/r: the step works in units of r (see ekf_step), so does the state buffer
+  const float* sp = p.state_p + n;   // P/r: the step works in units of r (see ekf_step), so does the state buffer (GEN: P)
   f.P = {sp[0], sp[N], sp[2 * N], sp[3 * N], sp[4 * N], sp[5 * N], sp[6 * N], sp[7 * N], sp[8 * N], sp[9 * N]};
   if (LPF) {
     const float* sl = p.state_lpf + n;
@@ -126,9 +150,9 @@ template <bool AUX> __device__ __forceinline__ AuxPtrs make_aux(const ReplayPara
   return a;
 }
 
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool GATE = false>
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool GATE = false, bool GEN = false>
 __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f, const float (&s)[kChannels], float h,
-                                            AuxPtrs& aux, GateRegsOf<GATE>& g) {
+                                            AuxPtrs& aux, GateRegsOf<GATE>& g, const GenRegsOf<GEN>* gr = nullptr) {
   Vec3<float> w = {s[0], s[1], s[2]}, a = {s[3], s[4], s[5]}, m = {s[6], s[7], s[8]};
   if (LPF) {   // SRV/KalmanFilter.cpp:285,298 -- filtered values feed Wahba, not renormalised
     if (p.alpha_acc >= 0.f) { lowpass<float>(f.la, a, p.alpha_acc, 1.f - p.alpha_acc); a = f.la; }
@@ -145,6 +169,10 @@ __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f
                                                        &g.gp, &gated);
     g.count += gated ? 1 : 0;
     if (g.out) { *g.out = gated ? 1 : 0; g.out += p.N; }
+  } else if constexpr (GEN) {
+    ekf_step<float, ALGO, AUX, false, false, false, false, true>(f.x, f.xlo, f.P, f.fc, w, a, m, StepH<float>(h), flip,
+                                                                aux.flips != nullptr, (AUX && !LPF && ALGO == WAHBA_QR2) ? &code : nullptr,
+                                                                nullptr, nullptr, (bool*)nullptr, &gr->m);
   } else {
     ekf_step<float, ALGO, AUX, COMP, INNOV, TAN>(f.x, f.xlo, f.P, f.fc, w, a, m, StepH<float>(h), flip, aux.flips != nullptr,
                                                  (AUX && !LPF && ALGO == WAHBA_QR2) ? &code : nullptr, INNOV ? &f.in : nullptr);
@@ -199,20 +227,23 @@ __device__ __forceinline__ void hold_step(const ReplayParams& p, const FilterReg
 // ---------------------------------------------------------------------------------------------
 // (INNOV: the innovation likelihood, TAN: its tangent-space form; their instantiations always have AUX and are built for
 //  3 CTAs per SM, <= 168 registers.  BATCH: per-stream dt columns and lengths, ReplayParams::dt_cols / n_valid)
-//  GATE: the innovation gate, its arguments in the pack ga (one GateArgs; empty in the other kernels))
+//  GATE: the innovation gate, its arguments in the pack ga (one GateArgs; empty in the other kernels).
+//  GEN: general Q and R matrices, the pack holds one GenQRArgs; plain variant, no innovation sums, no gate)
 template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false, bool GATE = false,
-          typename... GA>
-__global__ void __launch_bounds__(kThreads, (INNOV || GATE) ? 3 : ((ALGO == WAHBA_JACOBI || (COMP && LPF && AUX)) ? 4 : ((COMP || LPF) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
+          bool GEN = false, typename... GA>
+__global__ void __launch_bounds__(kThreads, (INNOV || GATE || GEN) ? 3 : ((ALGO == WAHBA_JACOBI || (COMP && LPF && AUX)) ? 4 : ((COMP || LPF) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
     replay_ldg_kernel(const ReplayParams p, GA... ga) {
   const int64_t n = (int64_t)blockIdx.x * kThreads + threadIdx.x;
   if (n >= p.N) return;
   const int64_t Ns = p.Ns;
   const int64_t col = (Ns == p.N) ? n : (n % Ns);
   FilterRegs f;
-  load_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, col, f);
+  load_filter<ALGO, LPF, COMP, INNOV, TAN, GEN>(p, n, col, f);
   AuxPtrs aux = make_aux<AUX>(p, n, col, true);
   [[maybe_unused]] GateRegsOf<GATE> g;
   if constexpr (GATE) load_gate<AUX>(p, gate_args_(ga...), n, g);
+  [[maybe_unused]] GenRegsOf<GEN> gr;
+  if constexpr (GEN) load_gen<ALGO>(gen_args_(ga...), n, f.fc, gr);
   const float* s = p.streams + col;
   const int64_t step_stride = kChannels * Ns;
   float cur[kChannels], nxt[kChannels];
@@ -231,7 +262,7 @@ __global__ void __launch_bounds__(kThreads, (INNOV || GATE) ? 3 : ((ALGO == WAHB
     for (int c = 0; c < kChannels; ++c) nxt[c] = ldg_stream(s + c * Ns);
     if (BATCH && dc) hnxt = ldg_stream(dc + (int64_t)(t + 1 < T ? t + 1 : t) * Ns);
     const float h = (BATCH && dc) ? hcur : (p.dt_per_step ? __ldg(p.dt + t) : dt0);
-    if (!BATCH || t < nv) filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE>(p, f, cur, h, aux, g);
+    if (!BATCH || t < nv) filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE, GEN>(p, f, cur, h, aux, g, &gr);
     else hold_step<ALGO, AUX, GATE>(p, f, aux, g);
 #pragma unroll
     for (int c = 0; c < kChannels; ++c) cur[c] = nxt[c];
@@ -283,8 +314,8 @@ struct __align__(128) TmaSmem {
 constexpr uint32_t kTileBytes = kTmaSteps * kChannels * kThreads * sizeof(float);
 
 template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false, bool GATE = false,
-          typename... GA>
-__global__ void __launch_bounds__(kThreads, (INNOV || GATE) ? 3 : (ALGO == WAHBA_JACOBI ? 4 : ((COMP && (LPF || AUX)) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
+          bool GEN = false, typename... GA>
+__global__ void __launch_bounds__(kThreads, (INNOV || GATE || GEN) ? 3 : (ALGO == WAHBA_JACOBI ? 4 : ((COMP && (LPF || AUX)) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
     replay_tma_kernel(const ReplayParams p, const __grid_constant__ CUtensorMap tmap, GA... ga) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   TmaSmem& sm = *reinterpret_cast<TmaSmem*>(smem_raw);
@@ -314,10 +345,12 @@ __global__ void __launch_bounds__(kThreads, (INNOV || GATE) ? 3 : (ALGO == WAHBA
   }
 
   FilterRegs f;
-  if (valid) load_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, (int64_t)col0 + tid, f);
+  if (valid) load_filter<ALGO, LPF, COMP, INNOV, TAN, GEN>(p, n, (int64_t)col0 + tid, f);
   AuxPtrs aux = make_aux<AUX>(p, n, (int64_t)col0 + tid, valid);
   [[maybe_unused]] GateRegsOf<GATE> g;
   if constexpr (GATE) { if (valid) load_gate<AUX>(p, gate_args_(ga...), n, g); }
+  [[maybe_unused]] GenRegsOf<GEN> gr;
+  if constexpr (GEN) { if (valid) load_gen<ALGO>(gen_args_(ga...), n, f.fc, gr); }
   const float dt0 = p.dt[0];
   // BATCH: this stream's length, and the time steps of the next tile held in registers (loaded one tile ahead: the
   // shared-memory ring has no room left at this kernel's occupancy)
@@ -357,10 +390,10 @@ __global__ void __launch_bounds__(kThreads, (INNOV || GATE) ? 3 : (ALGO == WAHBA
 #pragma unroll
           for (int c = 0; c < kChannels; ++c) s[c] = sm.tile[stage][tt][c][tid];
           if constexpr (BATCH) {
-            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE>(p, f, s, bt.cur[tt], aux, g);
+            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE, GEN>(p, f, s, bt.cur[tt], aux, g, &gr);
           } else {
             const float h = p.dt_per_step ? __ldg(p.dt + k * kTmaSteps + tt) : dt0;
-            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE>(p, f, s, h, aux, g);
+            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE, GEN>(p, f, s, h, aux, g, &gr);
           }
         }
       }

@@ -2,9 +2,10 @@
 """Registers, spills and stack of every kernel of the last library build, from the `-Xptxas -v` log that
 `poseestimationkf_b200/build.py` writes beside the library (build_ptxas.log), with demangled names.
 
-  python tools/ptxas_report.py [--match replay_] [--gated] [--out profiles/r06_gating_registers.json]
+  python tools/ptxas_report.py [--match replay_] [--gated | --general] [--out profiles/r06_gating_registers.json]
 
---gated keeps the replay kernels instantiated with the innovation gate (the GATE template flag set).
+--gated keeps the replay kernels instantiated with the innovation gate (the GATE template flag set), --general those
+instantiated with general Q and R matrices (the GEN flag of the scalar kernels set).
 """
 from __future__ import annotations
 
@@ -36,12 +37,20 @@ def entries(log_text: str):
     return out
 
 
-def is_gated(kernel: str) -> bool:
+def _flag(kernel: str, i: int) -> bool:
     m = re.search(r"replay_\w+_kernel<([^>]*)>", kernel)
     if not m:
         return False
     args = [a.strip() for a in m.group(1).split(",")]
-    return len(args) >= 8 and args[7] == "true"
+    return len(args) > i and args[i] == "true"
+
+
+def is_gated(kernel: str) -> bool:
+    return _flag(kernel, 7)
+
+
+def is_general(kernel: str) -> bool:
+    return _flag(kernel, 8)
 
 
 def main():
@@ -49,9 +58,11 @@ def main():
     ap.add_argument("--log", default=os.path.join(ROOT, "poseestimationkf_b200", "build_ptxas.log"))
     ap.add_argument("--match", default="")
     ap.add_argument("--gated", action="store_true")
+    ap.add_argument("--general", action="store_true")
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
-    ents = [e for e in entries(open(a.log).read()) if a.match in e["kernel"] and (not a.gated or is_gated(e["kernel"]))]
+    ents = [e for e in entries(open(a.log).read()) if a.match in e["kernel"] and (not a.gated or is_gated(e["kernel"]))
+            and (not a.general or is_general(e["kernel"]))]
     for e in ents:
         del e["mangled"]
     res = {"source": "ptxas -v of the sm_100a build (nvcc flags of poseestimationkf_b200/build.py)",
