@@ -325,6 +325,35 @@ int posekf_preprocess_f32(int64_t n_filters, int64_t n_steps, const float* gyro,
 int posekf_initial_values_f32(int64_t n_filters, int64_t n_samples, const float* samples, int normalize, float* out_mean,
                               float* out_var, void* stream);
 
+/* Raw event recordings -> the batch of posekf_replay_batch_f32 (what SRV/Parser.cpp:148-267 does per event, for a
+ * batch of recordings in one call; DESIGN section 5 f10).
+ * Input: n_rec recordings, each with a gyro, an accelerometer and a magnetometer event stream.  Per sensor s the
+ * streams are concatenated: t_s [M_s] int64 ns, v_s [3][M_s] float32, off_s [n_rec+1] int64; recording c owns events
+ * off_s[c] .. off_s[c+1]-1 and M_s = off_s[n_rec].  PRECONDITION (not checked here, like n_valid of
+ * posekf_replay_batch_f32): timestamps strictly increase within each recording's stream, and each recording has fewer
+ * than 2^31 gyro events.
+ *   acc_ref / mag_ref [3][n_rec]: the normalised means of the recording's first k_init acc / mag events (float64 sums in
+ *     arrival order, as posekf_initial_values_f32; k_init = 100 in SRV/Parser.cpp:5-7).  t_init: the later of the two
+ *     k_init-th timestamps.  A recording with fewer than k_init events of either sensor has length 0 and the
+ *     references (0,0,1) / (1,0,0).
+ *   lengths [n_rec] int32: the number of steps.  The steps are the gyro events g with t_g > t_init that both sensors
+ *     bracket (an event at t1 <= t_g and one at t2 > t_g); they are consecutive gyro events.
+ *   streams [t_out][9][n_rec]: step i of recording c is gyro event i of its steps, with acc and mag interpolated from
+ *     the LAST event at or before t_g and the FIRST event after it and normalised, with the operations of
+ *     posekf_preprocess_f32 (same device function); t2 - t1 and t_g - t1 are differenced in int64 ns, then converted
+ *     to float seconds as (float)(d * 1e-9) in double.
+ *   dt_cols [t_out][n_rec] seconds: (t_g(i) - t_g(i-1)) * 1e-9, and (t_g(0) - t_init) * 1e-9 for step 0, differenced
+ *     in int64 and rounded to float32 once.
+ *   Steps i >= lengths[c] (padding, never read by a replay with n_valid = lengths): the last step repeated with dt 0;
+ *     for a recording of length 0, gyro 0 and its reference vectors (the convention of logio.stack_logs).
+ * Query mode: streams NULL writes lengths only (the values, dt_cols and the references may be NULL), so that the caller
+ * can size t_out >= max(lengths) with one read-back.  With t_out < max(lengths) only the first t_out steps are written.
+ * POSEKF_EINVAL: n_rec < 0, t_out < 0, k_init < 1, or a NULL required pointer. */
+int posekf_align_events_f32(int64_t n_rec, int64_t k_init, const int64_t* gyro_t, const float* gyro_v, const int64_t* gyro_off,
+                            const int64_t* acc_t, const float* acc_v, const int64_t* acc_off, const int64_t* mag_t,
+                            const float* mag_v, const int64_t* mag_off, int64_t t_out, float* streams, float* dt_cols,
+                            int32_t* lengths, float* acc_ref, float* mag_ref, void* stream);
+
 /* Measurement stream for POSEKF_WAHBA_PRECOMPUTED.  The Wahba solution of a sample does not depend on Q or R,
  * so a tuning sweep that replays Ns trajectories N/Ns times solves it ONCE per (trajectory, step):
  *   streams [T][9][Ns] (gyro, acc, mag) -> out_streams [T][9][Ns]: rows 0-2 gyro, rows 3-6 the quaternion of

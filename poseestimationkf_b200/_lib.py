@@ -39,6 +39,8 @@ _SIGNATURES = {
     "posekf_measurement_stream_f32": [_i64, _i64, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _int, _vp],
     "posekf_initial_values_f32": [_i64, _i64, _vp, _int, _vp, _vp, _vp],
     "posekf_preprocess_f32": [_i64, _i64, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp],
+    "posekf_align_events_f32": [_i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp,
+                                _vp],
     "posekf_rot2quat_f32": [_i64, _vp, _vp, _vp],
     "posekf_predict_f32": [_i64, _vp, _vp, _int, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "posekf_correct_f32": [_i64, _vp, _vp, _vp, _vp, _int, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _int, _vp],

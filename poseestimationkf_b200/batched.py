@@ -798,6 +798,41 @@ def initial_values(samples, *, normalize: bool = True, want_variance: bool = Fal
     return mean, var
 
 
+def align_events(gyro_t, gyro_v, gyro_off, acc_t, acc_v, acc_off, mag_t, mag_v, mag_off, *, k_init: int = 100):
+    """Raw event recordings -> (streams [T,9,Ns], dt [T,Ns], lengths [Ns] int32, acc_ref [3,Ns], mag_ref [3,Ns]) on the
+    device (`posekf_align_events_f32`, whose header comment has the rules).  Per sensor: t [M] int64 ns, v [3,M] float32,
+    off [Ns+1] int64 CUDA tensors, recording c owning events off[c]..off[c+1]-1, timestamps strictly increasing within a
+    recording (checked by `logio.align_recordings`).  T = max(lengths), found with a first lengths-only call."""
+    ts, vs, offs = (gyro_t, acc_t, mag_t), (gyro_v, acc_v, mag_v), (gyro_off, acc_off, mag_off)
+    _require_cuda(*vs)
+    for t, v, off in zip(ts, vs, offs):
+        if not (t.is_cuda and off.is_cuda and t.dtype == torch.int64 and off.dtype == torch.int64):
+            raise TypeError("timestamps and offsets must be int64 CUDA tensors")
+        if not (t.is_contiguous() and off.is_contiguous()) or t.dim() != 1 or v.shape != (3, t.shape[0]):
+            raise ValueError("each sensor needs contiguous t [M] and v [3, M]")
+        if off.shape != gyro_off.shape or off.dim() != 1:
+            raise ValueError("the offsets of the three sensors must all be [Ns + 1]")
+    Ns = gyro_off.shape[0] - 1
+    dev = gyro_t.device
+    lib = _lib.load()
+    args = [Ns, int(k_init), _ptr(gyro_t), _ptr(gyro_v), _ptr(gyro_off), _ptr(acc_t), _ptr(acc_v), _ptr(acc_off), _ptr(mag_t),
+            _ptr(mag_v), _ptr(mag_off)]
+    lengths = torch.empty((max(Ns, 0),), dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.posekf_align_events_f32(*args, 0, None, None, _ptr(lengths), None, None, _stream()),
+                   "posekf_align_events_f32")
+        T = int(lengths.max().item()) if Ns > 0 else 0
+        # one row at least, whose pointer is passed: with T = 0 an empty tensor's NULL pointer would select the
+        # lengths-only call again, and the reference vectors would not be written
+        streams = torch.empty((max(T, 1), 9, Ns), dtype=torch.float32, device=dev)
+        dt = torch.empty((max(T, 1), Ns), dtype=torch.float32, device=dev)
+        acc_ref = torch.empty((3, Ns), dtype=torch.float32, device=dev)
+        mag_ref = torch.empty((3, Ns), dtype=torch.float32, device=dev)
+        _lib.check(lib.posekf_align_events_f32(*args, T, _ptr(streams), _ptr(dt), _ptr(lengths), _ptr(acc_ref), _ptr(mag_ref),
+                                               _stream()), "posekf_align_events_f32")
+    return streams[:T], dt[:T], lengths, acc_ref, mag_ref
+
+
 def traj2rpy(traj):
     """Quart2RPY over a stored trajectory [..., 4] -> degrees [..., 3]."""
     _require_cuda(traj)

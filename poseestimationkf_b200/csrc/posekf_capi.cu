@@ -721,6 +721,36 @@ int posekf_initial_values_f32(int64_t n_filters, int64_t n_samples, const float*
   return launch_status();
 }
 
+int posekf_align_events_f32(int64_t n_rec, int64_t k_init, const int64_t* gyro_t, const float* gyro_v, const int64_t* gyro_off,
+                            const int64_t* acc_t, const float* acc_v, const int64_t* acc_off, const int64_t* mag_t,
+                            const float* mag_v, const int64_t* mag_off, int64_t t_out, float* streams, float* dt_cols,
+                            int32_t* lengths, float* acc_ref, float* mag_ref, void* stream) {
+  if (n_rec < 0 || t_out < 0 || k_init < 1) return POSEKF_EINVAL;
+  if (n_rec == 0) return 0;
+  if (!gyro_t || !gyro_off || !acc_t || !acc_off || !mag_t || !mag_off || !lengths) return POSEKF_EINVAL;
+  const bool query = streams == nullptr;
+  if (!query && (!gyro_v || !acc_v || !mag_v || !dt_cols || !acc_ref || !mag_ref)) return POSEKF_EINVAL;
+  const int64_t col_tiles = (n_rec + kAlignTile - 1) / kAlignTile, step_tiles = (t_out + kAlignTile - 1) / kAlignTile;
+  if (blocks_for(n_rec, 256) > 0x7fffffffu || col_tiles * step_tiles > 0x7fffffffLL) return POSEKF_EINVAL;
+  cudaStream_t st = (cudaStream_t)stream;
+  AlignParams p{n_rec, t_out, k_init, gyro_t, acc_t, mag_t, gyro_v, acc_v, mag_v, gyro_off, acc_off, mag_off, lengths, nullptr,
+                acc_ref, mag_ref, streams, dt_cols};
+  if (query) {
+    align_bounds_kernel<<<blocks_for(n_rec, 256), 256, 0, st>>>(p);
+    return launch_status();
+  }
+  // the step-0 gyro index and t_init of every recording, from the first kernel to the second (stream-ordered scratch)
+  PKF_CUDA_TRY(cudaMallocAsync((void**)&p.bounds, (size_t)2 * n_rec * sizeof(int64_t), st));
+  align_bounds_kernel<<<blocks_for(n_rec, 256), 256, 0, st>>>(p);
+  int rc = launch_status();
+  if (rc == 0 && t_out > 0) {
+    align_events_kernel<<<(unsigned)(col_tiles * step_tiles), dim3(kAlignTile, kAlignWarps), 0, st>>>(p, col_tiles);
+    rc = launch_status();
+  }
+  const cudaError_t e = cudaFreeAsync(p.bounds, st);
+  return rc != 0 ? rc : (e == cudaSuccess ? 0 : (int)e);
+}
+
 int posekf_measurement_stream_f32(int64_t n_streams, int64_t n_steps, const float* streams, const float* acc_ref,
                                   const float* mag_ref, float lpf_alpha_acc, float lpf_alpha_mag, float* lpf_state,
                                   float* out_streams, int wahba_algo, void* stream) {

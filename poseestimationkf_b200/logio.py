@@ -108,6 +108,69 @@ def stack_logs(logs, device="cuda", pad_cols_to: int = 4) -> LogBatch:
     return LogBatch(t(streams), t(acc_ref), t(mag_ref), t(dt), t(lengths), K)
 
 
+@dataclass
+class SensorEvents:
+    """One sensor's event stream: t_ns [M] int64 timestamps in ns (strictly increasing), v [M,3] float32 values."""
+    t_ns: np.ndarray
+    v: np.ndarray
+
+
+@dataclass
+class RawRecording:
+    """A raw recording as a phone sends it: each sensor's events at its own rate and with its own timestamps."""
+    gyro: SensorEvents
+    acc: SensorEvents
+    mag: SensorEvents
+
+
+def _pack_sensor(events, name: str):
+    """Concatenate one sensor of every recording: (t [M] int64, v [3,M] float32, off [len+1] int64), host arrays."""
+    ts, vs = [], []
+    for c, e in enumerate(events):
+        t = np.asarray(e.t_ns)
+        v = np.asarray(e.v)
+        if t.dtype.kind not in "iu":
+            raise TypeError(f"recording {c}: {name} timestamps must be integer ns")
+        if t.ndim != 1 or v.shape != (t.shape[0], 3):
+            raise ValueError(f"recording {c}: {name} needs t_ns [M] and v [M,3], got {t.shape} and {v.shape}")
+        t = t.astype(np.int64)
+        if t.size > 1 and not (np.diff(t) > 0).all():
+            raise ValueError(f"recording {c}: {name} timestamps are not strictly increasing")
+        ts.append(t)
+        vs.append(np.asarray(v, dtype=np.float32))
+    off = np.zeros(len(ts) + 1, dtype=np.int64)
+    off[1:] = np.cumsum([t.size for t in ts])
+    t = np.concatenate(ts) if ts else np.zeros(0, dtype=np.int64)
+    v = np.concatenate(vs).T if vs else np.zeros((3, 0), dtype=np.float32)
+    return t, np.ascontiguousarray(v), off
+
+
+def align_recordings(recs, device="cuda", k_init: int = 100, pad_cols_to: int = 4) -> LogBatch:
+    """Raw event recordings (`RawRecording`) -> the `LogBatch` that `stack_logs` returns, aligned to each recording's
+    gyro clock on the device in one call (`batched.align_events`; the rules are `posekf_align_events_f32`'s in
+    include/posekf.h): reference vectors from the first `k_init` acc / mag events, one step per gyro event after them
+    that both sensors bracket, acc / mag interpolated to the gyro timestamp and normalised, dt from the gyro timestamps.
+    The number of columns is rounded up to a multiple of `pad_cols_to` with empty recordings, as in `stack_logs`.  The
+    replay's own low-pass (`lpf_alpha_acc/mag`) is not applied here."""
+    import torch
+    from . import batched as B
+    if int(k_init) < 1:
+        raise ValueError("k_init must be >= 1")
+    recs = list(recs)
+    K = len(recs)
+    Ns = -(-K // pad_cols_to) * pad_cols_to if pad_cols_to > 1 else K
+    empty = SensorEvents(np.zeros(0, dtype=np.int64), np.zeros((0, 3), dtype=np.float32))
+    packed = []
+    for name in ("gyro", "acc", "mag"):
+        t, v, off = _pack_sensor([getattr(r, name) for r in recs] + [empty] * (Ns - K), name)
+        if name == "gyro" and off.size > 1 and int(np.diff(off).max()) >= 2 ** 31:
+            raise ValueError("a recording has 2^31 gyro events or more")
+        dev = torch.device(device)
+        packed += [torch.from_numpy(t).to(dev), torch.from_numpy(v).to(dev), torch.from_numpy(off).to(dev)]
+    streams, dt, lengths, acc_ref, mag_ref = B.align_events(*packed, k_init=int(k_init))
+    return LogBatch(streams, acc_ref, mag_ref, dt, lengths, K)
+
+
 def _values(line: str):
     """ReadFile.py:14-21 (`getArray`): text after the first ':' split on ','."""
     return [float(v) for v in line.split(":")[1].split(",")]

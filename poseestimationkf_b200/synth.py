@@ -61,6 +61,27 @@ def _unit(v):
     return v / torch.linalg.vector_norm(v, dim=0, keepdim=True)
 
 
+def _reference_pair(U, N, az_range, f64):
+    """Gravity and field in the body frame at the start (float64 [3,N] each), drawn with the uniform sampler U."""
+    # initial tilt: gravity in the body frame has |z| = cos(tilt) in az_range, random azimuth
+    az = U(az_range[0] + 0.03, az_range[1] - 0.03, N) * torch.where(U(0, 1, N) < 0.5, -1.0, 1.0)
+    psi = U(0.0, 2 * math.pi, N)
+    s = torch.sqrt(1 - az * az)
+    acc0 = torch.stack((s * torch.cos(psi), s * torch.sin(psi), az))
+    # field: fixed angle to gravity (world: g=(0,0,1), m=normalize(0.4,0,-0.9165)); pick the
+    # horizontal direction at a random heading around gravity
+    mw = torch.tensor([0.4, 0.0, -0.9165], **f64)
+    mw = mw / torch.linalg.vector_norm(mw)
+    hdg = U(0.0, 2 * math.pi, N)
+    helper = torch.where((acc0[2].abs() < 0.9).unsqueeze(0),
+                         torch.tensor([0.0, 0.0, 1.0], **f64).unsqueeze(1).expand(3, N),
+                         torch.tensor([1.0, 0.0, 0.0], **f64).unsqueeze(1).expand(3, N))
+    e1 = _unit(torch.linalg.cross(acc0, helper, dim=0))
+    e2 = torch.linalg.cross(acc0, e1, dim=0)
+    horiz = torch.cos(hdg) * e1 + torch.sin(hdg) * e2
+    return acc0, _unit(mw[2] * acc0 + mw[0] * horiz)
+
+
 def make_imu(n_filters: int, n_steps: int, *, seed: int = 0, sigma: float = 0.0, dt: float = 0.01,
              device="cpu", keep_truth: bool = False, out: torch.Tensor | None = None,
              az_range=(0.02, 0.98)) -> SyntheticIMU:
@@ -83,24 +104,7 @@ def make_imu(n_filters: int, n_steps: int, *, seed: int = 0, sigma: float = 0.0,
         return lo + (hi - lo) * torch.rand(*shape, generator=g, **f64)
 
     amp, freq, phase = U(0.2, 1.0, 3, 3, N), U(0.05, 0.5, 3, 3, N), U(0.0, 2 * math.pi, 3, 3, N)
-
-    # initial tilt: gravity in the body frame has |z| = cos(tilt) in az_range, random azimuth
-    az = U(az_range[0] + 0.03, az_range[1] - 0.03, N) * torch.where(U(0, 1, N) < 0.5, -1.0, 1.0)
-    psi = U(0.0, 2 * math.pi, N)
-    s = torch.sqrt(1 - az * az)
-    acc0 = torch.stack((s * torch.cos(psi), s * torch.sin(psi), az))
-    # field: fixed angle to gravity (world: g=(0,0,1), m=normalize(0.4,0,-0.9165)); pick the
-    # horizontal direction at a random heading around gravity
-    mw = torch.tensor([0.4, 0.0, -0.9165], **f64)
-    mw = mw / torch.linalg.vector_norm(mw)
-    hdg = U(0.0, 2 * math.pi, N)
-    helper = torch.where((acc0[2].abs() < 0.9).unsqueeze(0),
-                         torch.tensor([0.0, 0.0, 1.0], **f64).unsqueeze(1).expand(3, N),
-                         torch.tensor([1.0, 0.0, 0.0], **f64).unsqueeze(1).expand(3, N))
-    e1 = _unit(torch.linalg.cross(acc0, helper, dim=0))
-    e2 = torch.linalg.cross(acc0, e1, dim=0)
-    horiz = torch.cos(hdg) * e1 + torch.sin(hdg) * e2
-    mag0 = _unit(mw[2] * acc0 + mw[0] * horiz)
+    acc0, mag0 = _reference_pair(U, N, az_range, f64)
 
     if out is None:
         out = torch.empty((T, N_CHANNELS, N), dtype=torch.float32, device=dev)
@@ -174,3 +178,89 @@ def add_disturbances(streams: torch.Tensor, *, seed: int = 1, n_mag: int = 3, n_
             streams[:, rows] = torch.where(on[:, None], v.to(torch.float32), streams[:, rows])
             mask |= on
     return mask
+
+
+@dataclass
+class SyntheticEvents:
+    """recordings : list of `logio.RawRecording` (int64 ns timestamps, float32 values)
+    truth      : list of [Mg, 4] float64 true attitudes at each gyro timestamp, or None
+    acc0, mag0 : [3, n_rec] float64 noise-free gravity and field in the body frame at rest"""
+    recordings: list
+    truth: list | None
+    acc0: torch.Tensor
+    mag0: torch.Tensor
+
+
+def make_events(n_rec: int, duration_s, *, rates=(200.0, 100.0, 100.0), jitter: float = 0.2, sigma: float = 0.0,
+                seed: int = 0, keep_truth: bool = False, still_s: float = 1.5, t0_ns: int = 1_700_000_000_000_000_000,
+                az_range=(0.02, 0.98)) -> SyntheticEvents:
+    """Asynchronous raw event recordings from `make_imu`'s motion model: the same body-rate model and reference
+    geometry, with the device at rest for the first `still_s` seconds (the phase whose first 100 acc / mag events make
+    the reference vectors) and the rate model running from then on.  Each sensor has its own sample clock: event k of
+    a sensor at rate f is at t0_ns + (phase + k + jitter * u_k) / f seconds, phase ~ U(0,1), u_k ~ U(-1/2,1/2), rounded
+    to integer ns; jitter < 1 keeps the timestamps strictly increasing.  `duration_s` and each entry of `rates` are
+    scalars or one value per recording.  Gyro events are the body rate at their timestamp, acc / mag the reference
+    vectors rotated into the body frame; noise sigma on all three, acc / mag renormalised; float64, rounded to float32
+    once.  The true attitude (body -> rest frame, identity at rest) is integrated with `make_imu`'s exact exponential of
+    the mid-point rate over the merged event times of each recording and kept at every gyro timestamp."""
+    from .logio import RawRecording, SensorEvents
+    if not 0.0 <= jitter < 1.0:
+        raise ValueError("jitter must be in [0, 1)")
+    g = torch.Generator(device="cpu")
+    g.manual_seed(seed)
+    f64 = dict(dtype=torch.float64)
+    N = n_rec
+
+    def U(lo, hi, *shape):
+        return lo + (hi - lo) * torch.rand(*shape, generator=g, **f64)
+
+    amp, freq, phase = U(0.2, 1.0, 3, 3, N), U(0.05, 0.5, 3, 3, N), U(0.0, 2 * math.pi, 3, 3, N)
+    acc0, mag0 = _reference_pair(U, N, az_range, f64)
+    per_rec = lambda x: torch.as_tensor(x, **f64).expand(N).clone()
+    dur = per_rec(duration_s)
+    rate = [per_rec(r) for r in rates]
+
+    def omega(c, t):
+        """body rate [3, n] of recording c at times t [n] (seconds since t0)"""
+        tm = (t - still_s).clamp_min(0.0)
+        w = (amp[:, :, c, None] * torch.sin(2 * math.pi * freq[:, :, c, None] * tm + phase[:, :, c, None])).sum(dim=1)
+        return torch.where(t >= still_s, w, torch.zeros_like(w))
+
+    def noisy(v):
+        return v if sigma == 0.0 else v + sigma * torch.randn(v.shape, generator=g, **f64)
+
+    recs, truth = [], [] if keep_truth else None
+    for c in range(N):
+        times = []
+        for f in rate:
+            fc = float(f[c])
+            n = int(math.floor(float(dur[c]) * fc))
+            k = torch.arange(n, **f64)
+            t = (U(0.0, 1.0, 1) + k + jitter * (U(0.0, 1.0, n) - 0.5)) / fc
+            times.append(torch.round(t * 1e9).to(torch.int64))                    # ns since t0
+        # attitude at the merged event times: the exact exponential of the mid-point rate over each interval
+        u = torch.unique(torch.cat(times))
+        us = u.to(torch.float64) * 1e-9
+        h = torch.diff(torch.cat((torch.zeros(1, **f64), us)))
+        w_mid = omega(c, us - 0.5 * h)
+        ang = torch.linalg.vector_norm(w_mid, dim=0) * h
+        half = 0.5 * ang
+        sinc = torch.where(ang > 1e-12, torch.sin(half) / ang.clamp_min(1e-300), torch.full_like(ang, 0.5))
+        dq = torch.cat((torch.cos(half)[None], w_mid * h * sinc), dim=0)          # [4, n]
+        q = torch.empty_like(dq)
+        cur = torch.tensor([1.0, 0.0, 0.0, 0.0], **f64)[:, None]
+        for i in range(dq.shape[1]):
+            cur = _quat_mul(cur, dq[:, i:i + 1])
+            cur = cur / torch.linalg.vector_norm(cur, dim=0, keepdim=True)
+            q[:, i] = cur[:, 0]
+        at = lambda t_ns: q[:, torch.searchsorted(u, t_ns)]
+        tg, ta, tm = times
+        qa, qm = at(ta), at(tm)
+        gyro = noisy(omega(c, tg.to(torch.float64) * 1e-9))
+        acc = _unit(noisy(_rotate_inverse(qa, acc0[:, c, None].expand(3, qa.shape[1]))))
+        mag = _unit(noisy(_rotate_inverse(qm, mag0[:, c, None].expand(3, qm.shape[1]))))
+        ev = lambda t, v: SensorEvents((t + t0_ns).numpy(), v.t().to(torch.float32).numpy())
+        recs.append(RawRecording(ev(tg, gyro), ev(ta, acc), ev(tm, mag)))
+        if keep_truth:
+            truth.append(at(tg).t().numpy())
+    return SyntheticEvents(recs, truth, acc0, mag0)

@@ -162,7 +162,13 @@ def build_multi_recording_sweep(logs, device, grid: int = C3_GRID, lo: float = -
     it with `run_c3(w, objective="innovation_tangent")` and read `pooled_innovation_surface`, whose argmin is the one
     (Q,R) that best explains every recording together."""
     from .logio import stack_logs
-    b = stack_logs(logs, device)
+    return build_batch_sweep(stack_logs(logs, device), grid, lo, step)
+
+
+def build_batch_sweep(b, grid: int = C3_GRID, lo: float = -7.0, step: float = 0.1) -> SweepWorkload:
+    """`build_multi_recording_sweep` over a `logio.LogBatch` that is already on the device, such as the one
+    `logio.align_recordings` makes from raw event recordings."""
+    device = b.streams.device
     Ns = b.streams.shape[2]
     hi = lo + step * (grid - 1)
     qs = torch.logspace(lo, hi, grid, device=device)
