@@ -221,6 +221,37 @@ int posekf_replay_gated_f32(int64_t n_filters, int64_t n_steps, const float* str
                             void* stream, const float* dt_cols, const int32_t* n_valid, float gate_nis3, int32_t* gate_count,
                             uint8_t* out_gated);
 
+/* Per-step innovation output: the replay of posekf_replay_gated_f32 (same parameters, same rules) that also writes the
+ * terms each step adds to the innovation sums, so that a recording can be scored step by step or window by window
+ * (where the filter is inconsistent, a gate threshold from a quantile of clean data, the likelihood of one segment).
+ *   out_innov   [2][T][N] float32 (planes innov_plane_stride elements apart), required unless n_steps * n_filters = 0
+ *               (NULL: POSEKF_EINVAL), 4-byte aligned (else POSEKF_EALIGN).  out_innov[0][t][n] = NIS_t, out_innov[innov_plane_stride + t N + n] =
+ *               ln det S_t of filter n, in the convention of innov_acc: natural log, true units, without the
+ *               (dof/2) ln 2 pi constant; the model is innov_model (POSEKF_INNOV_FULL: the 4-D terms,
+ *               POSEKF_INNOV_TANGENT: NIS3_t and ln det S3_t).  Filter index fastest, like out_gated.
+ *   innov_plane_stride  elements from plane 0 to plane 1, >= n_steps * n_filters (else POSEKF_EINVAL): a time chunk
+ *               t0..t1 of a replay can write straight into its slice of a full-length [2][T_total][N] buffer (plane
+ *               stride T_total N, base out_innov + t0 N).
+ *   innov_acc   may be NULL: the launch then writes the per-step terms only.  With a buffer, both.
+ * Held steps (t >= n_valid) write 0 to both planes, so for every filter sum_t out_innov[k][t][n] is what the launch adds
+ * to innov_acc[k][n] up to float32 summation: ln det S_t is the addend of the sum itself, NIS_t the product the sum's
+ * fused multiply-add adds, rounded on its own (one rounding per step apart).  Gated steps write their terms like any
+ * other step; with POSEKF_INNOV_TANGENT plane 0 is the statistic the gate thresholded (the gate compares r NIS3 with
+ * gate_nis3 r, so its decisions agree with out_innov[0] > gate_nis3 except at ties within rounding).
+ * gate_nis3 = +inf with gate_count and out_gated NULL is an ungated launch.  Every other output (state, P, trajectory,
+ * flips, loss, innov_acc, gate_count, out_gated) is bit-identical to the same launch without out_innov, and a chunked
+ * replay writes what the unchunked one writes.  All three Wahba modes, both variants, the low-pass, per-stream dt and
+ * lengths and the gate are supported; the scalar kernels run it (a packed staging runs the scalar TMA kernel, same bits).
+ * General Q and R matrices have no per-step output. */
+int posekf_replay_innovation_steps_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams,
+                                       const float* dt, int dt_per_step, const float* acc_ref, const float* mag_ref,
+                                       const float* q_scale, const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag,
+                                       float* state_x, float* state_x_lo, float* state_p, float* state_lpf, float* out_traj,
+                                       uint8_t* out_flip, const float* truth, float* loss_acc, float* innov_acc,
+                                       int innov_model, int wahba_algo, int staging, int state_flags, void* stream,
+                                       const float* dt_cols, const int32_t* n_valid, float gate_nis3, int32_t* gate_count,
+                                       uint8_t* out_gated, float* out_innov, int64_t innov_plane_stride);
+
 /* General Q and R matrices: the replay of posekf_replay_batch_f32 (same parameters and rules, minus q_scale / r_scale)
  * for filters whose process noise Q is any symmetric positive semidefinite 3x3 and whose measurement noise R is any
  * symmetric positive definite 4x4 -- the reference's KalmanFilter with its Q and R attributes assigned

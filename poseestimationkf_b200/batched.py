@@ -316,7 +316,7 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
            staging: str = "auto", keep_filter_frame: bool = False, allow_imprecise: bool = False,
            innovation: bool | torch.Tensor | None = None, innovation_model: str = "full",
            lengths: torch.Tensor | None = None, gate: float | None = None, gate_count: torch.Tensor | None = None,
-           out_gated: torch.Tensor | None = None):
+           out_gated: torch.Tensor | None = None, out_innovation: torch.Tensor | None = None):
     """Run T Prediction+Correction steps for N filters in one kernel launch.
 
     streams [T,9,Ns]; acc_ref, mag_ref [3,Ns]; dt: float seconds, [T] float32 CUDA tensor (one clock for every
@@ -370,6 +370,13 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     `gate_count`: [N] int32 CUDA tensor incremented by each filter's number of gated steps (created zeroed when None;
     pass `state.gate_count` back in for chunked replays); available as `state.gate_count`.  `out_gated`: a [T,N]
     uint8 CUDA tensor that receives 1 where a step was gated (0 elsewhere and on held steps).  Both need `gate`.
+    `out_innovation`: a [2,T,N] float32 CUDA tensor that receives the innovation terms of every step
+    (include/posekf.h, posekf_replay_innovation_steps_f32): [0] NIS_t, [1] ln det S_t of `innovation_model`, in the
+    convention of the sums (`workloads.window_innovation_nll` scores windows of it).  Held steps get 0, gated steps
+    their terms.  It needs neither `innovation` nor `gate` and changes no other output.  Its rows must be contiguous
+    (stride N along t, 1 along n); the plane stride may be larger, so a time-chunked replay passes each chunk the view
+    `out_innovation[:, t0:t1]` of one full-length buffer.  Not with general Q / R matrices; the precision rule is the
+    whole-batch one.
     Returns (state, traj [T,N,4] or None, flips [T,N] uint8 or None)."""
     if innovation_model not in _lib.INNOV_MODEL:
         raise ValueError("innovation_model is 'full' or 'tangent'")
@@ -403,8 +410,9 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
         wahba = "precomputed"
     general = _is_matrix(q) or _is_matrix(r)
     if general:
-        if (innovation is not None and innovation is not False) or gate is not None:
-            raise ValueError("general Q / R matrices: the replay has no innovation sums and no gate")
+        if (innovation is not None and innovation is not False) or gate is not None or out_innovation is not None:
+            raise ValueError("general Q / R matrices: the replay has no innovation sums, no per-step innovation output "
+                             "and no gate")
         if precise_state or (state is not None and state.x_lo is not None):
             raise ValueError("general Q / R matrices: the replay has no precise variant (precise_state, a two-float state)")
         q_tri, r_tri = general_qr_tri(q, r, N, dev)
@@ -427,7 +435,7 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     if precise_state is None:
         if not general and (isinstance(q, torch.Tensor) or isinstance(r, torch.Tensor)) and N > Ns and N % Ns == 0 \
                 and out_traj is None and not store_trajectory and not store_flips and not use_lpf and T > 0 \
-                and out_gated is None:
+                and out_gated is None and out_innovation is None:
             # a (Q,R) sweep: only the cells with r/q >= 100 or q/r >= 1e4 need the precise variant (+25 % time)
             mixed = _replay_sweep_mixed(streams, acc_ref, mag_ref, dt=dt, q=q, r=r, state=state, N=N, Ns=Ns, truth=truth,
                                         loss=loss, wahba=wahba, staging=staging, keep_filter_frame=keep_filter_frame,
@@ -478,6 +486,8 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     innov = _innovation_buffer(innovation, N, dev, state, innovation_model)
     if gate is not None:
         gate_count = _gate_buffers(gate_count, out_gated, N, T, dev)
+    if out_innovation is not None:
+        _check_innovation_steps(out_innovation, N, T)
     args = (N, T, _ptr(streams), Ns, _ptr(dt_t), per_step, _ptr(acc_ref), _ptr(mag_ref), _ptr(q_t), _ptr(r_t),
             -1.0 if lpf_alpha_acc is None else float(lpf_alpha_acc),
             -1.0 if lpf_alpha_mag is None else float(lpf_alpha_mag),
@@ -490,6 +500,11 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
             rc = _lib.load().posekf_replay_general_f32(
                 N, T, _ptr(streams), Ns, _ptr(dt_t), per_step, _ptr(acc_ref), _ptr(mag_ref), _ptr(q_tri), q_tri.shape[1],
                 _ptr(r_tri), r_tri.shape[1], *args[10:], None, _lib.INNOV_MODEL["full"], *tail, _ptr(dt_cols), _ptr(lengths))
+        elif out_innovation is not None:
+            rc = _lib.load().posekf_replay_innovation_steps_f32(
+                *args, _ptr(innov), _lib.INNOV_MODEL[innovation_model], *tail, _ptr(dt_cols), _ptr(lengths),
+                math.inf if gate is None else float(gate), _ptr(gate_count if gate is not None else None), _ptr(out_gated),
+                _ptr(out_innovation), out_innovation.stride(0))
         elif gate is not None:
             rc = _lib.load().posekf_replay_gated_f32(*args, _ptr(innov), _lib.INNOV_MODEL[innovation_model], *tail, _ptr(dt_cols),
                                                      _ptr(lengths), float(gate), _ptr(gate_count), _ptr(out_gated))
@@ -500,7 +515,8 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
             rc = _lib.load().posekf_replay_f32(*args, *tail)
         else:
             rc = _lib.load().posekf_replay_innovation_ex_f32(*args, _ptr(innov), _lib.INNOV_MODEL[innovation_model], *tail)
-    _lib.check(rc, "posekf_replay_general_f32" if general else "posekf_replay_gated_f32" if gate is not None else
+    _lib.check(rc, "posekf_replay_general_f32" if general else "posekf_replay_innovation_steps_f32" if out_innovation is not None
+               else "posekf_replay_gated_f32" if gate is not None else
                "posekf_replay_batch_f32" if batch else
                ("posekf_replay_f32" if innov is None else "posekf_replay_innovation_ex_f32"))
     if innov is not None:
@@ -542,6 +558,17 @@ def _gate_buffers(gate_count, out_gated, n: int, n_steps: int, device):
     if gate_count is None:
         gate_count = torch.zeros((n,), dtype=torch.int32, device=device)
     return gate_count
+
+
+def _check_innovation_steps(out, n: int, n_steps: int) -> None:
+    """replay(out_innovation=...): a [2,T,N] float32 CUDA tensor whose rows are contiguous (plane stride >= T N)."""
+    if not isinstance(out, torch.Tensor) or out.dtype != torch.float32 or tuple(out.shape) != (2, n_steps, n):
+        raise ValueError(f"out_innovation must be a float32 tensor of shape (2, {n_steps}, {n})")
+    if n and n_steps and (out.stride(2) != 1 or (n_steps > 1 and out.stride(1) != n) or out.stride(0) < n_steps * n):
+        raise ValueError("out_innovation must have contiguous [T, N] planes (strides (>= T N, N, 1)), e.g. a time slice "
+                         "out[:, t0:t1] of a contiguous buffer")
+    if not out.is_cuda:
+        raise _lib.PosekfError("poseestimationkf_b200 runs on CUDA tensors only (no CPU fallback)")
 
 
 def _innovation_buffer(innovation, n: int, device, state=None, model: str = "full"):

@@ -487,6 +487,12 @@ template <typename F> struct InnovAcc {
   F nis, logdet;
   F inv_r, log_rd;
 };
+// The terms one step adds (true units): NIS_t and ln det S_t (TAN: NIS3_t and ln det S3_t).  ln det S_t is the addend of
+// acc.logdet exactly; NIS_t is the product that acc.nis's fused multiply-add adds before its one rounding, here rounded
+// on its own.  Written only when the caller asks for them (per-step innovation output).
+template <typename F> struct InnovTerms {
+  F nis, logdet;
+};
 // 3 ln r, rounded once per lane: the packed lanes form it with scalar multiplications, which the compiler does not fuse
 // into the per-step addition (a packed product by 3 would be, and that fused sum differs from the scalar kernels' in the
 // last bit; 4 ln r is exact either way)
@@ -506,10 +512,10 @@ template <typename F> PKF_HD F log_pivots(F x0, F x1, F x2, F x3) {
   const F a = fma_(x0, x1, x0 + x1), b = fma_(x2, x3, x2 + x3);
   return log1p_(fma_(a, b, a + b));
 }
-// K = I - S~^-1 (the step's gain) and z are read by TAN only.
+// K = I - S~^-1 (the step's gain) and z are read by TAN only.  step: the step's own terms (see InnovTerms), or null.
 template <typename F, bool COMP, bool TAN = false>
 PKF_HD void innov_accumulate(InnovAcc<F>& acc, const InnovFactors<F>& f, const Sym4<F>& K, const Quat<F>& z,
-                             F e0, F e1, F e2, F e3) {
+                             F e0, F e1, F e2, F e3, InnovTerms<F>* step = nullptr) {
   const F t1 = fma_(f.n10, e0, e1);
   const F t2 = fma_(f.n21, e1, fma_(f.n20, e0, e2));
   const F t3 = fma_(f.n32, e2, fma_(f.n31, e1, fma_(f.n30, e0, e3)));
@@ -521,7 +527,9 @@ PKF_HD void innov_accumulate(InnovAcc<F>& acc, const InnovFactors<F>& f, const S
   }
   if constexpr (!TAN) {
     acc.nis = fma_(s, acc.inv_r, acc.nis);
-    acc.logdet = acc.logdet + (f.logdet + acc.log_rd);
+    const F ld = f.logdet + acc.log_rd;
+    acc.logdet = acc.logdet + ld;
+    if (step) { step->nis = s * acc.inv_r; step->logdet = ld; }
   } else {
     const F v1 = fma_(f.n10, z.w, z.x);
     const F v2 = fma_(f.n21, z.x, fma_(f.n20, z.w, z.y));
@@ -545,8 +553,11 @@ PKF_HD void innov_accumulate(InnovAcc<F>& acc, const InnovFactors<F>& f, const S
     const F iz2 = rcp_(dot4(z, z));
     const F kz = zkz * iz2;
     const F lc = sel_(kz < F(0.5), log1p_(-kz), log_(c * iz2));
-    acc.nis = fma_(fma_(-b, b * rcp_(c), s), acc.inv_r, acc.nis);
-    acc.logdet = acc.logdet + ((f.logdet + lc) + acc.log_rd);
+    const F nis_r = fma_(-b, b * rcp_(c), s);     // r NIS_3: the value tangent_nis_r gives the gate
+    acc.nis = fma_(nis_r, acc.inv_r, acc.nis);
+    const F ld = (f.logdet + lc) + acc.log_rd;
+    acc.logdet = acc.logdet + ld;
+    if (step) { step->nis = nis_r * acc.inv_r; step->logdet = ld; }
   }
 }
 
@@ -1508,12 +1519,14 @@ PKF_HD void ekf_update_general(Quat<F>& x, Sym4<F>& P, FilterConst<F>& fc, const
 // INNOV: the innovation likelihood of the step is added to *innov (see InnovAcc); the filter itself is unchanged.
 // TAN: its tangent-space form (see innov_accumulate).  GATE: the innovation gate (see GateParams), decision in *gated.
 // GEN: general Q and R from *gen (see GENERAL Q AND R); P is unscaled, plain variant only.
+// terms (INNOV): the step's own innovation terms (see InnovTerms), or null.
 template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, bool GATE = false, bool GEN = false,
           typename FlagT>
 PKF_HD void ekf_step_measured(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, const Vec3<F>& gyro,
                               const Quat<F>& y, F inv_norm, const StepH<F>& h, FlagT& flip, bool flip_wanted = true,
                               typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr,
-                              const GateParams<F>* gate = nullptr, FlagT* gated = nullptr, const GenQR<F>* gen = nullptr) {
+                              const GateParams<F>* gate = nullptr, FlagT* gated = nullptr, const GenQR<F>* gen = nullptr,
+                              InnovTerms<F>* terms = nullptr) {
   static_assert(!GEN || !(COMP || INNOV || GATE), "general Q and R: plain variant, no innovation sums, no gate");
   Sym4<F> K, Pm;
   Quat<F> inc, z;
@@ -1526,7 +1539,7 @@ PKF_HD void ekf_step_measured(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<
   if (WANT_FLIP && flip_wanted) flip = reference_flip_quat(fc, y, one_with_sign_(dyz), code);
   const F sn = copysign_(inv_norm, dyz);          // e = sg y/|y| - z, sg = sign(dot): the sign bit moves onto 1/|y| > 0  :76
   F e0 = fma_(sn, y.w, -z.w), e1 = fma_(sn, y.x, -z.x), e2 = fma_(sn, y.y, -z.y), e3 = fma_(sn, y.z, -z.z);
-  if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3);
+  if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3, terms);
   if constexpr (GATE) gate_apply<F, COMP>(*gate, fac, z, Pm, K, e0, e1, e2, e3, *gated);
   if constexpr (GEN) ekf_update_general(x, P, fc, gg, z, e0, e1, e2, e3);
   else ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);
@@ -1552,14 +1565,15 @@ template <typename F, int ALGO, bool WANT_FLIP, bool COMP, bool INNOV = false, b
 PKF_HD void ekf_step(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, const Vec3<F>& gyro,
                      const Vec3<F>& acc, const Vec3<F>& mag, const StepH<F>& h, FlagT& flip, bool flip_wanted = true,
                      typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr,
-                     const GateParams<F>* gate = nullptr, FlagT* gated = nullptr, const GenQR<F>* gen = nullptr) {
+                     const GateParams<F>* gate = nullptr, FlagT* gated = nullptr, const GenQR<F>* gen = nullptr,
+                     InnovTerms<F>* terms = nullptr) {
   // flip_wanted: launch-uniform run-time switch under WANT_FLIP -- a launch that stores the trajectory but
   // not the flip mask skips the reference's branch rule altogether
   if constexpr (ALGO == WAHBA_QR2) {
     F inv_norm;
     const Quat<F> y = measure_quat(fc, acc, mag, inv_norm);
     ekf_step_measured<F, WANT_FLIP, COMP, INNOV, TAN, GATE, GEN>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code,
-                                                                 innov, gate, gated, gen);
+                                                                 innov, gate, gated, gen, terms);
   } else {
     static_assert(!GEN || !(COMP || INNOV || GATE), "general Q and R: plain variant, no innovation sums, no gate");
     Sym4<F> K, Pm;
@@ -1601,7 +1615,7 @@ PKF_HD void ekf_step(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, c
         e2 = sel_(unrelated, yf.y - z.y, e2); e3 = sel_(unrelated, yf.z - z.z, e3);
       }
     }
-    if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3);
+    if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3, terms);
     if constexpr (GATE) gate_apply<F, COMP>(*gate, fac, z, Pm, K, e0, e1, e2, e3, *gated);
     if constexpr (GEN) ekf_update_general(x, P, fc, gg, z, e0, e1, e2, e3);
     else ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);

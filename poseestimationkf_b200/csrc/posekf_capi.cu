@@ -271,10 +271,43 @@ int launch_general_algo(const ReplayParams& p, const GenQRArgs& gq, int algo, bo
   return POSEKF_EINVAL;
 }
 
-// innov_model: POSEKF_INNOV_* of the sums in p.innov_acc (read only when it is set).  gate: run the gated kernels with
-// these arguments (null: the ungated ones).  gen: run the general-matrix kernels with these matrices.
+// Launches with per-step innovation output (posekf_replay_innovation_steps_f32): the scalar BATCH kernels with INNOV
+// (the statistic is needed whether or not the sums are) and AUX, gated or not, on the launch's staging.  A packed staging
+// runs the scalar TMA kernel with the same bits (the packed kernel has no per-step-output twin; DESIGN.md section 5,
+// f11).  ga: the pack's GateArgs (gated launches) and the InnovStepArgs.
+template <int ALGO, bool TAN, bool GATE, typename... GA>
+int launch_innov_steps(const ReplayParams& p, bool lpf, bool use_tma, cudaStream_t st, const GA&... ga) {
+  const bool comp = p.state_x_lo != nullptr;
+  if constexpr (ALGO != WAHBA_PRECOMPUTED) {
+    if (lpf) return comp ? launch_replay<ALGO, true, true, true, true, TAN, true, GATE>(p, use_tma, st, ga...)
+                         : launch_replay<ALGO, true, true, false, true, TAN, true, GATE>(p, use_tma, st, ga...);
+  }
+  return comp ? launch_replay<ALGO, false, true, true, true, TAN, true, GATE>(p, use_tma, st, ga...)
+              : launch_replay<ALGO, false, true, false, true, TAN, true, GATE>(p, use_tma, st, ga...);
+}
+
+template <int ALGO>
+int launch_innov_steps_model(const ReplayParams& p, const GateArgs* gate, const InnovStepArgs& ia, bool lpf, bool use_tma,
+                             int innov_model, cudaStream_t st) {
+  const bool tan = innov_model == POSEKF_INNOV_TANGENT;
+  if (gate) return tan ? launch_innov_steps<ALGO, true, true>(p, lpf, use_tma, st, *gate, ia)
+                       : launch_innov_steps<ALGO, false, true>(p, lpf, use_tma, st, *gate, ia);
+  return tan ? launch_innov_steps<ALGO, true, false>(p, lpf, use_tma, st, ia) : launch_innov_steps<ALGO, false, false>(p, lpf, use_tma, st, ia);
+}
+
+int launch_innov_steps_algo(const ReplayParams& p, const GateArgs* gate, const InnovStepArgs& ia, int algo, bool lpf, bool use_tma,
+                            int innov_model, cudaStream_t st) {
+  if (algo == POSEKF_WAHBA_QR2) return launch_innov_steps_model<WAHBA_QR2>(p, gate, ia, lpf, use_tma, innov_model, st);
+  if (algo == POSEKF_WAHBA_PRECOMPUTED) return launch_innov_steps_model<WAHBA_PRECOMPUTED>(p, gate, ia, lpf, use_tma, innov_model, st);
+  if (algo == POSEKF_WAHBA_JACOBI) return launch_innov_steps_model<WAHBA_JACOBI>(p, gate, ia, lpf, use_tma, innov_model, st);
+  return POSEKF_EINVAL;
+}
+
+// innov_model: POSEKF_INNOV_* of the sums in p.innov_acc (read only when it is set, or with steps).  gate: run the gated
+// kernels with these arguments (null: the ungated ones).  gen: run the general-matrix kernels with these matrices.
+// steps: run the innovation-steps kernels, which write the per-step terms there.
 int replay_dispatch(const ReplayParams& p, int algo, int staging, int innov_model, cudaStream_t st, const GateArgs* gate = nullptr,
-                    const GenQRArgs* gen = nullptr) {
+                    const GenQRArgs* gen = nullptr, const InnovStepArgs* steps = nullptr) {
   const bool lpf = (p.alpha_acc >= 0.f) || (p.alpha_mag >= 0.f);
   bool use_tma, packed = false;
   if (staging == POSEKF_STAGE_LDG) use_tma = false;
@@ -288,6 +321,7 @@ int replay_dispatch(const ReplayParams& p, int algo, int staging, int innov_mode
   } else return POSEKF_EINVAL;
   const bool batch = p.dt_cols != nullptr || p.n_valid != nullptr;
   int rc = gen ? launch_general_algo(p, *gen, algo, lpf, use_tma, st)
+           : steps ? launch_innov_steps_algo(p, gate, *steps, algo, lpf, use_tma, innov_model, st)
            : gate ? launch_gated_algo(p, *gate, algo, lpf, use_tma, packed, innov_model, st)
                 : batch ? launch_kernels<true>(p, algo, lpf, use_tma, packed, innov_model, st)
                         : launch_kernels<false>(p, algo, lpf, use_tma, packed, innov_model, st);
@@ -336,7 +370,8 @@ int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64
                  float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth, float* loss_acc,
                  float* innov_acc, int innov_model, int wahba_algo, int staging, int state_flags, void* stream,
                  const float* dt_cols = nullptr, const int32_t* n_valid = nullptr, bool gate = false, float gate_nis3 = 0.f,
-                 int32_t* gate_count = nullptr, uint8_t* out_gated = nullptr, const GenQRArgs* gen = nullptr) {
+                 int32_t* gate_count = nullptr, uint8_t* out_gated = nullptr, const GenQRArgs* gen = nullptr,
+                 const InnovStepArgs* steps = nullptr) {
   if (dt_cols && !dt) { dt = dt_cols; dt_per_step = 0; }    // (the kernels read dt[0] unconditionally; it is unused then)
   if (n_filters < 0 || n_steps < 0 || n_streams <= 0 && n_filters > 0) return POSEKF_EINVAL;
   if (state_flags & ~(POSEKF_STATE_IN_FILTER_FRAME | POSEKF_STATE_OUT_FILTER_FRAME)) return POSEKF_EINVAL;
@@ -372,7 +407,8 @@ int replay_entry(int64_t n_filters, int64_t n_steps, const float* streams, int64
   p.dt_cols = n_steps > 0 ? dt_cols : nullptr;
   p.n_valid = n_steps > 0 ? n_valid : nullptr;
   const GateArgs ga{gate_nis3, gate_count, out_gated};
-  return replay_dispatch(p, wahba_algo, staging, innov_model, (cudaStream_t)stream, gate && n_steps > 0 ? &ga : nullptr, gen);
+  return replay_dispatch(p, wahba_algo, staging, innov_model, (cudaStream_t)stream, gate && n_steps > 0 ? &ga : nullptr, gen,
+                         n_steps > 0 ? steps : nullptr);
 }
 }  // namespace
 
@@ -437,6 +473,30 @@ int posekf_replay_gated_f32(int64_t n_filters, int64_t n_steps, const float* str
                       lpf_alpha_mag, state_x, state_x_lo, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, innov_acc,
                       innov_model, wahba_algo, staging, state_flags, stream, dt_cols, n_valid, true, gate_nis3, gate_count,
                       out_gated);
+}
+
+int posekf_replay_innovation_steps_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams,
+                                       const float* dt, int dt_per_step, const float* acc_ref, const float* mag_ref,
+                                       const float* q_scale, const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag,
+                                       float* state_x, float* state_x_lo, float* state_p, float* state_lpf, float* out_traj,
+                                       uint8_t* out_flip, const float* truth, float* loss_acc, float* innov_acc,
+                                       int innov_model, int wahba_algo, int staging, int state_flags, void* stream,
+                                       const float* dt_cols, const int32_t* n_valid, float gate_nis3, int32_t* gate_count,
+                                       uint8_t* out_gated, float* out_innov, int64_t innov_plane_stride) {
+  if (innov_model != POSEKF_INNOV_FULL && innov_model != POSEKF_INNOV_TANGENT) return POSEKF_EINVAL;
+  if (gate_nis3 != gate_nis3) return POSEKF_EINVAL;
+  if (n_filters < 0 || n_steps < 0) return POSEKF_EINVAL;
+  if (n_filters > 0 && n_steps > 0) {     // (an empty launch writes nothing: its buffer may be NULL, as torch's empty tensors are)
+    if (!out_innov || n_steps > INT64_MAX / n_filters || innov_plane_stride < n_filters * n_steps) return POSEKF_EINVAL;
+  }
+  if ((reinterpret_cast<uintptr_t>(out_innov) & 3) != 0) return POSEKF_EALIGN;
+  // +inf with no gate buffer decides nothing and records nothing: the ungated kernels (the same bits)
+  const bool gate = !(gate_nis3 == INFINITY && !gate_count && !out_gated);
+  const InnovStepArgs ia{out_innov, innov_plane_stride};
+  return replay_entry(n_filters, n_steps, streams, n_streams, dt, dt_per_step, acc_ref, mag_ref, q_scale, r_scale, lpf_alpha_acc,
+                      lpf_alpha_mag, state_x, state_x_lo, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, innov_acc,
+                      innov_model, wahba_algo, staging, state_flags, stream, dt_cols, n_valid, gate, gate_nis3, gate_count,
+                      out_gated, nullptr, &ia);
 }
 
 int posekf_replay_general_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams, const float* dt,

@@ -68,6 +68,26 @@ template <bool AUX> __device__ __forceinline__ void load_gate(const ReplayParams
   g.out = (AUX && ga.out_gated) ? ga.out_gated + n : nullptr;
 }
 
+// Per-step innovation output (the innovation-steps kernels): the terms each step adds to the innovation sums, written to
+// out[0][t][n] (NIS_t) and out[plane][t][n] (ln det S_t), filter index fastest.  Like GateArgs it is a trailing kernel
+// parameter that only those kernels have (alone, or after the GateArgs of a gated launch); their per-filter pointer
+// lives in InnovStepRegs (empty NoInnovStepRegs elsewhere).  Those kernels always carry the statistic (INNOV) and take
+// innov_acc as optional: a launch may ask for the per-step terms, the sums or both.
+struct InnovStepArgs {
+  float* out;               // [2][T][N] with planes `plane` elements apart
+  int64_t plane;            // >= T N
+};
+template <typename... GA> constexpr bool kInnovSteps = (std::is_same<GA, InnovStepArgs>::value || ... || false);
+__device__ __forceinline__ InnovStepArgs innov_step_args_(const InnovStepArgs& a) { return a; }
+__device__ __forceinline__ InnovStepArgs innov_step_args_(const GateArgs&, const InnovStepArgs& a) { return a; }
+__device__ __forceinline__ GateArgs gate_args_(const GateArgs& g, const InnovStepArgs&) { return g; }
+struct InnovStepRegs {
+  float* out;               // this filter's slot in plane 0, advanced by N per step
+  int64_t plane;
+};
+struct NoInnovStepRegs {};
+template <bool OUT> using InnovStepRegsOf = typename std::conditional<OUT, InnovStepRegs, NoInnovStepRegs>::type;
+
 // General Q and R (GEN kernels): the upper triangles of the matrices, the last kernel parameter of those kernels only
 // (like GateArgs).  Filter n uses column (nq == 1 ? 0 : n) of q_tri and (nr == 1 ? 0 : n) of r_tri; the kernel carries
 // them in the filter frame, Q/4 and R in a register struct of their own (GenRegs; empty NoGenRegs elsewhere).
@@ -91,14 +111,18 @@ template <int ALGO> __device__ __forceinline__ void load_gen(const GenQRArgs& a,
   g.m = make_gen_qr<float>(fc, q, r, uses_filter_frame<ALGO>());
 }
 
-// (GEN: q_scale / r_scale are not read; the covariance is unscaled, the process noise scale fc.g is 1)
-template <int ALGO, bool LPF, bool COMP, bool INNOV = false, bool TAN = false, bool GEN = false>
+// (GEN: q_scale / r_scale are not read; the covariance is unscaled, the process noise scale fc.g is 1.  OPT_ACC:
+//  innov_acc may be null, the sums then start at 0 and are not stored)
+template <int ALGO, bool LPF, bool COMP, bool INNOV = false, bool TAN = false, bool GEN = false, bool OPT_ACC = false>
 __device__ __forceinline__ void load_filter(const ReplayParams& p, int64_t n, int64_t col, FilterRegs& f) {
   const int64_t N = p.N, Ns = p.Ns;
   Vec3<float> ra = {p.acc_ref[col], p.acc_ref[Ns + col], p.acc_ref[2 * Ns + col]};
   Vec3<float> rm = {p.mag_ref[col], p.mag_ref[Ns + col], p.mag_ref[2 * Ns + col]};
   f.fc = make_filter_const<float>(ra, rm, GEN ? 4.f : p.q_scale[n], GEN ? 1.f : p.r_scale[n]);
-  if (INNOV) f.in = make_innov_acc<float, TAN>(p.innov_acc[n], p.innov_acc[N + n], p.r_scale[n]);
+  if (INNOV) {
+    if (OPT_ACC && !p.innov_acc) f.in = make_innov_acc<float, TAN>(0.f, 0.f, p.r_scale[n]);
+    else f.in = make_innov_acc<float, TAN>(p.innov_acc[n], p.innov_acc[N + n], p.r_scale[n]);
+  }
   f.x = {p.state_x[n], p.state_x[N + n], p.state_x[2 * N + n], p.state_x[3 * N + n]};
   f.xlo = {0.f, 0.f, 0.f, 0.f};
   if (COMP) f.xlo = {p.state_x_lo[n], p.state_x_lo[N + n], p.state_x_lo[2 * N + n], p.state_x_lo[3 * N + n]};
@@ -114,7 +138,7 @@ __device__ __forceinline__ void load_filter(const ReplayParams& p, int64_t n, in
   if (uses_filter_frame<ALGO>() && !(p.state_flags & kStateInFilterFrame)) enter_filter_frame(f.fc, f.x, f.xlo, f.P, COMP);
 }
 
-template <int ALGO, bool LPF, bool COMP, bool INNOV = false, bool TAN = false>
+template <int ALGO, bool LPF, bool COMP, bool INNOV = false, bool TAN = false, bool OPT_ACC = false>
 __device__ __forceinline__ void store_filter(const ReplayParams& p, int64_t n, FilterRegs& f) {
   const int64_t N = p.N;
   if (uses_filter_frame<ALGO>() && !(p.state_flags & kStateOutFilterFrame)) leave_filter_frame(f.fc, f.x, f.xlo, f.P, COMP);
@@ -129,7 +153,7 @@ __device__ __forceinline__ void store_filter(const ReplayParams& p, int64_t n, F
     float* sl = p.state_lpf + n;
     sl[0] = f.la.x; sl[N] = f.la.y; sl[2 * N] = f.la.z; sl[3 * N] = f.lm.x; sl[4 * N] = f.lm.y; sl[5 * N] = f.lm.z;
   }
-  if (INNOV) { p.innov_acc[n] = f.in.nis; p.innov_acc[N + n] = f.in.logdet; }
+  if (INNOV && (!OPT_ACC || p.innov_acc)) { p.innov_acc[n] = f.in.nis; p.innov_acc[N + n] = f.in.logdet; }
 }
 
 // One filter step + optional outputs.  AUX = the launch has a trajectory and/or flip output.
@@ -150,9 +174,12 @@ template <bool AUX> __device__ __forceinline__ AuxPtrs make_aux(const ReplayPara
   return a;
 }
 
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool GATE = false, bool GEN = false>
+// OUT (innovation-steps kernels): the step's innovation terms go to io.out
+template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool GATE = false, bool GEN = false,
+          bool OUT = false>
 __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f, const float (&s)[kChannels], float h,
-                                            AuxPtrs& aux, GateRegsOf<GATE>& g, const GenRegsOf<GEN>* gr = nullptr) {
+                                            AuxPtrs& aux, GateRegsOf<GATE>& g, const GenRegsOf<GEN>* gr = nullptr,
+                                            InnovStepRegsOf<OUT>* io = nullptr) {
   Vec3<float> w = {s[0], s[1], s[2]}, a = {s[3], s[4], s[5]}, m = {s[6], s[7], s[8]};
   if (LPF) {   // SRV/KalmanFilter.cpp:285,298 -- filtered values feed Wahba, not renormalised
     if (p.alpha_acc >= 0.f) { lowpass<float>(f.la, a, p.alpha_acc, 1.f - p.alpha_acc); a = f.la; }
@@ -162,11 +189,12 @@ __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f
   // flip-mask byte: the float32 decision, plus the tie marker and per-branch alternatives that flip_fixup_kernel settles
   // in float64 after the launch (raw samples only: a low-passed sample is not in the stream any more)
   unsigned code = 0;
+  [[maybe_unused]] InnovTerms<float> it;
   if constexpr (GATE) {
     bool gated = false;
     ekf_step<float, ALGO, AUX, COMP, INNOV, TAN, true>(f.x, f.xlo, f.P, f.fc, w, a, m, StepH<float>(h), flip, aux.flips != nullptr,
                                                        (AUX && !LPF && ALGO == WAHBA_QR2) ? &code : nullptr, INNOV ? &f.in : nullptr,
-                                                       &g.gp, &gated);
+                                                       &g.gp, &gated, nullptr, OUT ? &it : nullptr);
     g.count += gated ? 1 : 0;
     if (g.out) { *g.out = gated ? 1 : 0; g.out += p.N; }
   } else if constexpr (GEN) {
@@ -175,7 +203,13 @@ __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f
                                                                 nullptr, nullptr, (bool*)nullptr, &gr->m);
   } else {
     ekf_step<float, ALGO, AUX, COMP, INNOV, TAN>(f.x, f.xlo, f.P, f.fc, w, a, m, StepH<float>(h), flip, aux.flips != nullptr,
-                                                 (AUX && !LPF && ALGO == WAHBA_QR2) ? &code : nullptr, INNOV ? &f.in : nullptr);
+                                                 (AUX && !LPF && ALGO == WAHBA_QR2) ? &code : nullptr, INNOV ? &f.in : nullptr,
+                                                 nullptr, (bool*)nullptr, nullptr, OUT ? &it : nullptr);
+  }
+  if constexpr (OUT) {     // [2][T][N]: a warp's store of one plane is one 128-byte line
+    __stcs(io->out, it.nis);
+    __stcs(io->out + io->plane, it.logdet);
+    io->out += p.N;
   }
   if (!(AUX && !LPF && ALGO == WAHBA_QR2)) code = flip ? 1u : 0u;
   if (AUX) {
@@ -206,9 +240,12 @@ __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f
 // A step at or past the length of the filter's stream (BATCH kernels): the filter is left as it is, the trajectory slot
 // gets the held state, the flip byte is 0 (unmarked: flip_fixup_kernel leaves it alone) and the objectives add nothing.
 // The step's sample and dt are not read.
-template <int ALGO, bool AUX, bool GATE = false>
-__device__ __forceinline__ void hold_step(const ReplayParams& p, const FilterRegs& f, AuxPtrs& aux, GateRegsOf<GATE>& g) {
+// (OUT: both innovation terms are 0)
+template <int ALGO, bool AUX, bool GATE = false, bool OUT = false>
+__device__ __forceinline__ void hold_step(const ReplayParams& p, const FilterRegs& f, AuxPtrs& aux, GateRegsOf<GATE>& g,
+                                          InnovStepRegsOf<OUT>* io = nullptr) {
   if constexpr (GATE) { if (g.out) { *g.out = 0; g.out += p.N; } }
+  if constexpr (OUT) { __stcs(io->out, 0.f); __stcs(io->out + io->plane, 0.f); io->out += p.N; }
   if (AUX) {
     if (aux.traj) {
       Quat<float> xr = f.x;
@@ -228,20 +265,25 @@ __device__ __forceinline__ void hold_step(const ReplayParams& p, const FilterReg
 // (INNOV: the innovation likelihood, TAN: its tangent-space form; their instantiations always have AUX and are built for
 //  3 CTAs per SM, <= 168 registers.  BATCH: per-stream dt columns and lengths, ReplayParams::dt_cols / n_valid)
 //  GATE: the innovation gate, its arguments in the pack ga (one GateArgs; empty in the other kernels).
-//  GEN: general Q and R matrices, the pack holds one GenQRArgs; plain variant, no innovation sums, no gate)
+//  GEN: general Q and R matrices, the pack holds one GenQRArgs; plain variant, no innovation sums, no gate.
+//  Innovation steps: the pack ends in an InnovStepArgs (OUT); INNOV kernels only, innov_acc optional)
 template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false, bool GATE = false,
           bool GEN = false, typename... GA>
 __global__ void __launch_bounds__(kThreads, (INNOV || GATE || GEN) ? 3 : ((ALGO == WAHBA_JACOBI || (COMP && LPF && AUX)) ? 4 : ((COMP || LPF) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
     replay_ldg_kernel(const ReplayParams p, GA... ga) {
+  constexpr bool OUT = kInnovSteps<GA...>;
+  static_assert(!OUT || INNOV, "per-step innovation output: INNOV kernels only");
   const int64_t n = (int64_t)blockIdx.x * kThreads + threadIdx.x;
   if (n >= p.N) return;
   const int64_t Ns = p.Ns;
   const int64_t col = (Ns == p.N) ? n : (n % Ns);
   FilterRegs f;
-  load_filter<ALGO, LPF, COMP, INNOV, TAN, GEN>(p, n, col, f);
+  load_filter<ALGO, LPF, COMP, INNOV, TAN, GEN, OUT>(p, n, col, f);
   AuxPtrs aux = make_aux<AUX>(p, n, col, true);
   [[maybe_unused]] GateRegsOf<GATE> g;
   if constexpr (GATE) load_gate<AUX>(p, gate_args_(ga...), n, g);
+  [[maybe_unused]] InnovStepRegsOf<OUT> io;
+  if constexpr (OUT) { const InnovStepArgs a = innov_step_args_(ga...); io = {a.out + n, a.plane}; }
   [[maybe_unused]] GenRegsOf<GEN> gr;
   if constexpr (GEN) load_gen<ALGO>(gen_args_(ga...), n, f.fc, gr);
   const float* s = p.streams + col;
@@ -262,13 +304,13 @@ __global__ void __launch_bounds__(kThreads, (INNOV || GATE || GEN) ? 3 : ((ALGO 
     for (int c = 0; c < kChannels; ++c) nxt[c] = ldg_stream(s + c * Ns);
     if (BATCH && dc) hnxt = ldg_stream(dc + (int64_t)(t + 1 < T ? t + 1 : t) * Ns);
     const float h = (BATCH && dc) ? hcur : (p.dt_per_step ? __ldg(p.dt + t) : dt0);
-    if (!BATCH || t < nv) filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE, GEN>(p, f, cur, h, aux, g, &gr);
-    else hold_step<ALGO, AUX, GATE>(p, f, aux, g);
+    if (!BATCH || t < nv) filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE, GEN, OUT>(p, f, cur, h, aux, g, &gr, &io);
+    else hold_step<ALGO, AUX, GATE, OUT>(p, f, aux, g, &io);
 #pragma unroll
     for (int c = 0; c < kChannels; ++c) cur[c] = nxt[c];
     if (BATCH) hcur = hnxt;
   }
-  store_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, f);
+  store_filter<ALGO, LPF, COMP, INNOV, TAN, OUT>(p, n, f);
   if (AUX && aux.truth) p.loss_acc[n] = aux.loss;
   if constexpr (GATE) { const GateArgs a = gate_args_(ga...); if (a.gate_count) a.gate_count[n] = g.count; }
 }
@@ -317,6 +359,8 @@ template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN 
           bool GEN = false, typename... GA>
 __global__ void __launch_bounds__(kThreads, (INNOV || GATE || GEN) ? 3 : (ALGO == WAHBA_JACOBI ? 4 : ((COMP && (LPF || AUX)) ? (kMinCtasPerSm > 5 ? 5 : kMinCtasPerSm) : kMinCtasPerSm)))
     replay_tma_kernel(const ReplayParams p, const __grid_constant__ CUtensorMap tmap, GA... ga) {
+  constexpr bool OUT = kInnovSteps<GA...>;     // (see replay_ldg_kernel)
+  static_assert(!OUT || INNOV, "per-step innovation output: INNOV kernels only");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   TmaSmem& sm = *reinterpret_cast<TmaSmem*>(smem_raw);
   const int tid = threadIdx.x;
@@ -345,10 +389,12 @@ __global__ void __launch_bounds__(kThreads, (INNOV || GATE || GEN) ? 3 : (ALGO =
   }
 
   FilterRegs f;
-  if (valid) load_filter<ALGO, LPF, COMP, INNOV, TAN, GEN>(p, n, (int64_t)col0 + tid, f);
+  if (valid) load_filter<ALGO, LPF, COMP, INNOV, TAN, GEN, OUT>(p, n, (int64_t)col0 + tid, f);
   AuxPtrs aux = make_aux<AUX>(p, n, (int64_t)col0 + tid, valid);
   [[maybe_unused]] GateRegsOf<GATE> g;
   if constexpr (GATE) { if (valid) load_gate<AUX>(p, gate_args_(ga...), n, g); }
+  [[maybe_unused]] InnovStepRegsOf<OUT> io;
+  if constexpr (OUT) { const InnovStepArgs a = innov_step_args_(ga...); io = {a.out + n, a.plane}; }
   [[maybe_unused]] GenRegsOf<GEN> gr;
   if constexpr (GEN) { if (valid) load_gen<ALGO>(gen_args_(ga...), n, f.fc, gr); }
   const float dt0 = p.dt[0];
@@ -384,16 +430,16 @@ __global__ void __launch_bounds__(kThreads, (INNOV || GATE || GEN) ? 3 : (ALGO =
       for (int tt = 0; tt < kTmaSteps; ++tt) {
         if (tt < steps) {
           if constexpr (BATCH) {
-            if (k * kTmaSteps + tt >= bt.nv) { hold_step<ALGO, AUX, GATE>(p, f, aux, g); continue; }
+            if (k * kTmaSteps + tt >= bt.nv) { hold_step<ALGO, AUX, GATE, OUT>(p, f, aux, g, &io); continue; }
           }
           float s[kChannels];
 #pragma unroll
           for (int c = 0; c < kChannels; ++c) s[c] = sm.tile[stage][tt][c][tid];
           if constexpr (BATCH) {
-            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE, GEN>(p, f, s, bt.cur[tt], aux, g, &gr);
+            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE, GEN, OUT>(p, f, s, bt.cur[tt], aux, g, &gr, &io);
           } else {
             const float h = p.dt_per_step ? __ldg(p.dt + k * kTmaSteps + tt) : dt0;
-            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE, GEN>(p, f, s, h, aux, g, &gr);
+            filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE, GEN, OUT>(p, f, s, h, aux, g, &gr, &io);
           }
         }
       }
@@ -402,7 +448,7 @@ __global__ void __launch_bounds__(kThreads, (INNOV || GATE || GEN) ? 3 : (ALGO =
     if ((tid & 31) == 0) mbar_arrive(&sm.empty[stage]);
     if (++stage == kTmaStages) { stage = 0; parity ^= 1; }
   }
-  if (valid) store_filter<ALGO, LPF, COMP, INNOV, TAN>(p, n, f);
+  if (valid) store_filter<ALGO, LPF, COMP, INNOV, TAN, OUT>(p, n, f);
   if constexpr (GATE) { const GateArgs a = gate_args_(ga...); if (valid && a.gate_count) a.gate_count[n] = g.count; }
   if (AUX && valid && aux.truth) p.loss_acc[n] = aux.loss;
 }
