@@ -242,7 +242,7 @@ int posekf_replay_gated_f32(int64_t n_filters, int64_t n_steps, const float* str
  * flips, loss, innov_acc, gate_count, out_gated) is bit-identical to the same launch without out_innov, and a chunked
  * replay writes what the unchunked one writes.  All three Wahba modes, both variants, the low-pass, per-stream dt and
  * lengths and the gate are supported; the scalar kernels run it (a packed staging runs the scalar TMA kernel, same bits).
- * General Q and R matrices have no per-step output. */
+ * With general Q and R matrices: posekf_replay_general_innovation_f32. */
 int posekf_replay_innovation_steps_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams,
                                        const float* dt, int dt_per_step, const float* acc_ref, const float* mag_ref,
                                        const float* q_scale, const float* r_scale, float lpf_alpha_acc, float lpf_alpha_mag,
@@ -266,9 +266,9 @@ int posekf_replay_innovation_steps_f32(int64_t n_filters, int64_t n_steps, const
  *           or n_filters.
  *   state_p holds P itself, NOT P/r as in the scalar entry points: convert when a state moves between the two.
  * Precondition (not checked here, like r > 0 and q >= 0 of the scalar entry points): R positive definite, Q positive
- * semidefinite, both symmetric.  POSEKF_EINVAL: innov_acc or state_x_lo non-NULL (no innovation sums and no precise
- * variant with general matrices), nq or nr neither 1 nor n_filters, q_tri or r_tri NULL, and everything
- * posekf_replay_batch_f32 refuses.  There is no gated twin.  The float64 flip fix-up, the tuning loss (truth/loss_acc),
+ * semidefinite, both symmetric.  POSEKF_EINVAL: innov_acc or state_x_lo non-NULL (no precise variant with general
+ * matrices; the innovation sums, their per-step terms and the gate are posekf_replay_general_innovation_f32's), nq or
+ * nr neither 1 nor n_filters, q_tri or r_tri NULL, and everything posekf_replay_batch_f32 refuses.  The float64 flip fix-up, the tuning loss (truth/loss_acc),
  * the low-pass, all three Wahba modes, per-stream dt / lengths and the filter-frame state flags work as in
  * posekf_replay_batch_f32.  A chunked replay equals the unchunked one bit for bit; every staging gives the same bits
  * (a packed staging runs the scalar TMA kernel).  The float32 step meets the 1e-5 rad tolerance of the float64
@@ -279,6 +279,39 @@ int posekf_replay_general_f32(int64_t n_filters, int64_t n_steps, const float* s
                               float* state_x_lo, float* state_p, float* state_lpf, float* out_traj, uint8_t* out_flip,
                               const float* truth, float* loss_acc, float* innov_acc, int innov_model, int wahba_algo,
                               int staging, int state_flags, void* stream, const float* dt_cols, const int32_t* n_valid);
+
+/* General Q and R matrices with the innovation likelihood, its per-step terms and the innovation gate: the replay of
+ * posekf_replay_general_f32 (same parameters, same rules for q_tri / nq / r_tri / nr, state_p holds P itself) plus the
+ * tail of posekf_replay_innovation_steps_f32.  The filter steps exactly as posekf_replay_general_f32; on that step:
+ *   4-D terms (innov_model POSEKF_INNOV_FULL)     NIS_t = e^T S^-1 e,  ln det S_t,   S = P^- + R,  e = sg y/|y| - z;
+ *   tangent terms (POSEKF_INNOV_TANGENT)          NIS3_t = e3^T S3^-1 e3,  ln det S3_t,  e3 = E^T e,  S3 = E^T S E, E any
+ *                                                 orthonormal basis of z-perp.
+ * True units (natural log, without the (dof/2) ln 2 pi constant), as in every innovation entry point.
+ *   innov_acc   [2][N] in/out or NULL: += sum_t NIS_t, sum_t ln det S_t.  Each sum adds exactly the float32 terms written
+ *               to out_innov (one addition per step).
+ *   out_innov, innov_plane_stride   as in posekf_replay_innovation_steps_f32, but out_innov may be NULL (no per-step
+ *               output); with a buffer the stride must be >= n_steps * n_filters (else POSEKF_EINVAL), 4-byte alignment
+ *               (else POSEKF_EALIGN).  Held steps write 0.
+ *   gate_nis3, gate_count, out_gated   the gate of posekf_replay_gated_f32 on the tangent-space NIS3 in true units: a live
+ *               step is gated iff NIS3_t > gate_nis3 (strict, NaN is never gated), and then keeps X_t = z_t/|z_t| and
+ *               P_t = P^-_t; the flip byte, the loss, the low-pass, the sums and the per-step terms still see it.  With
+ *               POSEKF_INNOV_TANGENT the decisions are exactly out_innov[0][t][n] > gate_nis3.  NaN gate_nis3:
+ *               POSEKF_EINVAL.  +inf with gate_count and out_gated NULL is an ungated launch.
+ * Every other output is bit-identical to posekf_replay_general_f32 on the same inputs when the launch is ungated, and a
+ * chunked replay equals the unchunked one bit for bit (sums, counts, per-step slices).  Any combination of innov_acc,
+ * out_innov and the gate may be asked for; with none of them the launch is posekf_replay_general_f32's.  All three Wahba
+ * modes, the low-pass, per-stream dt / lengths and the state flags work as there; every staging gives the same bits (a
+ * packed staging runs the scalar TMA kernel).  POSEKF_EINVAL also for state_x_lo non-NULL (no precise variant with
+ * general matrices) and an unknown innov_model. */
+int posekf_replay_general_innovation_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams,
+                                         const float* dt, int dt_per_step, const float* acc_ref, const float* mag_ref,
+                                         const float* q_tri, int64_t nq, const float* r_tri, int64_t nr, float lpf_alpha_acc,
+                                         float lpf_alpha_mag, float* state_x, float* state_x_lo, float* state_p,
+                                         float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth,
+                                         float* loss_acc, float* innov_acc, int innov_model, int wahba_algo, int staging,
+                                         int state_flags, void* stream, const float* dt_cols, const int32_t* n_valid,
+                                         float gate_nis3, int32_t* gate_count, uint8_t* out_gated, float* out_innov,
+                                         int64_t innov_plane_stride);
 
 /* Same replay with HOST buffers: streams_host [T][9][N] is streamed through the device in time
  * chunks (double-buffered H2D copies overlapped with the filter kernel, state carried across

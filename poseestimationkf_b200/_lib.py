@@ -32,6 +32,9 @@ _SIGNATURES = {
                                            _vp, _vp, _i64],
     "posekf_replay_general_f32": [_i64, _i64, _vp, _i64, _vp, _int, _vp, _vp, _vp, _i64, _vp, _i64, _f32, _f32, _vp, _vp, _vp,
                                   _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _int, _int, _vp, _vp, _vp],
+    "posekf_replay_general_innovation_f32": [_i64, _i64, _vp, _i64, _vp, _int, _vp, _vp, _vp, _i64, _vp, _i64, _f32, _f32,
+                                             _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _int, _int, _int, _int, _vp, _vp,
+                                             _vp, _f32, _vp, _vp, _vp, _i64],
     "posekf_replay_host_f32": [_i64, _i64, _vp, _f32, _vp, _vp, _vp, _vp, _f32, _f32, _vp, _vp, _vp, _vp, _vp, _i64,
                                _int, _int, _int, _vp],
     "posekf_host_workspace_create": [_int, _i64, _i64, _int, C.POINTER(C.c_void_p)],

@@ -324,9 +324,10 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     q, r: floats or [N] tensors (Q=q*I3, R=r*I4), or general matrices: q [3,3] / [N,3,3] and r [4,4] / [N,4,4] (numpy
     arrays or CUDA tensors; either may stay a float or [N] tensor).  A matrix runs the general-matrix replay
     (include/posekf.h, posekf_replay_general_f32): the reference's KalmanFilter with its Q and R attributes assigned,
-    symmetric Q positive semidefinite and R positive definite (checked, `general_qr_tri`).  It has no precise variant,
-    no innovation sums and no gate; trajectories, flips, the loss, the low-pass, every Wahba mode, per-stream dt and
-    lengths work as with scalars, and `state.p` then holds P itself (`state.r` = 1.0).  `n_filters` > Ns replays every trajectory
+    symmetric Q positive semidefinite and R positive definite (checked, `general_qr_tri`).  It has no precise variant;
+    its innovation sums, per-step innovation output and gate are `replay_general`'s.  Trajectories, flips, the loss,
+    the low-pass, every Wahba mode, per-stream dt and lengths work as with scalars, and `state.p` then holds P itself
+    (`state.r` = 1.0).  `n_filters` > Ns replays every trajectory
     N/Ns times (filter n reads column n % Ns) -- the Q/R sweep layout.  `state` is updated in place
     (created with the reference's initial values when None).  `truth` [T,Ns,4] enables the on-device
     tuning objective: `loss` [N] (created zeroed when None; pass it back in for chunked replays) is
@@ -375,9 +376,54 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     convention of the sums (`workloads.window_innovation_nll` scores windows of it).  Held steps get 0, gated steps
     their terms.  It needs neither `innovation` nor `gate` and changes no other output.  Its rows must be contiguous
     (stride N along t, 1 along n); the plane stride may be larger, so a time-chunked replay passes each chunk the view
-    `out_innovation[:, t0:t1]` of one full-length buffer.  Not with general Q / R matrices; the precision rule is the
-    whole-batch one.
+    `out_innovation[:, t0:t1]` of one full-length buffer.  With general Q / R matrices see `replay_general`; the
+    precision rule is the whole-batch one.
     Returns (state, traj [T,N,4] or None, flips [T,N] uint8 or None)."""
+    return _replay(streams, acc_ref, mag_ref, dt=dt, q=q, r=r, state=state, n_filters=n_filters, lpf_alpha_acc=lpf_alpha_acc,
+                   lpf_alpha_mag=lpf_alpha_mag, out_traj=out_traj, store_trajectory=store_trajectory, store_flips=store_flips,
+                   truth=truth, loss=loss, precise_state=precise_state, share_measurements=share_measurements, wahba=wahba,
+                   staging=staging, keep_filter_frame=keep_filter_frame, allow_imprecise=allow_imprecise,
+                   innovation=innovation, innovation_model=innovation_model, lengths=lengths, gate=gate,
+                   gate_count=gate_count, out_gated=out_gated, out_innovation=out_innovation, general_innovation=False)
+
+
+def replay_general(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, *, dt, q, r,
+                   state: ReplayState | None = None, n_filters: int | None = None, lpf_alpha_acc: float | None = None,
+                   lpf_alpha_mag: float | None = None, out_traj: torch.Tensor | None = None,
+                   store_trajectory: bool = False, store_flips: bool = False, truth: torch.Tensor | None = None,
+                   loss: torch.Tensor | None = None, precise_state: bool | None = None,
+                   share_measurements: bool | None = None, wahba: str = "qr2", staging: str = "auto",
+                   keep_filter_frame: bool = False, allow_imprecise: bool = False,
+                   innovation: bool | torch.Tensor | None = None, innovation_model: str = "full",
+                   lengths: torch.Tensor | None = None, gate: float | None = None, gate_count: torch.Tensor | None = None,
+                   out_gated: torch.Tensor | None = None, out_innovation: torch.Tensor | None = None):
+    """The general-matrix replay of `replay` (q [3,3] / [N,3,3] and/or r [4,4] / [N,4,4]; the other may stay a float or
+    [N] tensor) with the innovation likelihood, its per-step terms and the innovation gate (include/posekf.h,
+    posekf_replay_general_innovation_f32).  Every keyword means what it means in `replay`; `state.p` holds P itself.
+    `innovation` / `innovation_model`: the sums of the 4-D ("full") or tangent-space model, NIS_t = e^T S^-1 e and
+    ln det S_t with S = P^- + R in true units (`innovation_nll` and `state.innov` as for scalars).  `out_innovation`
+    [2,T,N]: the per-step terms (`workloads.window_innovation_nll` reads them).  `gate`: a live step whose tangent-space
+    NIS3 exceeds `gate` keeps its prediction and P^-; `gate_count`, `out_gated` and `state.gate_count` as in `replay`.
+    Without any of these the launch is exactly `replay`'s with the same matrices, and with them every other output
+    keeps those bits (ungated, or `gate=inf` without gate buffers).  There is no precise variant.  Scalar q and r are
+    refused: that is `replay`.  Returns (state, traj [T,N,4] or None, flips [T,N] uint8 or None)."""
+    if not (_is_matrix(q) or _is_matrix(r)):
+        raise ValueError("replay_general takes a [3,3] / [N,3,3] q or a [4,4] / [N,4,4] r; for Q = qI3 and R = rI4 use "
+                         "replay")
+    return _replay(streams, acc_ref, mag_ref, dt=dt, q=q, r=r, state=state, n_filters=n_filters, lpf_alpha_acc=lpf_alpha_acc,
+                   lpf_alpha_mag=lpf_alpha_mag, out_traj=out_traj, store_trajectory=store_trajectory, store_flips=store_flips,
+                   truth=truth, loss=loss, precise_state=precise_state, share_measurements=share_measurements, wahba=wahba,
+                   staging=staging, keep_filter_frame=keep_filter_frame, allow_imprecise=allow_imprecise,
+                   innovation=innovation, innovation_model=innovation_model, lengths=lengths, gate=gate,
+                   gate_count=gate_count, out_gated=out_gated, out_innovation=out_innovation, general_innovation=True)
+
+
+def _replay(streams, acc_ref, mag_ref, *, dt, q, r, state, n_filters, lpf_alpha_acc, lpf_alpha_mag, out_traj,
+            store_trajectory, store_flips, truth, loss, precise_state, share_measurements, wahba, staging,
+            keep_filter_frame, allow_imprecise, innovation, innovation_model, lengths, gate, gate_count, out_gated,
+            out_innovation, general_innovation: bool):
+    """The body of `replay` and `replay_general`.  general_innovation: matrices may come with the innovation sums, the
+    per-step terms and the gate (posekf_replay_general_innovation_f32)."""
     if innovation_model not in _lib.INNOV_MODEL:
         raise ValueError("innovation_model is 'full' or 'tangent'")
     if gate is None and (gate_count is not None or out_gated is not None):
@@ -410,9 +456,10 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
         wahba = "precomputed"
     general = _is_matrix(q) or _is_matrix(r)
     if general:
-        if (innovation is not None and innovation is not False) or gate is not None or out_innovation is not None:
-            raise ValueError("general Q / R matrices: the replay has no innovation sums, no per-step innovation output "
-                             "and no gate")
+        if not general_innovation and ((innovation is not None and innovation is not False) or gate is not None
+                                       or out_innovation is not None):
+            raise ValueError("general Q / R matrices: the innovation sums, the per-step innovation output and the gate "
+                             "are replay_general's (same keywords)")
         if precise_state or (state is not None and state.x_lo is not None):
             raise ValueError("general Q / R matrices: the replay has no precise variant (precise_state, a two-float state)")
         q_tri, r_tri = general_qr_tri(q, r, N, dev)
@@ -496,7 +543,14 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
     tail = (_lib.WAHBA[wahba], _lib.STAGING[staging], frame_flags, _stream())
     batch = dt_cols is not None or lengths is not None
     with torch.cuda.device(dev):
-        if general:
+        if general and general_innovation:
+            rc = _lib.load().posekf_replay_general_innovation_f32(
+                N, T, _ptr(streams), Ns, _ptr(dt_t), per_step, _ptr(acc_ref), _ptr(mag_ref), _ptr(q_tri), q_tri.shape[1],
+                _ptr(r_tri), r_tri.shape[1], *args[10:], _ptr(innov), _lib.INNOV_MODEL[innovation_model], *tail,
+                _ptr(dt_cols), _ptr(lengths), math.inf if gate is None else float(gate),
+                _ptr(gate_count if gate is not None else None), _ptr(out_gated), _ptr(out_innovation),
+                out_innovation.stride(0) if out_innovation is not None else 0)
+        elif general:
             rc = _lib.load().posekf_replay_general_f32(
                 N, T, _ptr(streams), Ns, _ptr(dt_t), per_step, _ptr(acc_ref), _ptr(mag_ref), _ptr(q_tri), q_tri.shape[1],
                 _ptr(r_tri), r_tri.shape[1], *args[10:], None, _lib.INNOV_MODEL["full"], *tail, _ptr(dt_cols), _ptr(lengths))
@@ -515,7 +569,8 @@ def replay(streams: torch.Tensor, acc_ref: torch.Tensor, mag_ref: torch.Tensor, 
             rc = _lib.load().posekf_replay_f32(*args, *tail)
         else:
             rc = _lib.load().posekf_replay_innovation_ex_f32(*args, _ptr(innov), _lib.INNOV_MODEL[innovation_model], *tail)
-    _lib.check(rc, "posekf_replay_general_f32" if general else "posekf_replay_innovation_steps_f32" if out_innovation is not None
+    _lib.check(rc, "posekf_replay_general_innovation_f32" if general and general_innovation else
+               "posekf_replay_general_f32" if general else "posekf_replay_innovation_steps_f32" if out_innovation is not None
                else "posekf_replay_gated_f32" if gate is not None else
                "posekf_replay_batch_f32" if batch else
                ("posekf_replay_f32" if innov is None else "posekf_replay_innovation_ex_f32"))

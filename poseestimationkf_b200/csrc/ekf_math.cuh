@@ -35,7 +35,7 @@
 
 #if defined(__CUDACC__)
 #define PKF_HD __host__ __device__ __forceinline__
-#define PKF_HD_RARE __host__ __device__ __noinline__      // rare paths: kept out of line so they cost the hot code no registers
+#define PKF_HD_RARE __host__ __device__ __noinline__ inline   // rare paths: kept out of line so they cost the hot code no registers
 #else
 #define PKF_HD inline
 #define PKF_HD_RARE inline
@@ -1402,6 +1402,16 @@ template <typename F> struct GainGen {
 struct NoGainGen {};
 template <typename F, bool GEN> struct GainGenOf { typedef GainGen<F> type; };   // (empty in the other instantiations)
 template <typename F> struct GainGenOf<F, false> { typedef NoGainGen type; };
+// GEN with INNOV or GATE: the pivots d_k of S = L D L^T (the innovation terms) and, gated only, P^- (see GEN INNOVATION
+// below).  Empty in every other instantiation, like GainGen: declared state that a kernel does not use still moves the
+// code of the others.
+template <typename F> struct GenInnov {
+  F d0, d1, d2, d3;   // pivots
+  F i0, i1, i2, i3;   // 1/d_k, as the gain uses them
+  Sym4<F> Pm;         // GATE only
+};
+template <typename F, bool ON> struct GenInnovOf { typedef GenInnov<F> type; };
+template <typename F> struct GenInnovOf<F, false> { typedef NoGainGen type; };
 
 // q [6], r [10]: the upper triangles of Q and R in the reference frame (row-major, the order of Sym4).  filter_frame:
 // express them in the filter frame of fc (p = conj(qE), Rot(p) = E^T).
@@ -1454,20 +1464,29 @@ PKF_HD Sym4<F> propagate_cov_general(const Sym4<F>& P, const Vec3<F>& hw, const 
 }
 
 // S = P^- + R = L D L^T, H = D^-1 L^-1 R and P^+ = R - (L^-1 R)^T H (see GENERAL Q AND R above).
-template <typename F> PKF_HD GainGen<F> kalman_gain_general(const Sym4<F>& Pm, const Sym4<F>& R) {
+// PIV: the pivots d_k also go to *gi.
+template <typename F, bool PIV = false>
+PKF_HD GainGen<F> kalman_gain_general(const Sym4<F>& Pm, const Sym4<F>& R, GenInnov<F>* gi = nullptr) {
   const F s00 = Pm.a00 + R.a00, s01 = Pm.a01 + R.a01, s02 = Pm.a02 + R.a02, s03 = Pm.a03 + R.a03;
   const F s11 = Pm.a11 + R.a11, s12 = Pm.a12 + R.a12, s13 = Pm.a13 + R.a13;
   const F s22 = Pm.a22 + R.a22, s23 = Pm.a23 + R.a23, s33 = Pm.a33 + R.a33;
   GainGen<F> g;
   const F i0 = rcp_(s00);
   g.l10 = s01 * i0; g.l20 = s02 * i0; g.l30 = s03 * i0;
-  const F i1 = rcp_(fma_(-g.l10, s01, s11));
+  const F d1 = fma_(-g.l10, s01, s11);
+  const F i1 = rcp_(d1);
   const F t21 = fma_(-g.l10, s02, s12), t31 = fma_(-g.l10, s03, s13);
   g.l21 = t21 * i1; g.l31 = t31 * i1;
-  const F i2 = rcp_(fma_(-g.l21, t21, fma_(-g.l20, s02, s22)));
+  const F d2 = fma_(-g.l21, t21, fma_(-g.l20, s02, s22));
+  const F i2 = rcp_(d2);
   const F t32 = fma_(-g.l21, t31, fma_(-g.l20, s03, s23));
   g.l32 = t32 * i2;
-  const F i3 = rcp_(fma_(-g.l32, t32, fma_(-g.l31, t31, fma_(-g.l30, s03, s33))));
+  const F d3 = fma_(-g.l32, t32, fma_(-g.l31, t31, fma_(-g.l30, s03, s33)));
+  const F i3 = rcp_(d3);
+  if constexpr (PIV) {
+    gi->d0 = s00; gi->d1 = d1; gi->d2 = d2; gi->d3 = d3;
+    gi->i0 = i0; gi->i1 = i1; gi->i2 = i2; gi->i3 = i3;
+  }
   const F Rm[4][4] = {{R.a00, R.a01, R.a02, R.a03}, {R.a01, R.a11, R.a12, R.a13}, {R.a02, R.a12, R.a22, R.a23},
                       {R.a03, R.a13, R.a23, R.a33}};
   F G[4][4];      // L^-1 R, column by column
@@ -1488,14 +1507,90 @@ template <typename F> PKF_HD GainGen<F> kalman_gain_general(const Sym4<F>& Pm, c
   return g;
 }
 
-// Prediction with general Q and R: the gain stage and the RK4 prediction z (plain-variant form)
-template <typename F>
+// Prediction with general Q and R: the gain stage and the RK4 prediction z (plain-variant form).
+// PIV: the pivots of S go to *gi (INNOV / GATE); PM: P^- too (GATE).
+template <typename F, bool PIV = false, bool PM = false>
 PKF_HD void ekf_predict_general(const Quat<F>& x, const Sym4<F>& P, const FilterConst<F>& fc, const GenQR<F>& gq,
-                                const Vec3<F>& gyro, const StepH<F>& h, GainGen<F>& gg, Quat<F>& z) {
+                                const Vec3<F>& gyro, const StepH<F>& h, GainGen<F>& gg, Quat<F>& z,
+                                GenInnov<F>* gi = nullptr) {
   Vec3<F> hw;
   hw.x = F(0.5) * gyro.x; hw.y = F(0.5) * gyro.y; hw.z = F(0.5) * gyro.z;
-  gg = kalman_gain_general(propagate_cov_general(P, hw, x, fc.gs, gq.q4), gq.R);     // :59-66
+  if constexpr (PIV) {
+    const Sym4<F> Pm = propagate_cov_general(P, hw, x, fc.gs, gq.q4);                  // :59-61
+    if constexpr (PM) gi->Pm = Pm;
+    gg = kalman_gain_general<F, true>(Pm, gq.R, gi);                                     // :63-66
+  } else {
+    gg = kalman_gain_general(propagate_cov_general(P, hw, x, fc.gs, gq.q4), gq.R);     // :59-66
+  }
   z = rk4_predict_fused(x, hw, h);                                                       // :62
+}
+
+// ------------------------------------------------------------------------------------------
+// GEN INNOVATION: the innovation terms and the gate of a filter with general Q and R, in true units (the covariance is
+// not scaled: no 1/r, no dof ln r).  S = P^- + R = L D L^T is already factored by the gain stage, and t = L^-1 e is the
+// quantity the update forms; S^-1 itself is never formed.
+//   4-D:      NIS = e^T S^-1 e = s = sum_k t_k^2 / d_k,      ln det S = sum_k ln d_k
+//   tangent:  v = L^-1 z,  c = z^T S^-1 z = sum_k v_k^2 / d_k,  b = z^T S^-1 e = sum_k v_k t_k / d_k;  for any orthonormal
+//             basis E of z-perp, e_3 = E^T e and S_3 = E^T S E,
+//               NIS_3 = e_3^T S_3^-1 e_3 = s - b^2/c                          (Schur complement of u = z/|z|)
+//               ln det S_3 = ln det S + ln(c/|z|^2)                           (det(E^T S E) = det S . u^T S^-1 u)
+// The log-determinant is summed from the logs of two pivot products, never the log of the product of four: pivots in
+// [1e-18, 1e18] then neither underflow nor overflow.  The sums add each step's terms as they are written out (one
+// addition each), so a sum is exactly the float32 running sum of its per-step terms.
+// Gate: gated <=> NIS_3 > gamma (strict: NaN is never gated).  A gated lane zeroes its innovation (X = z, normalised) and
+// keeps P^-, selected per lane.
+// ------------------------------------------------------------------------------------------
+template <typename F, bool TAN>
+PKF_HD void gen_innov_terms(const GainGen<F>& gg, const GenInnov<F>& gi, const Quat<F>& z, F e0, F e1, F e2, F e3,
+                            F& nis, F& logdet) {
+  const F t0 = e0;                                 // t = L^-1 e (the update's)
+  const F t1 = fma_(-gg.l10, t0, e1);
+  const F t2 = fma_(-gg.l21, t1, fma_(-gg.l20, t0, e2));
+  const F t3 = fma_(-gg.l32, t2, fma_(-gg.l31, t1, fma_(-gg.l30, t0, e3)));
+  const F u0 = gi.i0 * t0, u1 = gi.i1 * t1, u2 = gi.i2 * t2, u3 = gi.i3 * t3;
+  const F s = fma_(u3, t3, fma_(u2, t2, fma_(u1, t1, u0 * t0)));
+  const F ld = log_(gi.d0 * gi.d1) + log_(gi.d2 * gi.d3);
+  if constexpr (!TAN) {
+    nis = s;
+    logdet = ld;
+  } else {
+    const F v0 = z.w;                                // v = L^-1 z
+    const F v1 = fma_(-gg.l10, v0, z.x);
+    const F v2 = fma_(-gg.l21, v1, fma_(-gg.l20, v0, z.y));
+    const F v3 = fma_(-gg.l32, v2, fma_(-gg.l31, v1, fma_(-gg.l30, v0, z.z)));
+    const F g0 = gi.i0 * v0, g1 = gi.i1 * v1, g2 = gi.i2 * v2, g3 = gi.i3 * v3;
+    const F c = fma_(g3, v3, fma_(g2, v2, fma_(g1, v1, g0 * v0)));
+    const F b = fma_(g3, t3, fma_(g2, t2, fma_(g1, t1, g0 * t0)));
+    nis = fma_(-b, b * rcp_(c), s);
+    logdet = ld + log_(c * rcp_(dot4(z, z)));
+  }
+}
+
+// INNOV: the step's terms are added to *acc (acc.inv_r / acc.log_rd unused) and handed to *step when it is set
+template <typename F, bool TAN>
+PKF_HD void gen_innov_accumulate(InnovAcc<F>& acc, const GainGen<F>& gg, const GenInnov<F>& gi, const Quat<F>& z, F e0,
+                                 F e1, F e2, F e3, InnovTerms<F>* step = nullptr) {
+  F nis, ld;
+  gen_innov_terms<F, TAN>(gg, gi, z, e0, e1, e2, e3, nis, ld);
+  acc.nis = acc.nis + nis;
+  acc.logdet = acc.logdet + ld;
+  if (step) { step->nis = nis; step->logdet = ld; }
+}
+
+// GATE: the decision on NIS_3 (the same value as the tangent term), applied per lane to e and P^+
+template <typename F, typename FlagT>
+PKF_HD void gen_gate_apply(const GateParams<F>& gp, GainGen<F>& gg, const GenInnov<F>& gi, const Quat<F>& z, F& e0, F& e1,
+                           F& e2, F& e3, FlagT& gated) {
+  F nis3, ld;
+  gen_innov_terms<F, true>(gg, gi, z, e0, e1, e2, e3, nis3, ld);
+  const auto g = nis3 > gp.thr;
+  gated = g;
+  e0 = sel_(g, F(0), e0); e1 = sel_(g, F(0), e1); e2 = sel_(g, F(0), e2); e3 = sel_(g, F(0), e3);
+  Sym4<F>& P = gg.Pp;
+  const Sym4<F>& Pm = gi.Pm;
+  P.a00 = sel_(g, Pm.a00, P.a00); P.a01 = sel_(g, Pm.a01, P.a01); P.a02 = sel_(g, Pm.a02, P.a02); P.a03 = sel_(g, Pm.a03, P.a03);
+  P.a11 = sel_(g, Pm.a11, P.a11); P.a12 = sel_(g, Pm.a12, P.a12); P.a13 = sel_(g, Pm.a13, P.a13);
+  P.a22 = sel_(g, Pm.a22, P.a22); P.a23 = sel_(g, Pm.a23, P.a23); P.a33 = sel_(g, Pm.a33, P.a33);
 }
 
 // X = z + K e, normalised; P = P^+                                                         :77-79
@@ -1518,7 +1613,8 @@ PKF_HD void ekf_update_general(Quat<F>& x, Sym4<F>& P, FilterConst<F>& fc, const
 // Prediction + Correction with the measurement quaternion y (filter frame, any sign, norm 1/inv_norm) already computed.
 // INNOV: the innovation likelihood of the step is added to *innov (see InnovAcc); the filter itself is unchanged.
 // TAN: its tangent-space form (see innov_accumulate).  GATE: the innovation gate (see GateParams), decision in *gated.
-// GEN: general Q and R from *gen (see GENERAL Q AND R); P is unscaled, plain variant only.
+// GEN: general Q and R from *gen (see GENERAL Q AND R); P is unscaled, plain variant only.  With INNOV / GATE: the terms
+// and the gate of GEN INNOVATION.
 // terms (INNOV): the step's own innovation terms (see InnovTerms), or null.
 template <typename F, bool WANT_FLIP, bool COMP, bool INNOV = false, bool TAN = false, bool GATE = false, bool GEN = false,
           typename FlagT>
@@ -1527,20 +1623,27 @@ PKF_HD void ekf_step_measured(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<
                               typename FlipCodeOf<F>::type* code = nullptr, InnovAcc<F>* innov = nullptr,
                               const GateParams<F>* gate = nullptr, FlagT* gated = nullptr, const GenQR<F>* gen = nullptr,
                               InnovTerms<F>* terms = nullptr) {
-  static_assert(!GEN || !(COMP || INNOV || GATE), "general Q and R: plain variant, no innovation sums, no gate");
+  static_assert(!GEN || !COMP, "general Q and R: plain variant only");
   Sym4<F> K, Pm;
   Quat<F> inc, z;
   InnovFactors<F> fac;
   [[maybe_unused]] typename GainGenOf<F, GEN>::type gg;
-  if constexpr (GEN) ekf_predict_general(x, P, fc, *gen, gyro, h, gg, z);
+  [[maybe_unused]] typename GenInnovOf<F, GEN && (INNOV || GATE)>::type gi;
+  if constexpr (GEN && (INNOV || GATE)) ekf_predict_general<F, true, GATE>(x, P, fc, *gen, gyro, h, gg, z, &gi);
+  else if constexpr (GEN) ekf_predict_general(x, P, fc, *gen, gyro, h, gg, z);
   else ekf_predict<F, COMP, INNOV, GATE>(x, P, fc, gyro, h, K, inc, z, &fac, &Pm);
   const F dyz = dot4(y, z);                       // the comparator, literally: negate when dot(y, z) < 0  :73-75
   flip = FlagT();
   if (WANT_FLIP && flip_wanted) flip = reference_flip_quat(fc, y, one_with_sign_(dyz), code);
   const F sn = copysign_(inv_norm, dyz);          // e = sg y/|y| - z, sg = sign(dot): the sign bit moves onto 1/|y| > 0  :76
   F e0 = fma_(sn, y.w, -z.w), e1 = fma_(sn, y.x, -z.x), e2 = fma_(sn, y.y, -z.y), e3 = fma_(sn, y.z, -z.z);
-  if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3, terms);
-  if constexpr (GATE) gate_apply<F, COMP>(*gate, fac, z, Pm, K, e0, e1, e2, e3, *gated);
+  if constexpr (GEN) {
+    if constexpr (INNOV) gen_innov_accumulate<F, TAN>(*innov, gg, gi, z, e0, e1, e2, e3, terms);
+    if constexpr (GATE) gen_gate_apply(*gate, gg, gi, z, e0, e1, e2, e3, *gated);
+  } else {
+    if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3, terms);
+    if constexpr (GATE) gate_apply<F, COMP>(*gate, fac, z, Pm, K, e0, e1, e2, e3, *gated);
+  }
   if constexpr (GEN) ekf_update_general(x, P, fc, gg, z, e0, e1, e2, e3);
   else ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);
 }
@@ -1575,12 +1678,14 @@ PKF_HD void ekf_step(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, c
     ekf_step_measured<F, WANT_FLIP, COMP, INNOV, TAN, GATE, GEN>(x, xlo, P, fc, gyro, y, inv_norm, h, flip, flip_wanted, code,
                                                                  innov, gate, gated, gen, terms);
   } else {
-    static_assert(!GEN || !(COMP || INNOV || GATE), "general Q and R: plain variant, no innovation sums, no gate");
+    static_assert(!GEN || !COMP, "general Q and R: plain variant only");
     Sym4<F> K, Pm;
     Quat<F> inc, z;
     InnovFactors<F> fac;
     [[maybe_unused]] typename GainGenOf<F, GEN>::type gg;
-    if constexpr (GEN) ekf_predict_general(x, P, fc, *gen, gyro, h, gg, z);
+    [[maybe_unused]] typename GenInnovOf<F, GEN && (INNOV || GATE)>::type gi;
+    if constexpr (GEN && (INNOV || GATE)) ekf_predict_general<F, true, GATE>(x, P, fc, *gen, gyro, h, gg, z, &gi);
+    else if constexpr (GEN) ekf_predict_general(x, P, fc, *gen, gyro, h, gg, z);
     else ekf_predict<F, COMP, INNOV, GATE>(x, P, fc, gyro, h, K, inc, z, &fac, &Pm);
     // ---- Correction (PKF/ExtendedKalmanFilter.py:70-80) ----
     F e0, e1, e2, e3;
@@ -1615,8 +1720,13 @@ PKF_HD void ekf_step(Quat<F>& x, Quat<F>& xlo, Sym4<F>& P, FilterConst<F>& fc, c
         e2 = sel_(unrelated, yf.y - z.y, e2); e3 = sel_(unrelated, yf.z - z.z, e3);
       }
     }
-    if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3, terms);
-    if constexpr (GATE) gate_apply<F, COMP>(*gate, fac, z, Pm, K, e0, e1, e2, e3, *gated);
+    if constexpr (GEN) {
+      if constexpr (INNOV) gen_innov_accumulate<F, TAN>(*innov, gg, gi, z, e0, e1, e2, e3, terms);
+      if constexpr (GATE) gen_gate_apply(*gate, gg, gi, z, e0, e1, e2, e3, *gated);
+    } else {
+      if constexpr (INNOV) innov_accumulate<F, COMP, TAN>(*innov, fac, K, z, e0, e1, e2, e3, terms);
+      if constexpr (GATE) gate_apply<F, COMP>(*gate, fac, z, Pm, K, e0, e1, e2, e3, *gated);
+    }
     if constexpr (GEN) ekf_update_general(x, P, fc, gg, z, e0, e1, e2, e3);
     else ekf_update<F, COMP>(x, xlo, P, fc, K, z, inc, e0, e1, e2, e3);
   }

@@ -12,11 +12,14 @@
 //   * no tensor cores (per-filter matrices are 4x4), no inter-thread communication on the step;
 //   * filters are independent: multi-GPU = shard N, no collective on this path.
 //
-// Build: nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 --shared -Xcompiler -fPIC
+// Build: nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 --shared -Xcompiler -fPIC, with
+// replay_general_innovation.cu (poseestimationkf_b200/build.py compiles the two in parallel and links them)
 //
 // Files: ekf_math.cuh (per-filter arithmetic, scalar and packed), device_util.cuh (TMA / mbarrier /
 // streaming access helpers, tunables), replay_kernels.cuh (the three fused replay kernels),
-// ops_kernels.cuh (stand-alone operators), this file (launch logic and the extern "C" surface).
+// ops_kernels.cuh (stand-alone operators), replay_launch.cuh (launch helpers shared with
+// replay_general_innovation.cu, which launches the general-matrix innovation kernels in a device module of its own),
+// this file (launch logic and the extern "C" surface).
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -30,57 +33,15 @@
 #include "device_util.cuh"
 #include "replay_kernels.cuh"
 #include "ops_kernels.cuh"
+#include "replay_launch.cuh"
 
 using namespace pkf;
 using namespace pkf_dev;
+using namespace pkf_host;
 
 namespace {
 
-#define PKF_CUDA_TRY(expr)                           \
-  do {                                               \
-    cudaError_t _e = (expr);                         \
-    if (_e != cudaSuccess) return (int)_e;           \
-  } while (0)
-
 inline unsigned blocks_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
-
-inline int launch_status() {
-  cudaError_t e = cudaPeekAtLastError();
-  return e == cudaSuccess ? 0 : (int)e;
-}
-
-// ---------------------------------------------------------------------------------------------
-// launch logic
-// ---------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = []() -> EncodeTiledFn {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess) return nullptr;
-    if (q != cudaDriverEntryPointSuccess) return nullptr;
-    return (EncodeTiledFn)p;
-  }();
-  return fn;
-}
-
-// Tensor map over the stream [T][9][Ns] (float32) with a box of `columns` filters x 9 channels x `steps`
-// timesteps; out-of-range columns / steps are zero-filled by the TMA unit.
-int encode_stream_map(const ReplayParams& p, int columns, int steps, CUtensorMap* tmap) {
-  EncodeTiledFn enc = get_encode_fn();
-  if (!enc) return POSEKF_ENODEV;
-  const cuuint64_t dims[3] = {(cuuint64_t)p.Ns, (cuuint64_t)kChannels, (cuuint64_t)p.T};
-  const cuuint64_t strides[2] = {(cuuint64_t)p.Ns * sizeof(float), (cuuint64_t)p.Ns * kChannels * sizeof(float)};
-  const cuuint32_t box[3] = {(cuuint32_t)columns, (cuuint32_t)kChannels, (cuuint32_t)steps};
-  const cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(p.streams), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS ? 0 : POSEKF_EALIGN;
-}
 
 bool tma_eligible(const ReplayParams& p) {
   if ((reinterpret_cast<uintptr_t>(p.streams) & 15) != 0) return false;
@@ -89,25 +50,6 @@ bool tma_eligible(const ReplayParams& p) {
   if (p.Ns != p.N && (p.Ns % kThreads) != 0) return false;   // a CTA's 128 columns must not wrap
   if (p.T > INT32_MAX || p.Ns > INT32_MAX) return false;
   return true;
-}
-
-// ga: the gate's arguments (one GateArgs; GATE launches only) or the general Q and R (one GenQRArgs; GEN launches only);
-// the others pass none
-template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false, bool GATE = false,
-          bool GEN = false, typename... GA>
-int launch_replay(const ReplayParams& p, bool use_tma, cudaStream_t st, const GA&... ga) {
-  const unsigned grid = (unsigned)((p.N + kThreads - 1) / kThreads);
-  if (!use_tma) {
-    replay_ldg_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH, GATE, GEN, GA...><<<grid, kThreads, 0, st>>>(p, ga...);
-    return launch_status();
-  }
-  CUtensorMap tmap;
-  if (int rc = encode_stream_map(p, kThreads, kTmaSteps, &tmap)) return rc;
-  auto kern = replay_tma_kernel<ALGO, LPF, AUX, COMP, INNOV, TAN, BATCH, GATE, GEN, GA...>;
-  // idempotent; set on every launch (cheap) so that it holds on every device of a multi-GPU process
-  PKF_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TmaSmem)));
-  kern<<<grid, kThreads, sizeof(TmaSmem), st>>>(p, tmap, ga...);
-  return launch_status();
 }
 
 bool packed_eligible(const ReplayParams& p) {
@@ -305,7 +247,8 @@ int launch_innov_steps_algo(const ReplayParams& p, const GateArgs* gate, const I
 
 // innov_model: POSEKF_INNOV_* of the sums in p.innov_acc (read only when it is set, or with steps).  gate: run the gated
 // kernels with these arguments (null: the ungated ones).  gen: run the general-matrix kernels with these matrices.
-// steps: run the innovation-steps kernels, which write the per-step terms there.
+// steps: run the innovation-steps kernels, which write the per-step terms there (with gen: the general-matrix kernels
+// with the innovation terms, whose output there may be null).
 int replay_dispatch(const ReplayParams& p, int algo, int staging, int innov_model, cudaStream_t st, const GateArgs* gate = nullptr,
                     const GenQRArgs* gen = nullptr, const InnovStepArgs* steps = nullptr) {
   const bool lpf = (p.alpha_acc >= 0.f) || (p.alpha_mag >= 0.f);
@@ -320,7 +263,8 @@ int replay_dispatch(const ReplayParams& p, int algo, int staging, int innov_mode
     packed = use_tma && kAutoPrefersPacked && algo != POSEKF_WAHBA_JACOBI && packed_eligible(p);
   } else return POSEKF_EINVAL;
   const bool batch = p.dt_cols != nullptr || p.n_valid != nullptr;
-  int rc = gen ? launch_general_algo(p, *gen, algo, lpf, use_tma, st)
+  int rc = gen ? (steps ? launch_general_innov_algo(p, *gen, gate, *steps, algo, lpf, use_tma, innov_model, st)
+                        : launch_general_algo(p, *gen, algo, lpf, use_tma, st))
            : steps ? launch_innov_steps_algo(p, gate, *steps, algo, lpf, use_tma, innov_model, st)
            : gate ? launch_gated_algo(p, *gate, algo, lpf, use_tma, packed, innov_model, st)
                 : batch ? launch_kernels<true>(p, algo, lpf, use_tma, packed, innov_model, st)
@@ -514,6 +458,37 @@ int posekf_replay_general_f32(int64_t n_filters, int64_t n_steps, const float* s
                       lpf_alpha_mag, state_x, nullptr, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, nullptr,
                       innov_model, wahba_algo, staging, state_flags, stream, dt_cols, n_valid, false, 0.f, nullptr, nullptr,
                       &gq);
+}
+
+int posekf_replay_general_innovation_f32(int64_t n_filters, int64_t n_steps, const float* streams, int64_t n_streams,
+                                         const float* dt, int dt_per_step, const float* acc_ref, const float* mag_ref,
+                                         const float* q_tri, int64_t nq, const float* r_tri, int64_t nr, float lpf_alpha_acc,
+                                         float lpf_alpha_mag, float* state_x, float* state_x_lo, float* state_p,
+                                         float* state_lpf, float* out_traj, uint8_t* out_flip, const float* truth,
+                                         float* loss_acc, float* innov_acc, int innov_model, int wahba_algo, int staging,
+                                         int state_flags, void* stream, const float* dt_cols, const int32_t* n_valid,
+                                         float gate_nis3, int32_t* gate_count, uint8_t* out_gated, float* out_innov,
+                                         int64_t innov_plane_stride) {
+  if (innov_model != POSEKF_INNOV_FULL && innov_model != POSEKF_INNOV_TANGENT) return POSEKF_EINVAL;
+  if (gate_nis3 != gate_nis3) return POSEKF_EINVAL;
+  if (state_x_lo) return POSEKF_EINVAL;                  // no precise variant with general matrices
+  if (n_filters < 0 || n_steps < 0) return POSEKF_EINVAL;
+  if (n_filters > 0 && (!q_tri || !r_tri || (nq != 1 && nq != n_filters) || (nr != 1 && nr != n_filters))) return POSEKF_EINVAL;
+  if (out_innov && n_filters > 0 && n_steps > 0) {
+    if (n_steps > INT64_MAX / n_filters || innov_plane_stride < n_filters * n_steps) return POSEKF_EINVAL;
+  }
+  if ((reinterpret_cast<uintptr_t>(q_tri) & 3) != 0 || (reinterpret_cast<uintptr_t>(r_tri) & 3) != 0) return POSEKF_EALIGN;
+  if ((reinterpret_cast<uintptr_t>(out_innov) & 3) != 0) return POSEKF_EALIGN;
+  const GenQRArgs gq{q_tri, nq, r_tri, nr};
+  // +inf with no gate buffer decides nothing and records nothing: the ungated kernels (the same bits); a launch that
+  // asks for no innovation output at all is the plain general replay
+  const bool gate = !(gate_nis3 == INFINITY && !gate_count && !out_gated);
+  const InnovStepArgs ia{out_innov, innov_plane_stride};
+  const bool terms = innov_acc || out_innov || gate;
+  return replay_entry(n_filters, n_steps, streams, n_streams, dt, dt_per_step, acc_ref, mag_ref, nullptr, nullptr, lpf_alpha_acc,
+                      lpf_alpha_mag, state_x, nullptr, state_p, state_lpf, out_traj, out_flip, truth, loss_acc, innov_acc,
+                      innov_model, wahba_algo, staging, state_flags, stream, dt_cols, n_valid, gate, gate_nis3, gate_count,
+                      out_gated, &gq, terms ? &ia : nullptr);
 }
 
 // ---- host-buffer replay: workspace (device staging buffers, streams, events) ----------------------

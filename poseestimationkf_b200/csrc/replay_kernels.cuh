@@ -62,8 +62,10 @@ struct GateRegs {
 };
 struct NoGateRegs {};
 template <bool GATE> using GateRegsOf = typename std::conditional<GATE, GateRegs, NoGateRegs>::type;
-template <bool AUX> __device__ __forceinline__ void load_gate(const ReplayParams& p, const GateArgs& ga, int64_t n, GateRegs& g) {
-  g.gp = make_gate_params<float>(p.r_scale[n], ga.gate_nis3);
+// (GEN: the covariance is unscaled, the threshold is gamma itself)
+template <bool AUX, bool GEN = false>
+__device__ __forceinline__ void load_gate(const ReplayParams& p, const GateArgs& ga, int64_t n, GateRegs& g) {
+  g.gp = make_gate_params<float>(GEN ? 1.f : p.r_scale[n], ga.gate_nis3);
   g.count = ga.gate_count ? ga.gate_count[n] : 0;
   g.out = (AUX && ga.out_gated) ? ga.out_gated + n : nullptr;
 }
@@ -98,6 +100,13 @@ struct GenQRArgs {
   int64_t nr;
 };
 __device__ __forceinline__ GenQRArgs gen_args_(const GenQRArgs& g) { return g; }     // (GEN kernels: their one argument)
+// GEN kernels with the innovation terms: GenQRArgs, an optional GateArgs, then InnovStepArgs, whose `out` may be null
+// there (a launch that asks for the sums or the gate only; one launch-uniform branch per step)
+__device__ __forceinline__ GenQRArgs gen_args_(const GenQRArgs& g, const InnovStepArgs&) { return g; }
+__device__ __forceinline__ GenQRArgs gen_args_(const GenQRArgs& g, const GateArgs&, const InnovStepArgs&) { return g; }
+__device__ __forceinline__ GateArgs gate_args_(const GenQRArgs&, const GateArgs& g, const InnovStepArgs&) { return g; }
+__device__ __forceinline__ InnovStepArgs innov_step_args_(const GenQRArgs&, const InnovStepArgs& a) { return a; }
+__device__ __forceinline__ InnovStepArgs innov_step_args_(const GenQRArgs&, const GateArgs&, const InnovStepArgs& a) { return a; }
 struct GenRegs { GenQR<float> m; };
 struct NoGenRegs {};
 template <bool GEN> using GenRegsOf = typename std::conditional<GEN, GenRegs, NoGenRegs>::type;
@@ -120,8 +129,9 @@ __device__ __forceinline__ void load_filter(const ReplayParams& p, int64_t n, in
   Vec3<float> rm = {p.mag_ref[col], p.mag_ref[Ns + col], p.mag_ref[2 * Ns + col]};
   f.fc = make_filter_const<float>(ra, rm, GEN ? 4.f : p.q_scale[n], GEN ? 1.f : p.r_scale[n]);
   if (INNOV) {
-    if (OPT_ACC && !p.innov_acc) f.in = make_innov_acc<float, TAN>(0.f, 0.f, p.r_scale[n]);
-    else f.in = make_innov_acc<float, TAN>(p.innov_acc[n], p.innov_acc[N + n], p.r_scale[n]);
+    // (GEN: r = 1, true units: the sums add the terms as they are)
+    if (OPT_ACC && !p.innov_acc) f.in = make_innov_acc<float, TAN>(0.f, 0.f, GEN ? 1.f : p.r_scale[n]);
+    else f.in = make_innov_acc<float, TAN>(p.innov_acc[n], p.innov_acc[N + n], GEN ? 1.f : p.r_scale[n]);
   }
   f.x = {p.state_x[n], p.state_x[N + n], p.state_x[2 * N + n], p.state_x[3 * N + n]};
   f.xlo = {0.f, 0.f, 0.f, 0.f};
@@ -190,7 +200,18 @@ __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f
   // in float64 after the launch (raw samples only: a low-passed sample is not in the stream any more)
   unsigned code = 0;
   [[maybe_unused]] InnovTerms<float> it;
-  if constexpr (GATE) {
+  if constexpr (GEN && INNOV) {     // general Q and R with the innovation terms (GATE: and the gate)
+    [[maybe_unused]] bool gated = false;
+    const GateParams<float>* gp = nullptr;
+    if constexpr (GATE) gp = &g.gp;
+    ekf_step<float, ALGO, AUX, false, true, TAN, GATE, true>(f.x, f.xlo, f.P, f.fc, w, a, m, StepH<float>(h), flip,
+                                                           aux.flips != nullptr, (AUX && !LPF && ALGO == WAHBA_QR2) ? &code : nullptr,
+                                                           &f.in, gp, &gated, &gr->m, OUT ? &it : nullptr);
+    if constexpr (GATE) {
+      g.count += gated ? 1 : 0;
+      if (g.out) { *g.out = gated ? 1 : 0; g.out += p.N; }
+    }
+  } else if constexpr (GATE) {
     bool gated = false;
     ekf_step<float, ALGO, AUX, COMP, INNOV, TAN, true>(f.x, f.xlo, f.P, f.fc, w, a, m, StepH<float>(h), flip, aux.flips != nullptr,
                                                        (AUX && !LPF && ALGO == WAHBA_QR2) ? &code : nullptr, INNOV ? &f.in : nullptr,
@@ -207,9 +228,11 @@ __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f
                                                  nullptr, (bool*)nullptr, nullptr, OUT ? &it : nullptr);
   }
   if constexpr (OUT) {     // [2][T][N]: a warp's store of one plane is one 128-byte line
-    __stcs(io->out, it.nis);
-    __stcs(io->out + io->plane, it.logdet);
-    io->out += p.N;
+    if (!GEN || io->out) {
+      __stcs(io->out, it.nis);
+      __stcs(io->out + io->plane, it.logdet);
+      io->out += p.N;
+    }
   }
   if (!(AUX && !LPF && ALGO == WAHBA_QR2)) code = flip ? 1u : 0u;
   if (AUX) {
@@ -240,12 +263,14 @@ __device__ __forceinline__ void filter_step(const ReplayParams& p, FilterRegs& f
 // A step at or past the length of the filter's stream (BATCH kernels): the filter is left as it is, the trajectory slot
 // gets the held state, the flip byte is 0 (unmarked: flip_fixup_kernel leaves it alone) and the objectives add nothing.
 // The step's sample and dt are not read.
-// (OUT: both innovation terms are 0)
-template <int ALGO, bool AUX, bool GATE = false, bool OUT = false>
+// (OUT: both innovation terms are 0; GEN: when io->out is set)
+template <int ALGO, bool AUX, bool GATE = false, bool OUT = false, bool GEN = false>
 __device__ __forceinline__ void hold_step(const ReplayParams& p, const FilterRegs& f, AuxPtrs& aux, GateRegsOf<GATE>& g,
                                           InnovStepRegsOf<OUT>* io = nullptr) {
   if constexpr (GATE) { if (g.out) { *g.out = 0; g.out += p.N; } }
-  if constexpr (OUT) { __stcs(io->out, 0.f); __stcs(io->out + io->plane, 0.f); io->out += p.N; }
+  if constexpr (OUT) {
+    if (!GEN || io->out) { __stcs(io->out, 0.f); __stcs(io->out + io->plane, 0.f); io->out += p.N; }
+  }
   if (AUX) {
     if (aux.traj) {
       Quat<float> xr = f.x;
@@ -265,7 +290,8 @@ __device__ __forceinline__ void hold_step(const ReplayParams& p, const FilterReg
 // (INNOV: the innovation likelihood, TAN: its tangent-space form; their instantiations always have AUX and are built for
 //  3 CTAs per SM, <= 168 registers.  BATCH: per-stream dt columns and lengths, ReplayParams::dt_cols / n_valid)
 //  GATE: the innovation gate, its arguments in the pack ga (one GateArgs; empty in the other kernels).
-//  GEN: general Q and R matrices, the pack holds one GenQRArgs; plain variant, no innovation sums, no gate.
+//  GEN: general Q and R matrices, the pack holds one GenQRArgs; plain variant.  GEN with INNOV: the pack is GenQRArgs,
+//  an optional GateArgs (GATE) and an InnovStepArgs whose output, like innov_acc, is optional.
 //  Innovation steps: the pack ends in an InnovStepArgs (OUT); INNOV kernels only, innov_acc optional)
 template <int ALGO, bool LPF, bool AUX, bool COMP, bool INNOV = false, bool TAN = false, bool BATCH = false, bool GATE = false,
           bool GEN = false, typename... GA>
@@ -281,9 +307,12 @@ __global__ void __launch_bounds__(kThreads, (INNOV || GATE || GEN) ? 3 : ((ALGO 
   load_filter<ALGO, LPF, COMP, INNOV, TAN, GEN, OUT>(p, n, col, f);
   AuxPtrs aux = make_aux<AUX>(p, n, col, true);
   [[maybe_unused]] GateRegsOf<GATE> g;
-  if constexpr (GATE) load_gate<AUX>(p, gate_args_(ga...), n, g);
+  if constexpr (GATE) load_gate<AUX, GEN>(p, gate_args_(ga...), n, g);
   [[maybe_unused]] InnovStepRegsOf<OUT> io;
-  if constexpr (OUT) { const InnovStepArgs a = innov_step_args_(ga...); io = {a.out + n, a.plane}; }
+  if constexpr (OUT) {
+    const InnovStepArgs a = innov_step_args_(ga...);
+    io = {(!GEN || a.out) ? a.out + n : nullptr, a.plane};
+  }
   [[maybe_unused]] GenRegsOf<GEN> gr;
   if constexpr (GEN) load_gen<ALGO>(gen_args_(ga...), n, f.fc, gr);
   const float* s = p.streams + col;
@@ -305,7 +334,7 @@ __global__ void __launch_bounds__(kThreads, (INNOV || GATE || GEN) ? 3 : ((ALGO 
     if (BATCH && dc) hnxt = ldg_stream(dc + (int64_t)(t + 1 < T ? t + 1 : t) * Ns);
     const float h = (BATCH && dc) ? hcur : (p.dt_per_step ? __ldg(p.dt + t) : dt0);
     if (!BATCH || t < nv) filter_step<ALGO, LPF, AUX, COMP, INNOV, TAN, GATE, GEN, OUT>(p, f, cur, h, aux, g, &gr, &io);
-    else hold_step<ALGO, AUX, GATE, OUT>(p, f, aux, g, &io);
+    else hold_step<ALGO, AUX, GATE, OUT, GEN>(p, f, aux, g, &io);
 #pragma unroll
     for (int c = 0; c < kChannels; ++c) cur[c] = nxt[c];
     if (BATCH) hcur = hnxt;
@@ -392,9 +421,12 @@ __global__ void __launch_bounds__(kThreads, (INNOV || GATE || GEN) ? 3 : (ALGO =
   if (valid) load_filter<ALGO, LPF, COMP, INNOV, TAN, GEN, OUT>(p, n, (int64_t)col0 + tid, f);
   AuxPtrs aux = make_aux<AUX>(p, n, (int64_t)col0 + tid, valid);
   [[maybe_unused]] GateRegsOf<GATE> g;
-  if constexpr (GATE) { if (valid) load_gate<AUX>(p, gate_args_(ga...), n, g); }
+  if constexpr (GATE) { if (valid) load_gate<AUX, GEN>(p, gate_args_(ga...), n, g); }
   [[maybe_unused]] InnovStepRegsOf<OUT> io;
-  if constexpr (OUT) { const InnovStepArgs a = innov_step_args_(ga...); io = {a.out + n, a.plane}; }
+  if constexpr (OUT) {
+    const InnovStepArgs a = innov_step_args_(ga...);
+    io = {(!GEN || a.out) ? a.out + n : nullptr, a.plane};
+  }
   [[maybe_unused]] GenRegsOf<GEN> gr;
   if constexpr (GEN) { if (valid) load_gen<ALGO>(gen_args_(ga...), n, f.fc, gr); }
   const float dt0 = p.dt[0];
@@ -430,7 +462,7 @@ __global__ void __launch_bounds__(kThreads, (INNOV || GATE || GEN) ? 3 : (ALGO =
       for (int tt = 0; tt < kTmaSteps; ++tt) {
         if (tt < steps) {
           if constexpr (BATCH) {
-            if (k * kTmaSteps + tt >= bt.nv) { hold_step<ALGO, AUX, GATE, OUT>(p, f, aux, g, &io); continue; }
+            if (k * kTmaSteps + tt >= bt.nv) { hold_step<ALGO, AUX, GATE, OUT, GEN>(p, f, aux, g, &io); continue; }
           }
           float s[kChannels];
 #pragma unroll

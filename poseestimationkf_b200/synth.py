@@ -84,7 +84,7 @@ def _reference_pair(U, N, az_range, f64):
 
 def make_imu(n_filters: int, n_steps: int, *, seed: int = 0, sigma: float = 0.0, dt: float = 0.01,
              device="cpu", keep_truth: bool = False, out: torch.Tensor | None = None,
-             az_range=(0.02, 0.98)) -> SyntheticIMU:
+             az_range=(0.02, 0.98), gyro_sigma=None) -> SyntheticIMU:
     """Generate `n_filters` independent trajectories of `n_steps` samples.
 
     Body rate: omega_i(t) = sum_{j<3} A_ij sin(2 pi f_ij t + phi_ij), A~U(0.2,1) rad/s,
@@ -93,6 +93,8 @@ def make_imu(n_filters: int, n_steps: int, *, seed: int = 0, sigma: float = 0.0,
     random initial tilt drawn so that |acc_z| starts inside `az_range`.  Noise sigma is added to
     all three sensors, acc/mag are renormalised afterwards.  Everything is computed in float64 and
     rounded to float32 once; the oracle consumes exactly those float32 values.
+    `gyro_sigma`: (sx, sy, sz) per-body-axis gyro noise std that replaces `sigma` on the gyro (an anisotropic process
+    noise, e.g. a noisier yaw gyro); None keeps `sigma` and draws exactly the numbers it always did.
     """
     dev = torch.device(device)
     g = torch.Generator(device=dev)
@@ -116,6 +118,13 @@ def make_imu(n_filters: int, n_steps: int, *, seed: int = 0, sigma: float = 0.0,
             return v
         return v + sigma * torch.randn(v.shape, generator=g, **f64)
 
+    gyro_std = None if gyro_sigma is None else torch.as_tensor(gyro_sigma, **f64).reshape(3, 1)
+
+    def add_gyro_noise(v):
+        if gyro_std is None:
+            return add_noise(v)
+        return v + gyro_std * torch.randn(v.shape, generator=g, **f64)
+
     if sigma != 0.0:   # the references themselves are noisy samples, like a real log's sample 0
         acc0_meas, mag0_meas = _unit(add_noise(acc0)), _unit(add_noise(mag0))
     else:
@@ -136,7 +145,7 @@ def make_imu(n_filters: int, n_steps: int, *, seed: int = 0, sigma: float = 0.0,
         q = _quat_mul(q, dq)
         q = q / torch.linalg.vector_norm(q, dim=0, keepdim=True)
         # the gyro sample logged with step i is the body rate at that sample's timestamp
-        out[i, GYRO] = add_noise(w_end).to(torch.float32)
+        out[i, GYRO] = add_gyro_noise(w_end).to(torch.float32)
         out[i, ACC] = _unit(add_noise(_rotate_inverse(q, acc0))).to(torch.float32)
         out[i, MAG] = _unit(add_noise(_rotate_inverse(q, mag0))).to(torch.float32)
         if keep_truth:

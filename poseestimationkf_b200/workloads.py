@@ -179,18 +179,88 @@ def build_batch_sweep(b, grid: int = C3_GRID, lo: float = -7.0, step: float = 0.
     return SweepWorkload(b.streams, b.acc_ref, b.mag_ref, None, qs, rs, q, r, b.dt, b.lengths)
 
 
+def _pooled_innovation(streams, lengths, st: B.ReplayState, cells):
+    """(pooled NLL per step, pooled mean NIS) [*cells], float64, for a sweep whose cell c owns filters c Ns .. (c+1) Ns
+    (cells: the shape of the cell index, row-major): sum_k NLL_k / sum_k L_k and sum_k sum_t NIS / sum_k L_k."""
+    T, _, Ns = streams.shape
+    L = (lengths if lengths is not None else torch.full((Ns,), T, dtype=torch.int32, device=streams.device))
+    L = L.to(torch.float64)
+    n_steps = L.repeat(st.x.shape[1] // Ns)
+    nll, _ = B.innovation_nll(st, n_steps)
+    shape = tuple(cells) + (Ns,)
+    total = L.sum()
+    return nll.reshape(shape).sum(-1) / total, st.innov[0].to(torch.float64).reshape(shape).sum(-1) / total
+
+
 def pooled_innovation_surface(w: SweepWorkload, st: B.ReplayState):
     """([Gq, Gr] pooled innovation NLL per step, [Gq, Gr] pooled mean NIS) per cell, float64: the joint likelihood of
     all recordings of the sweep under the cell's one (Q,R), sum_k NLL_k / sum_k L_k, and sum_k sum_t NIS / sum_k L_k
     (L_k: the length of recording k; streams of length 0 add nothing).  Its argmin is the pooled tuning."""
-    T, _, Ns = w.streams.shape
-    L = (w.lengths if w.lengths is not None else torch.full((Ns,), T, dtype=torch.int32, device=w.streams.device))
-    L = L.to(torch.float64)
-    n_steps = L.repeat(st.x.shape[1] // Ns)
-    nll, _ = B.innovation_nll(st, n_steps)
-    shape = (w.qs.numel(), w.rs.numel(), Ns)
-    total = L.sum()
-    return nll.reshape(shape).sum(2) / total, st.innov[0].to(torch.float64).reshape(shape).sum(2) / total
+    return _pooled_innovation(w.streams, w.lengths, st, (w.qs.numel(), w.rs.numel()))
+
+
+# ------------------------------------------------------------------------------------------------
+# Matrix sweep: candidate Q and R matrices scored on recordings (B.replay_general)
+# ------------------------------------------------------------------------------------------------
+@dataclass
+class MatrixSweepWorkload:
+    streams: torch.Tensor      # [T, 9, Ns]
+    acc_ref: torch.Tensor
+    mag_ref: torch.Tensor
+    Q: torch.Tensor            # [M, 3, 3] float64 candidates (M = 1: one Q for every candidate)
+    R: torch.Tensor            # [M, 4, 4]
+    q: torch.Tensor            # [3, 3] or [M Ns, 3, 3] per filter: candidate m owns filters m Ns .. (m+1) Ns
+    r: torch.Tensor            # [4, 4] or [M Ns, 4, 4]
+    dt: float | torch.Tensor
+    lengths: torch.Tensor | None = None
+
+    @property
+    def n_candidates(self) -> int:
+        return max(self.Q.shape[0], self.R.shape[0])
+
+    @property
+    def n_filters(self) -> int:
+        return self.n_candidates * self.streams.shape[2]
+
+
+def build_matrix_sweep(b, q, r) -> MatrixSweepWorkload:
+    """Candidate matrices over the recordings of a `logio.LogBatch` (one recording: `logio.stack_logs([log], device)`):
+    q [M,3,3] or [3,3], r [M,4,4] or [4,4] (numpy arrays or tensors; a [3,3] / [4,4] matrix is shared by every
+    candidate, and two [M,...] stacks must agree on M).  N = M Ns filters, filter n replays recording n % Ns with the
+    matrices of candidate n // Ns.  Run it with `run_matrix_sweep` and read `matrix_innovation_surface`."""
+    device = b.streams.device
+    Q = torch.as_tensor(q, dtype=torch.float64, device=device)
+    R = torch.as_tensor(r, dtype=torch.float64, device=device)
+    Q = Q[None] if Q.dim() == 2 else Q
+    R = R[None] if R.dim() == 2 else R
+    if Q.dim() != 3 or Q.shape[1:] != (3, 3) or R.dim() != 3 or R.shape[1:] != (4, 4):
+        raise ValueError("q must be [M,3,3] or [3,3] and r [M,4,4] or [4,4]")
+    M = max(Q.shape[0], R.shape[0])
+    if Q.shape[0] not in (1, M) or R.shape[0] not in (1, M):
+        raise ValueError(f"q and r hold {Q.shape[0]} and {R.shape[0]} candidates: they must agree (or one be shared)")
+    Ns = b.streams.shape[2]
+    per_filter = lambda X: X[0] if X.shape[0] == 1 else X.repeat_interleave(Ns, dim=0).contiguous()
+    return MatrixSweepWorkload(b.streams, b.acc_ref, b.mag_ref, Q, R, per_filter(Q), per_filter(R), b.dt, b.lengths)
+
+
+def run_matrix_sweep(w: MatrixSweepWorkload, objective: str = "innovation_tangent", gate: float | None = None,
+                     out_innovation: torch.Tensor | None = None) -> B.ReplayState:
+    """One launch of the matrix sweep; returns the state with its innovation sums (`.innov`, objective "innovation"
+    for the 4-D model, "innovation_tangent" for the tangent-space one), `.gate_count` with `gate`, and the per-step
+    terms in `out_innovation` [2,T,N] when given (`window_innovation_nll` reads them)."""
+    model = {"innovation": "full", "innovation_tangent": "tangent"}.get(objective)
+    if model is None:
+        raise ValueError("objective is 'innovation' or 'innovation_tangent'")
+    st, _, _ = B.replay_general(w.streams, w.acc_ref, w.mag_ref, dt=w.dt, q=w.q, r=w.r, n_filters=w.n_filters,
+                                lengths=w.lengths, innovation=True, innovation_model=model,
+                                gate=gate, out_innovation=out_innovation)
+    return st
+
+
+def matrix_innovation_surface(w: MatrixSweepWorkload, st: B.ReplayState):
+    """(pooled innovation NLL per step [M], pooled mean NIS [M]) per candidate, float64: the `pooled_innovation_surface`
+    of the matrix sweep, sum_k NLL_k / sum_k L_k over its recordings.  The best candidate is the argmin of the first."""
+    return _pooled_innovation(w.streams, w.lengths, st, (w.n_candidates,))
 
 
 def window_innovation_nll(out_innovation: torch.Tensor, bounds, dof: int):

@@ -2,11 +2,13 @@
 """Registers, spills and stack of every kernel of the last library build, from the `-Xptxas -v` log that
 `poseestimationkf_b200/build.py` writes beside the library (build_ptxas.log), with demangled names.
 
-  python tools/ptxas_report.py [--match replay_] [--gated | --general | --innov-steps] [--out profiles/r06_gating_registers.json]
+  python tools/ptxas_report.py [--match replay_] [--gated | --general | --innov-steps | --general-innovation]
+                               [--out profiles/r06_gating_registers.json]
 
 --gated keeps the replay kernels instantiated with the innovation gate (the GATE template flag set), --general those
 instantiated with general Q and R matrices (the GEN flag of the scalar kernels set), --innov-steps those with the
-per-step innovation output (an InnovStepArgs in their parameter pack).
+per-step innovation output (an InnovStepArgs in their parameter pack), --general-innovation those with general matrices
+and the innovation terms (the GEN and INNOV flags both set).
 """
 from __future__ import annotations
 
@@ -54,6 +56,10 @@ def is_general(kernel: str) -> bool:
     return _flag(kernel, 8)
 
 
+def is_general_innovation(kernel: str) -> bool:
+    return _flag(kernel, 8) and _flag(kernel, 4)
+
+
 def is_innov_steps(kernel: str) -> bool:
     return "InnovStepArgs" in kernel
 
@@ -65,10 +71,12 @@ def main():
     ap.add_argument("--gated", action="store_true")
     ap.add_argument("--general", action="store_true")
     ap.add_argument("--innov-steps", action="store_true")
+    ap.add_argument("--general-innovation", action="store_true")
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
     ents = [e for e in entries(open(a.log).read()) if a.match in e["kernel"] and (not a.gated or is_gated(e["kernel"]))
-            and (not a.general or is_general(e["kernel"])) and (not a.innov_steps or is_innov_steps(e["kernel"]))]
+            and (not a.general or is_general(e["kernel"])) and (not a.innov_steps or is_innov_steps(e["kernel"]))
+            and (not a.general_innovation or is_general_innovation(e["kernel"]))]
     for e in ents:
         del e["mangled"]
     res = {"source": "ptxas -v of the sm_100a build (nvcc flags of poseestimationkf_b200/build.py)",
